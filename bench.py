@@ -14,6 +14,10 @@ carries: `roofline` (SURVEY 8d's algorithmic FLOPs of the reference traversal) a
 traversal executed), `traversal`, `frame_sha256` (one fixed-seed frame hashed through every product path: equal
 for every N), `other_configs` (C1, C3, C4, the author's native 2401x1601 depth-150 frame, C5 at its full 4096 spp),
 `cpu_baseline`.  Prints ONE JSON line on rank 0.
+
+`--dump-outputs DIR` writes the frame the last timed step left in device memory as DIR/rgb.npy (RGB8, float32) and, with one
+rank, DIR/sums.npy (the int32 PixelStats sums, float64), so that two builds can be compared output for output: the scene and
+the seeds depend only on the arguments.
 """
 import argparse
 import json
@@ -26,6 +30,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the checkout may be read-only: nothing is written into it
 
 import numpy as np  # noqa: E402
 
@@ -255,7 +260,7 @@ class Runner:
         for i in range(warmup):
             self.enqueue(handle, cam, spec, seed0 - 1000 + i)
         self.barrier()
-        out = {"ms": 0.0, "rays": 0, "paths": 0, "launches": 0, "main_ms": [], "main_rays": [], "degenerate": 0}
+        out = {"ms": 0.0, "rays": 0, "paths": 0, "launches": 0, "main_ms": [], "main_rays": [], "degenerate": 0, "last_seed": seed0 + steps - 1}
         for i in range(steps):
             self.flush.fill_(i & 0xFF)
             self.barrier()
@@ -276,6 +281,15 @@ class Runner:
             out["main_rays"].append(int(st.main_rays))
         return out
 
+    def device_frame(self, spec):
+        """The frame the last rt_comm_render left in device memory, copied to the host: RGB8 [rows, cols, 3] and, where this
+        rank holds all of them (one rank), the int32 PixelStats sums [rows, cols, 4].  Call after synchronising."""
+        d_rgb, d_sums = self.comm.frame_pointers()
+        host = lambda a: self.torch.as_tensor(a, device=self.dev).cpu().numpy()  # noqa: E731
+        rgb = host(DeviceArray(d_rgb, (spec.rows, spec.cols, 3), "|u1"))
+        sums = host(DeviceArray(d_sums, (spec.rows, spec.cols, 4), "<i4")) if self.world == 1 else None
+        return rgb, sums
+
     def counters(self, handle, cam, spec, seed=4000):
         """One untimed frame with RT_FLAG_COUNTERS (a slower kernel variant): the tests OUR traversal executes."""
         from ray_tracing_fsharp_b200 import abi
@@ -283,6 +297,37 @@ class Runner:
                                     flags=self.flags | abi.RT_FLAG_COUNTERS, want_rgb=False, want_sums=False, want_stats=True)
         rays, paths, box, prim = self.reduce([st.rays, st.paths, st.box_tests, st.prim_tests], "SUM")
         return {"rays": rays, "paths": paths, "box_tests": box, "prim_tests": prim}
+
+
+class DeviceArray:
+    """A buffer in device memory that the library owns, described by __cuda_array_interface__ so that torch can read it."""
+
+    def __init__(self, ptr, shape, typestr):
+        self.__cuda_array_interface__ = {"data": (ptr, False), "shape": shape, "typestr": typestr, "version": 2}
+
+
+DUMP_BYTES = 64_000_000  # all files together, .npy headers included
+
+
+def dump_outputs(out_dir, rgb, sums, seed=0):
+    """Writes the frame as out_dir/rgb.npy (float32) and out_dir/sums.npy (float64; omitted when None), both exact.  A frame
+    larger than DUMP_BYTES in all is cut to a fixed, seeded sample of its pixels ([n, 3] / [n, 4]), whose flat indices go to
+    out_dir/pixel_index.npy.  Returns {file name: shape}."""
+    arrays = {"rgb": rgb.astype(np.float32)}
+    if sums is not None:
+        arrays["sums"] = sums.astype(np.float64)
+    n_pixels = rgb.shape[0] * rgb.shape[1]
+    per_pixel = sum(a.nbytes for a in arrays.values()) // n_pixels
+    budget = DUMP_BYTES - 1024  # a .npy header is 128 bytes
+    if n_pixels * per_pixel > budget:
+        keep = budget // (per_pixel + 8)
+        idx = np.sort(np.random.default_rng(seed).choice(n_pixels, keep, replace=False))
+        arrays = {k: a.reshape(n_pixels, -1)[idx] for k, a in arrays.items()}
+        arrays["pixel_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    return {f"{name}.npy": list(a.shape) for name, a in arrays.items()}
 
 
 def n_planes_of(spec):
@@ -416,6 +461,10 @@ def run_ours(args):
     value = m["rays"] / secs / 1e6
     main_ms = sum(m["main_ms"]) / max(1, len(m["main_ms"]))
     main_rays = sum(m["main_rays"]) / max(1, len(m["main_rays"]))
+    dumped = None
+    if args.dump_outputs and rank == 0:  # before the next rt_comm_render replaces the frame
+        dumped = {"dir": os.path.abspath(args.dump_outputs), "frame_seed": m["last_seed"],
+                  "files": dump_outputs(args.dump_outputs, *r.device_frame(spec))}
 
     n_e2e = max(1, min(args.steps, 3))
     e2e = e2e_frames(r, spec, cam, n_e2e)
@@ -509,6 +558,8 @@ def run_ours(args):
             "traversal": {"box_tests_per_ray": trav["box_tests"] / max(1, trav["rays"]), "prim_tests_per_ray": trav["prim_tests"] / max(1, trav["rays"]),
                           "rays_per_path": trav["rays"] / max(1, trav["paths"])},
         }
+        if dumped:
+            line["dumped_outputs"] = dumped
         if hashes:
             line["frame_sha256"] = hashes
         if others:
@@ -551,7 +602,14 @@ def main():
     ap.add_argument("--other-configs", default="C1,C3,C4,native,C5", help="which of C1..C5 / native to measure after the headline config")
     ap.add_argument("--cpu-seconds", type=float, default=25.0)
     ap.add_argument("--flops-per-ray", type=float, default=0.0, help="FLOPs of the reference traversal per ray, used when the CPU sample does not run (default: the config's figure from DESIGN.md)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame of the last timed step as DIR/rgb.npy and DIR/sums.npy (at most 64 MB in all; a larger frame is a "
+                         "fixed, seeded sample of its pixels, indices in DIR/pixel_index.npy)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the frames of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

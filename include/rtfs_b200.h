@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define RT_ABI_VERSION 2
+#define RT_ABI_VERSION 3
 
 /* ---- error codes --------------------------------------------------------------------------- */
 #define RT_OK 0
@@ -235,6 +235,55 @@ int rt_host_unpin(void *ptr);
 int rt_render(RtScene *scene, const RtCamera *camera, int32_t max_width_coord,
               int32_t max_height_coord, const RtRenderOpts *opts, uint8_t *rgb_out,
               int32_t *sums_out, RtStats *stats);
+
+/* ---- progressive frames (host buffers; one GPU) -------------------------------------------------- */
+/* rt_render's frame in sample passes, with progress between them (the reference calls progressIncrement as rows finish,
+ * Scene.fs:232), an image to look at after every pass, early stopping and continuation to more samples.
+ *
+ * Open a frame once (rt_frame_begin: the probe phase, Scene.fs:172-188, and the compaction of the flagged pixels), then
+ * advance it in passes (rt_frame_advance: the third loop, Scene.fs:191-192, over a window of sample indices).  Every
+ * sample is keyed by (seed, pixel, sample index) and the sums are integers, so after any pass the frame's sums are bit for
+ * bit those of rt_render with samples_per_pixel = samples_done (same scene, camera, extents, seed, adaptive and flags).
+ * The rule's firstTrial = min(5, spp / 2) is the same at samples_done and at the target once the probe is done.
+ *
+ * Pass sizing.  A pass covers the sample window [samples_done, samples_done + k).  k is the smallest of max_samples
+ * (if > 0); the number of sample indices predicted to take target_ms of device time (if > 0), from the measured device
+ * time per sample index of the last pass, or of the probe for the first pass (a frame with adaptive = 0 has no probe:
+ * its first paced pass takes one sample index); and what is left.  k is never below 1.  max_samples = 0 and
+ * target_ms = 0 take everything that is left.  Only the number of passes depends on their sizes, never the result.
+ * Stopping.  A caller stops early by not calling rt_frame_advance again: one pass is the longest it waits.
+ * Extending.  rt_frame_extend raises (or lowers) the target to samples_per_pixel.  It accepts a value only if the target
+ *   it gives is >= samples_done, samples_per_pixel <= 2^22, and firstTrial stays what it is (6 -> 64 would change the
+ *   probe: RT_ERR_INVALID_ARGUMENT).  A frame opened at spp <= 2 firstTrial + 1 runs no main phase but keeps which pixels
+ *   would go on, so it can be extended.
+ * Modes.  RT_MODE_MEGAKERNEL only (RT_MODE_WAVEFRONT: RT_ERR_UNSUPPORTED); the RT_FLAG_* bits act as in rt_render.
+ * Ownership.  A frame owns its sum, flag, list and image buffers and its work counters: rt_render and other frames may
+ *   run on the same scene between two passes.  Every call returns with the device work it issued complete.  A frame is
+ *   not thread-safe (like its scene) and must be destroyed before its scene. */
+typedef struct RtFrame RtFrame;
+typedef struct RtFrameProgress {
+    int32_t samples_done;    /* every flagged pixel holds sample indices [0, samples_done): the frame equals
+                                rt_render's at samples_per_pixel = samples_done                                   */
+    int32_t samples_target;  /* max(2 firstTrial + 1, spp) with the early-out, spp without; or what rt_frame_extend set */
+    uint64_t paths_done;     /* traceOnce calls so far (probe + passes), from the device counters               */
+    uint64_t paths_target;   /* n_pixels * n_probe + pixels_flagged * (samples_target - n_probe); exact          */
+    uint64_t pixels_flagged; /* pixels that go on after the probe (every pixel without the early-out)             */
+    double last_pass_ms;     /* device time of the last pass (CUDA events)                                        */
+    double device_ms;        /* device time of the probe and compaction plus every pass so far                     */
+    int32_t passes;          /* rt_frame_advance calls that traced something                                      */
+    int32_t done;            /* samples_done == samples_target                                                    */
+} RtFrameProgress;
+/* probe + compaction, synchronous.  progress optional. */
+int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_width_coord,
+                   int32_t max_height_coord, const RtRenderOpts *opts, RtFrame **out,
+                   RtFrameProgress *progress);
+/* one pass (nothing when done).  progress optional. */
+int rt_frame_advance(RtFrame *frame, int32_t max_samples, double target_ms, RtFrameProgress *progress);
+/* the current image as rt_render gives it: rgb_out rows*cols*3 (gamma as opts->gamma of rt_render), sums_out
+ * rows*cols*4 int32 {sumR,sumG,sumB,count}; either may be NULL */
+int rt_frame_read(RtFrame *frame, int32_t gamma, uint8_t *rgb_out, int32_t *sums_out);
+int rt_frame_extend(RtFrame *frame, int32_t samples_per_pixel);
+void rt_frame_destroy(RtFrame *frame);
 
 /* The same frame split over the GPUs of this process (the F# host is one process): replicated scene,
  * sample-index split (Scene.fs:191-192 shared out by sample index), probe tiles shared out by tile.

@@ -5,7 +5,7 @@ struct against the values the compiled library reports.
 """
 import ctypes as C
 
-RT_ABI_VERSION = 2
+RT_ABI_VERSION = 3
 
 RT_OK = 0
 RT_ERR_INVALID_ARGUMENT = -1
@@ -123,4 +123,18 @@ class RtStats(C.Structure):
         ("main_ms", C.c_double),
         ("main_rays", C.c_uint64),
         ("degenerate_paths", C.c_uint64),
+    ]
+
+
+class RtFrameProgress(C.Structure):
+    _fields_ = [
+        ("samples_done", C.c_int32),
+        ("samples_target", C.c_int32),
+        ("paths_done", C.c_uint64),
+        ("paths_target", C.c_uint64),
+        ("pixels_flagged", C.c_uint64),
+        ("last_pass_ms", C.c_double),
+        ("device_ms", C.c_double),
+        ("passes", C.c_int32),
+        ("done", C.c_int32),
     ]

@@ -795,7 +795,7 @@ static int build_chunks(FrameParams &fp, int n_local, int boundary, size_t n_uni
     return RT_OK;
 }
 
-int launch_probe(DeviceScene *ds, FrameParams fp, bool count, bool no_smem, cudaStream_t st, int *launches) {
+int launch_probe(DeviceScene *ds, FrameParams fp, bool count, bool no_smem, cudaStream_t st, int *launches, bool raw_flags) {
     DeviceWorkspace *ws = ds->ws;
     const size_t n_pixels = size_t(fp.cam.rows) * fp.cam.cols;
     if (ws->probe_pixels < n_pixels) {
@@ -806,7 +806,7 @@ int launch_probe(DeviceScene *ds, FrameParams fp, bool count, bool no_smem, cuda
         ws->probe_pixels = n_pixels;
     }
     RT_CUDA(cudaMemsetAsync(ws->d_stats_b, 0, n_pixels * 4 * sizeof(int32_t), st));
-    RT_CUDA(cudaMemsetAsync(ws->d_counters + CN_WORK_PROBE, 0, sizeof(unsigned long long), st));
+    RT_CUDA(cudaMemsetAsync(fp.counters + CN_WORK_PROBE, 0, sizeof(unsigned long long), st));
     fp.stats_b = ws->d_stats_b;
     LaunchPlan plan;
     RenderKernelFn fn;
@@ -820,25 +820,29 @@ int launch_probe(DeviceScene *ds, FrameParams fp, bool count, bool no_smem, cuda
     ++*launches;
     probe_flags_kernel<<<unsigned((n_pixels + 255) / 256), 256, 0, st>>>(fp.stats, ws->d_stats_b, fp.flags, fp.cam.rows, fp.cam.cols, fp.tiles_x,
                                                                           fp.rank, fp.world, fp.first_trial, fp.n_probe,
-                                                                          fp.sample_end > fp.sample_begin ? 1 : 0);
+                                                                          (raw_flags || fp.sample_end > fp.sample_begin) ? 1 : 0);
     RT_CUDA(cudaGetLastError());
     ++*launches;
     return RT_OK;
 }
 
-int launch_main(DeviceScene *ds, FrameParams fp, const FlagsView &flags, bool count, bool no_smem, cudaStream_t st, int *launches) {
-    const size_t n_pixels = size_t(fp.cam.rows) * fp.cam.cols;
-    int rc = ensure_list(ds, n_pixels);
-    if (rc != RT_OK) return rc;
-    RT_CUDA(cudaMemsetAsync(ds->ws->d_counters + CN_LIST, 0, sizeof(unsigned long long), st));
-    RT_CUDA(cudaMemsetAsync(ds->ws->d_counters + CN_WORK_MAIN, 0, sizeof(unsigned long long), st));
-    compact_kernel<<<ds->ws->sm_count * 4, 256, 0, st>>>(flags, ds->ws->d_list, ds->ws->d_counters, fp.cam.rows, fp.cam.cols, fp.tiles_x, fp.tiles_y);
+// flags -> the flagged-pixel list `list`, its length in fp.counters[CN_LIST]; zeroes the main phase's work cursor
+int launch_compact(DeviceScene *ds, const FrameParams &fp, const FlagsView &flags, uint32_t *list, cudaStream_t st, int *launches) {
+    RT_CUDA(cudaMemsetAsync(fp.counters + CN_LIST, 0, sizeof(unsigned long long), st));
+    RT_CUDA(cudaMemsetAsync(fp.counters + CN_WORK_MAIN, 0, sizeof(unsigned long long), st));
+    compact_kernel<<<ds->ws->sm_count * 4, 256, 0, st>>>(flags, list, fp.counters, fp.cam.rows, fp.cam.cols, fp.tiles_x, fp.tiles_y);
     RT_CUDA(cudaGetLastError());
     ++*launches;
-    fp.list = ds->ws->d_list;
+    return RT_OK;
+}
+
+// The main phase over the sample window [fp.sample_begin, fp.sample_end) (this rank's share of it) for the pixels of
+// fp.list; the work cursor fp.counters[CN_WORK_MAIN] must be zero on entry
+int launch_samples(DeviceScene *ds, FrameParams fp, bool count, bool no_smem, cudaStream_t st, int *launches) {
+    const size_t n_pixels = size_t(fp.cam.rows) * fp.cam.cols;
     LaunchPlan plan;
     RenderKernelFn fn;
-    rc = plan_launch(ds, fp, false, count, no_smem, plan, fn);
+    int rc = plan_launch(ds, fp, false, count, no_smem, plan, fn);
     if (rc != RT_OK) return rc;
     int n_span = fp.sample_end - fp.sample_begin - fp.rank;
     int n_local = n_span > 0 ? (n_span + fp.world - 1) / fp.world : 0;
@@ -849,12 +853,21 @@ int launch_main(DeviceScene *ds, FrameParams fp, const FlagsView &flags, bool co
         rc = build_chunks(fp, std::min(kMaxLaunchSamples, n_local - base), -1, (n_pixels + 31) / 32, plan.blocks * (plan.threads / 32));
         if (rc != RT_OK) return rc;
         for (int k = 0; k < fp.n_chunks; ++k) fp.chunk_begin[k] += uint32_t(base);
-        if (base > 0) RT_CUDA(cudaMemsetAsync(ds->ws->d_counters + CN_WORK_MAIN, 0, sizeof(unsigned long long), st));
+        if (base > 0) RT_CUDA(cudaMemsetAsync(fp.counters + CN_WORK_MAIN, 0, sizeof(unsigned long long), st));
         fn<<<plan.blocks, plan.threads, plan.smem_bytes, st>>>(fp);
         RT_CUDA(cudaGetLastError());
         ++*launches;
     }
     return RT_OK;
+}
+
+int launch_main(DeviceScene *ds, FrameParams fp, const FlagsView &flags, bool count, bool no_smem, cudaStream_t st, int *launches) {
+    const size_t n_pixels = size_t(fp.cam.rows) * fp.cam.cols;
+    int rc = ensure_list(ds, n_pixels);
+    if (rc != RT_OK) return rc;
+    if ((rc = launch_compact(ds, fp, flags, ds->ws->d_list, st, launches)) != RT_OK) return rc;
+    fp.list = ds->ws->d_list;
+    return launch_samples(ds, fp, count, no_smem, st, launches);
 }
 
 void read_counters(DeviceScene *ds, RtStats *stats, size_t n_pixels, bool adaptive) {

@@ -171,8 +171,14 @@ inline FlagsView single_flags(const uint8_t *p) {
 
 int check_frame_args(const RtScene *scene, const RtCamera *camera, int max_w, int max_h, const RtRenderOpts *opts);
 void fill_frame(FrameParams &fp, DeviceScene *ds, const RtCamera &cam, int max_w, int max_h, const RtRenderOpts &opts, int rank, int world);
-int launch_probe(DeviceScene *ds, FrameParams fp, bool count, bool no_smem, cudaStream_t st, int *launches);
+// raw_flags: flag every pixel whose two probe means differ even where the frame has no main phase (progressive frames
+// keep them so that the frame can be extended to more samples); otherwise only where a main phase follows
+int launch_probe(DeviceScene *ds, FrameParams fp, bool count, bool no_smem, cudaStream_t st, int *launches, bool raw_flags = false);
+// compaction + the main phase over [fp.sample_begin, fp.sample_end); the two halves are also launched on their own
+// (progressive frames, rtfs_frame.cu: compaction once, then one launch_samples per pass)
 int launch_main(DeviceScene *ds, FrameParams fp, const FlagsView &flags, bool count, bool no_smem, cudaStream_t st, int *launches);
+int launch_compact(DeviceScene *ds, const FrameParams &fp, const FlagsView &flags, uint32_t *list, cudaStream_t st, int *launches);
+int launch_samples(DeviceScene *ds, FrameParams fp, bool count, bool no_smem, cudaStream_t st, int *launches);
 // makes sure the tree the frame will walk is on the device (the wide tree is built on first use for small scenes)
 int prepare_frame(RtScene *scene, const RtRenderOpts *opts);
 bool frame_walks_wide_tree(const DeviceScene *ds, int opt_flags, bool smem_fits);

@@ -1,0 +1,214 @@
+// rtfs_frame.cu — progressive frames (rt_frame_*): rt_render's frame on one device, cut into passes over windows of
+// sample indices.  The probe and the compaction run once, in rt_frame_begin; every rt_frame_advance is one
+// launch_samples over [samples_done, samples_done + k), i.e. the same render_kernel<PROBE = false> that rt_render's main
+// phase launches, with the same chunking.  Sums are integers keyed by (seed, pixel, sample index), so a frame that has
+// reached samples_done is bit for bit rt_render's frame at samples_per_pixel = samples_done (include/rtfs_b200.h).
+#include "rtfs_device.h"
+
+#include <algorithm>
+#include <cmath>
+#include <cstring>
+
+using namespace rtfs;
+
+// A frame owns everything a pass writes: sums, flags, the flagged-pixel list, the image and its own counter block
+// (paths, rays, the list length and the work cursors), so rt_render and other frames can use the scene between passes.
+struct RtFrame {
+    RtScene *scene = nullptr;
+    FrameParams fp;
+    bool count = false, no_smem = false;
+    size_t n_pixels = 0;
+    int32_t *d_stats = nullptr;
+    uint8_t *d_flags = nullptr;
+    uint32_t *d_list = nullptr;
+    uint8_t *d_rgb = nullptr;
+    unsigned long long *d_counters = nullptr;
+    unsigned long long h_counters[CN_SLOTS] = {};
+    cudaEvent_t ev[2] = {nullptr, nullptr};
+    int32_t samples_done = 0, samples_target = 0;
+    uint64_t pixels_flagged = 0;
+    double ms_per_sample = -1.0; // measured device time of one sample index of every flagged pixel (< 0: not known yet)
+    double last_pass_ms = 0.0, device_ms = 0.0;
+    int32_t passes = 0;
+};
+
+namespace {
+
+void frame_free(RtFrame *f) {
+    if (!f) return;
+    auto *ds = static_cast<DeviceScene *>(f->scene->dev);
+    cudaSetDevice(ds->device);
+    cudaStreamSynchronize(ds->ws->stream);
+    cudaFree(f->d_stats);
+    cudaFree(f->d_flags);
+    cudaFree(f->d_list);
+    cudaFree(f->d_rgb);
+    cudaFree(f->d_counters);
+    for (auto &e : f->ev)
+        if (e) cudaEventDestroy(e);
+    delete f;
+}
+
+// one small device->host copy of the frame's counters and a synchronisation of the scene's stream
+int frame_sync(RtFrame *f, cudaStream_t st) {
+    RT_CUDA(cudaMemcpyAsync(f->h_counters, f->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaStreamSynchronize(st));
+    return RT_OK;
+}
+
+void frame_progress(const RtFrame *f, RtFrameProgress *p) {
+    if (!p) return;
+    std::memset(p, 0, sizeof *p);
+    const uint64_t n_probe = uint64_t(f->fp.n_probe);
+    p->samples_done = f->samples_done;
+    p->samples_target = f->samples_target;
+    p->paths_done = f->h_counters[CN_PATHS];
+    p->paths_target = uint64_t(f->n_pixels) * n_probe + f->pixels_flagged * (uint64_t(f->samples_target) - n_probe);
+    p->pixels_flagged = f->pixels_flagged;
+    p->last_pass_ms = f->last_pass_ms;
+    p->device_ms = f->device_ms;
+    p->passes = f->passes;
+    p->done = f->samples_done == f->samples_target ? 1 : 0;
+}
+
+float elapsed_ms(cudaEvent_t a, cudaEvent_t b) {
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, a, b);
+    return ms;
+}
+
+} // namespace
+
+extern "C" {
+
+int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_t max_h, const RtRenderOpts *opts, RtFrame **out,
+                   RtFrameProgress *progress) {
+    int rc = check_frame_args(scene, camera, max_w, max_h, opts);
+    if (rc != RT_OK) return rc;
+    if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin: out is null");
+    *out = nullptr;
+    if (opts->mode == RT_MODE_WAVEFRONT) return fail(RT_ERR_UNSUPPORTED, "rt_frame_begin: progressive frames run the megakernel only");
+    if (opts->mode != RT_MODE_MEGAKERNEL) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin: unknown mode");
+    if ((rc = prepare_frame(scene, opts)) != RT_OK) return rc;
+    auto *ds = static_cast<DeviceScene *>(scene->dev);
+    RT_CUDA(cudaSetDevice(ds->device));
+    auto *f = new RtFrame();
+    f->scene = scene;
+    auto bail = [&](int code) {
+        frame_free(f);
+        return code;
+    };
+    const size_t n = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
+    f->n_pixels = n;
+    bool ok = cudaMalloc((void **)&f->d_stats, n * 4 * sizeof(int32_t)) == cudaSuccess && cudaMalloc((void **)&f->d_flags, n) == cudaSuccess &&
+              cudaMalloc((void **)&f->d_list, n * sizeof(uint32_t)) == cudaSuccess && cudaMalloc((void **)&f->d_rgb, n * 3) == cudaSuccess &&
+              cudaMalloc((void **)&f->d_counters, CN_SLOTS * sizeof(unsigned long long)) == cudaSuccess;
+    for (auto &e : f->ev) ok = ok && cudaEventCreate(&e) == cudaSuccess;
+    if (!ok) return bail(fail(RT_ERR_CUDA, std::string("rt_frame_begin: allocation failed: ") + cudaGetErrorString(cudaGetLastError())));
+
+    FrameParams &fp = f->fp;
+    fill_frame(fp, ds, *camera, max_w, max_h, *opts, 0, 1);
+    fp.stats = f->d_stats;
+    fp.flags = f->d_flags;
+    fp.list = f->d_list;
+    fp.counters = f->d_counters;
+    f->count = (opts->flags & RT_FLAG_COUNTERS) != 0;
+    f->no_smem = (opts->flags & RT_FLAG_NO_SMEM) != 0;
+    f->samples_done = fp.n_probe; // 0 without the early-out
+    f->samples_target = fp.sample_end;
+    cudaStream_t st = ds->ws->stream;
+    int launches = 0;
+    auto enqueue = [&]() -> int {
+        RT_CUDA(cudaMemsetAsync(f->d_counters, 0, CN_SLOTS * sizeof(unsigned long long), st));
+        RT_CUDA(cudaMemsetAsync(f->d_stats, 0, n * 4 * sizeof(int32_t), st));
+        RT_CUDA(cudaEventRecord(f->ev[0], st));
+        if (fp.adaptive) {
+            // the raw "means differ" flags, also where this target has no main phase: the frame can be extended
+            int rc2 = launch_probe(ds, fp, f->count, f->no_smem, st, &launches, true);
+            if (rc2 != RT_OK) return rc2;
+        } else {
+            RT_CUDA(cudaMemsetAsync(f->d_flags, 1, n, st));
+        }
+        int rc2 = launch_compact(ds, fp, single_flags(f->d_flags), f->d_list, st, &launches);
+        if (rc2 != RT_OK) return rc2;
+        RT_CUDA(cudaEventRecord(f->ev[1], st));
+        return frame_sync(f, st);
+    };
+    if ((rc = enqueue()) != RT_OK) return bail(rc);
+    f->pixels_flagged = f->h_counters[CN_LIST];
+    f->device_ms = elapsed_ms(f->ev[0], f->ev[1]);
+    // the probe traced n_probe samples of every pixel; a pass traces samples of the flagged pixels only
+    if (fp.adaptive) f->ms_per_sample = f->device_ms * double(f->pixels_flagged) / (double(n) * double(fp.n_probe));
+    *out = f;
+    frame_progress(f, progress);
+    return RT_OK;
+}
+
+int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameProgress *progress) {
+    if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_advance: null frame");
+    if (max_samples < 0 || !(target_ms >= 0.0)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_advance: max_samples and target_ms must be >= 0");
+    const int left = f->samples_target - f->samples_done;
+    if (left > 0) {
+        int k = left;
+        if (max_samples > 0) k = std::min(k, max_samples);
+        if (target_ms > 0.0) {
+            int paced = 1; // no rate known yet (no probe without the early-out): one sample index
+            if (f->ms_per_sample == 0.0) paced = left; // nothing to trace (no pixel is flagged)
+            else if (f->ms_per_sample > 0.0) paced = int(std::min(double(left), std::floor(target_ms / f->ms_per_sample)));
+            k = std::min(k, std::max(1, paced));
+        }
+        auto *ds = static_cast<DeviceScene *>(f->scene->dev);
+        RT_CUDA(cudaSetDevice(ds->device));
+        cudaStream_t st = ds->ws->stream;
+        FrameParams fp = f->fp;
+        fp.sample_begin = f->samples_done;
+        fp.sample_end = f->samples_done + k;
+        int launches = 0;
+        RT_CUDA(cudaMemsetAsync(f->d_counters + CN_WORK_MAIN, 0, sizeof(unsigned long long), st));
+        RT_CUDA(cudaEventRecord(f->ev[0], st));
+        int rc = launch_samples(ds, fp, f->count, f->no_smem, st, &launches);
+        if (rc != RT_OK) return rc;
+        RT_CUDA(cudaEventRecord(f->ev[1], st));
+        if ((rc = frame_sync(f, st)) != RT_OK) return rc;
+        f->samples_done += k;
+        f->passes += 1;
+        f->last_pass_ms = elapsed_ms(f->ev[0], f->ev[1]);
+        f->device_ms += f->last_pass_ms;
+        f->ms_per_sample = f->pixels_flagged ? f->last_pass_ms / k : 0.0;
+    }
+    frame_progress(f, progress);
+    return RT_OK;
+}
+
+int rt_frame_read(RtFrame *f, int32_t gamma, uint8_t *rgb_out, int32_t *sums_out) {
+    if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_read: null frame");
+    auto *ds = static_cast<DeviceScene *>(f->scene->dev);
+    RT_CUDA(cudaSetDevice(ds->device));
+    cudaStream_t st = ds->ws->stream;
+    if (rgb_out) {
+        int rc = rt_device_finalize(ds->device, f->d_stats, int32_t(f->n_pixels), gamma, f->d_rgb, st);
+        if (rc != RT_OK) return rc;
+        RT_CUDA(cudaMemcpyAsync(rgb_out, f->d_rgb, f->n_pixels * 3, cudaMemcpyDeviceToHost, st));
+    }
+    if (sums_out) RT_CUDA(cudaMemcpyAsync(sums_out, f->d_stats, f->n_pixels * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaStreamSynchronize(st));
+    return RT_OK;
+}
+
+int rt_frame_extend(RtFrame *f, int32_t spp) {
+    if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_extend: null frame");
+    if (spp < 1 || spp > (1 << 22)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_extend: samples_per_pixel must be in [1, 2^22]");
+    FrameParams &fp = f->fp;
+    if (fp.adaptive && std::min(5, spp / 2) != fp.first_trial) // Scene.fs:172
+        return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_extend: this samples_per_pixel changes firstTrial, i.e. the probe the frame already ran");
+    const int target = fp.adaptive ? std::max(fp.n_probe, spp) : spp;
+    if (target < f->samples_done) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_extend: the frame already holds more samples than that");
+    f->samples_target = target;
+    fp.sample_end = target;
+    fp.cam.spp = spp;
+    return RT_OK;
+}
+
+void rt_frame_destroy(RtFrame *f) { frame_free(f); }
+
+} // extern "C"

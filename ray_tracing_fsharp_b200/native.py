@@ -10,7 +10,7 @@ import os
 import numpy as np
 
 from . import abi
-from .abi import RtCamera, RtHittable, RtRenderOpts, RtStats, RtTexture
+from .abi import RtCamera, RtFrameProgress, RtHittable, RtRenderOpts, RtStats, RtTexture
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "librtfs_b200.so")
@@ -48,6 +48,12 @@ def _declare(lib):
         "rt_scene_device_bytes": (C.c_size_t, [_vp]),
         "rt_scene_shared_memory_bytes": (C.c_size_t, [_vp]),
         "rt_render": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _vp, _vp, C.POINTER(RtStats)]),
+        "rt_frame_begin": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), C.POINTER(_vp),
+                                     C.POINTER(RtFrameProgress)]),
+        "rt_frame_advance": (C.c_int, [_vp, _i32, C.c_double, C.POINTER(RtFrameProgress)]),
+        "rt_frame_read": (C.c_int, [_vp, _i32, _vp, _vp]),
+        "rt_frame_extend": (C.c_int, [_vp, _i32]),
+        "rt_frame_destroy": (None, [_vp]),
         "rt_render_multi": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i32, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _vp,
                                       _vp, C.POINTER(RtStats)]),
         "rt_multi_create": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i32, C.POINTER(_vp)]),
@@ -237,6 +243,10 @@ class SceneHandle:
         check(lib().rt_render(self.ptr, C.byref(camera), max_w, max_h, C.byref(opts), ptr(rgb), ptr(sums), C.byref(stats)))
         return rgb, sums, stats
 
+    def open_frame(self, camera, max_w, max_h, seed=0, adaptive=True, flags=0, mode=abi.RT_MODE_MEGAKERNEL):
+        """A progressive frame of this scene (rt_frame_begin: runs the probe).  See Frame."""
+        return Frame(self, camera, max_w, max_h, seed, adaptive, flags, mode)
+
     # ---- conformance ----
     def hit_object(self, o, d, traversal=0):
         o, d = f64(o, (-1, 3)), f64(d, (-1, 3))
@@ -277,6 +287,58 @@ class SceneHandle:
         check(lib().rt_test_trace_samples(self.ptr, C.byref(camera), max_w, max_h, seed, n, ptr(row_idx), ptr(col_idx), ptr(sample),
                                           ptr(colour), ptr(rays)))
         return colour, rays
+
+
+class Frame:
+    """Owner of an RtFrame* (rt_frame_begin / rt_frame_destroy): rt_render's frame advanced in passes over windows of
+    sample indices.  After every pass the frame is exactly rt_render's at samples_per_pixel = progress.samples_done.
+    Holds its scene handle, so the scene outlives it."""
+
+    def __init__(self, scene: SceneHandle, camera, max_w, max_h, seed=0, adaptive=True, flags=0, mode=abi.RT_MODE_MEGAKERNEL):
+        self.scene = scene
+        self.rows, self.cols = 2 * max_h + 1, 2 * max_w + 1
+        opts = RtRenderOpts(seed, int(adaptive), mode, 0, flags)
+        out = C.c_void_p()
+        self.progress = RtFrameProgress()
+        check(lib().rt_frame_begin(scene.ptr, C.byref(camera), max_w, max_h, C.byref(opts), C.byref(out), C.byref(self.progress)))
+        self.ptr = out
+
+    def advance(self, max_samples=0, target_ms=0.0) -> RtFrameProgress:
+        """One pass of at most `max_samples` sample indices (0: no limit) predicted to take about `target_ms` of device time
+        (0: no limit).  A no-op once the frame is done."""
+        progress = RtFrameProgress()
+        check(lib().rt_frame_advance(self.ptr, int(max_samples), float(target_ms), C.byref(progress)))
+        self.progress = progress
+        return progress
+
+    def read(self, gamma=False, want_sums=False, rgb_out=None):
+        """The current image (uint8 [rows, cols, 3]) and, with want_sums, the int32 sums [rows, cols, 4]."""
+        rgb = rgb_out if rgb_out is not None else _frame_buffer((self.rows, self.cols, 3))
+        sums = np.empty((self.rows, self.cols, 4), np.int32) if want_sums else None
+        check(lib().rt_frame_read(self.ptr, int(gamma), ptr(rgb), ptr(sums)))
+        return rgb, sums
+
+    def extend(self, spp):
+        """Raises the frame's target to `spp` samples per pixel (RtError RT_ERR_INVALID_ARGUMENT if that would change the
+        probe, or is below what the frame already holds)."""
+        check(lib().rt_frame_extend(self.ptr, int(spp)))
+
+    def close(self):
+        if getattr(self, "ptr", None):
+            lib().rt_frame_destroy(self.ptr)
+            self.ptr = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 class MultiHandle:

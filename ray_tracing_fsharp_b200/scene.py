@@ -6,6 +6,7 @@ reference's.  Everything that computes goes through the C ABI (native.py); nothi
   Camera.make_basic     RayTracing/Camera.fs:34-59
   Scene.make            RayTracing/Scene.fs:15-28
   Scene.render          RayTracing/Scene.fs:196-236
+  Scene.render_progressive  the same frame in sample passes, progress ticks as passes finish (native.Frame)
   Image / Image.render  RayTracing/Domain.fs:9-31
   ImageOutput.write_ppm RayTracing/ImageOutput.fs:163-197, PixelOutput.correct :11-18
 """
@@ -119,6 +120,64 @@ class Scene:
             return out
 
         return float(rows), Image([row_thunk(r) for r in range(rows)], rows, cols, all_rows)
+
+    @staticmethod
+    def render_progressive(progress_increment: Callable[[float], None], print_fn: Callable[[str], None], max_width_coord: int,
+                           max_height_coord: int, camera: abi.RtCamera, s: "Scene", seed: Optional[int] = None, adaptive: bool = True,
+                           target_ms: float = 250.0, on_pass: Optional[Callable[[abi.RtFrameProgress, "native.Frame"], object]] = None,
+                           flags: int = 0) -> np.ndarray:
+        """Scene.render's frame rendered in passes of about `target_ms` of device time each (native.Frame, one GPU).
+        `progress_increment(1.0)` is called as passes complete, in proportion to the paths traced so far out of the frame's
+        total, and exactly `rows` times in all, like the reference's one call per row (Scene.fs:232).  After every pass
+        `on_pass(progress, frame)` is called, if given: it may read the current image (`frame.read()`, exactly the frame of
+        `progress.samples_done` samples per pixel) and stops the frame by returning True.  Returns the pixels (uint8
+        [rows, cols, 3], before gamma): with the same seed, Scene.render's image, or that of the samples done when stopped.
+        `print_fn` is accepted and ignored as in Scene.render."""
+        if not isinstance(s._handle, native.SceneHandle):
+            raise NotImplementedError("progressive frames run on one GPU: make the scene with a single device")
+        rows = 2 * max_height_coord + 1
+        if seed is None:
+            seed = secrets.randbits(64)
+        ticks = ProgressTicks(rows)
+
+        def emit(n):
+            for _ in range(n):
+                progress_increment(1.0)
+
+        with s._handle.open_frame(camera, max_width_coord, max_height_coord, seed=seed, adaptive=adaptive, flags=flags) as frame:
+            progress = frame.progress
+            emit(ticks.update(progress.paths_done, progress.paths_target))  # the probe
+            while not progress.done:
+                progress = frame.advance(target_ms=target_ms)
+                if not progress.done:
+                    emit(ticks.update(progress.paths_done, progress.paths_target))
+                if on_pass is not None and on_pass(progress, frame):
+                    break
+            rgb, _ = frame.read()
+        emit(ticks.finish())  # the last pass's share, or the rest of the frame when on_pass stopped it
+        return rgb
+
+
+class ProgressTicks:
+    """Spreads `total` progress ticks over a quantity that grows towards a target: after update(done, target) the ticks
+    handed out so far are floor(total * done / target), so the fractional part carries into the next update, and
+    finish() hands out the rest.  However the updates fall, the ticks add up to exactly `total`."""
+
+    def __init__(self, total: int):
+        self.total = int(total)
+        self.emitted = 0
+
+    def update(self, done: int, target: int) -> int:
+        """Number of ticks to emit now."""
+        want = self.total if target <= 0 or done >= target else (self.total * int(done)) // int(target)
+        n = max(0, want - self.emitted)
+        self.emitted += n
+        return n
+
+    def finish(self) -> int:
+        n = self.total - self.emitted
+        self.emitted = self.total
+        return n
 
 
 class PixelOutput:

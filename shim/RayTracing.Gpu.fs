@@ -9,7 +9,8 @@
 // compile order, because it reads the private records `Sphere` (Sphere.fs:302-310) and
 // `InfinitePlane` (InfinitePlane.fs:101-106).  It adds `Scene.renderGpu`, with the signature of
 // `Scene.render` (Scene.fs:196-204), over a `GpuScene` built by `GpuScene.make : Hittable array -> GpuScene`
-// (the counterpart of `Scene.make`, Scene.fs:15-28).
+// (the counterpart of `Scene.make`, Scene.fs:15-28), and `SceneGpu.renderWithProgress`, the same frame traced in passes
+// with progress reported as they finish (a `GpuFrame`, rt_frame_*, for callers that want the passes themselves).
 namespace RayTracing
 
 open System
@@ -109,6 +110,18 @@ module internal Native =
         val mutable mainRays : uint64
         val mutable degeneratePaths : uint64
 
+    [<Struct ; StructLayout(LayoutKind.Sequential)>]
+    type RtFrameProgress =
+        val mutable samplesDone : int
+        val mutable samplesTarget : int
+        val mutable pathsDone : uint64
+        val mutable pathsTarget : uint64
+        val mutable pixelsFlagged : uint64
+        val mutable lastPassMs : float
+        val mutable deviceMs : float
+        val mutable passes : int
+        val mutable isDone : int // `done` in the header (a keyword in F#)
+
     [<DllImport(Lib)>]
     extern nativeint rt_last_error ()
 
@@ -123,6 +136,22 @@ module internal Native =
 
     [<DllImport(Lib)>]
     extern int rt_render (nativeint scene, RtCamera& camera, int maxWidthCoord, int maxHeightCoord, RtRenderOpts& opts, byte[] rgbOut, nativeint sumsOut, RtStats& stats)
+
+    // progressive frames on one device (include/rtfs_b200.h, rt_frame_*)
+    [<DllImport(Lib)>]
+    extern int rt_frame_begin (nativeint scene, RtCamera& camera, int maxWidthCoord, int maxHeightCoord, RtRenderOpts& opts, nativeint& frame, RtFrameProgress& progress)
+
+    [<DllImport(Lib)>]
+    extern int rt_frame_advance (nativeint frame, int maxSamples, float targetMs, RtFrameProgress& progress)
+
+    [<DllImport(Lib)>]
+    extern int rt_frame_read (nativeint frame, int gamma, byte[] rgbOut, nativeint sumsOut)
+
+    [<DllImport(Lib)>]
+    extern int rt_frame_extend (nativeint frame, int samplesPerPixel)
+
+    [<DllImport(Lib)>]
+    extern void rt_frame_destroy (nativeint frame)
 
     [<DllImport(Lib)>]
     extern int rt_multi_create (RtHittable[] objects, int nObjects, RtTexture[] textures, int nTextures, int[] devices, int nDevices, nativeint& multi)
@@ -412,6 +441,48 @@ module GpuScene =
 
     let make (objects : Hittable array) : GpuScene = makeOn [| 0 |] objects
 
+/// A frame in progress on a single-device GpuScene (rt_frame_*): advanced in passes over windows of sample indices.
+/// After every pass it is exactly the frame rt_render gives at `SamplesDone` samples per pixel with the same seed, so
+/// `Read` shows the image sharpening; a caller stops early by not advancing any more, and `Extend` continues a finished
+/// frame to more samples.  Dispose it before its scene.
+type GpuFrame internal (handle : nativeint, rows : int, cols : int, first : Native.RtFrameProgress) =
+    let mutable handle = handle
+    let mutable progress = first
+
+    member _.Rows = rows
+    member _.Cols = cols
+    member _.SamplesDone = progress.samplesDone
+    member _.SamplesTarget = progress.samplesTarget
+    /// traceOnce calls so far, and in the whole frame (exact from the start)
+    member _.PathsDone = progress.pathsDone
+    member _.PathsTarget = progress.pathsTarget
+    member _.LastPassMs = progress.lastPassMs
+    member _.Passes = progress.passes
+    member _.IsDone = progress.isDone <> 0
+
+    /// One pass of at most `maxSamples` sample indices (0: no limit) sized to take about `targetMs` of device time
+    /// (0: no limit).  Nothing happens once the frame is done.
+    member _.Advance (maxSamples : int, targetMs : float) : unit =
+        let mutable p = Native.RtFrameProgress ()
+        Native.rt_frame_advance (handle, maxSamples, targetMs, &p) |> Native.check
+        progress <- p
+
+    /// The current image as row-major RGB8, 3 * Rows * Cols bytes (PixelOutput.correct applied when `gamma`).
+    member _.Read (gamma : bool) : byte[] =
+        let rgb = Array.zeroCreate<byte> (3 * rows * cols)
+        Native.rt_frame_read (handle, (if gamma then 1 else 0), rgb, 0n) |> Native.check
+        rgb
+
+    /// Sets the target to `samplesPerPixel`; fails if that would change the probe already run (firstTrial) or is below
+    /// what the frame holds.
+    member _.Extend (samplesPerPixel : int) : unit =
+        Native.rt_frame_extend (handle, samplesPerPixel) |> Native.check
+
+    interface IDisposable with
+        member _.Dispose () =
+            Native.rt_frame_destroy handle
+            handle <- 0n
+
 [<RequireQualifiedAccess>]
 module SceneGpu =
 
@@ -499,6 +570,90 @@ module SceneGpu =
 
                         progressIncrement 1.0<progress>
                         return result
+                    }
+                )
+
+        1.0<progress> * float rowsIter, Image.make rowsIter colsIter rows
+
+    /// Opens a progressive frame (rt_frame_begin: the probe runs now).  Single-device scenes only.
+    let openFrame (maxWidthCoord : int) (maxHeightCoord : int) (camera : Camera) (seed : uint64) (s : GpuScene) : GpuFrame =
+        if s.IsMulti then
+            failwith "GPU backend: progressive frames run on a single-device GpuScene"
+
+        let mutable cam = marshalCamera camera
+        let mutable opts = Native.RtRenderOpts ()
+        opts.seed <- seed
+        opts.adaptive <- 1
+        let mutable handle = 0n
+        let mutable progress = Native.RtFrameProgress ()
+
+        Native.rt_frame_begin (s.Handle, &cam, maxWidthCoord, maxHeightCoord, &opts, &handle, &progress)
+        |> Native.check
+
+        new GpuFrame (handle, 2 * maxHeightCoord + 1, 2 * maxWidthCoord + 1, progress)
+
+    /// `render`'s signature and laziness, but the frame is traced in passes of about 250 ms of device time and
+    /// `progressIncrement 1.0<progress>` is called as passes finish, in proportion to the paths traced out of the frame's
+    /// total: `rows` calls in all, as the reference makes (Scene.fs:232).  Single-device scenes only.
+    let renderWithProgress
+        (progressIncrement : float<progress> -> unit)
+        (_print : string -> unit)
+        (maxWidthCoord : int)
+        (maxHeightCoord : int)
+        (camera : Camera)
+        (s : GpuScene)
+        : float<progress> * Image
+        =
+        let rowsIter = 2 * maxHeightCoord + 1
+        let colsIter = 2 * maxWidthCoord + 1
+
+        let frame =
+            lazy
+                (use f =
+                    openFrame maxWidthCoord maxHeightCoord camera (uint64 (Random().NextInt64 ())) s
+
+                 let ticked = ref 0
+
+                 // ticks so far = floor(rows * pathsDone / pathsTarget): the fraction carries to the next pass
+                 let tick () =
+                     let want =
+                         if f.IsDone || f.PathsTarget = 0UL then
+                             rowsIter
+                         else
+                             min rowsIter (int (float rowsIter * float f.PathsDone / float f.PathsTarget))
+
+                     for _ in ticked.Value + 1 .. want do
+                         progressIncrement 1.0<progress>
+
+                     ticked.Value <- max ticked.Value want
+
+                 tick ()
+
+                 while not f.IsDone do
+                     f.Advance (0, 250.0)
+                     tick ()
+
+                 f.Read false)
+
+        let rows =
+            Seq.init
+                rowsIter
+                (fun row ->
+                    async {
+                        let rgb = frame.Force ()
+
+                        return
+                            Array.init
+                                colsIter
+                                (fun col ->
+                                    let i = 3 * (row * colsIter + col)
+
+                                    {
+                                        Red = rgb.[i]
+                                        Green = rgb.[i + 1]
+                                        Blue = rgb.[i + 2]
+                                    }
+                                )
                     }
                 )
 

@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define RT_ABI_VERSION 3
+#define RT_ABI_VERSION 4
 
 /* ---- error codes --------------------------------------------------------------------------- */
 #define RT_OK 0
@@ -138,6 +138,9 @@ typedef struct RtRenderOpts {
                               slower than lockstep on B200 (DESIGN.md), kept selectable                          */
 #define RT_FLAG_NO_LEAN 64  /* do not pick the kernel specialised for scenes without FP64 unbounded objects and without
                               texture lookups even where the scene allows it (A/B tests; frames are bit-identical)      */
+#define RT_FLAG_NOISE 128   /* rt_frame_begin only: also keep per pixel the sum of r^2 + g^2 + b^2 over its samples, for the
+                              noise estimate of rt_frame_noise.  Not with RT_FLAG_FLOW or RT_FLAG_COUNTERS
+                              (RT_ERR_UNSUPPORTED).  Every other entry point ignores the bit                           */
 
 typedef struct RtStats {
     uint64_t paths;     /* traceOnce calls (Scene.fs:118)                                        */
@@ -256,7 +259,8 @@ int rt_render(RtScene *scene, const RtCamera *camera, int32_t max_width_coord,
  *   it gives is >= samples_done, samples_per_pixel <= 2^22, and firstTrial stays what it is (6 -> 64 would change the
  *   probe: RT_ERR_INVALID_ARGUMENT).  A frame opened at spp <= 2 firstTrial + 1 runs no main phase but keeps which pixels
  *   would go on, so it can be extended.
- * Modes.  RT_MODE_MEGAKERNEL only (RT_MODE_WAVEFRONT: RT_ERR_UNSUPPORTED); the RT_FLAG_* bits act as in rt_render.
+ * Modes.  RT_MODE_MEGAKERNEL only (RT_MODE_WAVEFRONT: RT_ERR_UNSUPPORTED); the RT_FLAG_* bits act as in rt_render, and
+ *   RT_FLAG_NOISE also keeps the per-pixel sum of squares for rt_frame_noise (below).
  * Ownership.  A frame owns its sum, flag, list and image buffers and its work counters: rt_render and other frames may
  *   run on the same scene between two passes.  Every call returns with the device work it issued complete.  A frame is
  *   not thread-safe (like its scene) and must be destroyed before its scene. */
@@ -284,6 +288,28 @@ int rt_frame_advance(RtFrame *frame, int32_t max_samples, double target_ms, RtFr
 int rt_frame_read(RtFrame *frame, int32_t gamma, uint8_t *rgb_out, int32_t *sums_out);
 int rt_frame_extend(RtFrame *frame, int32_t samples_per_pixel);
 void rt_frame_destroy(RtFrame *frame);
+
+/* Noise estimate of a progressive frame opened with RT_FLAG_NOISE.  Per pixel the frame holds, besides the channel sums
+ * T_c and the count n, Q = the sum over the pixel's samples of r^2 + g^2 + b^2 (8-bit levels).  Then
+ *     D = n Q - (T_r^2 + T_g^2 + T_b^2)          exact in int64 (every term < 3.5e18 at n <= 2^22)
+ *     E = sqrt(D / (3 n^2 (n - 1)))              in double, the denominator evaluated left to right as written
+ * is the RMS over the three channels of the standard error of the channel mean, in 8-bit levels; E = +inf where n < 2.
+ * Like the sums, Q is an integer keyed by (seed, pixel, sample index): it does not depend on how the frame was paced.
+ * rt_frame_noise returns, each optional: se_out rows*cols float E of every pixel, sq_out rows*cols uint64 Q, and the
+ * summary over the flagged pixels (those later passes still sample, in pixel order): how many, how many have
+ * E > tolerance, the largest and the mean E.  The summary is bit-identical from call to call (fixed-order reduction).
+ * RT_ERR_INVALID_ARGUMENT if the frame was opened without RT_FLAG_NOISE or tolerance is negative or NaN. */
+typedef struct RtFrameNoise {
+    uint64_t pixels;       /* flagged pixels (every pixel without the early-out)                        */
+    uint64_t pixels_above; /* of them, those with E > tolerance                                         */
+    double max_se;         /* the largest E over them (0 when there are none)                           */
+    double mean_se;        /* the mean E over them (0 when there are none)                              */
+    double tolerance;      /* as given                                                                  */
+} RtFrameNoise;
+int rt_frame_noise(RtFrame *frame, double tolerance, float *se_out, uint64_t *sq_out, RtFrameNoise *summary);
+/* The same E from saved moments, on the host (no device needed): sums n*4 int32 {T_r, T_g, T_b, n} as rt_render and
+ * rt_frame_read give them, sq n uint64 Q, se_out n float. */
+int rt_pixel_noise(const int32_t *sums, const uint64_t *sq, size_t n, float *se_out);
 
 /* The same frame split over the GPUs of this process (the F# host is one process): replicated scene,
  * sample-index split (Scene.fs:191-192 shared out by sample index), probe tiles shared out by tile.

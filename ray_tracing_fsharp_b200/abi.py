@@ -5,7 +5,7 @@ struct against the values the compiled library reports.
 """
 import ctypes as C
 
-RT_ABI_VERSION = 3
+RT_ABI_VERSION = 4
 
 RT_OK = 0
 RT_ERR_INVALID_ARGUMENT = -1
@@ -44,6 +44,7 @@ RT_FLAG_BVH2 = 8
 RT_FLAG_LOCKSTEP = 16
 RT_FLAG_FLOW = 32
 RT_FLAG_NO_LEAN = 64
+RT_FLAG_NOISE = 128  # rt_frame_begin only: keep the per-pixel sum of squares for rt_frame_noise
 
 RT_COMM_ID_BYTES = 128
 
@@ -137,4 +138,14 @@ class RtFrameProgress(C.Structure):
         ("device_ms", C.c_double),
         ("passes", C.c_int32),
         ("done", C.c_int32),
+    ]
+
+
+class RtFrameNoise(C.Structure):
+    _fields_ = [
+        ("pixels", C.c_uint64),
+        ("pixels_above", C.c_uint64),
+        ("max_se", C.c_double),
+        ("mean_se", C.c_double),
+        ("tolerance", C.c_double),
     ]

@@ -339,8 +339,16 @@ struct ItemSlot {
     unsigned acc_rg[32]; // sum of red | sum of green << 16
     unsigned acc_b[32];  // sum of blue
 };
-static_assert(sizeof(ItemSlot) % 16 == 0, "ItemSlot must be a multiple of 16 bytes");
-constexpr size_t warp_scratch_bytes(bool staged) { return size_t(item_slots(staged)) * sizeof(ItemSlot); } // per warp
+// The slot of the kernels that also sum r^2 + g^2 + b^2 per pixel (RT_FLAG_NOISE): one more word per lane, 528 bytes.  A chunk's
+// word stays below 3 x 255^2 x 256 < 2^26.
+struct NoiseItemSlot : ItemSlot {
+    unsigned acc_q[32]; // sum of r^2 + g^2 + b^2
+};
+static_assert(sizeof(ItemSlot) == 400 && sizeof(NoiseItemSlot) == 528, "item slot sizes");
+static_assert(sizeof(ItemSlot) % 16 == 0 && sizeof(NoiseItemSlot) % 16 == 0, "ItemSlot must be a multiple of 16 bytes");
+constexpr size_t warp_scratch_bytes(bool staged, bool noise = false) { // per warp
+    return size_t(item_slots(staged)) * (noise ? sizeof(NoiseItemSlot) : sizeof(ItemSlot));
+}
 
 __device__ __forceinline__ void flush_counters(unsigned long long *counters, uint32_t paths, uint32_t rays, TraversalCounters cn, bool count) {
     for (int off = 16; off > 0; off >>= 1) {
@@ -372,8 +380,12 @@ __device__ __forceinline__ void flush_counters(unsigned long long *counters, uin
 //                  remaining sample indices (Scene.fs:191-192).
 // A warp issues one instruction every ~7.6 cycles whatever the load, so the kernel ends one whole item after the
 // work runs out: hence chunks of decreasing length, the last ones a single sample (see build_chunks).
-template <bool PROBE, int SMEM, bool COUNT, bool SSTACK, bool WIDE>
+//   NOISE = true : also sum r^2 + g^2 + b^2 of every finished path per pixel (one more shared word per slot lane, flushed
+//                  with one 64-bit RED per pixel into fp.sq), for the noise estimate of progressive frames (rt_frame_noise).
+//                  The probe adds to the same sum whichever accumulator set its chunk belongs to.
+template <bool PROBE, int SMEM, bool COUNT, bool SSTACK, bool WIDE, bool NOISE = false>
 __global__ void __launch_bounds__(block_threads(SMEM), blocks_per_sm(SMEM)) render_kernel(const FrameParams fp) {
+    using Slot = typename std::conditional<NOISE, NoiseItemSlot, ItemSlot>::type;
     const SceneAccess<SMEM> sc = stage_scene<SMEM>(fp);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     typename std::conditional<SSTACK, SharedStack, LocalStack>::type stack;
@@ -383,7 +395,7 @@ __global__ void __launch_bounds__(block_threads(SMEM), blocks_per_sm(SMEM)) rend
         stack.levels = fp.stack_levels;
     }
     constexpr int kSlots = SMEM ? kItemSlots : kGlobalItemSlots;
-    ItemSlot *const slots = reinterpret_cast<ItemSlot *>(rtfs_smem + fp.s_warp) + warp * kSlots; // this warp's item slots
+    Slot *const slots = reinterpret_cast<Slot *>(rtfs_smem + fp.s_warp) + warp * kSlots; // this warp's item slots
     unsigned long long *work = fp.counters + (PROBE ? CN_WORK_PROBE : CN_WORK_MAIN);
     uint32_t n_paths = 0, n_rays = 0;
     TraversalCounters cn{0, 0};
@@ -393,7 +405,7 @@ __global__ void __launch_bounds__(block_threads(SMEM), blocks_per_sm(SMEM)) rend
     const unsigned long long n_items = (unsigned long long)n_units * (unsigned long long)fp.n_chunks;
 
     // Loads work item `item` into a slot: chunk-major numbering; this lane's pixel; the pool.  Returns the pool size.
-    auto load_item = [&](ItemSlot *sl, unsigned long long item, int &n_entries) -> int {
+    auto load_item = [&](Slot *sl, unsigned long long item, int &n_entries) -> int {
         const int k = int(item / n_units);
         const unsigned unit = unsigned(item - (unsigned long long)k * n_units);
         const int j_begin = int(fp.chunk_begin[k]), j_len = int(fp.chunk_len[k]);
@@ -410,6 +422,7 @@ __global__ void __launch_bounds__(block_threads(SMEM), blocks_per_sm(SMEM)) rend
             n_entries = int(min(32u, n_list - unit * 32u));
         }
         sl->acc_rg[lane] = 0u; sl->acc_b[lane] = 0u;
+        if constexpr (NOISE) sl->acc_q[lane] = 0u;
         sl->pix[lane] = my_pixel < 0 ? -1 : (((my_pixel / fp.cam.cols) << 16) | (my_pixel % fp.cam.cols));
         if (lane == 0) {
             sl->cursor = 0;
@@ -421,16 +434,18 @@ __global__ void __launch_bounds__(block_threads(SMEM), blocks_per_sm(SMEM)) rend
         return n_entries * j_len;
     };
     // Retires a slot whose paths have all finished: one RED per channel and pixel (PixelStats.add, Pixel.fs:87-95)
-    auto flush_item = [&](ItemSlot *sl) {
+    auto flush_item = [&](Slot *sl) {
         __syncwarp();
         const int rc = sl->pix[lane];
         if (rc >= 0) {
-            int *st = (sl->to_b ? fp.stats_b : fp.stats) + 4 * (size_t(rc >> 16) * size_t(fp.cam.cols) + size_t(rc & 0xffff));
+            const size_t p = size_t(rc >> 16) * size_t(fp.cam.cols) + size_t(rc & 0xffff);
+            int *st = (sl->to_b ? fp.stats_b : fp.stats) + 4 * p;
             const unsigned rg = sl->acc_rg[lane];
             atomicAdd(st + 0, int(rg & 0xffffu));
             atomicAdd(st + 1, int(rg >> 16));
             atomicAdd(st + 2, int(sl->acc_b[lane]));
             atomicAdd(st + 3, sl->j_len);
+            if constexpr (NOISE) atomicAdd(fp.sq + p, (unsigned long long)sl->acc_q[lane]);
         }
         __syncwarp();
     };
@@ -457,7 +472,7 @@ __global__ void __launch_bounds__(block_threads(SMEM), blocks_per_sm(SMEM)) rend
         int lane_slot = 0, my = 0; // my: slot index of this lane's path; lane_slot: its pixel within the item
         for (;;) {
             if (!active && !dry) {
-                ItemSlot *sl = &slots[cur];
+                Slot *sl = &slots[cur];
                 int q = atomicAdd(&sl->cursor, 1);
                 if (q >= pool) {
                     dry = true;
@@ -493,7 +508,7 @@ __global__ void __launch_bounds__(block_threads(SMEM), blocks_per_sm(SMEM)) rend
                     if (free_slot >= 0) {
                         item = __shfl_sync(0xffffffffu, prefetched, 0);
                         if (item < n_items) {
-                            ItemSlot *next = &slots[free_slot];
+                            Slot *next = &slots[free_slot];
                             pool = load_item(next, item, n_entries);
                             j_begin = next->j_begin;
                             prefetched = fetch_item();
@@ -513,9 +528,13 @@ __global__ void __launch_bounds__(block_threads(SMEM), blocks_per_sm(SMEM)) rend
                 ++n_rays;
                 if (path_step<SMEM, COUNT, decltype(stack), WIDE>(ps, sc, fp.cam.depth, result, cn, tracing, stack)) {
                     RTFS_BOUNDS(my >= 0 && my < kSlots && lane_slot >= 0 && lane_slot < 32);
-                    ItemSlot *mine = &slots[my]; // PixelStats.add into the item's accumulators
+                    Slot *mine = &slots[my]; // PixelStats.add into the item's accumulators
                     atomicAdd(&mine->acc_rg[lane_slot], ((result >> 16) & 255u) | ((result << 8) & 0x00ff0000u));
                     atomicAdd(&mine->acc_b[lane_slot], result & 255u);
+                    if constexpr (NOISE) {
+                        const unsigned r = (result >> 16) & 255u, g = (result >> 8) & 255u, b = result & 255u;
+                        atomicAdd(&mine->acc_q[lane_slot], r * r + g * g + b * b);
+                    }
                     if (result & kDegenerate) atomicAdd(fp.counters + CN_DEGENERATE, 1ull);
                     active = false;
                 }
@@ -609,24 +628,26 @@ struct LaunchPlan {
 };
 
 typedef void (*RenderKernelFn)(const FrameParams);
+// count and noise never come together (rt_frame_begin refuses RT_FLAG_NOISE with RT_FLAG_COUNTERS; plan_launch checks)
 template <bool PROBE, int SMEM, bool SSTACK, bool WIDE>
-static RenderKernelFn pick_count(bool count) {
+static RenderKernelFn pick_count(bool count, bool noise) {
+    if (noise) return render_kernel<PROBE, SMEM, false, SSTACK, WIDE, true>;
     return count ? render_kernel<PROBE, SMEM, true, SSTACK, WIDE> : render_kernel<PROBE, SMEM, false, SSTACK, WIDE>;
 }
 template <bool PROBE>
-static RenderKernelFn pick_global(bool sstack, bool wide, bool count) { // the scene is read from global memory
-    if (wide) return sstack ? pick_count<PROBE, 0, true, true>(count) : pick_count<PROBE, 0, false, true>(count);
-    return sstack ? pick_count<PROBE, 0, true, false>(count) : pick_count<PROBE, 0, false, false>(count);
+static RenderKernelFn pick_global(bool sstack, bool wide, bool count, bool noise) { // the scene is read from global memory
+    if (wide) return sstack ? pick_count<PROBE, 0, true, true>(count, noise) : pick_count<PROBE, 0, false, true>(count, noise);
+    return sstack ? pick_count<PROBE, 0, true, false>(count, noise) : pick_count<PROBE, 0, false, false>(count, noise);
 }
 template <bool PROBE>
 static RenderKernelFn pick_flow(bool smem, bool count) {
     if (smem) return count ? render_flow_kernel<PROBE, true, true> : render_flow_kernel<PROBE, true, false>;
     return count ? render_flow_kernel<PROBE, false, true> : render_flow_kernel<PROBE, false, false>;
 }
-static RenderKernelFn pick_kernel(bool probe, bool smem, bool lean, bool count, bool sstack, bool wide) {
-    if (smem && lean) return probe ? pick_count<true, 2, false, false>(count) : pick_count<false, 2, false, false>(count);
-    if (probe) return smem ? pick_count<true, 1, false, false>(count) : pick_global<true>(sstack, wide, count);
-    return smem ? pick_count<false, 1, false, false>(count) : pick_global<false>(sstack, wide, count);
+static RenderKernelFn pick_kernel(bool probe, bool smem, bool lean, bool count, bool sstack, bool wide, bool noise) {
+    if (smem && lean) return probe ? pick_count<true, 2, false, false>(count, noise) : pick_count<false, 2, false, false>(count, noise);
+    if (probe) return smem ? pick_count<true, 1, false, false>(count, noise) : pick_global<true>(sstack, wide, count, noise);
+    return smem ? pick_count<false, 1, false, false>(count, noise) : pick_global<false>(sstack, wide, count, noise);
 }
 
 // does a block with `bytes` of dynamic shared memory leave room for `per_sm` of its kind on an SM (1 KB reserved per block)
@@ -640,7 +661,10 @@ static int plan_launch(DeviceScene *ds, FrameParams &fp, bool probe, bool count,
     // the flow schedule (ring of rays per warp) on request only — measured slower than lockstep on B200 (DESIGN.md 5) —
     // and not with the wide tree (no flow variant) nor when the bounce budget does not fit the byte it shares with the colour
     const bool flow = (fp.opt_flags & RT_FLAG_FLOW) && !(fp.opt_flags & RT_FLAG_LOCKSTEP) && !wide_asked && fp.cam.depth <= kMaxFlowDepth;
-    size_t warp_q = (kBlockThreads / 32) * (flow ? sizeof(FlowWarp) : warp_scratch_bytes(true)) / 16;
+    // the sum of squares of progressive frames opened with RT_FLAG_NOISE: lockstep kernels without counters only
+    const bool noise = fp.sq != nullptr;
+    if (noise && (flow || count)) return fail(RT_ERR_UNSUPPORTED, "render: the noise estimate has no flow-schedule or counting kernel");
+    size_t warp_q = (kBlockThreads / 32) * (flow ? sizeof(FlowWarp) : warp_scratch_bytes(true, noise)) / 16;
     const size_t nodes_q = size_t(ds->g.n_nodes) * kStagedNodeQuads, sph_q = size_t(ds->g.n_bounded), mat_q = size_t(ds->g.n_bounded + ds->g.n_unbounded) * 2;
     const size_t scene_q = nodes_q + sph_q + mat_q;
     // stage the scene in shared memory when it fits beside the per-warp scratch (one block per SM)
@@ -650,7 +674,7 @@ static int plan_launch(DeviceScene *ds, FrameParams &fp, bool probe, bool count,
     // the launch shape follows from where the scene is read (rtfs_device.h); the flow kernels keep one block of 1024
     plan.threads = flow ? kBlockThreads : block_threads(smem);
     const int want_per_sm = flow ? 1 : blocks_per_sm(smem);
-    warp_q = size_t(plan.threads / 32) * (flow ? sizeof(FlowWarp) : warp_scratch_bytes(smem)) / 16;
+    warp_q = size_t(plan.threads / 32) * (flow ? sizeof(FlowWarp) : warp_scratch_bytes(smem, noise)) / 16;
     fp.s_nodes = 0;
     fp.s_spheres = uint32_t(nodes_q);
     fp.s_mats = uint32_t(nodes_q + sph_q);
@@ -661,7 +685,9 @@ static int plan_launch(DeviceScene *ds, FrameParams &fp, bool probe, bool count,
     // same change is within noise, 67.1 against 67.4 ms on C2, 137.7 against 136.7 on C4, so those kernels keep a local stack)
     const size_t used_q = (smem ? scene_q : 0) + warp_q;
     const size_t stack_q = size_t(wide ? 2 * (ds->wide_depth + 1) : ds->max_depth + 1) * size_t(plan.threads) * 4 / 16;
-    const bool sstack = !flow && !smem && ds->g.n_bounded > 0 && smem_fits(ds, (used_q + stack_q) * 16, want_per_sm);
+    // RTFS_LOCAL_STACK (A/B runs, tests): keep the walk stacks in local memory even where shared memory has room for them
+    static const bool local_stack = std::getenv("RTFS_LOCAL_STACK") != nullptr;
+    const bool sstack = !flow && !smem && !local_stack && ds->g.n_bounded > 0 && smem_fits(ds, (used_q + stack_q) * 16, want_per_sm);
     fp.s_stack = uint32_t(used_q);
     {
         static const int forced = [] {
@@ -672,7 +698,14 @@ static int plan_launch(DeviceScene *ds, FrameParams &fp, bool probe, bool count,
     }
     fp.stack_levels = int32_t(stack_q * 16 / (size_t(plan.threads) * 4));
     plan.smem_bytes = (used_q + (sstack ? stack_q : 0)) * 16;
-    fn = flow ? (probe ? pick_flow<true>(smem, count) : pick_flow<false>(smem, count)) : pick_kernel(probe, smem, ds->lean && !(fp.opt_flags & RT_FLAG_NO_LEAN), count, sstack, wide);
+    const bool lean = ds->lean && !(fp.opt_flags & RT_FLAG_NO_LEAN);
+    fn = flow ? (probe ? pick_flow<true>(smem, count) : pick_flow<false>(smem, count)) : pick_kernel(probe, smem, lean, count, sstack, wide, noise);
+    {
+        static const bool show = std::getenv("RTFS_DEBUG_PLAN") != nullptr;
+        if (show)
+            std::fprintf(stderr, "rtfs: plan probe=%d staged=%d lean=%d sstack=%d wide=%d flow=%d noise=%d smem_bytes=%zu threads=%d\n", int(probe),
+                         int(smem), int(smem && lean), int(sstack), int(wide), int(flow), int(noise), plan.smem_bytes, plan.threads);
+    }
     { // The dynamic shared-memory limit of a kernel is a per-function, per-device setting: it is only ever RAISED here
       // (to the largest size any scene has asked for), and the occupancy of a (kernel, size, device) triple is asked once.
         struct Known {

@@ -117,7 +117,7 @@ constexpr int kBlockThreads = RTFS_BLOCK_THREADS;
 constexpr int kBlocksPerSm = RTFS_BLOCKS_PER_SM;
 constexpr int kGlobalBlockThreads = RTFS_GLOBAL_BLOCK_THREADS;
 constexpr int kGlobalBlocksPerSm = RTFS_GLOBAL_BLOCKS_PER_SM;
-// Work-item slots per warp (rtfs_device.cu, 400 bytes each).  Four keep a warp fed best: on the 100 k-sphere scene (two blocks of
+// Work-item slots per warp (rtfs_device.cu, 400 bytes each, 528 with the sum of squares of RT_FLAG_NOISE).  Four keep a warp fed best: on the 100 k-sphere scene (two blocks of
 // 768 threads per SM) four slots 199.5 ms, three 202, two 222 (warps run dry).
 constexpr int kItemSlots = RTFS_ITEM_SLOTS, kGlobalItemSlots = RTFS_GLOBAL_ITEM_SLOTS;
 constexpr int item_slots(bool staged) { return staged ? kItemSlots : kGlobalItemSlots; }
@@ -152,6 +152,9 @@ struct FrameParams {
     int32_t opt_flags; // RtRenderOpts.flags
     int32_t stack_levels; // words per thread of the shared-memory walk stacks
     int32_t quantum;      // flow kernel: node visits between two schedule points
+    // last, so that no other parameter moves: rows*cols per-pixel sums of r^2 + g^2 + b^2 over the pixel's samples
+    // (progressive frames opened with RT_FLAG_NOISE; null otherwise, and then the kernels without that sum run)
+    unsigned long long *sq;
 };
 
 

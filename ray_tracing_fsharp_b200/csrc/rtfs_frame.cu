@@ -3,6 +3,8 @@
 // launch_samples over [samples_done, samples_done + k), i.e. the same render_kernel<PROBE = false> that rt_render's main
 // phase launches, with the same chunking.  Sums are integers keyed by (seed, pixel, sample index), so a frame that has
 // reached samples_done is bit for bit rt_render's frame at samples_per_pixel = samples_done (include/rtfs_b200.h).
+// A frame opened with RT_FLAG_NOISE also holds per pixel the sum of squares Q (render_kernel<NOISE = true>), from which
+// rt_frame_noise derives a per-pixel standard error and a summary over the flagged pixels.
 #include "rtfs_device.h"
 
 #include <algorithm>
@@ -10,6 +12,74 @@
 #include <cstring>
 
 using namespace rtfs;
+
+namespace rtfs {
+
+// E of a pixel from its moments: n samples, channel sums t0..t2, sum of squares q (include/rtfs_b200.h, rt_frame_noise).
+// D = n q - sum t_c^2 is exact in int64 for n <= 2^22 (each term < 3.5e18); the double arithmetic is the same, in the same
+// order, on the device and on the host (rt_pixel_noise), and IEEE division and square root round correctly on both.
+__host__ __device__ __forceinline__ double pixel_standard_error(int32_t n, int32_t t0, int32_t t1, int32_t t2, uint64_t q) {
+    if (n < 2) return HUGE_VAL;
+    // unsigned wrap-around arithmetic, then the int64 value: the same bits as the signed formula wherever that is defined
+    const uint64_t tt = uint64_t(int64_t(t0) * t0) + uint64_t(int64_t(t1) * t1) + uint64_t(int64_t(t2) * t2);
+    const int64_t d = int64_t(uint64_t(n) * q - tt);
+    const double nd = double(n);
+    return sqrt(double(d) / (3.0 * nd * nd * double(n - 1)));
+}
+
+// rt_frame_noise's reduction: a fixed grid, every block a fixed contiguous range of pixels, every thread a fixed stride of
+// it, then a fixed tree in shared memory, then one block over the partials in block order: no result depends on scheduling
+// (no floating-point atomics), so the summary is bit-identical from call to call.
+struct NoisePartial {
+    unsigned long long pixels, above;
+    double max_se, sum_se;
+};
+constexpr int kNoiseBlocks = 512, kNoiseThreads = 256;
+
+__device__ __forceinline__ void noise_combine(NoisePartial &a, const NoisePartial &b) {
+    a.pixels += b.pixels;
+    a.above += b.above;
+    a.max_se = fmax(a.max_se, b.max_se);
+    a.sum_se += b.sum_se;
+}
+
+__device__ __forceinline__ void noise_block_reduce(NoisePartial acc, NoisePartial *out) {
+    __shared__ NoisePartial part[kNoiseThreads];
+    part[threadIdx.x] = acc;
+    __syncthreads();
+    for (int half = kNoiseThreads / 2; half > 0; half >>= 1) {
+        if (int(threadIdx.x) < half) noise_combine(part[threadIdx.x], part[threadIdx.x + half]);
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *out = part[0];
+}
+
+__global__ void __launch_bounds__(kNoiseThreads) noise_kernel(const int4 *stats, const unsigned long long *sq, const uint8_t *flags, size_t n_pixels,
+                                                              double tolerance, float *se, NoisePartial *partial) {
+    const size_t per_block = (n_pixels + kNoiseBlocks - 1) / kNoiseBlocks;
+    const size_t begin = size_t(blockIdx.x) * per_block, end = begin + per_block < n_pixels ? begin + per_block : n_pixels;
+    NoisePartial acc{0ull, 0ull, 0.0, 0.0};
+    for (size_t p = begin + threadIdx.x; p < end; p += kNoiseThreads) {
+        const int4 s = stats[p];
+        const double e = pixel_standard_error(s.w, s.x, s.y, s.z, sq[p]);
+        if (se) se[p] = float(e);
+        if (flags[p]) {
+            acc.pixels += 1;
+            acc.above += e > tolerance ? 1 : 0;
+            acc.max_se = fmax(acc.max_se, e);
+            acc.sum_se += e;
+        }
+    }
+    noise_block_reduce(acc, partial + blockIdx.x);
+}
+
+__global__ void __launch_bounds__(kNoiseThreads) noise_summary_kernel(NoisePartial *partial) {
+    NoisePartial acc{0ull, 0ull, 0.0, 0.0};
+    for (int b = threadIdx.x; b < kNoiseBlocks; b += kNoiseThreads) noise_combine(acc, partial[b]);
+    noise_block_reduce(acc, partial + kNoiseBlocks);
+}
+
+} // namespace rtfs
 
 // A frame owns everything a pass writes: sums, flags, the flagged-pixel list, the image and its own counter block
 // (paths, rays, the list length and the work cursors), so rt_render and other frames can use the scene between passes.
@@ -23,6 +93,9 @@ struct RtFrame {
     uint32_t *d_list = nullptr;
     uint8_t *d_rgb = nullptr;
     unsigned long long *d_counters = nullptr;
+    unsigned long long *d_sq = nullptr; // RT_FLAG_NOISE: per pixel the sum of r^2 + g^2 + b^2 (null otherwise)
+    float *d_se = nullptr;              // rt_frame_noise's map, allocated on first use
+    NoisePartial *d_partial = nullptr;  // and its per-block partial summaries, then the summary (kNoiseBlocks + 1)
     unsigned long long h_counters[CN_SLOTS] = {};
     cudaEvent_t ev[2] = {nullptr, nullptr};
     int32_t samples_done = 0, samples_target = 0;
@@ -44,6 +117,9 @@ void frame_free(RtFrame *f) {
     cudaFree(f->d_list);
     cudaFree(f->d_rgb);
     cudaFree(f->d_counters);
+    cudaFree(f->d_sq);
+    cudaFree(f->d_se);
+    cudaFree(f->d_partial);
     for (auto &e : f->ev)
         if (e) cudaEventDestroy(e);
     delete f;
@@ -89,6 +165,9 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
     *out = nullptr;
     if (opts->mode == RT_MODE_WAVEFRONT) return fail(RT_ERR_UNSUPPORTED, "rt_frame_begin: progressive frames run the megakernel only");
     if (opts->mode != RT_MODE_MEGAKERNEL) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin: unknown mode");
+    const bool noise = (opts->flags & RT_FLAG_NOISE) != 0;
+    if (noise && (opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS)))
+        return fail(RT_ERR_UNSUPPORTED, "rt_frame_begin: RT_FLAG_NOISE has no flow-schedule or counting kernel");
     if ((rc = prepare_frame(scene, opts)) != RT_OK) return rc;
     auto *ds = static_cast<DeviceScene *>(scene->dev);
     RT_CUDA(cudaSetDevice(ds->device));
@@ -103,6 +182,7 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
     bool ok = cudaMalloc((void **)&f->d_stats, n * 4 * sizeof(int32_t)) == cudaSuccess && cudaMalloc((void **)&f->d_flags, n) == cudaSuccess &&
               cudaMalloc((void **)&f->d_list, n * sizeof(uint32_t)) == cudaSuccess && cudaMalloc((void **)&f->d_rgb, n * 3) == cudaSuccess &&
               cudaMalloc((void **)&f->d_counters, CN_SLOTS * sizeof(unsigned long long)) == cudaSuccess;
+    if (noise) ok = ok && cudaMalloc((void **)&f->d_sq, n * sizeof(unsigned long long)) == cudaSuccess;
     for (auto &e : f->ev) ok = ok && cudaEventCreate(&e) == cudaSuccess;
     if (!ok) return bail(fail(RT_ERR_CUDA, std::string("rt_frame_begin: allocation failed: ") + cudaGetErrorString(cudaGetLastError())));
 
@@ -112,6 +192,7 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
     fp.flags = f->d_flags;
     fp.list = f->d_list;
     fp.counters = f->d_counters;
+    fp.sq = f->d_sq; // non-null: plan_launch picks the kernels that also sum the squares
     f->count = (opts->flags & RT_FLAG_COUNTERS) != 0;
     f->no_smem = (opts->flags & RT_FLAG_NO_SMEM) != 0;
     f->samples_done = fp.n_probe; // 0 without the early-out
@@ -121,6 +202,7 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
     auto enqueue = [&]() -> int {
         RT_CUDA(cudaMemsetAsync(f->d_counters, 0, CN_SLOTS * sizeof(unsigned long long), st));
         RT_CUDA(cudaMemsetAsync(f->d_stats, 0, n * 4 * sizeof(int32_t), st));
+        if (f->d_sq) RT_CUDA(cudaMemsetAsync(f->d_sq, 0, n * sizeof(unsigned long long), st));
         RT_CUDA(cudaEventRecord(f->ev[0], st));
         if (fp.adaptive) {
             // the raw "means differ" flags, also where this target has no main phase: the frame can be extended
@@ -210,5 +292,41 @@ int rt_frame_extend(RtFrame *f, int32_t spp) {
 }
 
 void rt_frame_destroy(RtFrame *f) { frame_free(f); }
+
+int rt_frame_noise(RtFrame *f, double tolerance, float *se_out, uint64_t *sq_out, RtFrameNoise *summary) {
+    if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_noise: null frame");
+    if (!f->d_sq) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_noise: the frame was opened without RT_FLAG_NOISE");
+    if (!(tolerance >= 0.0)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_noise: tolerance must be >= 0");
+    auto *ds = static_cast<DeviceScene *>(f->scene->dev);
+    RT_CUDA(cudaSetDevice(ds->device));
+    cudaStream_t st = ds->ws->stream;
+    if (!f->d_partial) RT_CUDA(cudaMalloc((void **)&f->d_partial, (kNoiseBlocks + 1) * sizeof(NoisePartial)));
+    if (se_out && !f->d_se) RT_CUDA(cudaMalloc((void **)&f->d_se, f->n_pixels * sizeof(float)));
+    noise_kernel<<<kNoiseBlocks, kNoiseThreads, 0, st>>>(reinterpret_cast<const int4 *>(f->d_stats), f->d_sq, f->d_flags, f->n_pixels, tolerance,
+                                                         se_out ? f->d_se : nullptr, f->d_partial);
+    RT_CUDA(cudaGetLastError());
+    noise_summary_kernel<<<1, kNoiseThreads, 0, st>>>(f->d_partial);
+    RT_CUDA(cudaGetLastError());
+    NoisePartial total;
+    RT_CUDA(cudaMemcpyAsync(&total, f->d_partial + kNoiseBlocks, sizeof total, cudaMemcpyDeviceToHost, st));
+    if (se_out) RT_CUDA(cudaMemcpyAsync(se_out, f->d_se, f->n_pixels * sizeof(float), cudaMemcpyDeviceToHost, st));
+    if (sq_out) RT_CUDA(cudaMemcpyAsync(sq_out, f->d_sq, f->n_pixels * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaStreamSynchronize(st));
+    if (summary) {
+        summary->pixels = total.pixels;
+        summary->pixels_above = total.above;
+        summary->max_se = total.max_se;
+        summary->mean_se = total.pixels ? total.sum_se / double(total.pixels) : 0.0;
+        summary->tolerance = tolerance;
+    }
+    return RT_OK;
+}
+
+int rt_pixel_noise(const int32_t *sums, const uint64_t *sq, size_t n, float *se_out) {
+    if (n && (!sums || !sq || !se_out)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_pixel_noise: null buffer");
+    for (size_t p = 0; p < n; ++p)
+        se_out[p] = float(pixel_standard_error(sums[4 * p + 3], sums[4 * p], sums[4 * p + 1], sums[4 * p + 2], sq[p]));
+    return RT_OK;
+}
 
 } // extern "C"

@@ -10,7 +10,7 @@ import os
 import numpy as np
 
 from . import abi
-from .abi import RtCamera, RtFrameProgress, RtHittable, RtRenderOpts, RtStats, RtTexture
+from .abi import RtCamera, RtFrameNoise, RtFrameProgress, RtHittable, RtRenderOpts, RtStats, RtTexture
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "librtfs_b200.so")
@@ -54,6 +54,8 @@ def _declare(lib):
         "rt_frame_read": (C.c_int, [_vp, _i32, _vp, _vp]),
         "rt_frame_extend": (C.c_int, [_vp, _i32]),
         "rt_frame_destroy": (None, [_vp]),
+        "rt_frame_noise": (C.c_int, [_vp, C.c_double, _vp, _vp, C.POINTER(RtFrameNoise)]),
+        "rt_pixel_noise": (C.c_int, [_vp, _vp, C.c_size_t, _vp]),
         "rt_render_multi": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i32, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _vp,
                                       _vp, C.POINTER(RtStats)]),
         "rt_multi_create": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i32, C.POINTER(_vp)]),
@@ -323,6 +325,16 @@ class Frame:
         probe, or is below what the frame already holds)."""
         check(lib().rt_frame_extend(self.ptr, int(spp)))
 
+    def noise(self, tolerance, want_map=True, want_sq=False):
+        """The noise estimate of a frame opened with abi.RT_FLAG_NOISE (rt_frame_noise): (RtFrameNoise summary over the
+        flagged pixels against `tolerance`, the per-pixel standard error float32 [rows, cols] or None, the per-pixel sum of
+        r^2 + g^2 + b^2 uint64 [rows, cols] or None)."""
+        summary = RtFrameNoise()
+        se = np.empty((self.rows, self.cols), np.float32) if want_map else None
+        sq = np.empty((self.rows, self.cols), np.uint64) if want_sq else None
+        check(lib().rt_frame_noise(self.ptr, float(tolerance), ptr(se), ptr(sq), C.byref(summary)))
+        return summary, se, sq
+
     def close(self):
         if getattr(self, "ptr", None):
             lib().rt_frame_destroy(self.ptr)
@@ -516,6 +528,18 @@ def camera_make_basic(spp, focal, aspect, origin, view_dir, view_up):
     origin, view_dir, view_up = f64(origin), f64(view_dir), f64(view_up)
     check(lib().rt_camera_make_basic(spp, focal, aspect, ptr(origin), ptr(view_dir), ptr(view_up), C.byref(cam)))
     return cam
+
+
+def pixel_noise(sums, sq):
+    """rt_pixel_noise on the host: the per-pixel standard error (float32, the shape of `sq`) from saved moments, `sums`
+    int32 [..., 4] {sumR, sumG, sumB, count} and `sq` uint64 [...] (the sum of r^2 + g^2 + b^2).  Needs no device."""
+    sums = np.ascontiguousarray(sums, np.int32)
+    sq = np.ascontiguousarray(sq, np.uint64)
+    if sums.shape != sq.shape + (4,):
+        raise ValueError(f"sums {sums.shape} must be sq's shape {sq.shape} + (4,)")
+    se = np.empty(sq.shape, np.float32)
+    check(lib().rt_pixel_noise(ptr(sums), ptr(sq), sq.size, ptr(se)))
+    return se
 
 
 def ppm_format(rgb, gamma=False):

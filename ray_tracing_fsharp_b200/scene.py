@@ -125,14 +125,18 @@ class Scene:
     def render_progressive(progress_increment: Callable[[float], None], print_fn: Callable[[str], None], max_width_coord: int,
                            max_height_coord: int, camera: abi.RtCamera, s: "Scene", seed: Optional[int] = None, adaptive: bool = True,
                            target_ms: float = 250.0, on_pass: Optional[Callable[[abi.RtFrameProgress, "native.Frame"], object]] = None,
-                           flags: int = 0) -> np.ndarray:
+                           flags: int = 0, noise_tolerance: Optional[float] = None, noise_fraction: float = 0.0) -> np.ndarray:
         """Scene.render's frame rendered in passes of about `target_ms` of device time each (native.Frame, one GPU).
         `progress_increment(1.0)` is called as passes complete, in proportion to the paths traced so far out of the frame's
         total, and exactly `rows` times in all, like the reference's one call per row (Scene.fs:232).  After every pass
         `on_pass(progress, frame)` is called, if given: it may read the current image (`frame.read()`, exactly the frame of
         `progress.samples_done` samples per pixel) and stops the frame by returning True.  Returns the pixels (uint8
         [rows, cols, 3], before gamma): with the same seed, Scene.render's image, or that of the samples done when stopped.
-        `print_fn` is accepted and ignored as in Scene.render."""
+        `print_fn` is accepted and ignored as in Scene.render.
+        With `noise_tolerance` (8-bit levels) the frame also keeps its noise estimate (abi.RT_FLAG_NOISE, Frame.noise) and
+        stops at the first check where at most `noise_fraction` of the pixels still being sampled have a standard error
+        of the mean above the tolerance.  The check runs after the probe and after every pass (after `on_pass`); the image
+        returned is then rt_render's at the samples done."""
         if not isinstance(s._handle, native.SceneHandle):
             raise NotImplementedError("progressive frames run on one GPU: make the scene with a single device")
         rows = 2 * max_height_coord + 1
@@ -144,15 +148,26 @@ class Scene:
             for _ in range(n):
                 progress_increment(1.0)
 
+        if noise_tolerance is not None:
+            flags |= abi.RT_FLAG_NOISE
+
+        def converged(frame, progress):
+            if noise_tolerance is None or progress.done:
+                return False
+            summary, _, _ = frame.noise(noise_tolerance, want_map=False)
+            return summary.pixels_above <= noise_fraction * summary.pixels
+
         with s._handle.open_frame(camera, max_width_coord, max_height_coord, seed=seed, adaptive=adaptive, flags=flags) as frame:
             progress = frame.progress
             emit(ticks.update(progress.paths_done, progress.paths_target))  # the probe
-            while not progress.done:
+            stop = converged(frame, progress)
+            while not progress.done and not stop:
                 progress = frame.advance(target_ms=target_ms)
                 if not progress.done:
                     emit(ticks.update(progress.paths_done, progress.paths_target))
                 if on_pass is not None and on_pass(progress, frame):
                     break
+                stop = converged(frame, progress)
             rgb, _ = frame.read()
         emit(ticks.finish())  # the last pass's share, or the rest of the frame when on_pass stopped it
         return rgb

@@ -10,7 +10,8 @@
 // `InfinitePlane` (InfinitePlane.fs:101-106).  It adds `Scene.renderGpu`, with the signature of
 // `Scene.render` (Scene.fs:196-204), over a `GpuScene` built by `GpuScene.make : Hittable array -> GpuScene`
 // (the counterpart of `Scene.make`, Scene.fs:15-28), and `SceneGpu.renderWithProgress`, the same frame traced in passes
-// with progress reported as they finish (a `GpuFrame`, rt_frame_*, for callers that want the passes themselves).
+// with progress reported as they finish (a `GpuFrame`, rt_frame_*, for callers that want the passes themselves), and
+// `SceneGpu.renderWithProgressUntil`, which also stops the frame once its per-pixel noise estimate is below a tolerance.
 namespace RayTracing
 
 open System
@@ -122,6 +123,15 @@ module internal Native =
         val mutable passes : int
         val mutable isDone : int // `done` in the header (a keyword in F#)
 
+    [<Struct ; StructLayout(LayoutKind.Sequential)>]
+    type RtFrameNoise =
+        val mutable pixels : uint64
+        val mutable pixelsAbove : uint64
+        val mutable maxSe : float
+        val mutable meanSe : float
+        val mutable tolerance : float
+
+
     [<DllImport(Lib)>]
     extern nativeint rt_last_error ()
 
@@ -152,6 +162,12 @@ module internal Native =
 
     [<DllImport(Lib)>]
     extern void rt_frame_destroy (nativeint frame)
+
+    [<DllImport(Lib)>]
+    extern int rt_frame_noise (nativeint frame, float tolerance, float32[] seOut, uint64[] sqOut, RtFrameNoise& summary)
+
+    [<DllImport(Lib)>]
+    extern int rt_pixel_noise (int[] sums, uint64[] sq, unativeint n, float32[] seOut)
 
     [<DllImport(Lib)>]
     extern int rt_multi_create (RtHittable[] objects, int nObjects, RtTexture[] textures, int nTextures, int[] devices, int nDevices, nativeint& multi)
@@ -441,6 +457,25 @@ module GpuScene =
 
     let make (objects : Hittable array) : GpuScene = makeOn [| 0 |] objects
 
+/// RtRenderOpts.flags bits a caller may pass to SceneGpu.openFrameWith (include/rtfs_b200.h, RT_FLAG_*).
+[<RequireQualifiedAccess>]
+module FrameFlags =
+    /// RT_FLAG_NOISE: the frame also keeps the per-pixel sum of squares its noise estimate (GpuFrame.Noise) needs
+    [<Literal>]
+    let Noise = 128
+
+/// The noise estimate of a progressive frame over the pixels later passes still sample (RtFrameNoise of
+/// include/rtfs_b200.h, copied out of the native struct): how many there are, how many have a standard error of the mean
+/// above the tolerance (8-bit levels), the largest and the mean standard error, and the tolerance asked for.
+type FrameNoise =
+    {
+        Pixels : uint64
+        PixelsAbove : uint64
+        MaxSe : float
+        MeanSe : float
+        Tolerance : float
+    }
+
 /// A frame in progress on a single-device GpuScene (rt_frame_*): advanced in passes over windows of sample indices.
 /// After every pass it is exactly the frame rt_render gives at `SamplesDone` samples per pixel with the same seed, so
 /// `Read` shows the image sharpening; a caller stops early by not advancing any more, and `Extend` continues a finished
@@ -477,6 +512,23 @@ type GpuFrame internal (handle : nativeint, rows : int, cols : int, first : Nati
     /// what the frame holds.
     member _.Extend (samplesPerPixel : int) : unit =
         Native.rt_frame_extend (handle, samplesPerPixel) |> Native.check
+
+    /// The noise estimate of a frame opened with FrameFlags.Noise (rt_frame_noise): the summary over the pixels later
+    /// passes still sample, against `tolerance` (8-bit levels), and with `wantMap` the standard error of every pixel,
+    /// row-major Rows * Cols (null otherwise).
+    member _.Noise (tolerance : float, wantMap : bool) : FrameNoise * float32[] =
+        let map = if wantMap then Array.zeroCreate<float32> (rows * cols) else null
+        let mutable summary = Native.RtFrameNoise ()
+        Native.rt_frame_noise (handle, tolerance, map, null, &summary) |> Native.check
+
+        {
+            Pixels = summary.pixels
+            PixelsAbove = summary.pixelsAbove
+            MaxSe = summary.maxSe
+            MeanSe = summary.meanSe
+            Tolerance = summary.tolerance
+        },
+        map
 
     interface IDisposable with
         member _.Dispose () =
@@ -575,8 +627,9 @@ module SceneGpu =
 
         1.0<progress> * float rowsIter, Image.make rowsIter colsIter rows
 
-    /// Opens a progressive frame (rt_frame_begin: the probe runs now).  Single-device scenes only.
-    let openFrame (maxWidthCoord : int) (maxHeightCoord : int) (camera : Camera) (seed : uint64) (s : GpuScene) : GpuFrame =
+    /// Opens a progressive frame with RtRenderOpts.flags `flags` (e.g. FrameFlags.Noise for GpuFrame.Noise).
+    /// Single-device scenes only.
+    let openFrameWith (flags : int) (maxWidthCoord : int) (maxHeightCoord : int) (camera : Camera) (seed : uint64) (s : GpuScene) : GpuFrame =
         if s.IsMulti then
             failwith "GPU backend: progressive frames run on a single-device GpuScene"
 
@@ -584,6 +637,7 @@ module SceneGpu =
         let mutable opts = Native.RtRenderOpts ()
         opts.seed <- seed
         opts.adaptive <- 1
+        opts.flags <- flags
         let mutable handle = 0n
         let mutable progress = Native.RtFrameProgress ()
 
@@ -592,10 +646,16 @@ module SceneGpu =
 
         new GpuFrame (handle, 2 * maxHeightCoord + 1, 2 * maxWidthCoord + 1, progress)
 
-    /// `render`'s signature and laziness, but the frame is traced in passes of about 250 ms of device time and
-    /// `progressIncrement 1.0<progress>` is called as passes finish, in proportion to the paths traced out of the frame's
-    /// total: `rows` calls in all, as the reference makes (Scene.fs:232).  Single-device scenes only.
-    let renderWithProgress
+    /// Opens a progressive frame (rt_frame_begin: the probe runs now).  Single-device scenes only.
+    let openFrame (maxWidthCoord : int) (maxHeightCoord : int) (camera : Camera) (seed : uint64) (s : GpuScene) : GpuFrame =
+        openFrameWith 0 maxWidthCoord maxHeightCoord camera seed s
+
+    /// `renderWithProgress` with a stop on the noise estimate: with `Some (tolerance, fraction)` the frame stops at the
+    /// first check (after the probe, then after every pass) where at most `fraction` of the pixels still being sampled
+    /// have a standard error of the mean above `tolerance` (8-bit levels); the image is then rt_render's at the samples
+    /// done.  `None` is renderWithProgress.
+    let renderWithProgressUntil
+        (noiseStop : (float * float) option)
         (progressIncrement : float<progress> -> unit)
         (_print : string -> unit)
         (maxWidthCoord : int)
@@ -609,8 +669,10 @@ module SceneGpu =
 
         let frame =
             lazy
-                (use f =
-                    openFrame maxWidthCoord maxHeightCoord camera (uint64 (Random().NextInt64 ())) s
+                (let flags = if noiseStop.IsSome then FrameFlags.Noise else 0
+
+                 use f =
+                    openFrameWith flags maxWidthCoord maxHeightCoord camera (uint64 (Random().NextInt64 ())) s
 
                  let ticked = ref 0
 
@@ -627,12 +689,26 @@ module SceneGpu =
 
                      ticked.Value <- max ticked.Value want
 
-                 tick ()
+                 let converged () =
+                     match noiseStop with
+                     | Some (tolerance, fraction) when not f.IsDone ->
+                         let summary, _ = f.Noise (tolerance, false)
+                         float summary.PixelsAbove <= fraction * float summary.Pixels
+                     | _ -> false
 
-                 while not f.IsDone do
+                 tick ()
+                 let mutable stop = converged ()
+
+                 while not f.IsDone && not stop do
                      f.Advance (0, 250.0)
                      tick ()
+                     stop <- converged ()
 
+                 // a frame stopped on its noise hands out the rest of the rows' ticks
+                 for _ in ticked.Value + 1 .. rowsIter do
+                     progressIncrement 1.0<progress>
+
+                 ticked.Value <- rowsIter
                  f.Read false)
 
         let rows =
@@ -658,3 +734,17 @@ module SceneGpu =
                 )
 
         1.0<progress> * float rowsIter, Image.make rowsIter colsIter rows
+
+    /// `render`'s signature and laziness, but the frame is traced in passes of about 250 ms of device time and
+    /// `progressIncrement 1.0<progress>` is called as passes finish, in proportion to the paths traced out of the frame's
+    /// total: `rows` calls in all, as the reference makes (Scene.fs:232).  Single-device scenes only.
+    let renderWithProgress
+        (progressIncrement : float<progress> -> unit)
+        (print : string -> unit)
+        (maxWidthCoord : int)
+        (maxHeightCoord : int)
+        (camera : Camera)
+        (s : GpuScene)
+        : float<progress> * Image
+        =
+        renderWithProgressUntil None progressIncrement print maxWidthCoord maxHeightCoord camera s

@@ -703,8 +703,9 @@ static int plan_launch(DeviceScene *ds, FrameParams &fp, bool probe, bool count,
     {
         static const bool show = std::getenv("RTFS_DEBUG_PLAN") != nullptr;
         if (show)
-            std::fprintf(stderr, "rtfs: plan probe=%d staged=%d lean=%d sstack=%d wide=%d flow=%d noise=%d smem_bytes=%zu threads=%d\n", int(probe),
-                         int(smem), int(smem && lean), int(sstack), int(wide), int(flow), int(noise), plan.smem_bytes, plan.threads);
+            std::fprintf(stderr, "rtfs: plan probe=%d staged=%d lean=%d count=%d sstack=%d wide=%d flow=%d noise=%d smem_bytes=%zu threads=%d\n",
+                         int(probe), int(smem), int(smem && lean), int(count), int(sstack), int(wide), int(flow), int(noise), plan.smem_bytes,
+                         plan.threads);
     }
     { // The dynamic shared-memory limit of a kernel is a per-function, per-device setting: it is only ever RAISED here
       // (to the largest size any scene has asked for), and the occupancy of a (kernel, size, device) triple is asked once.

@@ -61,6 +61,83 @@ def small_random_spheres(n_side=4, seed=3):
     return sample_images.SceneSpec("reduced RTOW scene", objs, 32, 6.0, 1.5, (8.0, 2.0, -3.0), (0.0, 0.5, 0.0), (0.0, 1.0, 0.0), 60, 40, 50)
 
 
+# ---- frames rebuilt sample by sample --------------------------------------------------------------------------------------
+# Every sample is a pure function of (seed, pixel, sample index), so a frame's accumulators are the sums of the colours a
+# tracer (rt_test_trace_samples, or the oracle) gives for the pixel's sample indices.
+BATCH = 1 << 24  # paths per tracer call
+
+
+def sample_moments(tracer, cam, mw, mh, seed, pixels, s_begin, s_end):
+    """Per pixel, the colour sums ([n, 3] int64), the sum of r^2 + g^2 + b^2 ([n] int64) and the rays taken, of samples
+    s_begin .. s_end - 1."""
+    cols = 2 * mw + 1
+    m = s_end - s_begin
+    sums = np.zeros((len(pixels), 3), np.int64)
+    sq = np.zeros(len(pixels), np.int64)
+    rays = 0
+    if m <= 0 or len(pixels) == 0:
+        return sums, sq, rays
+    per_call = max(1, BATCH // m)
+    smp = np.arange(s_begin, s_end, dtype=np.int32)
+    for lo in range(0, len(pixels), per_call):
+        pix = pixels[lo:lo + per_call]
+        row = np.repeat((pix // cols).astype(np.int32), m)
+        col = np.repeat((pix % cols).astype(np.int32), m)
+        colour, r = tracer.trace_samples(cam, mw, mh, seed, row, col, np.tile(smp, len(pix)))
+        c = colour.astype(np.int64).reshape(len(pix), m, 3)
+        sums[lo:lo + len(pix)] = c.sum(1)
+        sq[lo:lo + len(pix)] = (c * c).sum((1, 2))
+        rays += int(r.sum(dtype=np.int64))
+    return sums, sq, rays
+
+
+def expected_sums(tracer, cam, max_w, max_h, seed, adaptive, pixels):
+    """What the frame's accumulators of the flat pixel ids `pixels` must hold: ([n, 4] int64 sums with the count in the last
+    column, the per-pixel count, the rays of all those samples).  renderPixel's rule (Scene.fs:157-194) exactly as fill_frame /
+    probe_flags_kernel and the oracle's render_pixel apply it: samples 0 .. firstTrial give the old mean, samples
+    0 .. 2 firstTrial the new one; a pixel whose truncated means differ takes samples up to spp - 1, if there are more."""
+    pixels = np.asarray(pixels, np.int64)
+    spp = int(cam.samples_per_pixel)
+    if adaptive:
+        ft = min(5, spp // 2)
+        n_probe = 2 * ft + 1
+        a, _, rays_a = sample_moments(tracer, cam, max_w, max_h, seed, pixels, 0, ft + 1)
+        b, _, rays_b = sample_moments(tracer, cam, max_w, max_h, seed, pixels, ft + 1, n_probe)
+        s = a + b
+        flagged = (np.abs(s // n_probe - a // (ft + 1)).sum(1) != 0) & (spp > n_probe)
+        more, _, rays_c = sample_moments(tracer, cam, max_w, max_h, seed, pixels[flagged], n_probe, spp)
+        s[flagged] += more
+        count = np.where(flagged, spp, n_probe)
+        rays = rays_a + rays_b + rays_c
+    else:
+        s, _, rays = sample_moments(tracer, cam, max_w, max_h, seed, pixels, 0, spp)
+        count = np.full(len(pixels), spp, np.int64)
+    return np.concatenate([s, count[:, None]], 1), count, rays
+
+
+def expected_moments(tracer, cam, mw, mh, seed, adaptive, pixels, samples_done):
+    """([n, 4] sums with the count, [n] Q) of the flat pixel ids `pixels` in a frame of cam.samples_per_pixel that has reached
+    samples_done.  renderPixel's rule: samples 0 .. firstTrial give the old mean, 0 .. 2 firstTrial the new one; a frame keeps
+    the raw "means differ" flags, and a flagged pixel holds sample indices 0 .. samples_done - 1."""
+    pixels = np.asarray(pixels, np.int64)
+    spp = int(cam.samples_per_pixel)
+    if adaptive:
+        ft = min(5, spp // 2)
+        n_probe = 2 * ft + 1
+        a, qa, _ = sample_moments(tracer, cam, mw, mh, seed, pixels, 0, ft + 1)
+        b, qb, _ = sample_moments(tracer, cam, mw, mh, seed, pixels, ft + 1, n_probe)
+        s, q = a + b, qa + qb
+        flagged = np.abs(s // n_probe - a // (ft + 1)).sum(1) != 0
+        more, qm, _ = sample_moments(tracer, cam, mw, mh, seed, pixels[flagged], n_probe, samples_done)
+        s[flagged] += more
+        q[flagged] += qm
+        count = np.where(flagged, samples_done, n_probe)
+    else:
+        s, q, _ = sample_moments(tracer, cam, mw, mh, seed, pixels, 0, samples_done)
+        count = np.full(len(pixels), samples_done, np.int64)
+    return np.concatenate([s, count[:, None]], 1), q
+
+
 def camera_sample_rays(spec, cam, rng, n):
     """Primary rays of random pixels as the oracle generates them: FP32-representable origins, unit directions in
     double (the oracle's formulas assume |d| = 1 to double precision, as the reference's UnitVector guarantees; the

@@ -18,11 +18,9 @@ import numpy as np
 import pytest
 
 import oracle
-from helpers import oracle_camera, small_random_spheres, unit
+from helpers import expected_sums, oracle_camera, small_random_spheres, unit
 from ray_tracing_fsharp_b200 import abi, sample_images
 from ray_tracing_fsharp_b200.domain import marshal
-
-BATCH = 1 << 24  # paths per tracer call
 
 
 class ParallelTracer:
@@ -41,50 +39,6 @@ class ParallelTracer:
             out = list(pool.map(lambda i: self.tracer.trace_samples(cam, max_w, max_h, seed, row[cut[i]:cut[i + 1]], col[cut[i]:cut[i + 1]],
                                                                     sample[cut[i]:cut[i + 1]]), range(parts)))
         return np.concatenate([c for c, _ in out]), np.concatenate([r for _, r in out])
-
-
-def _sample_sums(tracer, cam, max_w, max_h, seed, pixels, s_begin, s_end):
-    """Per pixel, the colour sums of samples s_begin .. s_end - 1 ([n, 3] int64), and the rays they took."""
-    cols = 2 * max_w + 1
-    m = s_end - s_begin
-    sums = np.zeros((len(pixels), 3), np.int64)
-    rays = 0
-    if m <= 0 or len(pixels) == 0:
-        return sums, rays
-    per_call = max(1, BATCH // m)
-    smp = np.arange(s_begin, s_end, dtype=np.int32)
-    for lo in range(0, len(pixels), per_call):
-        pix = pixels[lo:lo + per_call]
-        row = np.repeat((pix // cols).astype(np.int32), m)
-        col = np.repeat((pix % cols).astype(np.int32), m)
-        colour, r = tracer.trace_samples(cam, max_w, max_h, seed, row, col, np.tile(smp, len(pix)))
-        sums[lo:lo + len(pix)] = colour.reshape(len(pix), m, 3).sum(1, dtype=np.int64)
-        rays += int(r.sum(dtype=np.int64))
-    return sums, rays
-
-
-def expected_sums(tracer, cam, max_w, max_h, seed, adaptive, pixels):
-    """What the frame's accumulators of the flat pixel ids `pixels` must hold: ([n, 4] int64 sums with the count in the last
-    column, the per-pixel count, the rays of all those samples).  renderPixel's rule (Scene.fs:157-194) exactly as fill_frame /
-    probe_flags_kernel and the oracle's render_pixel apply it: samples 0 .. firstTrial give the old mean, samples
-    0 .. 2 firstTrial the new one; a pixel whose truncated means differ takes samples up to spp - 1, if there are more."""
-    pixels = np.asarray(pixels, np.int64)
-    spp = int(cam.samples_per_pixel)
-    if adaptive:
-        ft = min(5, spp // 2)
-        n_probe = 2 * ft + 1
-        a, rays_a = _sample_sums(tracer, cam, max_w, max_h, seed, pixels, 0, ft + 1)
-        b, rays_b = _sample_sums(tracer, cam, max_w, max_h, seed, pixels, ft + 1, n_probe)
-        s = a + b
-        flagged = (np.abs(s // n_probe - a // (ft + 1)).sum(1) != 0) & (spp > n_probe)
-        more, rays_c = _sample_sums(tracer, cam, max_w, max_h, seed, pixels[flagged], n_probe, spp)
-        s[flagged] += more
-        count = np.where(flagged, spp, n_probe)
-        rays = rays_a + rays_b + rays_c
-    else:
-        s, rays = _sample_sums(tracer, cam, max_w, max_h, seed, pixels, 0, spp)
-        count = np.full(len(pixels), spp, np.int64)
-    return np.concatenate([s, count[:, None]], 1), count, rays
 
 
 def assert_exact(sums, pixels, want, what):

@@ -2,7 +2,7 @@
 
 Every sample is a pure function of (seed, pixel, sample index) and rt_test_trace_samples reproduces it, so the per-pixel sum
 of squares Q a frame keeps is checked EXACTLY against the sum of r^2 + g^2 + b^2 over the pixel's sample indices, with
-renderPixel's early-out rule applied to the same colours (restated here from test_gpu_frame_reconstruction.py).  A frame
+renderPixel's early-out rule applied to the same colours (helpers.expected_moments).  A frame
 opened with the flag must still be rt_render's frame at samples_done, bit for bit; the estimate derived from Q must equal a
 numpy restatement; and render_progressive must stop at the first check that meets its rule."""
 import ctypes as C
@@ -15,7 +15,7 @@ import pytest
 
 if __name__ == "__main__":  # the child process of test_noise_kernels_with_local_walk_stacks
     sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from helpers import oracle_camera  # noqa: E402
+from helpers import expected_moments, oracle_camera  # noqa: E402
 from ray_tracing_fsharp_b200 import abi, native, sample_images  # noqa: E402
 from ray_tracing_fsharp_b200.domain import marshal  # noqa: E402
 from ray_tracing_fsharp_b200.scene import Image, Scene  # noqa: E402
@@ -23,7 +23,6 @@ from ray_tracing_fsharp_b200.scene import Image, Scene  # noqa: E402
 pytestmark = pytest.mark.gpu
 
 NOISE = abi.RT_FLAG_NOISE
-BATCH = 1 << 24  # paths per tracer call
 
 
 @pytest.fixture(scope="module")
@@ -64,51 +63,7 @@ def numpy_se(sums, sq):
     return np.where(n < 2, np.inf, e)
 
 
-# ---- reconstruction from single samples ----------------------------------------------------------------------------------
-def sample_moments(tracer, cam, mw, mh, seed, pixels, s_begin, s_end):
-    """Per pixel, the colour sums ([n, 3] int64) and the sum of r^2 + g^2 + b^2 ([n] int64) of samples s_begin .. s_end - 1."""
-    cols = 2 * mw + 1
-    m = s_end - s_begin
-    sums = np.zeros((len(pixels), 3), np.int64)
-    sq = np.zeros(len(pixels), np.int64)
-    if m <= 0 or len(pixels) == 0:
-        return sums, sq
-    per_call = max(1, BATCH // m)
-    smp = np.arange(s_begin, s_end, dtype=np.int32)
-    for lo in range(0, len(pixels), per_call):
-        pix = pixels[lo:lo + per_call]
-        row = np.repeat((pix // cols).astype(np.int32), m)
-        col = np.repeat((pix % cols).astype(np.int32), m)
-        colour, _ = tracer.trace_samples(cam, mw, mh, seed, row, col, np.tile(smp, len(pix)))
-        c = colour.astype(np.int64).reshape(len(pix), m, 3)
-        sums[lo:lo + len(pix)] = c.sum(1)
-        sq[lo:lo + len(pix)] = (c * c).sum((1, 2))
-    return sums, sq
-
-
-def expected_moments(tracer, cam, mw, mh, seed, adaptive, pixels, samples_done):
-    """([n, 4] sums with the count, [n] Q) of the flat pixel ids `pixels` in a frame of cam.samples_per_pixel that has reached
-    samples_done.  renderPixel's rule: samples 0 .. firstTrial give the old mean, 0 .. 2 firstTrial the new one; a frame keeps
-    the raw "means differ" flags, and a flagged pixel holds sample indices 0 .. samples_done - 1."""
-    pixels = np.asarray(pixels, np.int64)
-    spp = int(cam.samples_per_pixel)
-    if adaptive:
-        ft = min(5, spp // 2)
-        n_probe = 2 * ft + 1
-        a, qa = sample_moments(tracer, cam, mw, mh, seed, pixels, 0, ft + 1)
-        b, qb = sample_moments(tracer, cam, mw, mh, seed, pixels, ft + 1, n_probe)
-        s, q = a + b, qa + qb
-        flagged = np.abs(s // n_probe - a // (ft + 1)).sum(1) != 0
-        more, qm = sample_moments(tracer, cam, mw, mh, seed, pixels[flagged], n_probe, samples_done)
-        s[flagged] += more
-        q[flagged] += qm
-        count = np.where(flagged, samples_done, n_probe)
-    else:
-        s, q = sample_moments(tracer, cam, mw, mh, seed, pixels, 0, samples_done)
-        count = np.full(len(pixels), samples_done, np.int64)
-    return np.concatenate([s, count[:, None]], 1), q
-
-
+# ---- reconstruction from single samples (helpers.expected_moments) ----------------------------------------------------
 def row_subset(rows, cols, stride, n_random, seed):
     """Rows 0-3, the last four rows, every `stride`-th row between them, and `n_random` pixels anywhere (flat ids)."""
     picked = np.unique(np.concatenate([np.arange(4), np.arange(4, rows - 4, stride), np.arange(rows - 4, rows)]))

@@ -85,56 +85,6 @@ int nccl_api(NcclApi **out) {
     return RT_OK;
 }
 
-struct PeerReduceParams {
-    const int32_t *stats[kMaxDevices];
-    uint8_t *rgb[kMaxDevices];
-    int32_t world, n_pixels, quad_begin, quad_end, gamma;
-};
-// The fused tail of a frame for one rank's slice: sum over ranks (peer loads over NVLink) -> truncating mean -> gamma ->
-// RGB8 into every rank's frame (peer stores).  Four pixels per thread: the stores are whole 32-bit words.
-__global__ void peer_reduce_finalize_gather_kernel(const PeerReduceParams p) {
-    __shared__ uint8_t lut[256];
-    for (int i = threadIdx.x; i < 256; i += blockDim.x) {
-        int v = i;
-        if (p.gamma) {
-            v = __double2int_rn(sqrt(double(i) / 255.0) * 255.0); // Math.Round: half to even
-            if (v == 256) v = 255;
-        }
-        lut[i] = uint8_t(v);
-    }
-    __syncthreads();
-    const int quad = p.quad_begin + blockIdx.x * blockDim.x + threadIdx.x;
-    if (quad >= p.quad_end) return;
-    uint8_t out[12];
-    const int n_valid = min(4, p.n_pixels - 4 * quad);
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        int4 s = make_int4(0, 0, 0, 0);
-        if (k < n_valid) {
-            for (int r = 0; r < p.world; ++r) {
-                const int4 v = reinterpret_cast<const int4 *>(p.stats[r])[4 * quad + k];
-                s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
-            }
-        }
-        const int n = s.w > 0 ? s.w : 1;
-        out[3 * k + 0] = lut[(s.x / n) & 255];
-        out[3 * k + 1] = lut[(s.y / n) & 255];
-        out[3 * k + 2] = lut[(s.z / n) & 255];
-    }
-    const uint32_t w0 = uint32_t(out[0]) | (uint32_t(out[1]) << 8) | (uint32_t(out[2]) << 16) | (uint32_t(out[3]) << 24);
-    const uint32_t w1 = uint32_t(out[4]) | (uint32_t(out[5]) << 8) | (uint32_t(out[6]) << 16) | (uint32_t(out[7]) << 24);
-    const uint32_t w2 = uint32_t(out[8]) | (uint32_t(out[9]) << 8) | (uint32_t(out[10]) << 16) | (uint32_t(out[11]) << 24);
-    for (int r = 0; r < p.world; ++r) {
-        if (n_valid == 4) {
-            uint32_t *dst = reinterpret_cast<uint32_t *>(p.rgb[r] + 12 * size_t(quad));
-            dst[0] = w0; dst[1] = w1; dst[2] = w2;
-        } else {
-            for (int k = 0; k < 3 * n_valid; ++k) p.rgb[r][12 * size_t(quad) + k] = out[k];
-        }
-    }
-}
-
-
 #define RT_NCCL(api, expr)                                                                                    \
     do {                                                                                                      \
         ncclResult_t r__ = (expr);                                                                            \
@@ -150,7 +100,7 @@ struct RtComm {
     int rank = 0, world = 1, device = 0;
     cudaStream_t stream = nullptr;
     bool own_stream = false;
-    cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr}; // begin, zeroed, traced, end, main begin, main end
+    rtfs::FrameEvents ev;
     size_t last_pixels = 0;
     bool last_adaptive = false;
     int last_launches = 0;
@@ -253,8 +203,7 @@ void comm_free(RtComm *c) {
     cudaFree(c->d_stats);
     cudaFree(c->d_flags);
     cudaFree(c->d_rgb);
-    for (auto &e : c->ev)
-        if (e) cudaEventDestroy(e);
+    c->ev.destroy();
     if (c->own_stream && c->stream) cudaStreamDestroy(c->stream);
     delete c;
 }
@@ -284,6 +233,7 @@ int comm_workspace(RtComm *c, size_t n_pixels) {
     RT_CUDA(cudaMalloc((void **)&c->d_stats, padded * 4 * sizeof(int32_t)));
     RT_CUDA(cudaMalloc((void **)&c->d_flags, padded));
     RT_CUDA(cudaMalloc((void **)&c->d_rgb, padded * 3));
+    RT_CUDA(cudaMemset(c->d_stats, 0, padded * 4 * sizeof(int32_t))); // a frame clears its pixels only: the padding stays zero
     c->slice_px = slice;
     return peer_open(c);
 }
@@ -337,7 +287,7 @@ int rt_comm_create(const uint8_t *id, int32_t rank, int32_t world, int32_t devic
         ok = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) == cudaSuccess;
         c->own_stream = ok;
     }
-    for (auto &e : c->ev) ok = ok && cudaEventCreate(&e) == cudaSuccess;
+    ok = ok && c->ev.create();
     if (!ok) {
         comm_free(c);
         return fail(RT_ERR_CUDA, "rt_comm_create: stream / event creation failed");
@@ -370,69 +320,40 @@ int rt_comm_render(RtComm *c, RtScene *scene, const RtCamera *camera, int32_t ma
     RT_CUDA(cudaSetDevice(c->device));
     const size_t n_pixels = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
     if ((rc = comm_workspace(c, n_pixels)) != RT_OK) return rc;
-    const size_t padded = c->slice_px * size_t(c->world);
     cudaStream_t st = c->stream;
     NcclApi *api = c->api;
     FrameParams fp;
     fill_frame(fp, ds, *camera, max_w, max_h, *opts, c->rank, c->world);
     fp.stats = c->d_stats;
     fp.flags = c->d_flags;
-    const bool count = (opts->flags & RT_FLAG_COUNTERS) != 0, no_smem = (opts->flags & RT_FLAG_NO_SMEM) != 0;
     int launches = 0;
-    RT_CUDA(cudaEventRecord(c->ev[0], st));
-    RT_CUDA(cudaMemsetAsync(ds->ws->d_counters, 0, CN_SLOTS * sizeof(unsigned long long), st));
-    RT_CUDA(cudaMemsetAsync(c->d_stats, 0, padded * 4 * sizeof(int32_t), st));
-    RT_CUDA(cudaEventRecord(c->ev[1], st));
-    if (fp.adaptive) {
-        RT_CUDA(cudaMemsetAsync(c->d_flags, 0, padded, st));
-        if ((rc = launch_probe(ds, fp, count, no_smem, st, &launches)) != RT_OK) return rc;
-        if (c->world > 1) RT_NCCL(api, api->AllReduce(c->d_flags, c->d_flags, n_pixels, ncclUint8, ncclMax, c->comm, st));
-    } else {
-        RT_CUDA(cudaMemsetAsync(c->d_flags, 1, n_pixels, st));
-    }
-    RT_CUDA(cudaMemcpyAsync(ds->ws->h_counters + CN_SLOTS, ds->ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    RT_CUDA(cudaEventRecord(c->ev[4], st));
-    if ((rc = launch_main(ds, fp, single_flags(c->d_flags), count, no_smem, st, &launches)) != RT_OK) return rc;
-    RT_CUDA(cudaEventRecord(c->ev[5], st));
-    RT_CUDA(cudaEventRecord(c->ev[2], st));
+    if ((rc = frame_probe(ds, fp, st, &c->ev, &launches)) != RT_OK) return rc;
+    if (fp.adaptive && c->world > 1) RT_NCCL(api, api->AllReduce(c->d_flags, c->d_flags, n_pixels, ncclUint8, ncclMax, c->comm, st));
+    if ((rc = frame_main(ds, fp, st, c->ev, &launches)) != RT_OK) return rc;
     if (c->world == 1 || sums_out) {
         // every rank returns the sums: all-reduce them, then divide the whole frame locally
         if (c->world > 1) RT_NCCL(api, api->AllReduce(c->d_stats, c->d_stats, n_pixels * 4, ncclInt32, ncclSum, c->comm, st));
-        if ((rc = rt_device_finalize(c->device, c->d_stats, int32_t(n_pixels), opts->gamma, c->d_rgb, st)) != RT_OK) return rc;
-        ++launches;
+        if ((rc = launch_finalize(c->d_stats, n_pixels, opts->gamma, c->d_rgb, st, &launches)) != RT_OK) return rc;
     } else if (c->peer) {
-        // one kernel over peer memory between two 4-byte barriers
+        // one kernel over peer memory between two 4-byte barriers: this rank's slice into every rank's frame
         RT_NCCL(api, api->AllReduce(c->d_sync, c->d_sync, 1, ncclInt32, ncclSum, c->comm, st)); // every rank's sums are final
-        PeerReduceParams rp{};
+        ReduceTargets t{};
         for (int r = 0; r < c->world; ++r) {
-            rp.stats[r] = c->peer_stats[r];
-            rp.rgb[r] = c->peer_rgb[r];
+            t.stats[r] = c->peer_stats[r];
+            t.rgb[r] = c->peer_rgb[r];
         }
-        const int n_quads = int((n_pixels + 3) / 4);
-        rp.world = c->world;
-        rp.n_pixels = int(n_pixels);
-        rp.quad_begin = int((long long)n_quads * c->rank / c->world);
-        rp.quad_end = int((long long)n_quads * (c->rank + 1) / c->world);
-        rp.gamma = opts->gamma;
-        if (rp.quad_end > rp.quad_begin) {
-            peer_reduce_finalize_gather_kernel<<<(rp.quad_end - rp.quad_begin + 255) / 256, 256, 0, st>>>(rp);
-            RT_CUDA(cudaGetLastError());
-            ++launches;
-        }
+        t.world = t.n_rgb = c->world;
+        if ((rc = launch_reduce_finalize(t, c->rank, n_pixels, opts->gamma, st, &launches)) != RT_OK) return rc;
         RT_NCCL(api, api->AllReduce(c->d_sync, c->d_sync, 1, ncclInt32, ncclSum, c->comm, st)); // every slice has landed everywhere
     } else {
         // reduce-scatter (in place: rank r's totals land in its own slice), divide the slice, all-gather RGB8 (in place)
         int32_t *slice_stats = c->d_stats + size_t(c->rank) * c->slice_px * 4;
         uint8_t *slice_rgb = c->d_rgb + size_t(c->rank) * c->slice_px * 3;
         RT_NCCL(api, api->ReduceScatter(c->d_stats, slice_stats, c->slice_px * 4, ncclInt32, ncclSum, c->comm, st));
-        if ((rc = rt_device_finalize(c->device, slice_stats, int32_t(c->slice_px), opts->gamma, slice_rgb, st)) != RT_OK) return rc;
-        ++launches;
+        if ((rc = launch_finalize(slice_stats, c->slice_px, opts->gamma, slice_rgb, st, &launches)) != RT_OK) return rc;
         RT_NCCL(api, api->AllGather(slice_rgb, c->d_rgb, c->slice_px * 3, ncclUint8, c->comm, st));
     }
-    if (rgb_out) RT_CUDA(cudaMemcpyAsync(rgb_out, c->d_rgb, n_pixels * 3, cudaMemcpyDeviceToHost, st));
-    if (sums_out) RT_CUDA(cudaMemcpyAsync(sums_out, c->d_stats, n_pixels * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    RT_CUDA(cudaEventRecord(c->ev[3], st));
-    RT_CUDA(cudaMemcpyAsync(ds->ws->h_counters, ds->ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    if ((rc = frame_finish(ds, fp, c->d_rgb, rgb_out, sums_out, st, c->ev)) != RT_OK) return rc;
     c->last_pixels = n_pixels;
     c->last_adaptive = fp.adaptive != 0;
     c->last_launches = launches;
@@ -447,19 +368,8 @@ int rt_comm_last_stats(RtComm *c, RtScene *scene, RtStats *stats) {
     auto *ds = static_cast<DeviceScene *>(scene->dev);
     if (!c->last_pixels) return fail(RT_ERR_INVALID_ARGUMENT, "rt_comm_last_stats: no frame has been rendered on this communicator");
     RT_CUDA(cudaSetDevice(c->device));
-    RT_CUDA(cudaEventSynchronize(c->ev[3]));
-    RT_CUDA(cudaStreamSynchronize(c->stream)); // the counter copy follows the last event
-    std::memset(stats, 0, sizeof *stats);
-    read_counters(ds, stats, c->last_pixels, c->last_adaptive); // this rank's paths and rays
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, c->ev[1], c->ev[2]);
-    stats->kernel_ms = ms;
-    cudaEventElapsedTime(&ms, c->ev[0], c->ev[3]);
-    stats->total_ms = ms;
-    cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]);
-    stats->main_ms = ms;
-    stats->main_rays = ds->ws->h_counters[CN_RAYS] - ds->ws->h_counters[CN_SLOTS + CN_RAYS];
-    stats->launches = c->last_launches;
+    RT_CUDA(cudaEventSynchronize(c->ev.ev[FrameEvents::END])); // the counter copy precedes it
+    read_stats(ds, c->last_pixels, c->last_adaptive, c->last_launches, &c->ev, stats); // this rank's paths and rays
     return RT_OK;
 }
 

@@ -33,8 +33,7 @@ static void workspace_destroy(DeviceWorkspace *ws) {
     cudaFree(ws->d_blob);
     if (ws->h_blob) cudaFreeHost(ws->h_blob);
     if (ws->h_counters) cudaFreeHost(ws->h_counters);
-    for (auto &e : ws->ev)
-        if (e) cudaEventDestroy(e);
+    ws->ev.destroy();
     if (ws->stream) cudaStreamDestroy(ws->stream);
     delete ws;
 }
@@ -59,8 +58,7 @@ int workspace_acquire(int device, DeviceWorkspace **out) {
         ws->smem_optin = prop.sharedMemPerBlockOptin;
         ok = cudaMalloc((void **)&ws->d_counters, CN_SLOTS * sizeof(unsigned long long)) == cudaSuccess &&
              cudaMallocHost((void **)&ws->h_counters, 2 * CN_SLOTS * sizeof(unsigned long long)) == cudaSuccess &&
-             cudaStreamCreateWithFlags(&ws->stream, cudaStreamNonBlocking) == cudaSuccess;
-        for (auto &e : ws->ev) ok = ok && cudaEventCreate(&e) == cudaSuccess;
+             cudaStreamCreateWithFlags(&ws->stream, cudaStreamNonBlocking) == cudaSuccess && ws->ev.create();
     }
     if (!ok) {
         std::string why = cudaGetErrorString(cudaGetLastError());
@@ -589,22 +587,10 @@ __global__ void compact_kernel(const FlagsView flags, uint32_t *list, unsigned l
 // PixelStats.mean (Pixel.fs:103-108) and, optionally, PixelOutput.correct (ImageOutput.fs:11-18)
 __global__ void finalize_kernel(const int32_t *stats, int n_pixels, int gamma, uint8_t *rgb) {
     __shared__ uint8_t lut[256];
-    for (int i = threadIdx.x; i < 256; i += blockDim.x) {
-        int v = i;
-        if (gamma) {
-            v = __double2int_rn(sqrt(double(i) / 255.0) * 255.0); // Math.Round: half to even
-            if (v == 256) v = 255;
-        }
-        lut[i] = uint8_t(v);
-    }
-    __syncthreads();
+    fill_gamma_lut(lut, gamma);
     int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n_pixels) return;
-    int4 s = reinterpret_cast<const int4 *>(stats)[p];
-    int n = s.w > 0 ? s.w : 1;
-    rgb[3 * size_t(p) + 0] = lut[(s.x / n) & 255];
-    rgb[3 * size_t(p) + 1] = lut[(s.y / n) & 255];
-    rgb[3 * size_t(p) + 2] = lut[(s.z / n) & 255];
+    pixel_rgb8(reinterpret_cast<const int4 *>(stats)[p], lut, rgb + 3 * size_t(p));
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -655,8 +641,20 @@ static bool smem_fits(const DeviceScene *ds, size_t bytes, int per_sm) {
     return (bytes + 1024) * size_t(per_sm) <= ds->ws->smem_optin + (per_sm > 1 ? 1024 : 0);
 }
 
+// 16-byte quads of the scene a staged block holds: nodes | spheres | materials
+static size_t staged_scene_quads(const DeviceScene *ds) {
+    return size_t(ds->g.n_nodes) * kStagedNodeQuads + size_t(ds->g.n_bounded) + size_t(ds->g.n_bounded + ds->g.n_unbounded) * 2;
+}
+
+// the scene is staged in shared memory when it fits beside `warp_bytes` of scratch per warp (one block of kBlockThreads per SM)
+static bool scene_staged(const DeviceScene *ds, size_t warp_bytes) {
+    const size_t warp_q = (kBlockThreads / 32) * warp_bytes / 16;
+    return smem_fits(ds, (staged_scene_quads(ds) + warp_q) * 16, kBlocksPerSm) && ds->g.n_bounded > 0;
+}
+
 // lays out shared memory and sizes the persistent grid
-static int plan_launch(DeviceScene *ds, FrameParams &fp, bool probe, bool count, bool no_smem, LaunchPlan &plan, RenderKernelFn &fn) {
+static int plan_launch(DeviceScene *ds, FrameParams &fp, bool probe, LaunchPlan &plan, RenderKernelFn &fn) {
+    const bool count = (fp.opt_flags & RT_FLAG_COUNTERS) != 0, no_smem = (fp.opt_flags & RT_FLAG_NO_SMEM) != 0;
     const bool wide_asked = frame_walks_wide_tree(ds, fp.opt_flags, true);
     // the flow schedule (ring of rays per warp) on request only — measured slower than lockstep on B200 (DESIGN.md 5) —
     // and not with the wide tree (no flow variant) nor when the bounce budget does not fit the byte it shares with the colour
@@ -664,17 +662,15 @@ static int plan_launch(DeviceScene *ds, FrameParams &fp, bool probe, bool count,
     // the sum of squares of progressive frames opened with RT_FLAG_NOISE: lockstep kernels without counters only
     const bool noise = fp.sq != nullptr;
     if (noise && (flow || count)) return fail(RT_ERR_UNSUPPORTED, "render: the noise estimate has no flow-schedule or counting kernel");
-    size_t warp_q = (kBlockThreads / 32) * (flow ? sizeof(FlowWarp) : warp_scratch_bytes(true, noise)) / 16;
-    const size_t nodes_q = size_t(ds->g.n_nodes) * kStagedNodeQuads, sph_q = size_t(ds->g.n_bounded), mat_q = size_t(ds->g.n_bounded + ds->g.n_unbounded) * 2;
-    const size_t scene_q = nodes_q + sph_q + mat_q;
-    // stage the scene in shared memory when it fits beside the per-warp scratch (one block per SM)
-    bool smem = smem_fits(ds, (scene_q + warp_q) * 16, kBlocksPerSm) && ds->g.n_bounded > 0;
+    const size_t nodes_q = size_t(ds->g.n_nodes) * kStagedNodeQuads, sph_q = size_t(ds->g.n_bounded);
+    const size_t scene_q = staged_scene_quads(ds);
+    bool smem = scene_staged(ds, flow ? sizeof(FlowWarp) : warp_scratch_bytes(true, noise));
     const bool wide = frame_walks_wide_tree(ds, fp.opt_flags, smem);
     if (no_smem || wide) smem = false;
     // the launch shape follows from where the scene is read (rtfs_device.h); the flow kernels keep one block of 1024
     plan.threads = flow ? kBlockThreads : block_threads(smem);
     const int want_per_sm = flow ? 1 : blocks_per_sm(smem);
-    warp_q = size_t(plan.threads / 32) * (flow ? sizeof(FlowWarp) : warp_scratch_bytes(smem, noise)) / 16;
+    const size_t warp_q = size_t(plan.threads / 32) * (flow ? sizeof(FlowWarp) : warp_scratch_bytes(smem, noise)) / 16;
     fp.s_nodes = 0;
     fp.s_spheres = uint32_t(nodes_q);
     fp.s_mats = uint32_t(nodes_q + sph_q);
@@ -744,13 +740,39 @@ static int plan_launch(DeviceScene *ds, FrameParams &fp, bool probe, bool count,
     return RT_OK;
 }
 
-static int ensure_list(DeviceScene *ds, size_t n_pixels) {
-    if (ds->ws->list_pixels >= n_pixels) return RT_OK;
-    cudaFree(ds->ws->d_list);
-    ds->ws->d_list = nullptr;
-    ds->ws->list_pixels = 0;
-    RT_CUDA(cudaMalloc((void **)&ds->ws->d_list, n_pixels * sizeof(uint32_t)));
-    ds->ws->list_pixels = n_pixels;
+int ensure_frame_buffers(DeviceWorkspace *ws, size_t n_pixels) {
+    if (ws->ws_pixels >= n_pixels) return RT_OK;
+    cudaFree(ws->d_stats);
+    cudaFree(ws->d_flags);
+    cudaFree(ws->d_rgb);
+    ws->d_stats = nullptr;
+    ws->d_flags = nullptr;
+    ws->d_rgb = nullptr;
+    ws->ws_pixels = 0;
+    RT_CUDA(cudaMalloc((void **)&ws->d_stats, n_pixels * 4 * sizeof(int32_t)));
+    RT_CUDA(cudaMalloc((void **)&ws->d_flags, n_pixels));
+    RT_CUDA(cudaMalloc((void **)&ws->d_rgb, n_pixels * 3));
+    ws->ws_pixels = n_pixels;
+    return RT_OK;
+}
+
+int ensure_list(DeviceWorkspace *ws, size_t n_pixels) {
+    if (ws->list_pixels >= n_pixels) return RT_OK;
+    cudaFree(ws->d_list);
+    ws->d_list = nullptr;
+    ws->list_pixels = 0;
+    RT_CUDA(cudaMalloc((void **)&ws->d_list, n_pixels * sizeof(uint32_t)));
+    ws->list_pixels = n_pixels;
+    return RT_OK;
+}
+
+int ensure_probe_sums(DeviceWorkspace *ws, size_t n_pixels) {
+    if (ws->probe_pixels >= n_pixels) return RT_OK;
+    cudaFree(ws->d_stats_b);
+    ws->d_stats_b = nullptr;
+    ws->probe_pixels = 0;
+    RT_CUDA(cudaMalloc((void **)&ws->d_stats_b, n_pixels * 4 * sizeof(int32_t)));
+    ws->probe_pixels = n_pixels;
     return RT_OK;
 }
 
@@ -829,32 +851,30 @@ static int build_chunks(FrameParams &fp, int n_local, int boundary, size_t n_uni
     return RT_OK;
 }
 
-int launch_probe(DeviceScene *ds, FrameParams fp, bool count, bool no_smem, cudaStream_t st, int *launches, bool raw_flags) {
+int launch_probe(DeviceScene *ds, FrameParams fp, cudaStream_t st, int *launches, bool raw_flags) {
     DeviceWorkspace *ws = ds->ws;
     const size_t n_pixels = size_t(fp.cam.rows) * fp.cam.cols;
-    if (ws->probe_pixels < n_pixels) {
-        cudaFree(ws->d_stats_b);
-        ws->d_stats_b = nullptr;
-        ws->probe_pixels = 0;
-        RT_CUDA(cudaMalloc((void **)&ws->d_stats_b, n_pixels * 4 * sizeof(int32_t)));
-        ws->probe_pixels = n_pixels;
-    }
+    int rc = ensure_probe_sums(ws, n_pixels);
+    if (rc != RT_OK) return rc;
     RT_CUDA(cudaMemsetAsync(ws->d_stats_b, 0, n_pixels * 4 * sizeof(int32_t), st));
     RT_CUDA(cudaMemsetAsync(fp.counters + CN_WORK_PROBE, 0, sizeof(unsigned long long), st));
     fp.stats_b = ws->d_stats_b;
     LaunchPlan plan;
     RenderKernelFn fn;
-    int rc = plan_launch(ds, fp, true, count, no_smem, plan, fn);
-    if (rc != RT_OK) return rc;
+    if ((rc = plan_launch(ds, fp, true, plan, fn)) != RT_OK) return rc;
     const size_t n_units = size_t((fp.tiles_x * fp.tiles_y - fp.rank + fp.world - 1) / fp.world);
     rc = build_chunks(fp, fp.n_probe, fp.first_trial + 1, n_units, plan.blocks * (plan.threads / 32));
     if (rc != RT_OK) return rc;
     fn<<<plan.blocks, plan.threads, plan.smem_bytes, st>>>(fp);
     RT_CUDA(cudaGetLastError());
     ++*launches;
-    probe_flags_kernel<<<unsigned((n_pixels + 255) / 256), 256, 0, st>>>(fp.stats, ws->d_stats_b, fp.flags, fp.cam.rows, fp.cam.cols, fp.tiles_x,
-                                                                          fp.rank, fp.world, fp.first_trial, fp.n_probe,
-                                                                          (raw_flags || fp.sample_end > fp.sample_begin) ? 1 : 0);
+    return launch_probe_flags(fp, ws->d_stats_b, raw_flags || fp.sample_end > fp.sample_begin, st, launches);
+}
+
+int launch_probe_flags(const FrameParams &fp, const int32_t *stats_b, bool more, cudaStream_t st, int *launches) {
+    const size_t n_pixels = size_t(fp.cam.rows) * fp.cam.cols;
+    probe_flags_kernel<<<unsigned((n_pixels + 255) / 256), 256, 0, st>>>(fp.stats, stats_b, fp.flags, fp.cam.rows, fp.cam.cols, fp.tiles_x,
+                                                                          fp.rank, fp.world, fp.first_trial, fp.n_probe, more ? 1 : 0);
     RT_CUDA(cudaGetLastError());
     ++*launches;
     return RT_OK;
@@ -872,11 +892,11 @@ int launch_compact(DeviceScene *ds, const FrameParams &fp, const FlagsView &flag
 
 // The main phase over the sample window [fp.sample_begin, fp.sample_end) (this rank's share of it) for the pixels of
 // fp.list; the work cursor fp.counters[CN_WORK_MAIN] must be zero on entry
-int launch_samples(DeviceScene *ds, FrameParams fp, bool count, bool no_smem, cudaStream_t st, int *launches) {
+int launch_samples(DeviceScene *ds, FrameParams fp, cudaStream_t st, int *launches) {
     const size_t n_pixels = size_t(fp.cam.rows) * fp.cam.cols;
     LaunchPlan plan;
     RenderKernelFn fn;
-    int rc = plan_launch(ds, fp, false, count, no_smem, plan, fn);
+    int rc = plan_launch(ds, fp, false, plan, fn);
     if (rc != RT_OK) return rc;
     int n_span = fp.sample_end - fp.sample_begin - fp.rank;
     int n_local = n_span > 0 ? (n_span + fp.world - 1) / fp.world : 0;
@@ -895,23 +915,80 @@ int launch_samples(DeviceScene *ds, FrameParams fp, bool count, bool no_smem, cu
     return RT_OK;
 }
 
-int launch_main(DeviceScene *ds, FrameParams fp, const FlagsView &flags, bool count, bool no_smem, cudaStream_t st, int *launches) {
-    const size_t n_pixels = size_t(fp.cam.rows) * fp.cam.cols;
-    int rc = ensure_list(ds, n_pixels);
+int launch_main(DeviceScene *ds, FrameParams fp, const FlagsView &flags, cudaStream_t st, int *launches) {
+    int rc = ensure_list(ds->ws, size_t(fp.cam.rows) * fp.cam.cols);
     if (rc != RT_OK) return rc;
     if ((rc = launch_compact(ds, fp, flags, ds->ws->d_list, st, launches)) != RT_OK) return rc;
     fp.list = ds->ws->d_list;
-    return launch_samples(ds, fp, count, no_smem, st, launches);
+    return launch_samples(ds, fp, st, launches);
 }
 
-void read_counters(DeviceScene *ds, RtStats *stats, size_t n_pixels, bool adaptive) {
-    stats->paths = ds->ws->h_counters[CN_PATHS];
-    stats->rays = ds->ws->h_counters[CN_RAYS];
-    stats->box_tests = ds->ws->h_counters[CN_BOX];
-    stats->prim_tests = ds->ws->h_counters[CN_PRIM];
-    stats->pixels_early_out = adaptive ? (unsigned long long)n_pixels - ds->ws->h_counters[CN_LIST] : 0;
-    stats->degenerate_paths = ds->ws->h_counters[CN_DEGENERATE];
-    if (std::getenv("RTFS_DEBUG_BLOCKS")) std::fprintf(stderr, "rtfs: blocks that found work (probe + main): %llu\n", ds->ws->h_counters[CN_BUSY_BLOCKS]);
+int launch_finalize(const int32_t *stats, size_t n_pixels, int gamma, uint8_t *rgb, cudaStream_t st, int *launches) {
+    finalize_kernel<<<unsigned((n_pixels + 255) / 256), 256, 0, st>>>(stats, int(n_pixels), gamma, rgb);
+    RT_CUDA(cudaGetLastError());
+    ++*launches;
+    return RT_OK;
+}
+
+int frame_probe(DeviceScene *ds, const FrameParams &fp, cudaStream_t st, FrameEvents *ev, int *launches) {
+    const size_t n_pixels = size_t(fp.cam.rows) * fp.cam.cols;
+    if (ev) RT_CUDA(ev->record(FrameEvents::BEGIN, st));
+    RT_CUDA(cudaMemsetAsync(fp.counters, 0, CN_SLOTS * sizeof(unsigned long long), st));
+    RT_CUDA(cudaMemsetAsync(fp.stats, 0, n_pixels * 4 * sizeof(int32_t), st));
+    if (fp.sq) RT_CUDA(cudaMemsetAsync(fp.sq, 0, n_pixels * sizeof(unsigned long long), st));
+    if (ev) RT_CUDA(ev->record(FrameEvents::ZEROED, st));
+    if (!fp.adaptive) {
+        RT_CUDA(cudaMemsetAsync(fp.flags, 1, n_pixels, st));
+        return RT_OK;
+    }
+    if (fp.world > 1) RT_CUDA(cudaMemsetAsync(fp.flags, 0, n_pixels, st));
+    return launch_probe(ds, fp, st, launches, fp.counters != ds->ws->d_counters);
+}
+
+int frame_main(DeviceScene *ds, const FrameParams &fp, cudaStream_t st, FrameEvents &ev, int *launches) {
+    RT_CUDA(cudaMemcpyAsync(ds->ws->h_counters + CN_SLOTS, fp.counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    RT_CUDA(ev.record(FrameEvents::MAIN_BEGIN, st));
+    int rc = launch_main(ds, fp, single_flags(fp.flags), st, launches);
+    if (rc != RT_OK) return rc;
+    RT_CUDA(ev.record(FrameEvents::MAIN_END, st));
+    RT_CUDA(ev.record(FrameEvents::TRACED, st));
+    return RT_OK;
+}
+
+int frame_finish(DeviceScene *ds, const FrameParams &fp, const uint8_t *d_rgb, uint8_t *rgb_out, int32_t *sums_out, cudaStream_t st,
+                 FrameEvents &ev) {
+    const size_t n_pixels = size_t(fp.cam.rows) * fp.cam.cols;
+    if (rgb_out) RT_CUDA(cudaMemcpyAsync(rgb_out, d_rgb, n_pixels * 3, cudaMemcpyDeviceToHost, st));
+    if (sums_out) RT_CUDA(cudaMemcpyAsync(sums_out, fp.stats, n_pixels * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaMemcpyAsync(ds->ws->h_counters, fp.counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    RT_CUDA(ev.record(FrameEvents::END, st));
+    return RT_OK;
+}
+
+void read_stats(const DeviceScene *ds, size_t n_pixels, bool adaptive, int launches, const FrameEvents *ev, RtStats *stats) {
+    const unsigned long long *h = ds->ws->h_counters;
+    std::memset(stats, 0, sizeof *stats);
+    stats->paths = h[CN_PATHS];
+    stats->rays = h[CN_RAYS];
+    stats->box_tests = h[CN_BOX];
+    stats->prim_tests = h[CN_PRIM];
+    stats->pixels_early_out = adaptive ? (unsigned long long)n_pixels - h[CN_LIST] : 0;
+    stats->degenerate_paths = h[CN_DEGENERATE];
+    stats->launches = launches;
+    if (ev) {
+        stats->kernel_ms = ev->ms(FrameEvents::ZEROED, FrameEvents::TRACED);
+        stats->total_ms = ev->ms(FrameEvents::BEGIN, FrameEvents::END);
+        stats->main_ms = ev->ms(FrameEvents::MAIN_BEGIN, FrameEvents::MAIN_END);
+        stats->main_rays = h[CN_RAYS] - h[CN_SLOTS + CN_RAYS];
+    }
+    if (std::getenv("RTFS_DEBUG_BLOCKS")) std::fprintf(stderr, "rtfs: blocks that found work (probe + main): %llu\n", h[CN_BUSY_BLOCKS]);
+}
+
+// one device->host copy of the counters into ds->ws->h_counters and a synchronisation of the stream
+static int sync_counters(DeviceScene *ds, cudaStream_t st) {
+    RT_CUDA(cudaMemcpyAsync(ds->ws->h_counters, ds->ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaStreamSynchronize(st));
+    return RT_OK;
 }
 
 // implemented in rtfs_wavefront.cu
@@ -956,10 +1033,8 @@ int rt_device_count(void) {
 size_t rt_scene_shared_memory_bytes(const RtScene *scene) {
     if (!scene || !scene->dev) return 0;
     auto *ds = static_cast<const DeviceScene *>(scene->dev);
-    const size_t warp_q = (kBlockThreads / 32) * warp_scratch_bytes(true) / 16; // the default (lockstep) schedule's per-warp scratch
-    const size_t scene_q = size_t(ds->g.n_nodes) * kStagedNodeQuads + size_t(ds->g.n_bounded) + size_t(ds->g.n_bounded + ds->g.n_unbounded) * 2;
-    bool smem = smem_fits(ds, (scene_q + warp_q) * 16, kBlocksPerSm) && ds->g.n_bounded > 0;
-    return smem ? scene_q * 16 : 0;
+    // with the default (lockstep) schedule's per-warp scratch
+    return scene_staged(ds, warp_scratch_bytes(true)) ? staged_scene_quads(ds) * 16 : 0;
 }
 
 int rt_device_probe(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_t max_h, const RtRenderOpts *opts, int32_t rank,
@@ -981,16 +1056,12 @@ int rt_device_probe(RtScene *scene, const RtCamera *camera, int32_t max_w, int32
     if (!fp.adaptive) {
         // no probe phase: every pixel takes all its samples in the main phase (rank 0 raises the flags once)
         if (rank == 0) RT_CUDA(cudaMemsetAsync(d_flags, 1, n_pixels, st));
-    } else {
-        rc = launch_probe(ds, fp, (opts->flags & RT_FLAG_COUNTERS) != 0, (opts->flags & RT_FLAG_NO_SMEM) != 0, st, &launches);
-        if (rc != RT_OK) return rc;
+    } else if ((rc = launch_probe(ds, fp, st, &launches, false)) != RT_OK) {
+        return rc;
     }
     if (stats) {
-        RT_CUDA(cudaMemcpyAsync(ds->ws->h_counters, ds->ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-        RT_CUDA(cudaStreamSynchronize(st));
-        std::memset(stats, 0, sizeof *stats);
-        read_counters(ds, stats, n_pixels, false);
-        stats->launches = launches;
+        if ((rc = sync_counters(ds, st)) != RT_OK) return rc;
+        read_stats(ds, n_pixels, false, launches, nullptr, stats);
     }
     return RT_OK;
 }
@@ -1008,16 +1079,11 @@ int rt_device_main(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
     fill_frame(fp, ds, *camera, max_w, max_h, *opts, rank, world);
     fp.stats = d_stats;
     fp.flags = const_cast<uint8_t *>(d_flags);
-    const size_t n_pixels = size_t(fp.cam.rows) * fp.cam.cols;
     int launches = 0;
-    rc = launch_main(ds, fp, single_flags(d_flags), (opts->flags & RT_FLAG_COUNTERS) != 0, (opts->flags & RT_FLAG_NO_SMEM) != 0, st, &launches);
-    if (rc != RT_OK) return rc;
+    if ((rc = launch_main(ds, fp, single_flags(d_flags), st, &launches)) != RT_OK) return rc;
     if (stats) {
-        RT_CUDA(cudaMemcpyAsync(ds->ws->h_counters, ds->ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-        RT_CUDA(cudaStreamSynchronize(st));
-        std::memset(stats, 0, sizeof *stats);
-        read_counters(ds, stats, n_pixels, fp.adaptive != 0);
-        stats->launches = launches;
+        if ((rc = sync_counters(ds, st)) != RT_OK) return rc;
+        read_stats(ds, size_t(fp.cam.rows) * fp.cam.cols, fp.adaptive != 0, launches, nullptr, stats);
     }
     return RT_OK;
 }
@@ -1028,9 +1094,8 @@ int rt_device_counters(RtScene *scene, void *stream, RtStats *stats) {
     if (!scene->dev) return fail(RT_ERR_NO_DEVICE, "rt_device_counters: the scene has no device");
     auto *ds = static_cast<DeviceScene *>(scene->dev);
     RT_CUDA(cudaSetDevice(ds->device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    RT_CUDA(cudaMemcpyAsync(ds->ws->h_counters, ds->ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    RT_CUDA(cudaStreamSynchronize(st));
+    int rc = sync_counters(ds, static_cast<cudaStream_t>(stream));
+    if (rc != RT_OK) return rc;
     std::memset(stats, 0, sizeof *stats);
     stats->paths = ds->ws->h_counters[CN_PATHS];
     stats->rays = ds->ws->h_counters[CN_RAYS];
@@ -1044,9 +1109,8 @@ int rt_device_finalize(int32_t device, const int32_t *d_stats, int32_t n_pixels,
     int rc = require_device(device);
     if (rc != RT_OK) return rc;
     if (!d_stats || !d_rgb || n_pixels <= 0) return fail(RT_ERR_INVALID_ARGUMENT, "rt_device_finalize: bad argument");
-    finalize_kernel<<<(n_pixels + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(d_stats, n_pixels, gamma, d_rgb);
-    RT_CUDA(cudaGetLastError());
-    return RT_OK;
+    int launches = 0;
+    return launch_finalize(d_stats, size_t(n_pixels), gamma, d_rgb, static_cast<cudaStream_t>(stream), &launches);
 }
 
 int rt_render(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_t max_h, const RtRenderOpts *opts, uint8_t *rgb_out,
@@ -1059,64 +1123,21 @@ int rt_render(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_t max
     if ((rc = prepare_frame(scene, opts)) != RT_OK) return rc;
     auto *ds = static_cast<DeviceScene *>(scene->dev);
     RT_CUDA(cudaSetDevice(ds->device));
+    DeviceWorkspace *ws = ds->ws;
     const size_t n_pixels = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
-    if (ds->ws->ws_pixels < n_pixels) {
-        cudaFree(ds->ws->d_stats);
-        cudaFree(ds->ws->d_flags);
-        cudaFree(ds->ws->d_rgb);
-        ds->ws->d_stats = nullptr;
-        ds->ws->d_flags = nullptr;
-        ds->ws->d_rgb = nullptr;
-        ds->ws->ws_pixels = 0;
-        RT_CUDA(cudaMalloc((void **)&ds->ws->d_stats, n_pixels * 4 * sizeof(int32_t)));
-        RT_CUDA(cudaMalloc((void **)&ds->ws->d_flags, n_pixels));
-        RT_CUDA(cudaMalloc((void **)&ds->ws->d_rgb, n_pixels * 3));
-        ds->ws->ws_pixels = n_pixels;
-    }
-    cudaStream_t st = ds->ws->stream;
+    if ((rc = ensure_frame_buffers(ws, n_pixels)) != RT_OK) return rc;
+    cudaStream_t st = ws->stream;
     FrameParams fp;
     fill_frame(fp, ds, *camera, max_w, max_h, *opts, 0, 1);
-    fp.stats = ds->ws->d_stats;
-    fp.flags = ds->ws->d_flags;
-    const bool count = (opts->flags & RT_FLAG_COUNTERS) != 0, no_smem = (opts->flags & RT_FLAG_NO_SMEM) != 0;
+    fp.stats = ws->d_stats;
+    fp.flags = ws->d_flags;
     int launches = 0;
-    RT_CUDA(cudaEventRecord(ds->ws->ev[0], st));
-    RT_CUDA(cudaMemsetAsync(ds->ws->d_counters, 0, CN_SLOTS * sizeof(unsigned long long), st));
-    RT_CUDA(cudaMemsetAsync(ds->ws->d_stats, 0, n_pixels * 4 * sizeof(int32_t), st));
-    RT_CUDA(cudaEventRecord(ds->ws->ev[1], st));
-    if (fp.adaptive) {
-        rc = launch_probe(ds, fp, count, no_smem, st, &launches);
-        if (rc != RT_OK) return rc;
-    } else {
-        RT_CUDA(cudaMemsetAsync(ds->ws->d_flags, 1, n_pixels, st));
-    }
-    RT_CUDA(cudaMemcpyAsync(ds->ws->h_counters + CN_SLOTS, ds->ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    RT_CUDA(cudaEventRecord(ds->ws->ev[4], st));
-    rc = launch_main(ds, fp, single_flags(ds->ws->d_flags), count, no_smem, st, &launches);
-    if (rc != RT_OK) return rc;
-    RT_CUDA(cudaEventRecord(ds->ws->ev[5], st));
-    RT_CUDA(cudaEventRecord(ds->ws->ev[2], st));
-    finalize_kernel<<<unsigned((n_pixels + 255) / 256), 256, 0, st>>>(ds->ws->d_stats, int(n_pixels), opts->gamma, ds->ws->d_rgb);
-    RT_CUDA(cudaGetLastError());
-    ++launches;
-    RT_CUDA(cudaMemcpyAsync(rgb_out, ds->ws->d_rgb, n_pixels * 3, cudaMemcpyDeviceToHost, st));
-    if (sums_out) RT_CUDA(cudaMemcpyAsync(sums_out, ds->ws->d_stats, n_pixels * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    RT_CUDA(cudaMemcpyAsync(ds->ws->h_counters, ds->ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    RT_CUDA(cudaEventRecord(ds->ws->ev[3], st));
+    if ((rc = frame_probe(ds, fp, st, &ws->ev, &launches)) != RT_OK) return rc;
+    if ((rc = frame_main(ds, fp, st, ws->ev, &launches)) != RT_OK) return rc;
+    if ((rc = launch_finalize(ws->d_stats, n_pixels, opts->gamma, ws->d_rgb, st, &launches)) != RT_OK) return rc;
+    if ((rc = frame_finish(ds, fp, ws->d_rgb, rgb_out, sums_out, st, ws->ev)) != RT_OK) return rc;
     RT_CUDA(cudaStreamSynchronize(st));
-    if (stats) {
-        std::memset(stats, 0, sizeof *stats);
-        read_counters(ds, stats, n_pixels, fp.adaptive != 0);
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, ds->ws->ev[1], ds->ws->ev[2]);
-        stats->kernel_ms = ms;
-        cudaEventElapsedTime(&ms, ds->ws->ev[0], ds->ws->ev[3]);
-        stats->total_ms = ms;
-        cudaEventElapsedTime(&ms, ds->ws->ev[4], ds->ws->ev[5]);
-        stats->main_ms = ms;
-        stats->main_rays = ds->ws->h_counters[CN_RAYS] - ds->ws->h_counters[CN_SLOTS + CN_RAYS];
-        stats->launches = launches;
-    }
+    if (stats) read_stats(ds, n_pixels, fp.adaptive != 0, launches, &ws->ev, stats);
     return RT_OK;
 }
 

@@ -36,6 +36,29 @@ enum CounterSlot { CN_PATHS = 0, CN_RAYS = 1, CN_BOX = 2, CN_PRIM = 3, CN_LIST =
 // (the last slot of the pinned copy is a scratch word of the wavefront driver; the pinned buffer holds a second set of
 // CN_SLOTS words: the snapshot taken between the probe and the main phase)
 
+// The events a frame records on its stream, in stream order: BEGIN; ZEROED once the counters and sums are cleared;
+// MAIN_BEGIN and MAIN_END around the main phase; TRACED once the last render kernel is done; END once the results and
+// the counters are copied.  RtStats: kernel_ms = ZEROED -> TRACED, main_ms = MAIN_BEGIN -> MAIN_END, total_ms = BEGIN -> END.
+struct FrameEvents {
+    enum Which { BEGIN, ZEROED, MAIN_BEGIN, MAIN_END, TRACED, END, COUNT };
+    cudaEvent_t ev[COUNT] = {};
+    bool create() {
+        bool ok = true;
+        for (auto &e : ev) ok = ok && cudaEventCreate(&e) == cudaSuccess;
+        return ok;
+    }
+    void destroy() {
+        for (auto &e : ev)
+            if (e) cudaEventDestroy(e);
+    }
+    cudaError_t record(Which w, cudaStream_t st) { return cudaEventRecord(ev[w], st); }
+    float ms(Which from, Which to) const {
+        float t = 0.f;
+        cudaEventElapsedTime(&t, ev[from], ev[to]);
+        return t;
+    }
+};
+
 // Frame buffers, scratch, stream and events of one device.  Allocating these costs milliseconds, so they are
 // pooled: a scene handle borrows one for its lifetime and returns it on destroy (handles stay independent of
 // one another; nothing is shared between two live handles).
@@ -59,10 +82,14 @@ struct DeviceWorkspace {
     unsigned long long *d_counters = nullptr;
     unsigned long long *h_counters = nullptr; // pinned
     cudaStream_t stream = nullptr;
-    cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr}; // begin, zeroed, traced, end, main begin, main end
+    FrameEvents ev;
 };
 int workspace_acquire(int device, DeviceWorkspace **out);
 void workspace_release(DeviceWorkspace *ws);
+// grow-only: the sums, flags and RGB8 of rt_render's frame; the flagged-pixel list; the probe's second accumulator set
+int ensure_frame_buffers(DeviceWorkspace *ws, size_t n_pixels);
+int ensure_list(DeviceWorkspace *ws, size_t n_pixels);
+int ensure_probe_sums(DeviceWorkspace *ws, size_t n_pixels);
 
 struct PooledTexture { // an image texture's array + texture object, pooled by (device, width, height)
     int device, w, h;
@@ -174,18 +201,71 @@ inline FlagsView single_flags(const uint8_t *p) {
 
 int check_frame_args(const RtScene *scene, const RtCamera *camera, int max_w, int max_h, const RtRenderOpts *opts);
 void fill_frame(FrameParams &fp, DeviceScene *ds, const RtCamera &cam, int max_w, int max_h, const RtRenderOpts &opts, int rank, int world);
+// The launch helpers pick their kernels from fp.opt_flags (RT_FLAG_COUNTERS, RT_FLAG_NO_SMEM, ...) and count what they
+// launch in *launches.
 // raw_flags: flag every pixel whose two probe means differ even where the frame has no main phase (progressive frames
 // keep them so that the frame can be extended to more samples); otherwise only where a main phase follows
-int launch_probe(DeviceScene *ds, FrameParams fp, bool count, bool no_smem, cudaStream_t st, int *launches, bool raw_flags = false);
+int launch_probe(DeviceScene *ds, FrameParams fp, cudaStream_t st, int *launches, bool raw_flags);
+// merges the probe's two accumulator sets (fp.stats += stats_b) and raises fp.flags on the pixels of this rank's tiles
+// whose two means differ (more: only if samples follow)
+int launch_probe_flags(const FrameParams &fp, const int32_t *stats_b, bool more, cudaStream_t st, int *launches);
 // compaction + the main phase over [fp.sample_begin, fp.sample_end); the two halves are also launched on their own
 // (progressive frames, rtfs_frame.cu: compaction once, then one launch_samples per pass)
-int launch_main(DeviceScene *ds, FrameParams fp, const FlagsView &flags, bool count, bool no_smem, cudaStream_t st, int *launches);
+int launch_main(DeviceScene *ds, FrameParams fp, const FlagsView &flags, cudaStream_t st, int *launches);
 int launch_compact(DeviceScene *ds, const FrameParams &fp, const FlagsView &flags, uint32_t *list, cudaStream_t st, int *launches);
-int launch_samples(DeviceScene *ds, FrameParams fp, bool count, bool no_smem, cudaStream_t st, int *launches);
+int launch_samples(DeviceScene *ds, FrameParams fp, cudaStream_t st, int *launches);
+// PixelStats.mean + the optional gamma of a whole frame: sums -> RGB8
+int launch_finalize(const int32_t *stats, size_t n_pixels, int gamma, uint8_t *rgb, cudaStream_t st, int *launches);
+
+// One rank's frame, in three steps on its stream; fp.stats, fp.flags and fp.counters (and fp.sq) are the frame's.
+// frame_probe: BEGIN, zero the counters, the sums (and fp.sq), ZEROED, then the probe, or every flag raised without the
+//   early-out.  A split probe (fp.world > 1) writes the flags of its own tiles only, so the others are cleared first;
+//   a frame with its own counter block (progressive frames) keeps the raw flags.  ev may be null: no events.
+// frame_main: the counter snapshot into ws->h_counters + CN_SLOTS, MAIN_BEGIN, compaction + samples over the flags in
+//   fp.flags, MAIN_END, TRACED.
+// frame_finish: RGB8 (from d_rgb) and sums to the host if asked, the counters into ws->h_counters, END.
+int frame_probe(DeviceScene *ds, const FrameParams &fp, cudaStream_t st, FrameEvents *ev, int *launches);
+int frame_main(DeviceScene *ds, const FrameParams &fp, cudaStream_t st, FrameEvents &ev, int *launches);
+int frame_finish(DeviceScene *ds, const FrameParams &fp, const uint8_t *d_rgb, uint8_t *rgb_out, int32_t *sums_out, cudaStream_t st,
+                 FrameEvents &ev);
+// RtStats from the counters last copied into ds->ws->h_counters; with ev, also the frame's times and main_rays
+void read_stats(const DeviceScene *ds, size_t n_pixels, bool adaptive, int launches, const FrameEvents *ev, RtStats *stats);
+
+// The tail of a frame split over ranks, for one rank's slice of the pixels: sum the ranks' sums (peer loads over NVLink),
+// truncating mean, gamma, RGB8 into each of rgb[0, n_rgb) and, if given, the summed int4 into sums.  Four pixels per
+// thread, so that the RGB8 stores are whole 32-bit words.  (rtfs_multi.cu)
+struct ReduceTargets {
+    const int32_t *stats[kMaxDevices];
+    int32_t world;
+    uint8_t *rgb[kMaxDevices];
+    int32_t n_rgb;
+    int32_t *sums;
+};
+int launch_reduce_finalize(const ReduceTargets &t, int rank, size_t n_pixels, int gamma, cudaStream_t st, int *launches);
+
+// PixelOutput.correct (ImageOutput.fs:11-18): the block fills `lut` with the 8-bit output of every mean, gamma or not
+__device__ __forceinline__ void fill_gamma_lut(uint8_t *lut, int gamma) {
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) {
+        int v = i;
+        if (gamma) {
+            v = __double2int_rn(sqrt(double(i) / 255.0) * 255.0); // Math.Round: half to even
+            if (v == 256) v = 255;
+        }
+        lut[i] = uint8_t(v);
+    }
+    __syncthreads();
+}
+// PixelStats.mean (Pixel.fs:103-108): the truncating mean of each channel, through the table
+__device__ __forceinline__ void pixel_rgb8(int4 s, const uint8_t *lut, uint8_t *out) {
+    int n = s.w > 0 ? s.w : 1;
+    out[0] = lut[(s.x / n) & 255];
+    out[1] = lut[(s.y / n) & 255];
+    out[2] = lut[(s.z / n) & 255];
+}
+
 // makes sure the tree the frame will walk is on the device (the wide tree is built on first use for small scenes)
 int prepare_frame(RtScene *scene, const RtRenderOpts *opts);
 bool frame_walks_wide_tree(const DeviceScene *ds, int opt_flags, bool smem_fits);
-void read_counters(DeviceScene *ds, RtStats *stats, size_t n_pixels, bool adaptive);
 
 inline DevCamera make_dev_camera(const RtCamera &c, int max_w, int max_h) {
     DevCamera d{};

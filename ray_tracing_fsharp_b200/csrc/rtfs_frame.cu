@@ -86,7 +86,6 @@ __global__ void __launch_bounds__(kNoiseThreads) noise_summary_kernel(NoiseParti
 struct RtFrame {
     RtScene *scene = nullptr;
     FrameParams fp;
-    bool count = false, no_smem = false;
     size_t n_pixels = 0;
     int32_t *d_stats = nullptr;
     uint8_t *d_flags = nullptr;
@@ -97,7 +96,7 @@ struct RtFrame {
     float *d_se = nullptr;              // rt_frame_noise's map, allocated on first use
     NoisePartial *d_partial = nullptr;  // and its per-block partial summaries, then the summary (kNoiseBlocks + 1)
     unsigned long long h_counters[CN_SLOTS] = {};
-    cudaEvent_t ev[2] = {nullptr, nullptr};
+    FrameEvents ev; // rt_frame_begin: ZEROED -> TRACED; a pass: BEGIN -> END
     int32_t samples_done = 0, samples_target = 0;
     uint64_t pixels_flagged = 0;
     double ms_per_sample = -1.0; // measured device time of one sample index of every flagged pixel (< 0: not known yet)
@@ -120,8 +119,7 @@ void frame_free(RtFrame *f) {
     cudaFree(f->d_sq);
     cudaFree(f->d_se);
     cudaFree(f->d_partial);
-    for (auto &e : f->ev)
-        if (e) cudaEventDestroy(e);
+    f->ev.destroy();
     delete f;
 }
 
@@ -145,12 +143,6 @@ void frame_progress(const RtFrame *f, RtFrameProgress *p) {
     p->device_ms = f->device_ms;
     p->passes = f->passes;
     p->done = f->samples_done == f->samples_target ? 1 : 0;
-}
-
-float elapsed_ms(cudaEvent_t a, cudaEvent_t b) {
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, a, b);
-    return ms;
 }
 
 } // namespace
@@ -183,7 +175,7 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
               cudaMalloc((void **)&f->d_list, n * sizeof(uint32_t)) == cudaSuccess && cudaMalloc((void **)&f->d_rgb, n * 3) == cudaSuccess &&
               cudaMalloc((void **)&f->d_counters, CN_SLOTS * sizeof(unsigned long long)) == cudaSuccess;
     if (noise) ok = ok && cudaMalloc((void **)&f->d_sq, n * sizeof(unsigned long long)) == cudaSuccess;
-    for (auto &e : f->ev) ok = ok && cudaEventCreate(&e) == cudaSuccess;
+    ok = ok && f->ev.create();
     if (!ok) return bail(fail(RT_ERR_CUDA, std::string("rt_frame_begin: allocation failed: ") + cudaGetErrorString(cudaGetLastError())));
 
     FrameParams &fp = f->fp;
@@ -193,32 +185,22 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
     fp.list = f->d_list;
     fp.counters = f->d_counters;
     fp.sq = f->d_sq; // non-null: plan_launch picks the kernels that also sum the squares
-    f->count = (opts->flags & RT_FLAG_COUNTERS) != 0;
-    f->no_smem = (opts->flags & RT_FLAG_NO_SMEM) != 0;
     f->samples_done = fp.n_probe; // 0 without the early-out
     f->samples_target = fp.sample_end;
     cudaStream_t st = ds->ws->stream;
     int launches = 0;
+    // with its own counter block, the frame's probe keeps the raw "means differ" flags, also where this target has no main
+    // phase: the frame can be extended
     auto enqueue = [&]() -> int {
-        RT_CUDA(cudaMemsetAsync(f->d_counters, 0, CN_SLOTS * sizeof(unsigned long long), st));
-        RT_CUDA(cudaMemsetAsync(f->d_stats, 0, n * 4 * sizeof(int32_t), st));
-        if (f->d_sq) RT_CUDA(cudaMemsetAsync(f->d_sq, 0, n * sizeof(unsigned long long), st));
-        RT_CUDA(cudaEventRecord(f->ev[0], st));
-        if (fp.adaptive) {
-            // the raw "means differ" flags, also where this target has no main phase: the frame can be extended
-            int rc2 = launch_probe(ds, fp, f->count, f->no_smem, st, &launches, true);
-            if (rc2 != RT_OK) return rc2;
-        } else {
-            RT_CUDA(cudaMemsetAsync(f->d_flags, 1, n, st));
-        }
-        int rc2 = launch_compact(ds, fp, single_flags(f->d_flags), f->d_list, st, &launches);
+        int rc2 = frame_probe(ds, fp, st, &f->ev, &launches);
         if (rc2 != RT_OK) return rc2;
-        RT_CUDA(cudaEventRecord(f->ev[1], st));
+        if ((rc2 = launch_compact(ds, fp, single_flags(f->d_flags), f->d_list, st, &launches)) != RT_OK) return rc2;
+        RT_CUDA(f->ev.record(FrameEvents::TRACED, st));
         return frame_sync(f, st);
     };
     if ((rc = enqueue()) != RT_OK) return bail(rc);
     f->pixels_flagged = f->h_counters[CN_LIST];
-    f->device_ms = elapsed_ms(f->ev[0], f->ev[1]);
+    f->device_ms = f->ev.ms(FrameEvents::ZEROED, FrameEvents::TRACED);
     // the probe traced n_probe samples of every pixel; a pass traces samples of the flagged pixels only
     if (fp.adaptive) f->ms_per_sample = f->device_ms * double(f->pixels_flagged) / (double(n) * double(fp.n_probe));
     *out = f;
@@ -247,14 +229,14 @@ int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameP
         fp.sample_end = f->samples_done + k;
         int launches = 0;
         RT_CUDA(cudaMemsetAsync(f->d_counters + CN_WORK_MAIN, 0, sizeof(unsigned long long), st));
-        RT_CUDA(cudaEventRecord(f->ev[0], st));
-        int rc = launch_samples(ds, fp, f->count, f->no_smem, st, &launches);
+        RT_CUDA(f->ev.record(FrameEvents::BEGIN, st));
+        int rc = launch_samples(ds, fp, st, &launches);
         if (rc != RT_OK) return rc;
-        RT_CUDA(cudaEventRecord(f->ev[1], st));
+        RT_CUDA(f->ev.record(FrameEvents::END, st));
         if ((rc = frame_sync(f, st)) != RT_OK) return rc;
         f->samples_done += k;
         f->passes += 1;
-        f->last_pass_ms = elapsed_ms(f->ev[0], f->ev[1]);
+        f->last_pass_ms = f->ev.ms(FrameEvents::BEGIN, FrameEvents::END);
         f->device_ms += f->last_pass_ms;
         f->ms_per_sample = f->pixels_flagged ? f->last_pass_ms / k : 0.0;
     }
@@ -268,7 +250,8 @@ int rt_frame_read(RtFrame *f, int32_t gamma, uint8_t *rgb_out, int32_t *sums_out
     RT_CUDA(cudaSetDevice(ds->device));
     cudaStream_t st = ds->ws->stream;
     if (rgb_out) {
-        int rc = rt_device_finalize(ds->device, f->d_stats, int32_t(f->n_pixels), gamma, f->d_rgb, st);
+        int launches = 0;
+        int rc = launch_finalize(f->d_stats, f->n_pixels, gamma, f->d_rgb, st, &launches);
         if (rc != RT_OK) return rc;
         RT_CUDA(cudaMemcpyAsync(rgb_out, f->d_rgb, f->n_pixels * 3, cudaMemcpyDeviceToHost, st));
     }

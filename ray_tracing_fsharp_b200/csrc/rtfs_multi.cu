@@ -36,56 +36,36 @@ struct RtMulti {
 namespace rtfs {
 namespace {
 
-struct ReduceParams {
-    const int32_t *stats[kMaxDevices];
-    int32_t world;
-    int32_t n_pixels;
-    int32_t quad_begin, quad_end; // this device's slice, in groups of four pixels
-    int32_t gamma;
-    uint8_t *rgb;   // n_pixels * 3, host-mapped
-    int32_t *sums;  // optional, n_pixels * 4, host-mapped
-};
-
-// sum over ranks (peer loads) -> truncating mean -> gamma -> RGB8; four pixels per thread so that the
-// stores are whole 32-bit words
-__global__ void reduce_finalize_kernel(const ReduceParams p) {
+__global__ void reduce_finalize_kernel(const ReduceTargets t, int n_pixels, int quad_begin, int quad_end, int gamma) {
     __shared__ uint8_t lut[256];
-    for (int i = threadIdx.x; i < 256; i += blockDim.x) {
-        int v = i;
-        if (p.gamma) {
-            v = __double2int_rn(sqrt(double(i) / 255.0) * 255.0);
-            if (v == 256) v = 255;
-        }
-        lut[i] = uint8_t(v);
-    }
-    __syncthreads();
-    int quad = p.quad_begin + blockIdx.x * blockDim.x + threadIdx.x;
-    if (quad >= p.quad_end) return;
+    fill_gamma_lut(lut, gamma);
+    const int quad = quad_begin + blockIdx.x * blockDim.x + threadIdx.x;
+    if (quad >= quad_end) return;
     uint8_t out[12];
-    int n_valid = min(4, p.n_pixels - 4 * quad);
+    const int n_valid = min(4, n_pixels - 4 * quad);
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-        int px = 4 * quad + k;
+        const int px = 4 * quad + k;
         int4 s = make_int4(0, 0, 0, 0);
         if (k < n_valid) {
-            for (int r = 0; r < p.world; ++r) {
-                int4 v = reinterpret_cast<const int4 *>(p.stats[r])[px];
+            for (int r = 0; r < t.world; ++r) {
+                const int4 v = reinterpret_cast<const int4 *>(t.stats[r])[px];
                 s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
             }
-            if (p.sums) reinterpret_cast<int4 *>(p.sums)[px] = s;
+            if (t.sums) reinterpret_cast<int4 *>(t.sums)[px] = s;
         }
-        int n = s.w > 0 ? s.w : 1;
-        out[3 * k + 0] = lut[(s.x / n) & 255];
-        out[3 * k + 1] = lut[(s.y / n) & 255];
-        out[3 * k + 2] = lut[(s.z / n) & 255];
+        pixel_rgb8(s, lut, out + 3 * k);
     }
-    if (n_valid == 4) {
-        uint32_t *dst = reinterpret_cast<uint32_t *>(p.rgb + 12 * size_t(quad));
-        dst[0] = uint32_t(out[0]) | (uint32_t(out[1]) << 8) | (uint32_t(out[2]) << 16) | (uint32_t(out[3]) << 24);
-        dst[1] = uint32_t(out[4]) | (uint32_t(out[5]) << 8) | (uint32_t(out[6]) << 16) | (uint32_t(out[7]) << 24);
-        dst[2] = uint32_t(out[8]) | (uint32_t(out[9]) << 8) | (uint32_t(out[10]) << 16) | (uint32_t(out[11]) << 24);
-    } else {
-        for (int k = 0; k < 3 * n_valid; ++k) p.rgb[12 * size_t(quad) + k] = out[k];
+    const uint32_t w0 = uint32_t(out[0]) | (uint32_t(out[1]) << 8) | (uint32_t(out[2]) << 16) | (uint32_t(out[3]) << 24);
+    const uint32_t w1 = uint32_t(out[4]) | (uint32_t(out[5]) << 8) | (uint32_t(out[6]) << 16) | (uint32_t(out[7]) << 24);
+    const uint32_t w2 = uint32_t(out[8]) | (uint32_t(out[9]) << 8) | (uint32_t(out[10]) << 16) | (uint32_t(out[11]) << 24);
+    for (int r = 0; r < t.n_rgb; ++r) {
+        if (n_valid == 4) {
+            uint32_t *dst = reinterpret_cast<uint32_t *>(t.rgb[r] + 12 * size_t(quad));
+            dst[0] = w0; dst[1] = w1; dst[2] = w2;
+        } else {
+            for (int k = 0; k < 3 * n_valid; ++k) t.rgb[r][12 * size_t(quad) + k] = out[k];
+        }
     }
 }
 
@@ -139,6 +119,17 @@ int multi_workspace(RtMulti *m, size_t n_pixels, bool want_sums) {
 }
 
 } // namespace
+
+int launch_reduce_finalize(const ReduceTargets &t, int rank, size_t n_pixels, int gamma, cudaStream_t st, int *launches) {
+    const long long n_quads = (long long)(n_pixels + 3) / 4;
+    const int quad_begin = int(n_quads * rank / t.world), quad_end = int(n_quads * (rank + 1) / t.world);
+    if (quad_end <= quad_begin) return RT_OK;
+    reduce_finalize_kernel<<<(quad_end - quad_begin + 255) / 256, 256, 0, st>>>(t, int(n_pixels), quad_begin, quad_end, gamma);
+    RT_CUDA(cudaGetLastError());
+    ++*launches;
+    return RT_OK;
+}
+
 } // namespace rtfs
 
 using namespace rtfs;
@@ -214,7 +205,6 @@ int rt_multi_render(RtMulti *m, const RtCamera *camera, int32_t max_w, int32_t m
     if (rc != RT_OK) return rc;
     for (RtScene *s : m->scenes)
         if ((rc = prepare_frame(s, opts)) != RT_OK) return rc;
-    const bool count = (opts->flags & RT_FLAG_COUNTERS) != 0, no_smem = (opts->flags & RT_FLAG_NO_SMEM) != 0;
     std::vector<int> launches(world, 0);
     std::vector<FrameParams> fps(world);
     FlagsView flags{};
@@ -230,15 +220,7 @@ int rt_multi_render(RtMulti *m, const RtCamera *camera, int32_t max_w, int32_t m
         fps[i].stats = m->d_stats[i];
         fps[i].flags = m->d_flags[i];
         RT_CUDA(cudaEventRecord(m->ev_begin[i], st));
-        RT_CUDA(cudaMemsetAsync(ds->ws->d_counters, 0, CN_SLOTS * sizeof(unsigned long long), st));
-        RT_CUDA(cudaMemsetAsync(m->d_stats[i], 0, n_pixels * 4 * sizeof(int32_t), st));
-        if (fps[i].adaptive) {
-            RT_CUDA(cudaMemsetAsync(m->d_flags[i], 0, n_pixels, st));
-            rc = launch_probe(ds, fps[i], count, no_smem, st, &launches[i]);
-            if (rc != RT_OK) return rc;
-        } else {
-            RT_CUDA(cudaMemsetAsync(m->d_flags[i], 1, n_pixels, st));
-        }
+        if ((rc = frame_probe(ds, fps[i], st, nullptr, &launches[i])) != RT_OK) return rc;
         RT_CUDA(cudaEventRecord(m->ev_probe[i], st));
     }
     // phase 2: needs everyone's flags
@@ -248,34 +230,23 @@ int rt_multi_render(RtMulti *m, const RtCamera *camera, int32_t max_w, int32_t m
         cudaStream_t st = m->streams[i];
         for (int j = 0; j < world; ++j)
             if (j != i) RT_CUDA(cudaStreamWaitEvent(st, m->ev_probe[j], 0));
-        rc = launch_main(ds, fps[i], flags, count, no_smem, st, &launches[i]);
-        if (rc != RT_OK) return rc;
+        if ((rc = launch_main(ds, fps[i], flags, st, &launches[i])) != RT_OK) return rc;
         RT_CUDA(cudaMemcpyAsync(ds->ws->h_counters, ds->ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
         RT_CUDA(cudaEventRecord(m->ev_main[i], st));
     }
     // reduce + finalize: needs everyone's sums; each device owns a slice of the pixels
-    const int n_quads = int((n_pixels + 3) / 4);
+    ReduceTargets t{};
+    for (int j = 0; j < world; ++j) t.stats[j] = m->d_stats[j];
+    t.world = world;
+    t.n_rgb = 1;
     for (int i = 0; i < world; ++i) {
         RT_CUDA(cudaSetDevice(m->devices[i]));
         cudaStream_t st = m->streams[i];
         for (int j = 0; j < world; ++j)
             if (j != i) RT_CUDA(cudaStreamWaitEvent(st, m->ev_main[j], 0));
-        ReduceParams rp{};
-        for (int j = 0; j < world; ++j) rp.stats[j] = m->d_stats[j];
-        rp.world = world;
-        rp.n_pixels = int(n_pixels);
-        rp.quad_begin = int((long long)n_quads * i / world);
-        rp.quad_end = int((long long)n_quads * (i + 1) / world);
-        rp.gamma = opts->gamma;
-        RT_CUDA(cudaHostGetDevicePointer((void **)&rp.rgb, m->h_rgb, 0));
-        rp.sums = nullptr;
-        if (sums_out) RT_CUDA(cudaHostGetDevicePointer((void **)&rp.sums, m->h_sums, 0));
-        int nq = rp.quad_end - rp.quad_begin;
-        if (nq > 0) {
-            reduce_finalize_kernel<<<(nq + 255) / 256, 256, 0, st>>>(rp);
-            RT_CUDA(cudaGetLastError());
-            ++launches[i];
-        }
+        RT_CUDA(cudaHostGetDevicePointer((void **)&t.rgb[0], m->h_rgb, 0));
+        if (sums_out) RT_CUDA(cudaHostGetDevicePointer((void **)&t.sums, m->h_sums, 0));
+        if ((rc = launch_reduce_finalize(t, i, n_pixels, opts->gamma, st, &launches[i])) != RT_OK) return rc;
         RT_CUDA(cudaEventRecord(m->ev_end[i], st));
     }
     for (int i = 0; i < world; ++i) {
@@ -286,23 +257,20 @@ int rt_multi_render(RtMulti *m, const RtCamera *camera, int32_t max_w, int32_t m
     if (sums_out) std::memcpy(sums_out, m->h_sums, n_pixels * 4 * sizeof(int32_t));
     if (stats) {
         std::memset(stats, 0, sizeof *stats);
-        double kernel_ms = 0.0;
-        unsigned long long listed = 0;
         for (int i = 0; i < world; ++i) {
-            auto *ds = static_cast<DeviceScene *>(m->scenes[i]->dev);
-            stats->paths += ds->ws->h_counters[CN_PATHS];
-            stats->rays += ds->ws->h_counters[CN_RAYS];
-            stats->box_tests += ds->ws->h_counters[CN_BOX];
-            stats->prim_tests += ds->ws->h_counters[CN_PRIM];
-            stats->degenerate_paths += ds->ws->h_counters[CN_DEGENERATE];
-            listed = ds->ws->h_counters[CN_LIST];
-            stats->launches += launches[i];
+            RtStats d;
+            read_stats(static_cast<DeviceScene *>(m->scenes[i]->dev), n_pixels, opts->adaptive != 0, launches[i], nullptr, &d);
+            stats->paths += d.paths;
+            stats->rays += d.rays;
+            stats->box_tests += d.box_tests;
+            stats->prim_tests += d.prim_tests;
+            stats->degenerate_paths += d.degenerate_paths;
+            stats->launches += d.launches;
+            stats->pixels_early_out = d.pixels_early_out; // every device compacted the same flags
             float ms = 0.f;
             cudaEventElapsedTime(&ms, m->ev_begin[i], m->ev_end[i]);
-            kernel_ms = std::max(kernel_ms, double(ms));
+            stats->kernel_ms = std::max(stats->kernel_ms, double(ms)); // device time of the slowest GPU, probe -> reduce
         }
-        stats->pixels_early_out = opts->adaptive ? (unsigned long long)n_pixels - listed : 0;
-        stats->kernel_ms = kernel_ms; // device time of the slowest GPU, probe -> reduce
         stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     }
     return RT_OK;

@@ -14,6 +14,7 @@
 #include "rtfs_device.h"
 
 #include <cstring>
+#include <memory>
 
 namespace rtfs {
 namespace {
@@ -172,18 +173,6 @@ __global__ void __launch_bounds__(kWfThreads) wf_shade(const WfParams p) {
     }
 }
 
-// end of the probe phase: Scene.fs:177-188 — merge the two accumulator sets, flag pixels whose truncated means differ
-__global__ void wf_probe_flags(int32_t *stats_a, const int32_t *stats_b, uint8_t *flags, int n_pixels, int first_trial, int n_probe, int more) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_pixels) return;
-    int4 a = reinterpret_cast<int4 *>(stats_a)[i], b = reinterpret_cast<const int4 *>(stats_b)[i];
-    int n_old = first_trial + 1;
-    int4 s = make_int4(a.x + b.x, a.y + b.y, a.z + b.z, n_probe);
-    int diff = abs(s.x / n_probe - a.x / n_old) + abs(s.y / n_probe - a.y / n_old) + abs(s.z / n_probe - a.z / n_old);
-    reinterpret_cast<int4 *>(stats_a)[i] = s;
-    flags[i] = (diff != 0 && more) ? 1 : 0;
-}
-
 int wf_reserve(DeviceWorkspace *ws, WfState &st, size_t capacity) {
     // the state block is not pooled: the wavefront mode is a measurement variant, not the default path
     (void)ws;
@@ -210,36 +199,19 @@ int render_wavefront(RtScene *scene, const RtCamera *camera, int32_t max_w, int3
     RT_CUDA(cudaSetDevice(ds->device));
     cudaStream_t st = ws->stream;
     const size_t n_pixels = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
-    if (ws->ws_pixels < n_pixels) {
-        cudaFree(ws->d_stats); cudaFree(ws->d_flags); cudaFree(ws->d_rgb);
-        ws->d_stats = nullptr; ws->d_flags = nullptr; ws->d_rgb = nullptr; ws->ws_pixels = 0;
-        RT_CUDA(cudaMalloc((void **)&ws->d_stats, n_pixels * 4 * sizeof(int32_t)));
-        RT_CUDA(cudaMalloc((void **)&ws->d_flags, n_pixels));
-        RT_CUDA(cudaMalloc((void **)&ws->d_rgb, n_pixels * 3));
-        ws->ws_pixels = n_pixels;
-    }
-    if (ws->list_pixels < n_pixels) {
-        cudaFree(ws->d_list);
-        ws->d_list = nullptr; ws->list_pixels = 0;
-        RT_CUDA(cudaMalloc((void **)&ws->d_list, n_pixels * sizeof(uint32_t)));
-        ws->list_pixels = n_pixels;
-    }
+    int rc = ensure_frame_buffers(ws, n_pixels);
+    if (rc == RT_OK) rc = ensure_list(ws, n_pixels);
+    if (rc == RT_OK) rc = ensure_probe_sums(ws, n_pixels);
+    if (rc != RT_OK) return rc;
     FrameParams fp;
     fill_frame(fp, ds, *camera, max_w, max_h, *opts, 0, 1);
+    fp.stats = ws->d_stats;
+    fp.flags = ws->d_flags;
 
     const size_t batch = size_t(8) << 20; // paths in flight
     WfState wf;
-    int32_t *stats_b = nullptr;
-    auto cleanup = [&]() {
-        cudaFree(wf.block);
-        cudaFree(stats_b);
-    };
-    int rc = wf_reserve(ws, wf, batch);
-    if (rc != RT_OK) return rc;
-    if (cudaMalloc((void **)&stats_b, n_pixels * 4 * sizeof(int32_t)) != cudaSuccess) {
-        cleanup();
-        return fail(RT_ERR_CUDA, "wavefront: accumulator allocation failed");
-    }
+    if ((rc = wf_reserve(ws, wf, batch)) != RT_OK) return rc;
+    const std::unique_ptr<void, cudaError_t (*)(void *)> free_state(wf.block, cudaFree);
 
     // shared-memory staging plan (persistent grid-stride blocks)
     const bool no_smem = (opts->flags & RT_FLAG_NO_SMEM) != 0;
@@ -272,7 +244,7 @@ int render_wavefront(RtScene *scene, const RtCamera *camera, int32_t max_w, int3
     p.s_spheres = uint32_t(nodes_q);
     p.s_mats = uint32_t(nodes_q + sph_q);
     p.stats_a = ws->d_stats;
-    p.stats_b = stats_b;
+    p.stats_b = ws->d_stats_b;
 
     cudaError_t err = cudaSuccess;
     auto run_phase = [&](bool probe, unsigned long long n_paths, uint32_t n_list) -> int {
@@ -307,68 +279,38 @@ int render_wavefront(RtScene *scene, const RtCamera *camera, int32_t max_w, int3
         return RT_OK;
     };
     auto fail_cuda = [&](const char *what) {
-        std::string msg = std::string(what) + ": " + cudaGetErrorString(err != cudaSuccess ? err : cudaGetLastError());
-        cleanup();
-        return fail(RT_ERR_CUDA, msg);
+        return fail(RT_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(err != cudaSuccess ? err : cudaGetLastError()));
     };
 
-    cudaEventRecord(ws->ev[0], st);
+    FrameEvents &ev = ws->ev;
+    ev.record(FrameEvents::BEGIN, st);
     cudaMemsetAsync(ws->d_counters, 0, CN_SLOTS * sizeof(unsigned long long), st);
     cudaMemsetAsync(ws->d_stats, 0, n_pixels * 4 * sizeof(int32_t), st);
-    cudaMemsetAsync(stats_b, 0, n_pixels * 4 * sizeof(int32_t), st);
-    cudaEventRecord(ws->ev[1], st);
-    unsigned long long n_list = n_pixels;
+    cudaMemsetAsync(ws->d_stats_b, 0, n_pixels * 4 * sizeof(int32_t), st);
+    ev.record(FrameEvents::ZEROED, st);
     if (fp.adaptive) {
         if (run_phase(true, (unsigned long long)n_pixels * fp.n_probe, 0) != RT_OK) return fail_cuda("wavefront probe phase");
-        wf_probe_flags<<<unsigned((n_pixels + 255) / 256), 256, 0, st>>>(ws->d_stats, stats_b, ws->d_flags, int(n_pixels), fp.first_trial, fp.n_probe,
-                                                                          fp.sample_end > fp.sample_begin ? 1 : 0);
-        ++launches;
+        launch_probe_flags(fp, ws->d_stats_b, fp.sample_end > fp.sample_begin, st, &launches);
     } else {
         cudaMemsetAsync(ws->d_flags, 1, n_pixels, st);
     }
     // the flagged-pixel list (same kernel as the megakernel path uses)
-    {
-        FrameParams f2 = fp;
-        f2.stats = ws->d_stats;
-        f2.flags = ws->d_flags;
-        f2.sample_end = fp.sample_begin; // no samples: launch_main then only compacts
-        rc = launch_main(ds, f2, single_flags(ws->d_flags), false, true, st, &launches);
-        if (rc != RT_OK) {
-            cleanup();
-            return rc;
-        }
-        cudaMemcpyAsync(ws->h_counters, ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
-        if ((err = cudaStreamSynchronize(st)) != cudaSuccess) return fail_cuda("wavefront compaction");
-        n_list = ws->h_counters[CN_LIST];
-    }
+    launch_compact(ds, fp, single_flags(ws->d_flags), ws->d_list, st, &launches);
+    cudaMemcpyAsync(ws->h_counters, ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
+    if ((err = cudaStreamSynchronize(st)) != cudaSuccess) return fail_cuda("wavefront compaction");
+    const unsigned long long n_list = ws->h_counters[CN_LIST];
     const int n_main = fp.sample_end - fp.sample_begin;
     if (n_main > 0 && n_list > 0)
         if (run_phase(false, n_list * (unsigned long long)n_main, uint32_t(n_list)) != RT_OK) return fail_cuda("wavefront main phase");
-    cudaEventRecord(ws->ev[2], st);
-    rc = rt_device_finalize(ds->device, ws->d_stats, int32_t(n_pixels), opts->gamma, ws->d_rgb, st);
-    ++launches;
-    if (rc != RT_OK) {
-        cleanup();
-        return rc;
+    ev.record(FrameEvents::TRACED, st);
+    if ((rc = launch_finalize(ws->d_stats, n_pixels, opts->gamma, ws->d_rgb, st, &launches)) != RT_OK) return rc;
+    if ((rc = frame_finish(ds, fp, ws->d_rgb, rgb_out, sums_out, st, ev)) != RT_OK) return rc;
+    RT_CUDA(cudaStreamSynchronize(st));
+    if (stats) { // no main_ms: the main phase is many launches with host synchronisations between them
+        read_stats(ds, n_pixels, fp.adaptive != 0, launches, nullptr, stats);
+        stats->kernel_ms = ev.ms(FrameEvents::ZEROED, FrameEvents::TRACED);
+        stats->total_ms = ev.ms(FrameEvents::BEGIN, FrameEvents::END);
     }
-    cudaMemcpyAsync(rgb_out, ws->d_rgb, n_pixels * 3, cudaMemcpyDeviceToHost, st);
-    if (sums_out) cudaMemcpyAsync(sums_out, ws->d_stats, n_pixels * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, st);
-    cudaMemcpyAsync(ws->h_counters, ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
-    cudaEventRecord(ws->ev[3], st);
-    if ((err = cudaStreamSynchronize(st)) != cudaSuccess) return fail_cuda("wavefront frame");
-    if (stats) {
-        std::memset(stats, 0, sizeof *stats);
-        stats->paths = ws->h_counters[CN_PATHS];
-        stats->rays = ws->h_counters[CN_RAYS];
-        stats->pixels_early_out = fp.adaptive ? (unsigned long long)n_pixels - n_list : 0;
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, ws->ev[1], ws->ev[2]);
-        stats->kernel_ms = ms;
-        cudaEventElapsedTime(&ms, ws->ev[0], ws->ev[3]);
-        stats->total_ms = ms;
-        stats->launches = launches;
-    }
-    cleanup();
     return RT_OK;
 }
 

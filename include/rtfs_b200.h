@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define RT_ABI_VERSION 4
+#define RT_ABI_VERSION 5
 
 /* ---- error codes --------------------------------------------------------------------------- */
 #define RT_OK 0
@@ -310,6 +310,38 @@ int rt_frame_noise(RtFrame *frame, double tolerance, float *se_out, uint64_t *sq
 /* The same E from saved moments, on the host (no device needed): sums n*4 int32 {T_r, T_g, T_b, n} as rt_render and
  * rt_frame_read give them, sq n uint64 Q, se_out n float. */
 int rt_pixel_noise(const int32_t *sums, const uint64_t *sq, size_t n, float *se_out);
+
+/* Convergence rule of a progressive frame opened with RT_FLAG_NOISE: stop sampling each pixel once its E has converged.
+ * rt_frame_set_convergence(tolerance tau, min_samples m, interval k) before the first pass; a second call before it
+ * replaces the rule.  RT_ERR_INVALID_ARGUMENT without RT_FLAG_NOISE, after a pass, for tau negative or NaN, k < 1,
+ * m < 2 or m <= samples_done (the probe's samples).
+ *   Checkpoints are the sample counts c = m + j k (j >= 0), a fixed lattice: they do not depend on the target, the
+ *   pacing or rt_frame_extend.  A pass never crosses one: rt_frame_advance also cuts its window at the next checkpoint.
+ *   When a pass ends on a checkpoint c, the same rt_frame_advance call runs the check: every pixel still being sampled
+ *   whose E over samples [0, c) is <= tau (E in double, exactly as rt_frame_noise computes it: the complement of its
+ *   summary's E > tolerance) stops there, with its sums, count and Q.
+ *   So every pixel p holds samples [0, n_p): n_p = n_probe for a pixel the probe stopped, the first checkpoint at which it
+ *   converged, or samples_done for a pixel still being sampled; bit for bit rt_render's pixel p at samples_per_pixel =
+ *   n_p.  n_p is a function of the frame's inputs and the rule only: the frame is the same whatever the pacing, and a
+ *   frame extended from 256 to 512 samples is the frame opened at 512.
+ *   Progress: samples_done is the count of the pixels still being sampled; pixels_flagged keeps its meaning;
+ *   paths_target = paths_done + pixels_active (samples_target - samples_done), exact if nothing more converges, so it
+ *   never grows between two rt_frame_extend calls; when a check leaves no pixel active, samples_done becomes
+ *   samples_target (done) without a launch.  rt_frame_noise's summary covers the pixels still being sampled: right after
+ *   a check, pixels_above == pixels at tolerance tau.  The check (one thread per pixel, then the compaction of the
+ *   remaining flags) is part of its pass's last_pass_ms.
+ * rt_frame_convergence fails (RT_ERR_INVALID_ARGUMENT) on a frame without a rule. */
+typedef struct RtFrameConvergence {
+    double tolerance;          /* tau, as set                                                                        */
+    int32_t min_samples;       /* m                                                                                  */
+    int32_t interval;          /* k                                                                                  */
+    int32_t next_check;        /* the first checkpoint above samples_done                                            */
+    int32_t checks;            /* checks run so far                                                                  */
+    uint64_t pixels_active;    /* pixels still being sampled (pixels_flagged before the first check)                 */
+    uint64_t pixels_converged; /* pixels stopped by a check; pixels_active + pixels_converged == pixels_flagged       */
+} RtFrameConvergence;
+int rt_frame_set_convergence(RtFrame *frame, double tolerance, int32_t min_samples, int32_t interval);
+int rt_frame_convergence(RtFrame *frame, RtFrameConvergence *out);
 
 /* The same frame split over the GPUs of this process (the F# host is one process): replicated scene,
  * sample-index split (Scene.fs:191-192 shared out by sample index), probe tiles shared out by tile.

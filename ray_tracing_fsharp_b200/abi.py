@@ -5,7 +5,7 @@ struct against the values the compiled library reports.
 """
 import ctypes as C
 
-RT_ABI_VERSION = 4
+RT_ABI_VERSION = 5
 
 RT_OK = 0
 RT_ERR_INVALID_ARGUMENT = -1
@@ -148,4 +148,16 @@ class RtFrameNoise(C.Structure):
         ("max_se", C.c_double),
         ("mean_se", C.c_double),
         ("tolerance", C.c_double),
+    ]
+
+
+class RtFrameConvergence(C.Structure):
+    _fields_ = [
+        ("tolerance", C.c_double),
+        ("min_samples", C.c_int32),
+        ("interval", C.c_int32),
+        ("next_check", C.c_int32),
+        ("checks", C.c_int32),
+        ("pixels_active", C.c_uint64),
+        ("pixels_converged", C.c_uint64),
     ]

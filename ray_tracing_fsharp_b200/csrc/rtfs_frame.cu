@@ -4,7 +4,8 @@
 // phase launches, with the same chunking.  Sums are integers keyed by (seed, pixel, sample index), so a frame that has
 // reached samples_done is bit for bit rt_render's frame at samples_per_pixel = samples_done (include/rtfs_b200.h).
 // A frame opened with RT_FLAG_NOISE also holds per pixel the sum of squares Q (render_kernel<NOISE = true>), from which
-// rt_frame_noise derives a per-pixel standard error and a summary over the flagged pixels.
+// rt_frame_noise derives a per-pixel standard error and a summary over the flagged pixels, and with which a convergence rule
+// (rt_frame_set_convergence) stops sampling each pixel once its estimate is within a tolerance.
 #include "rtfs_device.h"
 
 #include <algorithm>
@@ -79,6 +80,17 @@ __global__ void __launch_bounds__(kNoiseThreads) noise_summary_kernel(NoiseParti
     noise_block_reduce(acc, partial + kNoiseBlocks);
 }
 
+// The check of a convergence rule at a checkpoint: a pixel still being sampled whose E over the samples it holds is <= the
+// tolerance stops there (its flag is cleared; the compaction that follows drops it from the list).  E is rt_frame_noise's,
+// so `<=` is exactly the complement of its summary's `e > tolerance`.
+__global__ void __launch_bounds__(256) converge_kernel(const int4 *stats, const unsigned long long *sq, uint8_t *flags, size_t n_pixels,
+                                                       double tolerance) {
+    const size_t p = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (p >= n_pixels || !flags[p]) return;
+    const int4 s = stats[p];
+    if (pixel_standard_error(s.w, s.x, s.y, s.z, sq[p]) <= tolerance) flags[p] = 0;
+}
+
 } // namespace rtfs
 
 // A frame owns everything a pass writes: sums, flags, the flagged-pixel list, the image and its own counter block
@@ -102,6 +114,10 @@ struct RtFrame {
     double ms_per_sample = -1.0; // measured device time of one sample index of every flagged pixel (< 0: not known yet)
     double last_pass_ms = 0.0, device_ms = 0.0;
     int32_t passes = 0;
+    // convergence rule (rt_frame_set_convergence; conv_interval == 0: none): checkpoints conv_min + j conv_interval
+    double conv_tolerance = 0.0;
+    int32_t conv_min = 0, conv_interval = 0, conv_checks = 0;
+    uint64_t pixels_active = 0; // pixels still being sampled: the list's length (pixels_flagged until a check)
 };
 
 namespace {
@@ -130,6 +146,12 @@ int frame_sync(RtFrame *f, cudaStream_t st) {
     return RT_OK;
 }
 
+// the first checkpoint of the frame's rule above samples_done (int64: m + j k may pass INT32_MAX)
+int64_t next_checkpoint(const RtFrame *f) {
+    const int64_t m = f->conv_min, k = f->conv_interval, s = f->samples_done;
+    return s < m ? m : m + ((s - m) / k + 1) * k;
+}
+
 void frame_progress(const RtFrame *f, RtFrameProgress *p) {
     if (!p) return;
     std::memset(p, 0, sizeof *p);
@@ -138,6 +160,8 @@ void frame_progress(const RtFrame *f, RtFrameProgress *p) {
     p->samples_target = f->samples_target;
     p->paths_done = f->h_counters[CN_PATHS];
     p->paths_target = uint64_t(f->n_pixels) * n_probe + f->pixels_flagged * (uint64_t(f->samples_target) - n_probe);
+    // with a rule: exact if nothing more converges, so it only shrinks at a check
+    if (f->conv_interval) p->paths_target = p->paths_done + f->pixels_active * uint64_t(f->samples_target - f->samples_done);
     p->pixels_flagged = f->pixels_flagged;
     p->last_pass_ms = f->last_pass_ms;
     p->device_ms = f->device_ms;
@@ -199,7 +223,7 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
         return frame_sync(f, st);
     };
     if ((rc = enqueue()) != RT_OK) return bail(rc);
-    f->pixels_flagged = f->h_counters[CN_LIST];
+    f->pixels_flagged = f->pixels_active = f->h_counters[CN_LIST];
     f->device_ms = f->ev.ms(FrameEvents::ZEROED, FrameEvents::TRACED);
     // the probe traced n_probe samples of every pixel; a pass traces samples of the flagged pixels only
     if (fp.adaptive) f->ms_per_sample = f->device_ms * double(f->pixels_flagged) / (double(n) * double(fp.n_probe));
@@ -211,6 +235,8 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
 int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameProgress *progress) {
     if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_advance: null frame");
     if (max_samples < 0 || !(target_ms >= 0.0)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_advance: max_samples and target_ms must be >= 0");
+    const bool rule = f->conv_interval > 0;
+    if (rule && f->pixels_active == 0) f->samples_done = f->samples_target; // every pixel has stopped: nothing to trace
     const int left = f->samples_target - f->samples_done;
     if (left > 0) {
         int k = left;
@@ -221,6 +247,8 @@ int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameP
             else if (f->ms_per_sample > 0.0) paced = int(std::min(double(left), std::floor(target_ms / f->ms_per_sample)));
             k = std::min(k, std::max(1, paced));
         }
+        if (rule) k = int(std::min<int64_t>(k, next_checkpoint(f) - f->samples_done)); // a pass never crosses a checkpoint
+        const bool check = rule && f->samples_done + k == next_checkpoint(f);
         auto *ds = static_cast<DeviceScene *>(f->scene->dev);
         RT_CUDA(cudaSetDevice(ds->device));
         cudaStream_t st = ds->ws->stream;
@@ -232,13 +260,26 @@ int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameP
         RT_CUDA(f->ev.record(FrameEvents::BEGIN, st));
         int rc = launch_samples(ds, fp, st, &launches);
         if (rc != RT_OK) return rc;
+        if (check) { // the pass ends on a checkpoint: stop the converged pixels and list the others
+            converge_kernel<<<unsigned((f->n_pixels + 255) / 256), 256, 0, st>>>(reinterpret_cast<const int4 *>(f->d_stats), f->d_sq, f->d_flags,
+                                                                                 f->n_pixels, f->conv_tolerance);
+            RT_CUDA(cudaGetLastError());
+            if ((rc = launch_compact(ds, fp, single_flags(f->d_flags), f->d_list, st, &launches)) != RT_OK) return rc;
+        }
         RT_CUDA(f->ev.record(FrameEvents::END, st));
         if ((rc = frame_sync(f, st)) != RT_OK) return rc;
         f->samples_done += k;
         f->passes += 1;
         f->last_pass_ms = f->ev.ms(FrameEvents::BEGIN, FrameEvents::END);
         f->device_ms += f->last_pass_ms;
-        f->ms_per_sample = f->pixels_flagged ? f->last_pass_ms / k : 0.0;
+        const uint64_t before = f->pixels_active;
+        if (check) {
+            f->pixels_active = f->h_counters[CN_LIST];
+            f->conv_checks += 1;
+            if (f->pixels_active == 0) f->samples_done = f->samples_target; // done, without a launch
+        }
+        // the next pass traces the pixels still listed
+        f->ms_per_sample = before ? f->last_pass_ms / k * (double(f->pixels_active) / double(before)) : 0.0;
     }
     frame_progress(f, progress);
     return RT_OK;
@@ -302,6 +343,33 @@ int rt_frame_noise(RtFrame *f, double tolerance, float *se_out, uint64_t *sq_out
         summary->mean_se = total.pixels ? total.sum_se / double(total.pixels) : 0.0;
         summary->tolerance = tolerance;
     }
+    return RT_OK;
+}
+
+int rt_frame_set_convergence(RtFrame *f, double tolerance, int32_t min_samples, int32_t interval) {
+    if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_set_convergence: null frame");
+    if (!f->d_sq) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_set_convergence: the frame was opened without RT_FLAG_NOISE");
+    if (f->passes > 0) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_set_convergence: a pass has already run");
+    if (!(tolerance >= 0.0)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_set_convergence: tolerance must be >= 0");
+    if (interval < 1) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_set_convergence: interval must be >= 1");
+    if (min_samples < 2 || min_samples <= f->samples_done)
+        return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_set_convergence: min_samples must be >= 2 and above the probe's samples");
+    f->conv_tolerance = tolerance;
+    f->conv_min = min_samples;
+    f->conv_interval = interval;
+    return RT_OK;
+}
+
+int rt_frame_convergence(RtFrame *f, RtFrameConvergence *out) {
+    if (!f || !out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_convergence: null frame or output");
+    if (!f->conv_interval) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_convergence: the frame has no convergence rule");
+    out->tolerance = f->conv_tolerance;
+    out->min_samples = f->conv_min;
+    out->interval = f->conv_interval;
+    out->next_check = int32_t(std::min<int64_t>(next_checkpoint(f), INT32_MAX));
+    out->checks = f->conv_checks;
+    out->pixels_active = f->pixels_active;
+    out->pixels_converged = f->pixels_flagged - f->pixels_active;
     return RT_OK;
 }
 

@@ -10,7 +10,7 @@ import os
 import numpy as np
 
 from . import abi
-from .abi import RtCamera, RtFrameNoise, RtFrameProgress, RtHittable, RtRenderOpts, RtStats, RtTexture
+from .abi import RtCamera, RtFrameConvergence, RtFrameNoise, RtFrameProgress, RtHittable, RtRenderOpts, RtStats, RtTexture
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "librtfs_b200.so")
@@ -55,6 +55,8 @@ def _declare(lib):
         "rt_frame_extend": (C.c_int, [_vp, _i32]),
         "rt_frame_destroy": (None, [_vp]),
         "rt_frame_noise": (C.c_int, [_vp, C.c_double, _vp, _vp, C.POINTER(RtFrameNoise)]),
+        "rt_frame_set_convergence": (C.c_int, [_vp, C.c_double, _i32, _i32]),
+        "rt_frame_convergence": (C.c_int, [_vp, C.POINTER(RtFrameConvergence)]),
         "rt_pixel_noise": (C.c_int, [_vp, _vp, C.c_size_t, _vp]),
         "rt_render_multi": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i32, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _vp,
                                       _vp, C.POINTER(RtStats)]),
@@ -334,6 +336,18 @@ class Frame:
         sq = np.empty((self.rows, self.cols), np.uint64) if want_sq else None
         check(lib().rt_frame_noise(self.ptr, float(tolerance), ptr(se), ptr(sq), C.byref(summary)))
         return summary, se, sq
+
+    def set_convergence(self, tolerance, min_samples=64, interval=64):
+        """Stops sampling each pixel once its noise estimate is within `tolerance` (8-bit levels), checked at the sample
+        counts min_samples + j * interval (rt_frame_set_convergence).  Only on a frame opened with abi.RT_FLAG_NOISE, before
+        its first pass.  Every pixel is then exactly rt_render's pixel at the sample count it stopped at."""
+        check(lib().rt_frame_set_convergence(self.ptr, float(tolerance), int(min_samples), int(interval)))
+
+    def convergence(self) -> RtFrameConvergence:
+        """The rule and its state (rt_frame_convergence): next checkpoint, checks run, pixels still sampled and stopped."""
+        out = RtFrameConvergence()
+        check(lib().rt_frame_convergence(self.ptr, C.byref(out)))
+        return out
 
     def close(self):
         if getattr(self, "ptr", None):

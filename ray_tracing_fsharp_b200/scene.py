@@ -125,7 +125,9 @@ class Scene:
     def render_progressive(progress_increment: Callable[[float], None], print_fn: Callable[[str], None], max_width_coord: int,
                            max_height_coord: int, camera: abi.RtCamera, s: "Scene", seed: Optional[int] = None, adaptive: bool = True,
                            target_ms: float = 250.0, on_pass: Optional[Callable[[abi.RtFrameProgress, "native.Frame"], object]] = None,
-                           flags: int = 0, noise_tolerance: Optional[float] = None, noise_fraction: float = 0.0) -> np.ndarray:
+                           flags: int = 0, noise_tolerance: Optional[float] = None, noise_fraction: float = 0.0,
+                           converge_tolerance: Optional[float] = None, converge_min_samples: int = 64,
+                           converge_interval: int = 64) -> np.ndarray:
         """Scene.render's frame rendered in passes of about `target_ms` of device time each (native.Frame, one GPU).
         `progress_increment(1.0)` is called as passes complete, in proportion to the paths traced so far out of the frame's
         total, and exactly `rows` times in all, like the reference's one call per row (Scene.fs:232).  After every pass
@@ -136,7 +138,11 @@ class Scene:
         With `noise_tolerance` (8-bit levels) the frame also keeps its noise estimate (abi.RT_FLAG_NOISE, Frame.noise) and
         stops at the first check where at most `noise_fraction` of the pixels still being sampled have a standard error
         of the mean above the tolerance.  The check runs after the probe and after every pass (after `on_pass`); the image
-        returned is then rt_render's at the samples done."""
+        returned is then rt_render's at the samples done.
+        With `converge_tolerance` (8-bit levels) each pixel stops being sampled once its standard error is within it, checked
+        at converge_min_samples + j * converge_interval samples (Frame.set_convergence): every pixel is then rt_render's pixel
+        at the sample count it stopped at.  It composes with the `noise_tolerance` stop, whose summary then covers the pixels
+        still being sampled."""
         if not isinstance(s._handle, native.SceneHandle):
             raise NotImplementedError("progressive frames run on one GPU: make the scene with a single device")
         rows = 2 * max_height_coord + 1
@@ -148,7 +154,7 @@ class Scene:
             for _ in range(n):
                 progress_increment(1.0)
 
-        if noise_tolerance is not None:
+        if noise_tolerance is not None or converge_tolerance is not None:
             flags |= abi.RT_FLAG_NOISE
 
         def converged(frame, progress):
@@ -158,6 +164,8 @@ class Scene:
             return summary.pixels_above <= noise_fraction * summary.pixels
 
         with s._handle.open_frame(camera, max_width_coord, max_height_coord, seed=seed, adaptive=adaptive, flags=flags) as frame:
+            if converge_tolerance is not None:
+                frame.set_convergence(converge_tolerance, converge_min_samples, converge_interval)
             progress = frame.progress
             emit(ticks.update(progress.paths_done, progress.paths_target))  # the probe
             stop = converged(frame, progress)

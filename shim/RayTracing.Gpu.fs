@@ -11,7 +11,8 @@
 // `Scene.render` (Scene.fs:196-204), over a `GpuScene` built by `GpuScene.make : Hittable array -> GpuScene`
 // (the counterpart of `Scene.make`, Scene.fs:15-28), and `SceneGpu.renderWithProgress`, the same frame traced in passes
 // with progress reported as they finish (a `GpuFrame`, rt_frame_*, for callers that want the passes themselves), and
-// `SceneGpu.renderWithProgressUntil`, which also stops the frame once its per-pixel noise estimate is below a tolerance.
+// `SceneGpu.renderWithProgressUntil`, which also stops the frame once its per-pixel noise estimate is below a tolerance,
+// and `SceneGpu.renderConverging`, which stops sampling each pixel once its own estimate is.
 namespace RayTracing
 
 open System
@@ -131,6 +132,16 @@ module internal Native =
         val mutable meanSe : float
         val mutable tolerance : float
 
+    [<Struct ; StructLayout(LayoutKind.Sequential)>]
+    type RtFrameConvergence =
+        val mutable tolerance : float
+        val mutable minSamples : int
+        val mutable interval : int
+        val mutable nextCheck : int
+        val mutable checks : int
+        val mutable pixelsActive : uint64
+        val mutable pixelsConverged : uint64
+
 
     [<DllImport(Lib)>]
     extern nativeint rt_last_error ()
@@ -165,6 +176,12 @@ module internal Native =
 
     [<DllImport(Lib)>]
     extern int rt_frame_noise (nativeint frame, float tolerance, float32[] seOut, uint64[] sqOut, RtFrameNoise& summary)
+
+    [<DllImport(Lib)>]
+    extern int rt_frame_set_convergence (nativeint frame, float tolerance, int minSamples, int interval)
+
+    [<DllImport(Lib)>]
+    extern int rt_frame_convergence (nativeint frame, RtFrameConvergence& out)
 
     [<DllImport(Lib)>]
     extern int rt_pixel_noise (int[] sums, uint64[] sq, unativeint n, float32[] seOut)
@@ -476,6 +493,20 @@ type FrameNoise =
         Tolerance : float
     }
 
+/// The convergence rule of a progressive frame and its state (RtFrameConvergence of include/rtfs_b200.h): the tolerance
+/// (8-bit levels), the checkpoints MinSamples + j * Interval, the next one, the checks run so far, the pixels still being
+/// sampled and those a check has stopped.
+type FrameConvergence =
+    {
+        Tolerance : float
+        MinSamples : int
+        Interval : int
+        NextCheck : int
+        Checks : int
+        PixelsActive : uint64
+        PixelsConverged : uint64
+    }
+
 /// A frame in progress on a single-device GpuScene (rt_frame_*): advanced in passes over windows of sample indices.
 /// After every pass it is exactly the frame rt_render gives at `SamplesDone` samples per pixel with the same seed, so
 /// `Read` shows the image sharpening; a caller stops early by not advancing any more, and `Extend` continues a finished
@@ -529,6 +560,27 @@ type GpuFrame internal (handle : nativeint, rows : int, cols : int, first : Nati
             Tolerance = summary.tolerance
         },
         map
+
+    /// Stops sampling each pixel once its standard error is within `tolerance` (8-bit levels), checked at the sample
+    /// counts minSamples + j * interval (rt_frame_set_convergence).  Only on a frame opened with FrameFlags.Noise, before
+    /// its first pass.  Every pixel is then exactly rt_render's pixel at the sample count it stopped at.
+    member _.SetConvergence (tolerance : float, minSamples : int, interval : int) : unit =
+        Native.rt_frame_set_convergence (handle, tolerance, minSamples, interval) |> Native.check
+
+    /// The rule set by SetConvergence and its state (rt_frame_convergence).
+    member _.Convergence () : FrameConvergence =
+        let mutable c = Native.RtFrameConvergence ()
+        Native.rt_frame_convergence (handle, &c) |> Native.check
+
+        {
+            Tolerance = c.tolerance
+            MinSamples = c.minSamples
+            Interval = c.interval
+            NextCheck = c.nextCheck
+            Checks = c.checks
+            PixelsActive = c.pixelsActive
+            PixelsConverged = c.pixelsConverged
+        }
 
     interface IDisposable with
         member _.Dispose () =
@@ -650,11 +702,10 @@ module SceneGpu =
     let openFrame (maxWidthCoord : int) (maxHeightCoord : int) (camera : Camera) (seed : uint64) (s : GpuScene) : GpuFrame =
         openFrameWith 0 maxWidthCoord maxHeightCoord camera seed s
 
-    /// `renderWithProgress` with a stop on the noise estimate: with `Some (tolerance, fraction)` the frame stops at the
-    /// first check (after the probe, then after every pass) where at most `fraction` of the pixels still being sampled
-    /// have a standard error of the mean above `tolerance` (8-bit levels); the image is then rt_render's at the samples
-    /// done.  `None` is renderWithProgress.
-    let renderWithProgressUntil
+    // the frame of renderWithProgressUntil and renderConverging: passes of about 250 ms with progress ticks, an optional
+    // convergence rule (tolerance, minSamples, interval) and an optional stop on the noise summary (tolerance, fraction)
+    let private renderInPasses
+        (rule : (float * int * int) option)
         (noiseStop : (float * float) option)
         (progressIncrement : float<progress> -> unit)
         (_print : string -> unit)
@@ -669,10 +720,14 @@ module SceneGpu =
 
         let frame =
             lazy
-                (let flags = if noiseStop.IsSome then FrameFlags.Noise else 0
+                (let flags = if noiseStop.IsSome || rule.IsSome then FrameFlags.Noise else 0
 
                  use f =
                     openFrameWith flags maxWidthCoord maxHeightCoord camera (uint64 (Random().NextInt64 ())) s
+
+                 match rule with
+                 | Some (tolerance, minSamples, interval) -> f.SetConvergence (tolerance, minSamples, interval)
+                 | None -> ()
 
                  let ticked = ref 0
 
@@ -734,6 +789,37 @@ module SceneGpu =
                 )
 
         1.0<progress> * float rowsIter, Image.make rowsIter colsIter rows
+
+    /// `renderWithProgress` with a stop on the noise estimate: with `Some (tolerance, fraction)` the frame stops at the
+    /// first check (after the probe, then after every pass) where at most `fraction` of the pixels still being sampled
+    /// have a standard error of the mean above `tolerance` (8-bit levels); the image is then rt_render's at the samples
+    /// done.  `None` is renderWithProgress.
+    let renderWithProgressUntil
+        (noiseStop : (float * float) option)
+        (progressIncrement : float<progress> -> unit)
+        (print : string -> unit)
+        (maxWidthCoord : int)
+        (maxHeightCoord : int)
+        (camera : Camera)
+        (s : GpuScene)
+        : float<progress> * Image
+        =
+        renderInPasses None noiseStop progressIncrement print maxWidthCoord maxHeightCoord camera s
+
+    /// `renderWithProgress` where each pixel stops being sampled once its standard error of the mean is within
+    /// `tolerance` (8-bit levels), checked at minSamples + j * interval samples (GpuFrame.SetConvergence, e.g. 64 and 64):
+    /// every pixel is rt_render's pixel at the sample count it stopped at, and smooth regions cost fewer paths.
+    let renderConverging
+        (tolerance : float, minSamples : int, interval : int)
+        (progressIncrement : float<progress> -> unit)
+        (print : string -> unit)
+        (maxWidthCoord : int)
+        (maxHeightCoord : int)
+        (camera : Camera)
+        (s : GpuScene)
+        : float<progress> * Image
+        =
+        renderInPasses (Some (tolerance, minSamples, interval)) None progressIncrement print maxWidthCoord maxHeightCoord camera s
 
     /// `render`'s signature and laziness, but the frame is traced in passes of about 250 ms of device time and
     /// `progressIncrement 1.0<progress>` is called as passes finish, in proportion to the paths traced out of the frame's

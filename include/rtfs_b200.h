@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define RT_ABI_VERSION 5
+#define RT_ABI_VERSION 6
 
 /* ---- error codes --------------------------------------------------------------------------- */
 #define RT_OK 0
@@ -238,6 +238,32 @@ int rt_host_unpin(void *ptr);
 int rt_render(RtScene *scene, const RtCamera *camera, int32_t max_width_coord,
               int32_t max_height_coord, const RtRenderOpts *opts, uint8_t *rgb_out,
               int32_t *sums_out, RtStats *stats);
+
+/* ---- many views of one scene (host buffers; one GPU) -------------------------------------------- */
+/* n_views frames of one scene, same extents, in one submission: a turntable, a camera path, stereo pairs, a contact sheet
+ * of previews.  The views are stacked as one tall frame of n_views * rows rows, so the batch pays rt_render's fixed costs
+ * once (the launches of one probe, one main phase and one output tail, the tail of the persistent kernel, one device->host
+ * copy and one synchronisation) instead of once per view.
+ *
+ * View v is cameras[v] with seed seeds[v] (seeds NULL: opts->seed for every view).  rgb_out: n_views*rows*cols*3, view v at
+ * offset v*rows*cols*3; sums_out (optional) n_views*rows*cols*4 int32, view v at offset v*rows*cols*4.  Every sample is
+ * keyed by (seed, pixel, sample index) with the pixel counted within its view, and the sums are integers, so view v's bytes
+ * are bit for bit rt_render(scene, &cameras[v], max_w, max_h, opts with seed = seeds[v]).
+ * What may differ between views: origin, view direction, axes, viewport width and height, focal length, seed.
+ * What must be the same: samples_per_pixel and bounce_depth on every camera (the probe's firstTrial and the chunk table are
+ *   shared): RT_ERR_INVALID_ARGUMENT otherwise.
+ * Other argument errors (RT_ERR_INVALID_ARGUMENT): n_views < 1; cameras or rgb_out NULL; n_views * rows * cols >= 2^31;
+ *   and those of rt_render.
+ * Options.  RT_MODE_WAVEFRONT, RT_FLAG_FLOW and RT_FLAG_COUNTERS: RT_ERR_UNSUPPORTED (no batched wavefront, flow-schedule
+ *   or counting kernels).  RT_FLAG_NOISE is ignored, as rt_render ignores it.  RT_FLAG_NO_SMEM, RT_FLAG_WIDE_BVH,
+ *   RT_FLAG_BVH2, RT_FLAG_NO_LEAN, RT_FLAG_LOCKSTEP, adaptive and gamma act as in rt_render.
+ * Stats (optional): paths, rays, degenerate_paths and pixels_early_out are sums over the views; the _ms fields and
+ *   launches describe the batch; box_tests and prim_tests are 0.
+ * Like rt_render, the call returns with its device work complete, and rt_render or progressive frames may use the scene
+ * between two batches. */
+int rt_render_views(RtScene *scene, const RtCamera *cameras, const uint64_t *seeds, int32_t n_views,
+                    int32_t max_width_coord, int32_t max_height_coord, const RtRenderOpts *opts,
+                    uint8_t *rgb_out, int32_t *sums_out, RtStats *stats);
 
 /* ---- progressive frames (host buffers; one GPU) -------------------------------------------------- */
 /* rt_render's frame in sample passes, with progress between them (the reference calls progressIncrement as rows finish,

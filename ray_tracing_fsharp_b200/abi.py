@@ -5,7 +5,7 @@ struct against the values the compiled library reports.
 """
 import ctypes as C
 
-RT_ABI_VERSION = 5
+RT_ABI_VERSION = 6
 
 RT_OK = 0
 RT_ERR_INVALID_ARGUMENT = -1

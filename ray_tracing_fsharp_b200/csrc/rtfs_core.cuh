@@ -1099,18 +1099,20 @@ RTFS_HD ScatterResult scatter(const SceneAccess<SMEM> &sc, int prim, int last, f
 // `begin` starts a camera sample; `step` performs one hitObject + Reflection and reports whether the
 // path ended.  The render kernels call `step` from a single flat loop so that the lanes of a warp stay
 // converged on the traversal while their paths are at different bounces (path regeneration).
-struct PathState {
+// Rng: CounterRng, or a generator with the same draws that finds its key and pixel word another way (rtfs_views.cu); it
+// has the counter words `bounce` and `retry` and a `next()`.
+template <class Rng = CounterRng>
+struct PathStateT {
     float3 o, d;
     uint32_t colour;
     int32_t last; // the primitive the ray leaves, as a ref (see ref_of_prim)
     int32_t bounces;
-    CounterRng rng;
+    Rng rng;
 };
-RTFS_HD bool path_begin(PathState &p, const DevCamera &cam, uint32_t k0, uint32_t k1, int row_idx, int col_idx, uint32_t sample) {
-    p.rng.k0 = k0;
-    p.rng.k1 = k1;
-    p.rng.pixel = uint32_t(row_idx * cam.cols + col_idx);
-    p.rng.sample = sample;
+using PathState = PathStateT<>;
+// the camera sample of a path whose generator already holds its key, pixel and sample index
+template <class Rng>
+RTFS_HD bool path_start(PathStateT<Rng> &p, const DevCamera &cam, int row_idx, int col_idx) {
     p.rng.bounce = 0;
     p.rng.retry = 0;
     float4 u = p.rng.next(); // rand.GetTwo (), Scene.fs:129
@@ -1121,10 +1123,17 @@ RTFS_HD bool path_begin(PathState &p, const DevCamera &cam, uint32_t k0, uint32_
     int col = col_idx - cam.max_w;     // Scene.fs:226
     return camera_ray(cam, row, col, u.x, u.y, p.o, p.d);
 }
+RTFS_HD bool path_begin(PathState &p, const DevCamera &cam, uint32_t k0, uint32_t k1, int row_idx, int col_idx, uint32_t sample) {
+    p.rng.k0 = k0;
+    p.rng.k1 = k1;
+    p.rng.pixel = uint32_t(row_idx * cam.cols + col_idx);
+    p.rng.sample = sample;
+    return path_start(p, cam, row_idx, col_idx);
+}
 // the part of a step that follows hitObject: Reflection, bounce count (Scene.fs:102-114).
 // Returns true when the path is finished; `result` is then its Pixel.
-template <int SMEM>
-RTFS_HD bool path_after_hit(PathState &p, const SceneAccess<SMEM> &sc, const Hit &h, int max_count, uint32_t &result) {
+template <int SMEM, class Rng>
+RTFS_HD bool path_after_hit(PathStateT<Rng> &p, const SceneAccess<SMEM> &sc, const Hit &h, int max_count, uint32_t &result) {
     if (h.prim == kNoPrim) { // the ray goes off into the distance
         result = kBlack;
         return true;
@@ -1149,8 +1158,8 @@ RTFS_HD bool path_after_hit(PathState &p, const SceneAccess<SMEM> &sc, const Hit
     return false;
 }
 // one whole step: hitObject + Reflection; returns true when the path is finished
-template <int SMEM, bool COUNT, class Stack, bool WIDE = false>
-RTFS_HD bool path_step(PathState &p, const SceneAccess<SMEM> &sc, int max_count, uint32_t &result, TraversalCounters &cn, unsigned lanes,
+template <int SMEM, bool COUNT, class Stack, bool WIDE = false, class Rng>
+RTFS_HD bool path_step(PathStateT<Rng> &p, const SceneAccess<SMEM> &sc, int max_count, uint32_t &result, TraversalCounters &cn, unsigned lanes,
                        Stack &stack) {
     Hit h = closest_hit_from<SMEM, COUNT, Stack, WIDE>(sc, p.o, p.d, p.last, cn, lanes, stack);
     return path_after_hit<SMEM>(p, sc, h, max_count, result);

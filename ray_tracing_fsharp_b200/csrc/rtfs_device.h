@@ -59,6 +59,12 @@ struct FrameEvents {
     }
 };
 
+// one view of a batch (rt_render_views): its camera and its Philox key
+struct ViewCamera {
+    DevCamera cam;
+    uint32_t k0, k1;
+};
+
 // Frame buffers, scratch, stream and events of one device.  Allocating these costs milliseconds, so they are
 // pooled: a scene handle borrows one for its lifetime and returns it on destroy (handles stay independent of
 // one another; nothing is shared between two live handles).
@@ -79,6 +85,8 @@ struct DeviceWorkspace {
     void *d_blob = nullptr;
     void *h_blob = nullptr;
     size_t blob_cap = 0;
+    size_t views_cap = 0; // the per-view cameras and keys of rt_render_views
+    ViewCamera *d_views = nullptr;
     unsigned long long *d_counters = nullptr;
     unsigned long long *h_counters = nullptr; // pinned
     cudaStream_t stream = nullptr;
@@ -182,6 +190,12 @@ struct FrameParams {
     // last, so that no other parameter moves: rows*cols per-pixel sums of r^2 + g^2 + b^2 over the pixel's samples
     // (progressive frames opened with RT_FLAG_NOISE; null otherwise, and then the kernels without that sum run)
     unsigned long long *sq;
+    // a batch of views (rt_render_views, rtfs_views.cu): n_views views of view_pixels pixels each, stacked as one tall frame
+    // (cam.rows = n_views x the rows of a view), and the camera and key of every view; null otherwise, and then the kernels
+    // of one frame run
+    const ViewCamera *views;
+    int32_t n_views;
+    int32_t view_pixels;
 };
 
 
@@ -214,6 +228,10 @@ int launch_probe_flags(const FrameParams &fp, const int32_t *stats_b, bool more,
 int launch_main(DeviceScene *ds, FrameParams fp, const FlagsView &flags, cudaStream_t st, int *launches);
 int launch_compact(DeviceScene *ds, const FrameParams &fp, const FlagsView &flags, uint32_t *list, cudaStream_t st, int *launches);
 int launch_samples(DeviceScene *ds, FrameParams fp, cudaStream_t st, int *launches);
+// the kernel of a batch of views (rtfs_views.cu) for the launch plan_launch has decided: scene staged in shared memory
+// (and lean), or read from global memory with shared or local walk stacks over the binary or the 8-wide tree
+typedef void (*RenderKernelFn)(const FrameParams);
+RenderKernelFn pick_views_kernel(bool probe, bool smem, bool lean, bool sstack, bool wide);
 // PixelStats.mean + the optional gamma of a whole frame: sums -> RGB8
 int launch_finalize(const int32_t *stats, size_t n_pixels, int gamma, uint8_t *rgb, cudaStream_t st, int *launches);
 

@@ -48,6 +48,7 @@ def _declare(lib):
         "rt_scene_device_bytes": (C.c_size_t, [_vp]),
         "rt_scene_shared_memory_bytes": (C.c_size_t, [_vp]),
         "rt_render": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _vp, _vp, C.POINTER(RtStats)]),
+        "rt_render_views": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(RtRenderOpts), _vp, _vp, C.POINTER(RtStats)]),
         "rt_frame_begin": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), C.POINTER(_vp),
                                      C.POINTER(RtFrameProgress)]),
         "rt_frame_advance": (C.c_int, [_vp, _i32, C.c_double, C.POINTER(RtFrameProgress)]),
@@ -245,6 +246,26 @@ class SceneHandle:
         opts = RtRenderOpts(seed, int(adaptive), mode, int(gamma), flags)
         stats = RtStats()
         check(lib().rt_render(self.ptr, C.byref(camera), max_w, max_h, C.byref(opts), ptr(rgb), ptr(sums), C.byref(stats)))
+        return rgb, sums, stats
+
+    def render_views(self, cameras, max_w, max_h, seeds=None, adaptive=True, gamma=False, flags=0, want_sums=False, seed=0):
+        """n views of this scene in one submission (rt_render_views): `cameras` a sequence of RtCamera (same
+        samples_per_pixel and bounce_depth), `seeds` one per view or None (then `seed` for every view).  Returns
+        (uint8 [n, rows, cols, 3], int32 [n, rows, cols, 4] or None, RtStats of the batch); view v is exactly
+        render(cameras[v], max_w, max_h, seed=seeds[v]).  RtError RT_ERR_INVALID_ARGUMENT for an empty batch."""
+        n = len(cameras)
+        rows, cols = 2 * max_h + 1, 2 * max_w + 1
+        cams = (RtCamera * max(1, n))(*cameras)
+        sd = None
+        if seeds is not None:
+            if len(seeds) != n:
+                raise ValueError(f"{len(seeds)} seeds for {n} cameras")
+            sd = np.ascontiguousarray([int(x) for x in seeds], np.uint64)
+        rgb = _frame_buffer((n, rows, cols, 3))
+        sums = np.empty((n, rows, cols, 4), np.int32) if want_sums else None
+        opts = RtRenderOpts(seed, int(adaptive), abi.RT_MODE_MEGAKERNEL, int(gamma), flags)
+        stats = RtStats()
+        check(lib().rt_render_views(self.ptr, cams, ptr(sd), n, max_w, max_h, C.byref(opts), ptr(rgb), ptr(sums), C.byref(stats)))
         return rgb, sums, stats
 
     def open_frame(self, camera, max_w, max_h, seed=0, adaptive=True, flags=0, mode=abi.RT_MODE_MEGAKERNEL):

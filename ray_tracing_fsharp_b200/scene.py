@@ -6,6 +6,7 @@ reference's.  Everything that computes goes through the C ABI (native.py); nothi
   Camera.make_basic     RayTracing/Camera.fs:34-59
   Scene.make            RayTracing/Scene.fs:15-28
   Scene.render          RayTracing/Scene.fs:196-236
+  Scene.render_views    Scene.render of many cameras of one scene in one submission (rt_render_views)
   Scene.render_progressive  the same frame in sample passes, progress ticks as passes finish (native.Frame)
   Image / Image.render  RayTracing/Domain.fs:9-31
   ImageOutput.write_ppm RayTracing/ImageOutput.fs:163-197, PixelOutput.correct :11-18
@@ -120,6 +121,48 @@ class Scene:
             return out
 
         return float(rows), Image([row_thunk(r) for r in range(rows)], rows, cols, all_rows)
+
+    @staticmethod
+    def render_views(progress_increment: Callable[[float], None], print_fn: Callable[[str], None], max_width_coord: int,
+                     max_height_coord: int, cameras: Sequence[abi.RtCamera], s: "Scene", seed: Optional[int] = None,
+                     seeds: Optional[Sequence[int]] = None, adaptive: bool = True, flags: int = 0):
+        """Scene.render for every camera of `cameras` (same samples_per_pixel and bounce_depth; a turntable, a fly-through,
+        stereo pairs, previews), rendered together by one GPU (native.SceneHandle.render_views).  Returns (total progress,
+        [Image per camera]); lazy like Scene.render: the first forced row renders every view.  The progress ticks total
+        rows * len(cameras), one per row forced.  `seeds`: one RNG key per view; otherwise `seed` (None: one drawn from the
+        OS) for every view.  With the same camera and seed, view v is Scene.render's image.  `print_fn` is ignored."""
+        if not isinstance(s._handle, native.SceneHandle):
+            raise NotImplementedError("a batch of views runs on one GPU: make the scene with a single device")
+        rows, cols = 2 * max_height_coord + 1, 2 * max_width_coord + 1
+        n = len(cameras)
+        if seed is None and seeds is None:
+            seed = secrets.randbits(64)
+        state = {}
+
+        def frames():
+            if "rgb" not in state:
+                rgb, _, stats = s._handle.render_views(list(cameras), max_width_coord, max_height_coord, seeds=seeds, seed=seed or 0,
+                                                       adaptive=adaptive, flags=flags)
+                s.last_stats = stats
+                state["rgb"] = rgb
+            return state["rgb"]
+
+        def image(v):
+            def row_thunk(r):
+                def force():
+                    out = frames()[v, r]
+                    progress_increment(1.0)
+                    return out
+                return force
+
+            def all_rows():
+                out = frames()[v]
+                for _ in range(rows):
+                    progress_increment(1.0)
+                return out
+            return Image([row_thunk(r) for r in range(rows)], rows, cols, all_rows)
+
+        return float(rows * n), [image(v) for v in range(n)]
 
     @staticmethod
     def render_progressive(progress_increment: Callable[[float], None], print_fn: Callable[[str], None], max_width_coord: int,

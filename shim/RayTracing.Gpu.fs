@@ -158,6 +158,10 @@ module internal Native =
     [<DllImport(Lib)>]
     extern int rt_render (nativeint scene, RtCamera& camera, int maxWidthCoord, int maxHeightCoord, RtRenderOpts& opts, byte[] rgbOut, nativeint sumsOut, RtStats& stats)
 
+    // many views of one scene in one submission (include/rtfs_b200.h, rt_render_views); seeds may be null
+    [<DllImport(Lib)>]
+    extern int rt_render_views (nativeint scene, RtCamera[] cameras, uint64[] seeds, int nViews, int maxWidthCoord, int maxHeightCoord, RtRenderOpts& opts, byte[] rgbOut, nativeint sumsOut, RtStats& stats)
+
     // progressive frames on one device (include/rtfs_b200.h, rt_frame_*)
     [<DllImport(Lib)>]
     extern int rt_frame_begin (nativeint scene, RtCamera& camera, int maxWidthCoord, int maxHeightCoord, RtRenderOpts& opts, nativeint& frame, RtFrameProgress& progress)
@@ -678,6 +682,71 @@ module SceneGpu =
                 )
 
         1.0<progress> * float rowsIter, Image.make rowsIter colsIter rows
+
+    /// Scene.render for every camera of `cameras` (same SamplesPerPixel and BounceDepth; a turntable, a fly-through,
+    /// stereo pairs, previews), rendered together in one rt_render_views call on a single-device scene: one Image per
+    /// camera, lazy like `render` (the first forced row of any view renders them all).  Every row of every view reports
+    /// progress once: rows * cameras.Length in all.  One fresh seed per view, as `render` draws one per frame.
+    let renderViews
+        (progressIncrement : float<progress> -> unit)
+        (_print : string -> unit)
+        (maxWidthCoord : int)
+        (maxHeightCoord : int)
+        (cameras : Camera array)
+        (s : GpuScene)
+        : float<progress> * Image array
+        =
+        if s.IsMulti then
+            failwith "GPU backend: a batch of views runs on a single-device GpuScene"
+
+        let rowsIter = 2 * maxHeightCoord + 1
+        let colsIter = 2 * maxWidthCoord + 1
+        let n = cameras.Length
+
+        let frames =
+            lazy
+                (let rgb = Array.zeroCreate<byte> (3 * rowsIter * colsIter * n)
+                 let cams = cameras |> Array.map marshalCamera
+                 let seeds = Array.init n (fun _ -> uint64 (Random().NextInt64 ()))
+                 let mutable opts = Native.RtRenderOpts ()
+                 opts.adaptive <- 1
+                 let mutable stats = Native.RtStats ()
+
+                 Native.rt_render_views (s.Handle, cams, seeds, n, maxWidthCoord, maxHeightCoord, &opts, rgb, 0n, &stats)
+                 |> Native.check
+
+                 rgb)
+
+        let image (view : int) =
+            let rows =
+                Seq.init
+                    rowsIter
+                    (fun row ->
+                        async {
+                            let rgb = frames.Force ()
+                            let start = 3 * ((view * rowsIter + row) * colsIter)
+
+                            let result =
+                                Array.init
+                                    colsIter
+                                    (fun col ->
+                                        let i = start + 3 * col
+
+                                        {
+                                            Red = rgb.[i]
+                                            Green = rgb.[i + 1]
+                                            Blue = rgb.[i + 2]
+                                        }
+                                    )
+
+                            progressIncrement 1.0<progress>
+                            return result
+                        }
+                    )
+
+            Image.make rowsIter colsIter rows
+
+        1.0<progress> * float (rowsIter * n), Array.init n image
 
     /// Opens a progressive frame with RtRenderOpts.flags `flags` (e.g. FrameFlags.Noise for GpuFrame.Noise).
     /// Single-device scenes only.

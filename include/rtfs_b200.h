@@ -255,7 +255,8 @@ int rt_render(RtScene *scene, const RtCamera *camera, int32_t max_width_coord,
  * Other argument errors (RT_ERR_INVALID_ARGUMENT): n_views < 1; cameras or rgb_out NULL; n_views * rows * cols >= 2^31;
  *   and those of rt_render.
  * Options.  RT_MODE_WAVEFRONT, RT_FLAG_FLOW and RT_FLAG_COUNTERS: RT_ERR_UNSUPPORTED (no batched wavefront, flow-schedule
- *   or counting kernels).  RT_FLAG_NOISE is ignored, as rt_render ignores it.  RT_FLAG_NO_SMEM, RT_FLAG_WIDE_BVH,
+ *   or counting kernels).  RT_FLAG_NOISE is ignored, as rt_render ignores it (a batch that keeps its noise estimate is a
+ *   progressive frame: rt_frame_begin_views, below).  RT_FLAG_NO_SMEM, RT_FLAG_WIDE_BVH,
  *   RT_FLAG_BVH2, RT_FLAG_NO_LEAN, RT_FLAG_LOCKSTEP, adaptive and gamma act as in rt_render.
  * Stats (optional): paths, rays, degenerate_paths and pixels_early_out are sums over the views; the _ms fields and
  *   launches describe the batch; box_tests and prim_tests are 0.
@@ -368,6 +369,39 @@ typedef struct RtFrameConvergence {
 } RtFrameConvergence;
 int rt_frame_set_convergence(RtFrame *frame, double tolerance, int32_t min_samples, int32_t interval);
 int rt_frame_convergence(RtFrame *frame, RtFrameConvergence *out);
+
+/* ---- progressive frames of many views (host buffers; one GPU) ------------------------------------ */
+/* A progressive frame whose pixels are a batch of views: rt_render_views' tall frame (n_views * rows rows, view v at
+ * offset v*rows*cols) driven in passes, with the noise estimate and the convergence rule above.  A turntable rendered to
+ * a noise target pays each pass's fixed costs (the tail of the persistent kernel, a synchronisation, a counter copy) once
+ * for the batch instead of once per view.
+ *
+ * These two functions were added without a change of RT_ABI_VERSION (still 6): no struct and no existing prototype
+ * changed.  A caller detects the feature by the presence of the symbol rt_frame_begin_views.
+ *
+ * rt_frame_begin_views returns an ordinary RtFrame: rt_frame_advance, _read, _extend, _noise, _set_convergence,
+ * _convergence and _destroy accept it unchanged.  rt_frame_read writes n_views*rows*cols*3 bytes (sums
+ * n_views*rows*cols*4); rt_frame_noise's maps and its summary cover the whole batch; the counts of RtFrameProgress and
+ * RtFrameConvergence are sums over the views.
+ *   Arguments as rt_render_views: n_views >= 1, cameras non-NULL, the same samples_per_pixel and bounce_depth on every
+ *   camera, n_views * rows * cols < 2^31 (RT_ERR_INVALID_ARGUMENT otherwise); seeds NULL: opts->seed for every view.
+ *   Modes as rt_frame_begin: RT_MODE_MEGAKERNEL only; RT_FLAG_FLOW and RT_FLAG_COUNTERS: RT_ERR_UNSUPPORTED, with or
+ *   without RT_FLAG_NOISE.
+ *   The frame owns its table of view cameras and keys: rt_render_views, rt_render and other frames may run on the scene
+ *   between two passes.
+ * Exactness.  Every sample is keyed by (view seed, pixel within the view, sample index) and the sums, Q and counts are
+ *   integers, so after any pass view v is bit for bit the progressive frame of cameras[v] and seeds[v] at the same
+ *   samples_done (and rt_render's frame at that samples_per_pixel).  Under a convergence rule each pixel's stopping count
+ *   depends only on its own samples and the checkpoint lattice: view v of a converging batch is a converging frame of
+ *   camera v with the same rule, whatever the pacing of either.
+ * rt_frame_view_noise fills per_view[0 .. n_views) (n_views = 1 for a frame of rt_frame_begin): view v's summary over its
+ *   pixels still being sampled, bit for bit rt_frame_noise's summary of the frame of camera v and seed v in the same state
+ *   (the same fixed-order reduction over the view's pixels).  pixels == 0: the view is finished.  RT_ERR_INVALID_ARGUMENT
+ *   for a frame opened without RT_FLAG_NOISE, a NULL per_view, or a negative or NaN tolerance. */
+int rt_frame_begin_views(RtScene *scene, const RtCamera *cameras, const uint64_t *seeds, int32_t n_views,
+                         int32_t max_width_coord, int32_t max_height_coord, const RtRenderOpts *opts,
+                         RtFrame **out, RtFrameProgress *progress);
+int rt_frame_view_noise(RtFrame *frame, double tolerance, RtFrameNoise *per_view /* n_views entries */);
 
 /* The same frame split over the GPUs of this process (the F# host is one process): replicated scene,
  * sample-index split (Scene.fs:191-192 shared out by sample index), probe tiles shared out by tile.

@@ -447,9 +447,10 @@ static int plan_launch(DeviceScene *ds, FrameParams &fp, bool probe, LaunchPlan 
     // the sum of squares of progressive frames opened with RT_FLAG_NOISE: lockstep kernels without counters only
     const bool noise = fp.sq != nullptr;
     if (noise && (flow || count)) return fail(RT_ERR_UNSUPPORTED, "render: the noise estimate has no flow-schedule or counting kernel");
-    // a batch of views (rt_render_views): lockstep kernels without counters or the sum of squares
+    // a batch of views (rt_render_views, rt_frame_begin_views): lockstep kernels without counters, with or without the sum
+    // of squares
     const bool views = fp.views != nullptr;
-    if (views && (flow || count || noise)) return fail(RT_ERR_UNSUPPORTED, "render: a batch of views has no flow-schedule, counting or noise kernel");
+    if (views && (flow || count)) return fail(RT_ERR_UNSUPPORTED, "render: a batch of views has no flow-schedule or counting kernel");
     const size_t nodes_q = size_t(ds->g.n_nodes) * kStagedNodeQuads, sph_q = size_t(ds->g.n_bounded);
     const size_t scene_q = staged_scene_quads(ds);
     bool smem = scene_staged(ds, flow ? sizeof(FlowWarp) : warp_scratch_bytes(true, noise));
@@ -483,7 +484,7 @@ static int plan_launch(DeviceScene *ds, FrameParams &fp, bool probe, LaunchPlan 
     fp.stack_levels = int32_t(stack_q * 16 / (size_t(plan.threads) * 4));
     plan.smem_bytes = (used_q + (sstack ? stack_q : 0)) * 16;
     const bool lean = ds->lean && !(fp.opt_flags & RT_FLAG_NO_LEAN);
-    if (views) fn = pick_views_kernel(probe, smem, lean, sstack, wide);
+    if (views) fn = pick_views_kernel(probe, smem, lean, sstack, wide, noise);
     else fn = flow ? (probe ? pick_flow<true>(smem, count) : pick_flow<false>(smem, count)) : pick_kernel(probe, smem, lean, count, sstack, wide, noise);
     {
         static const bool show = std::getenv("RTFS_DEBUG_PLAN") != nullptr;

@@ -229,9 +229,10 @@ int launch_main(DeviceScene *ds, FrameParams fp, const FlagsView &flags, cudaStr
 int launch_compact(DeviceScene *ds, const FrameParams &fp, const FlagsView &flags, uint32_t *list, cudaStream_t st, int *launches);
 int launch_samples(DeviceScene *ds, FrameParams fp, cudaStream_t st, int *launches);
 // the kernel of a batch of views (rtfs_views.cu) for the launch plan_launch has decided: scene staged in shared memory
-// (and lean), or read from global memory with shared or local walk stacks over the binary or the 8-wide tree
+// (and lean), or read from global memory with shared or local walk stacks over the binary or the 8-wide tree; with noise,
+// the kernel that also sums the squares (progressive frames of a batch opened with RT_FLAG_NOISE)
 typedef void (*RenderKernelFn)(const FrameParams);
-RenderKernelFn pick_views_kernel(bool probe, bool smem, bool lean, bool sstack, bool wide);
+RenderKernelFn pick_views_kernel(bool probe, bool smem, bool lean, bool sstack, bool wide, bool noise);
 // PixelStats.mean + the optional gamma of a whole frame: sums -> RGB8
 int launch_finalize(const int32_t *stats, size_t n_pixels, int gamma, uint8_t *rgb, cudaStream_t st, int *launches);
 

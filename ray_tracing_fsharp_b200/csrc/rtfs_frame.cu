@@ -6,6 +6,9 @@
 // A frame opened with RT_FLAG_NOISE also holds per pixel the sum of squares Q (render_kernel<NOISE = true>), from which
 // rt_frame_noise derives a per-pixel standard error and a summary over the flagged pixels, and with which a convergence rule
 // (rt_frame_set_convergence) stops sampling each pixel once its estimate is within a tolerance.
+// rt_frame_begin_views opens the same frame over rt_render_views' tall frame of a batch of views (its kernels are in
+// rtfs_views.cu); the probe flags, the compaction, the checks and the output tail work per pixel and need no change for it,
+// and rt_frame_view_noise reduces each view as rt_frame_noise reduces a frame of its own.
 #include "rtfs_device.h"
 
 #include <algorithm>
@@ -55,10 +58,13 @@ __device__ __forceinline__ void noise_block_reduce(NoisePartial acc, NoisePartia
     if (threadIdx.x == 0) *out = part[0];
 }
 
+// blockIdx.y is the view of a batch (rt_frame_view_noise: n_pixels is then one view's pixels, view v starts at v n_pixels, and
+// its partials and summary at v (kNoiseBlocks + 1)): each view is reduced exactly as a frame of its own pixels would be.
 __global__ void __launch_bounds__(kNoiseThreads) noise_kernel(const int4 *stats, const unsigned long long *sq, const uint8_t *flags, size_t n_pixels,
                                                               double tolerance, float *se, NoisePartial *partial) {
-    const size_t per_block = (n_pixels + kNoiseBlocks - 1) / kNoiseBlocks;
-    const size_t begin = size_t(blockIdx.x) * per_block, end = begin + per_block < n_pixels ? begin + per_block : n_pixels;
+    const size_t per_block = (n_pixels + kNoiseBlocks - 1) / kNoiseBlocks, base = size_t(blockIdx.y) * n_pixels;
+    const size_t begin = base + size_t(blockIdx.x) * per_block;
+    const size_t end = size_t(blockIdx.x) * per_block + per_block < n_pixels ? begin + per_block : base + n_pixels;
     NoisePartial acc{0ull, 0ull, 0.0, 0.0};
     for (size_t p = begin + threadIdx.x; p < end; p += kNoiseThreads) {
         const int4 s = stats[p];
@@ -71,10 +77,12 @@ __global__ void __launch_bounds__(kNoiseThreads) noise_kernel(const int4 *stats,
             acc.sum_se += e;
         }
     }
-    noise_block_reduce(acc, partial + blockIdx.x);
+    noise_block_reduce(acc, partial + size_t(blockIdx.y) * (kNoiseBlocks + 1) + blockIdx.x);
 }
 
+// one block per view (blockIdx.x) over that view's partials, in block order
 __global__ void __launch_bounds__(kNoiseThreads) noise_summary_kernel(NoisePartial *partial) {
+    partial += size_t(blockIdx.x) * (kNoiseBlocks + 1);
     NoisePartial acc{0ull, 0ull, 0.0, 0.0};
     for (int b = threadIdx.x; b < kNoiseBlocks; b += kNoiseThreads) noise_combine(acc, partial[b]);
     noise_block_reduce(acc, partial + kNoiseBlocks);
@@ -106,7 +114,11 @@ struct RtFrame {
     unsigned long long *d_counters = nullptr;
     unsigned long long *d_sq = nullptr; // RT_FLAG_NOISE: per pixel the sum of r^2 + g^2 + b^2 (null otherwise)
     float *d_se = nullptr;              // rt_frame_noise's map, allocated on first use
-    NoisePartial *d_partial = nullptr;  // and its per-block partial summaries, then the summary (kNoiseBlocks + 1)
+    NoisePartial *d_partial = nullptr;  // and its per-block partial summaries, then the summary (kNoiseBlocks + 1 per view)
+    // a batch of views (rt_frame_begin_views): the frame's own table of view cameras and keys, since rt_render_views
+    // rewrites the workspace's between two passes; null for a frame of one camera
+    ViewCamera *d_views = nullptr;
+    int32_t n_views = 1;
     unsigned long long h_counters[CN_SLOTS] = {};
     FrameEvents ev; // rt_frame_begin: ZEROED -> TRACED; a pass: BEGIN -> END
     int32_t samples_done = 0, samples_target = 0;
@@ -135,6 +147,7 @@ void frame_free(RtFrame *f) {
     cudaFree(f->d_sq);
     cudaFree(f->d_se);
     cudaFree(f->d_partial);
+    cudaFree(f->d_views);
     f->ev.destroy();
     delete f;
 }
@@ -169,22 +182,13 @@ void frame_progress(const RtFrame *f, RtFrameProgress *p) {
     p->done = f->samples_done == f->samples_target ? 1 : 0;
 }
 
-} // namespace
-
-extern "C" {
-
-int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_t max_h, const RtRenderOpts *opts, RtFrame **out,
-                   RtFrameProgress *progress) {
-    int rc = check_frame_args(scene, camera, max_w, max_h, opts);
-    if (rc != RT_OK) return rc;
-    if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin: out is null");
-    *out = nullptr;
-    if (opts->mode == RT_MODE_WAVEFRONT) return fail(RT_ERR_UNSUPPORTED, "rt_frame_begin: progressive frames run the megakernel only");
-    if (opts->mode != RT_MODE_MEGAKERNEL) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin: unknown mode");
+// rt_frame_begin (views empty) and rt_frame_begin_views, once their arguments are checked: allocates the frame, and runs
+// the probe and the compaction.  A batch's frame is the tall frame of rt_render_views (rtfs_views.cu) with its own table.
+int frame_open(RtScene *scene, const RtCamera &camera, const std::vector<ViewCamera> &views, int32_t max_w, int32_t max_h,
+               const RtRenderOpts *opts, RtFrame **out, RtFrameProgress *progress, const char *who) {
     const bool noise = (opts->flags & RT_FLAG_NOISE) != 0;
-    if (noise && (opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS)))
-        return fail(RT_ERR_UNSUPPORTED, "rt_frame_begin: RT_FLAG_NOISE has no flow-schedule or counting kernel");
-    if ((rc = prepare_frame(scene, opts)) != RT_OK) return rc;
+    int rc = prepare_frame(scene, opts);
+    if (rc != RT_OK) return rc;
     auto *ds = static_cast<DeviceScene *>(scene->dev);
     RT_CUDA(cudaSetDevice(ds->device));
     auto *f = new RtFrame();
@@ -193,17 +197,31 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
         frame_free(f);
         return code;
     };
-    const size_t n = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
+    const size_t view_pixels = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
+    const size_t n = view_pixels * std::max<size_t>(1, views.size());
     f->n_pixels = n;
     bool ok = cudaMalloc((void **)&f->d_stats, n * 4 * sizeof(int32_t)) == cudaSuccess && cudaMalloc((void **)&f->d_flags, n) == cudaSuccess &&
               cudaMalloc((void **)&f->d_list, n * sizeof(uint32_t)) == cudaSuccess && cudaMalloc((void **)&f->d_rgb, n * 3) == cudaSuccess &&
               cudaMalloc((void **)&f->d_counters, CN_SLOTS * sizeof(unsigned long long)) == cudaSuccess;
     if (noise) ok = ok && cudaMalloc((void **)&f->d_sq, n * sizeof(unsigned long long)) == cudaSuccess;
+    if (!views.empty()) ok = ok && cudaMalloc((void **)&f->d_views, views.size() * sizeof(ViewCamera)) == cudaSuccess;
     ok = ok && f->ev.create();
-    if (!ok) return bail(fail(RT_ERR_CUDA, std::string("rt_frame_begin: allocation failed: ") + cudaGetErrorString(cudaGetLastError())));
+    if (!ok) return bail(fail(RT_ERR_CUDA, std::string(who) + ": allocation failed: " + cudaGetErrorString(cudaGetLastError())));
 
+    cudaStream_t st = ds->ws->stream;
     FrameParams &fp = f->fp;
-    fill_frame(fp, ds, *camera, max_w, max_h, *opts, 0, 1);
+    fill_frame(fp, ds, camera, max_w, max_h, *opts, 0, 1);
+    if (!views.empty()) {
+        // (from pageable memory: staged before the call returns; the probe below follows it on the stream)
+        if (cudaMemcpyAsync(f->d_views, views.data(), views.size() * sizeof(ViewCamera), cudaMemcpyHostToDevice, st) != cudaSuccess)
+            return bail(fail(RT_ERR_CUDA, std::string(who) + ": view table upload failed: " + cudaGetErrorString(cudaGetLastError())));
+        f->n_views = int32_t(views.size());
+        fp.cam.rows *= f->n_views; // the tall frame: probe tiles, flags, list, sums and Q run over it as over one frame
+        fp.tiles_y = (fp.cam.rows + kTileH - 1) / kTileH;
+        fp.views = f->d_views;
+        fp.n_views = f->n_views;
+        fp.view_pixels = int32_t(view_pixels);
+    }
     fp.stats = f->d_stats;
     fp.flags = f->d_flags;
     fp.list = f->d_list;
@@ -211,7 +229,6 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
     fp.sq = f->d_sq; // non-null: plan_launch picks the kernels that also sum the squares
     f->samples_done = fp.n_probe; // 0 without the early-out
     f->samples_target = fp.sample_end;
-    cudaStream_t st = ds->ws->stream;
     int launches = 0;
     // with its own counter block, the frame's probe keeps the raw "means differ" flags, also where this target has no main
     // phase: the frame can be extended
@@ -230,6 +247,75 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
     *out = f;
     frame_progress(f, progress);
     return RT_OK;
+}
+
+// rt_frame_view_noise reduces at most this many views per launch: the grid's y extent stays far below its limit (65535),
+// and the partials stay at most 16.8 MB however many views a batch of small extents has
+constexpr int32_t kNoiseViewChunk = 1024;
+
+// the noise reductions' partial summaries, kNoiseBlocks + 1 per view of one chunk of views, allocated on first use
+int ensure_partials(RtFrame *f) {
+    const size_t views = size_t(std::min(f->n_views, kNoiseViewChunk));
+    if (!f->d_partial) RT_CUDA(cudaMalloc((void **)&f->d_partial, views * (kNoiseBlocks + 1) * sizeof(NoisePartial)));
+    return RT_OK;
+}
+
+void fill_noise(const NoisePartial &total, double tolerance, RtFrameNoise *out) {
+    out->pixels = total.pixels;
+    out->pixels_above = total.above;
+    out->max_se = total.max_se;
+    out->mean_se = total.pixels ? total.sum_se / double(total.pixels) : 0.0;
+    out->tolerance = tolerance;
+}
+
+// the refusals of both openers, after their own argument checks
+int check_frame_mode(const RtRenderOpts *opts, const char *who) {
+    if (opts->mode == RT_MODE_WAVEFRONT) return fail(RT_ERR_UNSUPPORTED, std::string(who) + ": progressive frames run the megakernel only");
+    if (opts->mode != RT_MODE_MEGAKERNEL) return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": unknown mode");
+    return RT_OK;
+}
+
+} // namespace
+
+extern "C" {
+
+int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_t max_h, const RtRenderOpts *opts, RtFrame **out,
+                   RtFrameProgress *progress) {
+    int rc = check_frame_args(scene, camera, max_w, max_h, opts);
+    if (rc != RT_OK) return rc;
+    if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin: out is null");
+    *out = nullptr;
+    if ((rc = check_frame_mode(opts, "rt_frame_begin")) != RT_OK) return rc;
+    if ((opts->flags & RT_FLAG_NOISE) && (opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS)))
+        return fail(RT_ERR_UNSUPPORTED, "rt_frame_begin: RT_FLAG_NOISE has no flow-schedule or counting kernel");
+    return frame_open(scene, *camera, {}, max_w, max_h, opts, out, progress, "rt_frame_begin");
+}
+
+int rt_frame_begin_views(RtScene *scene, const RtCamera *cameras, const uint64_t *seeds, int32_t n_views, int32_t max_w, int32_t max_h,
+                         const RtRenderOpts *opts, RtFrame **out, RtFrameProgress *progress) {
+    // rt_render_views' checks, then rt_frame_begin's
+    if (n_views < 1) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin_views: n_views must be >= 1");
+    if (!cameras) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin_views: cameras is null");
+    int rc = check_frame_args(scene, &cameras[0], max_w, max_h, opts);
+    if (rc != RT_OK) return rc;
+    for (int32_t v = 1; v < n_views; ++v)
+        if (cameras[v].samples_per_pixel != cameras[0].samples_per_pixel || cameras[v].bounce_depth != cameras[0].bounce_depth)
+            return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin_views: every camera must have the same samples_per_pixel and bounce_depth");
+    if (size_t(2 * max_w + 1) * size_t(2 * max_h + 1) * size_t(n_views) >= (size_t(1) << 31))
+        return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin_views: n_views x rows x cols must be below 2^31");
+    if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin_views: out is null");
+    *out = nullptr;
+    if ((rc = check_frame_mode(opts, "rt_frame_begin_views")) != RT_OK) return rc;
+    if (opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS))
+        return fail(RT_ERR_UNSUPPORTED, "rt_frame_begin_views: a batch of views has no flow-schedule or counting kernel");
+    std::vector<ViewCamera> table(n_views);
+    for (int32_t v = 0; v < n_views; ++v) {
+        const uint64_t seed = seeds ? seeds[v] : opts->seed;
+        table[v].cam = make_dev_camera(cameras[v], max_w, max_h);
+        table[v].k0 = uint32_t(seed);
+        table[v].k1 = uint32_t(seed >> 32);
+    }
+    return frame_open(scene, cameras[0], table, max_w, max_h, opts, out, progress, "rt_frame_begin_views");
 }
 
 int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameProgress *progress) {
@@ -324,7 +410,8 @@ int rt_frame_noise(RtFrame *f, double tolerance, float *se_out, uint64_t *sq_out
     auto *ds = static_cast<DeviceScene *>(f->scene->dev);
     RT_CUDA(cudaSetDevice(ds->device));
     cudaStream_t st = ds->ws->stream;
-    if (!f->d_partial) RT_CUDA(cudaMalloc((void **)&f->d_partial, (kNoiseBlocks + 1) * sizeof(NoisePartial)));
+    int rc = ensure_partials(f);
+    if (rc != RT_OK) return rc;
     if (se_out && !f->d_se) RT_CUDA(cudaMalloc((void **)&f->d_se, f->n_pixels * sizeof(float)));
     noise_kernel<<<kNoiseBlocks, kNoiseThreads, 0, st>>>(reinterpret_cast<const int4 *>(f->d_stats), f->d_sq, f->d_flags, f->n_pixels, tolerance,
                                                          se_out ? f->d_se : nullptr, f->d_partial);
@@ -336,13 +423,36 @@ int rt_frame_noise(RtFrame *f, double tolerance, float *se_out, uint64_t *sq_out
     if (se_out) RT_CUDA(cudaMemcpyAsync(se_out, f->d_se, f->n_pixels * sizeof(float), cudaMemcpyDeviceToHost, st));
     if (sq_out) RT_CUDA(cudaMemcpyAsync(sq_out, f->d_sq, f->n_pixels * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
     RT_CUDA(cudaStreamSynchronize(st));
-    if (summary) {
-        summary->pixels = total.pixels;
-        summary->pixels_above = total.above;
-        summary->max_se = total.max_se;
-        summary->mean_se = total.pixels ? total.sum_se / double(total.pixels) : 0.0;
-        summary->tolerance = tolerance;
+    if (summary) fill_noise(total, tolerance, summary);
+    return RT_OK;
+}
+
+int rt_frame_view_noise(RtFrame *f, double tolerance, RtFrameNoise *per_view) {
+    if (!f || !per_view) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_view_noise: null frame or output");
+    if (!f->d_sq) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_view_noise: the frame was opened without RT_FLAG_NOISE");
+    if (!(tolerance >= 0.0)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_view_noise: tolerance must be >= 0");
+    auto *ds = static_cast<DeviceScene *>(f->scene->dev);
+    RT_CUDA(cudaSetDevice(ds->device));
+    cudaStream_t st = ds->ws->stream;
+    int rc = ensure_partials(f);
+    if (rc != RT_OK) return rc;
+    // every view reduced as rt_frame_noise reduces a frame of its pixels: the same 512 ranges, tree and block order
+    const size_t view_pixels = f->n_pixels / size_t(f->n_views);
+    std::vector<NoisePartial> totals(size_t(f->n_views));
+    for (int32_t v0 = 0; v0 < f->n_views; v0 += kNoiseViewChunk) {
+        const int32_t nv = std::min(kNoiseViewChunk, f->n_views - v0);
+        const size_t at = size_t(v0) * view_pixels;
+        noise_kernel<<<dim3(kNoiseBlocks, unsigned(nv)), kNoiseThreads, 0, st>>>(reinterpret_cast<const int4 *>(f->d_stats) + at, f->d_sq + at,
+                                                                                  f->d_flags + at, view_pixels, tolerance, nullptr, f->d_partial);
+        RT_CUDA(cudaGetLastError());
+        noise_summary_kernel<<<unsigned(nv), kNoiseThreads, 0, st>>>(f->d_partial);
+        RT_CUDA(cudaGetLastError());
+        // (the next chunk's kernels follow this copy on the stream before they overwrite the partials)
+        RT_CUDA(cudaMemcpy2DAsync(totals.data() + v0, sizeof(NoisePartial), f->d_partial + kNoiseBlocks, (kNoiseBlocks + 1) * sizeof(NoisePartial),
+                                  sizeof(NoisePartial), size_t(nv), cudaMemcpyDeviceToHost, st));
     }
+    RT_CUDA(cudaStreamSynchronize(st));
+    for (int32_t v = 0; v < f->n_views; ++v) fill_noise(totals[size_t(v)], tolerance, per_view + v);
     return RT_OK;
 }
 

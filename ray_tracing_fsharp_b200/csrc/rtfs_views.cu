@@ -51,14 +51,26 @@ __global__ void __launch_bounds__(block_threads(SMEM), blocks_per_sm(SMEM)) rend
     render_items<PROBE, SMEM, false, SSTACK, WIDE, false>(fp, ViewPixels{fp});
 }
 
-template <bool PROBE>
-static RenderKernelFn pick_views(bool smem, bool lean, bool sstack, bool wide) {
-    if (smem) return lean ? render_views_kernel<PROBE, 2, false, false> : render_views_kernel<PROBE, 1, false, false>;
-    if (wide) return sstack ? render_views_kernel<PROBE, 0, true, true> : render_views_kernel<PROBE, 0, false, true>;
-    return sstack ? render_views_kernel<PROBE, 0, true, false> : render_views_kernel<PROBE, 0, false, false>;
+// The same twelve shapes that also sum r^2 + g^2 + b^2 per pixel into fp.sq, as render_kernel<..., NOISE = true>: the
+// progressive frames of a batch opened with RT_FLAG_NOISE (rt_frame_begin_views).  A kernel of its own rather than a
+// parameter of render_views_kernel, whose twelve instantiations stay what they are.
+template <bool PROBE, int SMEM, bool SSTACK, bool WIDE>
+__global__ void __launch_bounds__(block_threads(SMEM), blocks_per_sm(SMEM)) render_views_noise_kernel(const FrameParams fp) {
+    render_items<PROBE, SMEM, false, SSTACK, WIDE, true>(fp, ViewPixels{fp});
 }
-RenderKernelFn pick_views_kernel(bool probe, bool smem, bool lean, bool sstack, bool wide) {
-    return probe ? pick_views<true>(smem, lean, sstack, wide) : pick_views<false>(smem, lean, sstack, wide);
+
+template <bool PROBE, int SMEM, bool SSTACK, bool WIDE>
+static RenderKernelFn pick_noise(bool noise) {
+    return noise ? render_views_noise_kernel<PROBE, SMEM, SSTACK, WIDE> : render_views_kernel<PROBE, SMEM, SSTACK, WIDE>;
+}
+template <bool PROBE>
+static RenderKernelFn pick_views(bool smem, bool lean, bool sstack, bool wide, bool noise) {
+    if (smem) return lean ? pick_noise<PROBE, 2, false, false>(noise) : pick_noise<PROBE, 1, false, false>(noise);
+    if (wide) return sstack ? pick_noise<PROBE, 0, true, true>(noise) : pick_noise<PROBE, 0, false, true>(noise);
+    return sstack ? pick_noise<PROBE, 0, true, false>(noise) : pick_noise<PROBE, 0, false, false>(noise);
+}
+RenderKernelFn pick_views_kernel(bool probe, bool smem, bool lean, bool sstack, bool wide, bool noise) {
+    return probe ? pick_views<true>(smem, lean, sstack, wide, noise) : pick_views<false>(smem, lean, sstack, wide, noise);
 }
 
 // grow-only, like the frame buffers

@@ -58,6 +58,9 @@ def _declare(lib):
         "rt_frame_noise": (C.c_int, [_vp, C.c_double, _vp, _vp, C.POINTER(RtFrameNoise)]),
         "rt_frame_set_convergence": (C.c_int, [_vp, C.c_double, _i32, _i32]),
         "rt_frame_convergence": (C.c_int, [_vp, C.POINTER(RtFrameConvergence)]),
+        "rt_frame_begin_views": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(RtRenderOpts), C.POINTER(_vp),
+                                           C.POINTER(RtFrameProgress)]),
+        "rt_frame_view_noise": (C.c_int, [_vp, C.c_double, _vp]),
         "rt_pixel_noise": (C.c_int, [_vp, _vp, C.c_size_t, _vp]),
         "rt_render_multi": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i32, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _vp,
                                       _vp, C.POINTER(RtStats)]),
@@ -272,6 +275,28 @@ class SceneHandle:
         """A progressive frame of this scene (rt_frame_begin: runs the probe).  See Frame."""
         return Frame(self, camera, max_w, max_h, seed, adaptive, flags, mode)
 
+    def open_frame_views(self, cameras, max_w, max_h, seeds=None, seed=0, adaptive=True, flags=0):
+        """A progressive frame of a batch of views of this scene (rt_frame_begin_views: runs the probe), cameras and seeds as
+        render_views.  A Frame whose read, noise and sums have shape [n_views, rows, cols, ...]; view v is exactly
+        open_frame(cameras[v], max_w, max_h, seed=seeds[v]) at the same samples_done, and Frame.view_noise summarises
+        each view.  RtError RT_ERR_INVALID_ARGUMENT for an empty batch."""
+        n = len(cameras)
+        cams = (RtCamera * max(1, n))(*cameras)
+        sd = None
+        if seeds is not None:
+            if len(seeds) != n:
+                raise ValueError(f"{len(seeds)} seeds for {n} cameras")
+            sd = np.ascontiguousarray([int(x) for x in seeds], np.uint64)
+        opts = RtRenderOpts(seed, int(adaptive), abi.RT_MODE_MEGAKERNEL, 0, flags)
+        out = C.c_void_p()
+        progress = RtFrameProgress()
+        check(lib().rt_frame_begin_views(self.ptr, cams, ptr(sd), n, max_w, max_h, C.byref(opts), C.byref(out), C.byref(progress)))
+        frame = Frame.__new__(Frame)
+        frame.scene, frame.ptr, frame.progress = self, out, progress
+        frame.rows, frame.cols = 2 * max_h + 1, 2 * max_w + 1
+        frame.n_views = n
+        return frame
+
     # ---- conformance ----
     def hit_object(self, o, d, traversal=0):
         o, d = f64(o, (-1, 3)), f64(d, (-1, 3))
@@ -317,7 +342,13 @@ class SceneHandle:
 class Frame:
     """Owner of an RtFrame* (rt_frame_begin / rt_frame_destroy): rt_render's frame advanced in passes over windows of
     sample indices.  After every pass the frame is exactly rt_render's at samples_per_pixel = progress.samples_done.
-    Holds its scene handle, so the scene outlives it."""
+    Holds its scene handle, so the scene outlives it.  A frame of a batch of views (SceneHandle.open_frame_views) has
+    n_views set, and its images, sums and maps carry a leading view axis."""
+
+    n_views = None  # a frame of one camera
+
+    def _shape(self, *tail):
+        return ((self.n_views,) if self.n_views is not None else ()) + (self.rows, self.cols) + tail
 
     def __init__(self, scene: SceneHandle, camera, max_w, max_h, seed=0, adaptive=True, flags=0, mode=abi.RT_MODE_MEGAKERNEL):
         self.scene = scene
@@ -338,8 +369,8 @@ class Frame:
 
     def read(self, gamma=False, want_sums=False, rgb_out=None):
         """The current image (uint8 [rows, cols, 3]) and, with want_sums, the int32 sums [rows, cols, 4]."""
-        rgb = rgb_out if rgb_out is not None else _frame_buffer((self.rows, self.cols, 3))
-        sums = np.empty((self.rows, self.cols, 4), np.int32) if want_sums else None
+        rgb = rgb_out if rgb_out is not None else _frame_buffer(self._shape(3))
+        sums = np.empty(self._shape(4), np.int32) if want_sums else None
         check(lib().rt_frame_read(self.ptr, int(gamma), ptr(rgb), ptr(sums)))
         return rgb, sums
 
@@ -353,10 +384,18 @@ class Frame:
         flagged pixels against `tolerance`, the per-pixel standard error float32 [rows, cols] or None, the per-pixel sum of
         r^2 + g^2 + b^2 uint64 [rows, cols] or None)."""
         summary = RtFrameNoise()
-        se = np.empty((self.rows, self.cols), np.float32) if want_map else None
-        sq = np.empty((self.rows, self.cols), np.uint64) if want_sq else None
+        se = np.empty(self._shape(), np.float32) if want_map else None
+        sq = np.empty(self._shape(), np.uint64) if want_sq else None
         check(lib().rt_frame_noise(self.ptr, float(tolerance), ptr(se), ptr(sq), C.byref(summary)))
         return summary, se, sq
+
+    def view_noise(self, tolerance):
+        """One RtFrameNoise per view (rt_frame_view_noise; one for a frame of one camera): view v's summary over its pixels
+        still being sampled, bit for bit noise(tolerance)[0] of the frame of camera v alone.  pixels == 0: the view is
+        finished."""
+        out = (RtFrameNoise * (self.n_views or 1))()
+        check(lib().rt_frame_view_noise(self.ptr, float(tolerance), out))
+        return list(out)
 
     def set_convergence(self, tolerance, min_samples=64, interval=64):
         """Stops sampling each pixel once its noise estimate is within `tolerance` (8-bit levels), checked at the sample

@@ -8,6 +8,7 @@ reference's.  Everything that computes goes through the C ABI (native.py); nothi
   Scene.render          RayTracing/Scene.fs:196-236
   Scene.render_views    Scene.render of many cameras of one scene in one submission (rt_render_views)
   Scene.render_progressive  the same frame in sample passes, progress ticks as passes finish (native.Frame)
+  Scene.render_views_progressive  Scene.render_views in sample passes, as one progressive frame of the batch
   Image / Image.render  RayTracing/Domain.fs:9-31
   ImageOutput.write_ppm RayTracing/ImageOutput.fs:163-197, PixelOutput.correct :11-18
 """
@@ -222,6 +223,51 @@ class Scene:
             rgb, _ = frame.read()
         emit(ticks.finish())  # the last pass's share, or the rest of the frame when on_pass stopped it
         return rgb
+
+    @staticmethod
+    def render_views_progressive(progress_increment: Callable[[float], None], print_fn: Callable[[str], None], max_width_coord: int,
+                                 max_height_coord: int, cameras: Sequence[abi.RtCamera], s: "Scene", seeds: Optional[Sequence[int]] = None,
+                                 seed: Optional[int] = None, adaptive: bool = True, target_ms: float = 250.0,
+                                 on_pass: Optional[Callable[[abi.RtFrameProgress, "native.Frame"], object]] = None, flags: int = 0,
+                                 converge_tolerance: Optional[float] = None, converge_min_samples: int = 64,
+                                 converge_interval: int = 64) -> List[np.ndarray]:
+        """render_progressive for every camera of `cameras` (same samples_per_pixel and bounce_depth), as one progressive frame
+        of the batch (native.SceneHandle.open_frame_views): each pass of about `target_ms` of device time advances every view.
+        The progress ticks total rows * len(cameras), spread over the paths traced as in render_progressive.  `on_pass(progress,
+        frame)` after every pass may read the views (`frame.read()`, [n, rows, cols, 3]) and stops the batch by returning True.
+        `seeds`: one RNG key per view; otherwise `seed` (None: one drawn from the OS) for every view.  With
+        `converge_tolerance` every pixel of every view stops once its standard error is within it, checked at
+        converge_min_samples + j * converge_interval samples (Frame.set_convergence).  Returns one uint8 [rows, cols, 3] image
+        per view (before gamma): with the same camera and seed, view v is render_progressive's image of camera v with the same
+        rule, or, stopped early, that of the samples done.  `print_fn` is ignored."""
+        if not isinstance(s._handle, native.SceneHandle):
+            raise NotImplementedError("progressive frames run on one GPU: make the scene with a single device")
+        rows, n = 2 * max_height_coord + 1, len(cameras)
+        if seed is None and seeds is None:
+            seed = secrets.randbits(64)
+        ticks = ProgressTicks(rows * n)
+
+        def emit(k):
+            for _ in range(k):
+                progress_increment(1.0)
+
+        if converge_tolerance is not None:
+            flags |= abi.RT_FLAG_NOISE
+        with s._handle.open_frame_views(list(cameras), max_width_coord, max_height_coord, seeds=seeds, seed=seed or 0, adaptive=adaptive,
+                                        flags=flags) as frame:
+            if converge_tolerance is not None:
+                frame.set_convergence(converge_tolerance, converge_min_samples, converge_interval)
+            progress = frame.progress
+            emit(ticks.update(progress.paths_done, progress.paths_target))  # the probe
+            while not progress.done:
+                progress = frame.advance(target_ms=target_ms)
+                if not progress.done:
+                    emit(ticks.update(progress.paths_done, progress.paths_target))
+                if on_pass is not None and on_pass(progress, frame):
+                    break
+            rgb, _ = frame.read()
+        emit(ticks.finish())
+        return [rgb[v] for v in range(n)]
 
 
 class ProgressTicks:

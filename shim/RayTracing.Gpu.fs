@@ -187,6 +187,13 @@ module internal Native =
     [<DllImport(Lib)>]
     extern int rt_frame_convergence (nativeint frame, RtFrameConvergence& out)
 
+    // progressive frames of a batch of views (include/rtfs_b200.h, rt_frame_begin_views; ABI 6 still: detect by the symbol)
+    [<DllImport(Lib)>]
+    extern int rt_frame_begin_views (nativeint scene, RtCamera[] cameras, uint64[] seeds, int nViews, int maxWidthCoord, int maxHeightCoord, RtRenderOpts& opts, nativeint& frame, RtFrameProgress& progress)
+
+    [<DllImport(Lib)>]
+    extern int rt_frame_view_noise (nativeint frame, float tolerance, [<Out>] RtFrameNoise[] perView)
+
     [<DllImport(Lib)>]
     extern int rt_pixel_noise (int[] sums, uint64[] sq, unativeint n, float32[] seOut)
 
@@ -514,13 +521,24 @@ type FrameConvergence =
 /// A frame in progress on a single-device GpuScene (rt_frame_*): advanced in passes over windows of sample indices.
 /// After every pass it is exactly the frame rt_render gives at `SamplesDone` samples per pixel with the same seed, so
 /// `Read` shows the image sharpening; a caller stops early by not advancing any more, and `Extend` continues a finished
-/// frame to more samples.  Dispose it before its scene.
-type GpuFrame internal (handle : nativeint, rows : int, cols : int, first : Native.RtFrameProgress) =
+/// frame to more samples.  Dispose it before its scene.  A frame of a batch of views (SceneGpu.openFrameViews) holds `Views`
+/// images of Rows * Cols pixels one after the other; the progress and convergence counts are sums over them.
+type GpuFrame internal (handle : nativeint, rows : int, cols : int, views : int, first : Native.RtFrameProgress) =
     let mutable handle = handle
     let mutable progress = first
 
+    let noise (s : Native.RtFrameNoise) : FrameNoise =
+        {
+            Pixels = s.pixels
+            PixelsAbove = s.pixelsAbove
+            MaxSe = s.maxSe
+            MeanSe = s.meanSe
+            Tolerance = s.tolerance
+        }
+
     member _.Rows = rows
     member _.Cols = cols
+    member _.Views = views
     member _.SamplesDone = progress.samplesDone
     member _.SamplesTarget = progress.samplesTarget
     /// traceOnce calls so far, and in the whole frame (exact from the start)
@@ -537,9 +555,9 @@ type GpuFrame internal (handle : nativeint, rows : int, cols : int, first : Nati
         Native.rt_frame_advance (handle, maxSamples, targetMs, &p) |> Native.check
         progress <- p
 
-    /// The current image as row-major RGB8, 3 * Rows * Cols bytes (PixelOutput.correct applied when `gamma`).
+    /// The current image as row-major RGB8, 3 * Rows * Cols bytes per view (PixelOutput.correct applied when `gamma`).
     member _.Read (gamma : bool) : byte[] =
-        let rgb = Array.zeroCreate<byte> (3 * rows * cols)
+        let rgb = Array.zeroCreate<byte> (3 * views * rows * cols)
         Native.rt_frame_read (handle, (if gamma then 1 else 0), rgb, 0n) |> Native.check
         rgb
 
@@ -550,20 +568,19 @@ type GpuFrame internal (handle : nativeint, rows : int, cols : int, first : Nati
 
     /// The noise estimate of a frame opened with FrameFlags.Noise (rt_frame_noise): the summary over the pixels later
     /// passes still sample, against `tolerance` (8-bit levels), and with `wantMap` the standard error of every pixel,
-    /// row-major Rows * Cols (null otherwise).
+    /// row-major Rows * Cols per view (null otherwise).
     member _.Noise (tolerance : float, wantMap : bool) : FrameNoise * float32[] =
-        let map = if wantMap then Array.zeroCreate<float32> (rows * cols) else null
+        let map = if wantMap then Array.zeroCreate<float32> (views * rows * cols) else null
         let mutable summary = Native.RtFrameNoise ()
         Native.rt_frame_noise (handle, tolerance, map, null, &summary) |> Native.check
+        noise summary, map
 
-        {
-            Pixels = summary.pixels
-            PixelsAbove = summary.pixelsAbove
-            MaxSe = summary.maxSe
-            MeanSe = summary.meanSe
-            Tolerance = summary.tolerance
-        },
-        map
+    /// One summary per view (rt_frame_view_noise): view v's pixels still being sampled, exactly `Noise`'s summary of the
+    /// frame of that view alone.  Pixels = 0: the view is finished.
+    member _.ViewNoise (tolerance : float) : FrameNoise[] =
+        let out = Array.zeroCreate<Native.RtFrameNoise> views
+        Native.rt_frame_view_noise (handle, tolerance, out) |> Native.check
+        out |> Array.map noise
 
     /// Stops sampling each pixel once its standard error is within `tolerance` (8-bit levels), checked at the sample
     /// counts minSamples + j * interval (rt_frame_set_convergence).  Only on a frame opened with FrameFlags.Noise, before
@@ -765,11 +782,33 @@ module SceneGpu =
         Native.rt_frame_begin (s.Handle, &cam, maxWidthCoord, maxHeightCoord, &opts, &handle, &progress)
         |> Native.check
 
-        new GpuFrame (handle, 2 * maxHeightCoord + 1, 2 * maxWidthCoord + 1, progress)
+        new GpuFrame (handle, 2 * maxHeightCoord + 1, 2 * maxWidthCoord + 1, 1, progress)
 
     /// Opens a progressive frame (rt_frame_begin: the probe runs now).  Single-device scenes only.
     let openFrame (maxWidthCoord : int) (maxHeightCoord : int) (camera : Camera) (seed : uint64) (s : GpuScene) : GpuFrame =
         openFrameWith 0 maxWidthCoord maxHeightCoord camera seed s
+
+    /// Opens a progressive frame of a batch of views (rt_frame_begin_views: the probe of every view runs now) with
+    /// RtRenderOpts.flags `flags`: `cameras` with the same SamplesPerPixel and BounceDepth, one seed per view.  View v is
+    /// exactly the frame openFrameWith gives for cameras.[v] and seeds.[v].  Single-device scenes only.
+    let openFrameViews (flags : int) (maxWidthCoord : int) (maxHeightCoord : int) (cameras : Camera array) (seeds : uint64 array) (s : GpuScene) : GpuFrame =
+        if s.IsMulti then
+            failwith "GPU backend: progressive frames run on a single-device GpuScene"
+
+        if seeds.Length <> cameras.Length then
+            invalidArg "seeds" "one seed per camera"
+
+        let cams = cameras |> Array.map marshalCamera
+        let mutable opts = Native.RtRenderOpts ()
+        opts.adaptive <- 1
+        opts.flags <- flags
+        let mutable handle = 0n
+        let mutable progress = Native.RtFrameProgress ()
+
+        Native.rt_frame_begin_views (s.Handle, cams, seeds, cams.Length, maxWidthCoord, maxHeightCoord, &opts, &handle, &progress)
+        |> Native.check
+
+        new GpuFrame (handle, 2 * maxHeightCoord + 1, 2 * maxWidthCoord + 1, cameras.Length, progress)
 
     // the frame of renderWithProgressUntil and renderConverging: passes of about 250 ms with progress ticks, an optional
     // convergence rule (tolerance, minSamples, interval) and an optional stop on the noise summary (tolerance, fraction)
@@ -903,3 +942,78 @@ module SceneGpu =
         : float<progress> * Image
         =
         renderWithProgressUntil None progressIncrement print maxWidthCoord maxHeightCoord camera s
+
+    /// `renderViews` traced as one converging progressive frame of the batch (openFrameViews): passes of about 250 ms of
+    /// device time advance every view, and each pixel stops being sampled once its standard error of the mean is within
+    /// `tolerance` (8-bit levels), checked at minSamples + j * interval samples.  View v is exactly `renderConverging`'s
+    /// image of cameras.[v] with the same seed and rule; a batch pays each pass's fixed cost once instead of once per view.
+    /// rows * cameras.Length progress calls in all, as passes finish.  One fresh seed per view.
+    let renderViewsConverging
+        (tolerance : float, minSamples : int, interval : int)
+        (progressIncrement : float<progress> -> unit)
+        (_print : string -> unit)
+        (maxWidthCoord : int)
+        (maxHeightCoord : int)
+        (cameras : Camera array)
+        (s : GpuScene)
+        : float<progress> * Image array
+        =
+        let rowsIter = 2 * maxHeightCoord + 1
+        let colsIter = 2 * maxWidthCoord + 1
+        let n = cameras.Length
+        let total = rowsIter * n
+
+        let frames =
+            lazy
+                (let seeds = Array.init n (fun _ -> uint64 (Random().NextInt64 ()))
+                 use f = openFrameViews FrameFlags.Noise maxWidthCoord maxHeightCoord cameras seeds s
+                 f.SetConvergence (tolerance, minSamples, interval)
+                 let ticked = ref 0
+
+                 let tick () =
+                     let want =
+                         if f.IsDone || f.PathsTarget = 0UL then
+                             total
+                         else
+                             min total (int (float total * float f.PathsDone / float f.PathsTarget))
+
+                     for _ in ticked.Value + 1 .. want do
+                         progressIncrement 1.0<progress>
+
+                     ticked.Value <- max ticked.Value want
+
+                 tick ()
+
+                 while not f.IsDone do
+                     f.Advance (0, 250.0)
+                     tick ()
+
+                 f.Read false)
+
+        let image (view : int) =
+            let rows =
+                Seq.init
+                    rowsIter
+                    (fun row ->
+                        async {
+                            let rgb = frames.Force ()
+                            let start = 3 * ((view * rowsIter + row) * colsIter)
+
+                            return
+                                Array.init
+                                    colsIter
+                                    (fun col ->
+                                        let i = start + 3 * col
+
+                                        {
+                                            Red = rgb.[i]
+                                            Green = rgb.[i + 1]
+                                            Blue = rgb.[i + 2]
+                                        }
+                                    )
+                        }
+                    )
+
+            Image.make rowsIter colsIter rows
+
+        1.0<progress> * float total, Array.init n image

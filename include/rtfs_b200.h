@@ -403,6 +403,43 @@ int rt_frame_begin_views(RtScene *scene, const RtCamera *cameras, const uint64_t
                          RtFrame **out, RtFrameProgress *progress);
 int rt_frame_view_noise(RtFrame *frame, double tolerance, RtFrameNoise *per_view /* n_views entries */);
 
+/* ---- a window of a frame (host buffers; one GPU) ------------------------------------------------- */
+/* Any rectangle of rt_render's frame, bit for bit, without tracing the rest: a closer look at one part of the image (a
+ * caustic, a reflection) at the frame's own camera, or a tile of a frame rendered by several processes, which assemble
+ * into the frame with nothing to blend at the seams.
+ *
+ * These two functions were added without a change of RT_ABI_VERSION (still 6): no struct and no existing prototype
+ * changed.  A caller detects the feature by the presence of the symbol rt_render_window.
+ *
+ * The window is [row0, row0 + rows) x [col0, col0 + cols), rows and cols counted as rt_render's output (row 0 = top row;
+ * the frame is (2 max_h + 1) x (2 max_w + 1)).  rgb_out rows*cols*3, sums_out (optional) rows*cols*4 int32, row-major over
+ * the window.
+ * Exactness.  Every sample is keyed by (seed, frame pixel, sample index), a path depends only on that key and the camera's
+ *   full extents, and the sums are integers; the probe's flag of a pixel depends only on its own samples.  So window pixel
+ *   (r, c) is bit for bit pixel (row0 + r, col0 + c) of rt_render(scene, camera, max_w, max_h, opts): sums, RGB8 and gamma
+ *   RGB8, whatever the window, and tiles of any grid reassemble into rt_render's frame.
+ * Argument errors (RT_ERR_INVALID_ARGUMENT): rows < 1 or cols < 1; row0 < 0 or col0 < 0; row0 + rows > 2 max_h + 1 or
+ *   col0 + cols > 2 max_w + 1; rgb_out (or out) NULL; and those of rt_render.
+ * Options.  RT_MODE_WAVEFRONT, RT_FLAG_FLOW and RT_FLAG_COUNTERS: RT_ERR_UNSUPPORTED (no window wavefront, flow-schedule or
+ *   counting kernels).  RT_FLAG_NO_SMEM, RT_FLAG_WIDE_BVH, RT_FLAG_BVH2, RT_FLAG_NO_LEAN, RT_FLAG_LOCKSTEP, adaptive and
+ *   gamma act as in rt_render; RT_FLAG_NOISE acts as in rt_frame_begin, and rt_render_window ignores it.
+ * Stats (optional): the window's own paths, rays, degenerate_paths and pixels_early_out (of its pixels); the _ms fields and
+ *   launches describe the call; box_tests and prim_tests are 0.  A window that is the whole frame is rt_render in every
+ *   output, stats included.
+ * Like rt_render, the call returns with its device work complete. */
+int rt_render_window(RtScene *scene, const RtCamera *camera, int32_t max_width_coord, int32_t max_height_coord,
+                     int32_t row0, int32_t col0, int32_t rows, int32_t cols, const RtRenderOpts *opts,
+                     uint8_t *rgb_out, int32_t *sums_out, RtStats *stats);
+/* A progressive frame over that window: an ordinary RtFrame (rt_frame_advance, _read, _extend, _noise, _view_noise,
+ * _set_convergence, _convergence and _destroy take it unchanged; read and the noise maps are rows*cols, and
+ * rt_frame_view_noise gives one entry).  The counts of RtFrameProgress and RtFrameConvergence cover the window's pixels.
+ * Arguments and modes as rt_render_window.  After any pass, and under a convergence rule, window pixel (r, c) is bit for
+ * bit pixel (row0 + r, col0 + c) of rt_frame_begin's frame of the same camera, extents, opts and rule: sums, counts, Q and
+ * the E map (each pixel's stopping count depends only on its own samples and the checkpoint lattice). */
+int rt_frame_begin_window(RtScene *scene, const RtCamera *camera, int32_t max_width_coord, int32_t max_height_coord,
+                          int32_t row0, int32_t col0, int32_t rows, int32_t cols, const RtRenderOpts *opts,
+                          RtFrame **out, RtFrameProgress *progress);
+
 /* The same frame split over the GPUs of this process (the F# host is one process): replicated scene,
  * sample-index split (Scene.fs:191-192 shared out by sample index), probe tiles shared out by tile.
  * The devices exchange flags and sums through NVLink peer memory inside the kernels that consume them

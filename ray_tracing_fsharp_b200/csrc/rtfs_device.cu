@@ -451,6 +451,9 @@ static int plan_launch(DeviceScene *ds, FrameParams &fp, bool probe, LaunchPlan 
     // of squares
     const bool views = fp.views != nullptr;
     if (views && (flow || count)) return fail(RT_ERR_UNSUPPORTED, "render: a batch of views has no flow-schedule or counting kernel");
+    // a window of one frame (rt_render_window, rt_frame_begin_window): the same kernels as a batch, over the window's pixels
+    const bool window = fp.window != 0;
+    if (window && (flow || count)) return fail(RT_ERR_UNSUPPORTED, "render: a window has no flow-schedule or counting kernel");
     const size_t nodes_q = size_t(ds->g.n_nodes) * kStagedNodeQuads, sph_q = size_t(ds->g.n_bounded);
     const size_t scene_q = staged_scene_quads(ds);
     bool smem = scene_staged(ds, flow ? sizeof(FlowWarp) : warp_scratch_bytes(true, noise));
@@ -485,15 +488,18 @@ static int plan_launch(DeviceScene *ds, FrameParams &fp, bool probe, LaunchPlan 
     plan.smem_bytes = (used_q + (sstack ? stack_q : 0)) * 16;
     const bool lean = ds->lean && !(fp.opt_flags & RT_FLAG_NO_LEAN);
     if (views) fn = pick_views_kernel(probe, smem, lean, sstack, wide, noise);
+    else if (window) fn = pick_window_kernel(probe, smem, lean, sstack, wide, noise);
     else fn = flow ? (probe ? pick_flow<true>(smem, count) : pick_flow<false>(smem, count)) : pick_kernel(probe, smem, lean, count, sstack, wide, noise);
     {
         static const bool show = std::getenv("RTFS_DEBUG_PLAN") != nullptr;
         if (show) {
             char views_field[24] = ""; // a batch of views adds its size to the line
             if (views) std::snprintf(views_field, sizeof views_field, " views=%d", fp.n_views);
-            std::fprintf(stderr, "rtfs: plan probe=%d staged=%d lean=%d count=%d sstack=%d wide=%d flow=%d noise=%d smem_bytes=%zu threads=%d%s\n",
+            char window_field[64] = ""; // a window adds its size and offset
+            if (window) std::snprintf(window_field, sizeof window_field, " window=%dx%d@%d,%d", fp.cam.rows, fp.cam.cols, fp.win_row0, fp.win_col0);
+            std::fprintf(stderr, "rtfs: plan probe=%d staged=%d lean=%d count=%d sstack=%d wide=%d flow=%d noise=%d smem_bytes=%zu threads=%d%s%s\n",
                          int(probe), int(smem), int(smem && lean), int(count), int(sstack), int(wide), int(flow), int(noise), plan.smem_bytes,
-                         plan.threads, views_field);
+                         plan.threads, views_field, window_field);
         }
     }
     { // The dynamic shared-memory limit of a kernel is a per-function, per-device setting: it is only ever RAISED here

@@ -196,7 +196,21 @@ struct FrameParams {
     const ViewCamera *views;
     int32_t n_views;
     int32_t view_pixels;
+    // a window of rt_render's frame (rt_render_window, rt_frame_begin_window: rtfs_window.cu): cam.rows x cam.cols are the
+    // window's, at row win_row0 and column win_col0 of the (2 max_h + 1) x (2 max_w + 1) frame; window = 0 otherwise, and
+    // then the kernels of one frame run
+    int32_t window;
+    int32_t win_row0, win_col0;
 };
+
+// a window of rt_render's frame: rows x cols pixels from (row0, col0), counted as rt_render's output (row 0 = top row)
+struct FrameWindow {
+    int32_t row0, col0, rows, cols;
+};
+// RT_ERR_INVALID_ARGUMENT unless the window is non-empty and lies inside the (2 max_h + 1) x (2 max_w + 1) frame
+int check_window(const FrameWindow &w, int max_w, int max_h, const char *who);
+// narrows a frame filled by fill_frame to the window: probe tiles, flags, list, sums and the output tail run over its pixels
+void set_window(FrameParams &fp, const FrameWindow &w);
 
 
 constexpr int kMaxDevices = 16;
@@ -233,6 +247,8 @@ int launch_samples(DeviceScene *ds, FrameParams fp, cudaStream_t st, int *launch
 // the kernel that also sums the squares (progressive frames of a batch opened with RT_FLAG_NOISE)
 typedef void (*RenderKernelFn)(const FrameParams);
 RenderKernelFn pick_views_kernel(bool probe, bool smem, bool lean, bool sstack, bool wide, bool noise);
+// the same choice among the kernels of a window of one frame (rtfs_window.cu)
+RenderKernelFn pick_window_kernel(bool probe, bool smem, bool lean, bool sstack, bool wide, bool noise);
 // PixelStats.mean + the optional gamma of a whole frame: sums -> RGB8
 int launch_finalize(const int32_t *stats, size_t n_pixels, int gamma, uint8_t *rgb, cudaStream_t st, int *launches);
 

@@ -9,6 +9,8 @@
 // rt_frame_begin_views opens the same frame over rt_render_views' tall frame of a batch of views (its kernels are in
 // rtfs_views.cu); the probe flags, the compaction, the checks and the output tail work per pixel and need no change for it,
 // and rt_frame_view_noise reduces each view as rt_frame_noise reduces a frame of its own.
+// rt_frame_begin_window opens it over a window of rt_render's frame (its kernels are in rtfs_window.cu): the frame's buffers,
+// maps and counts are the window's, and every per-pixel kernel runs over the window unchanged.
 #include "rtfs_device.h"
 
 #include <algorithm>
@@ -182,10 +184,11 @@ void frame_progress(const RtFrame *f, RtFrameProgress *p) {
     p->done = f->samples_done == f->samples_target ? 1 : 0;
 }
 
-// rt_frame_begin (views empty) and rt_frame_begin_views, once their arguments are checked: allocates the frame, and runs
-// the probe and the compaction.  A batch's frame is the tall frame of rt_render_views (rtfs_views.cu) with its own table.
-int frame_open(RtScene *scene, const RtCamera &camera, const std::vector<ViewCamera> &views, int32_t max_w, int32_t max_h,
-               const RtRenderOpts *opts, RtFrame **out, RtFrameProgress *progress, const char *who) {
+// rt_frame_begin (views empty, no window), rt_frame_begin_views and rt_frame_begin_window, once their arguments are checked:
+// allocates the frame, and runs the probe and the compaction.  A batch's frame is the tall frame of rt_render_views
+// (rtfs_views.cu) with its own table; a window's frame holds the window's pixels only (rtfs_window.cu).
+int frame_open(RtScene *scene, const RtCamera &camera, const std::vector<ViewCamera> &views, const FrameWindow *window, int32_t max_w,
+               int32_t max_h, const RtRenderOpts *opts, RtFrame **out, RtFrameProgress *progress, const char *who) {
     const bool noise = (opts->flags & RT_FLAG_NOISE) != 0;
     int rc = prepare_frame(scene, opts);
     if (rc != RT_OK) return rc;
@@ -198,7 +201,7 @@ int frame_open(RtScene *scene, const RtCamera &camera, const std::vector<ViewCam
         return code;
     };
     const size_t view_pixels = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
-    const size_t n = view_pixels * std::max<size_t>(1, views.size());
+    const size_t n = window ? size_t(window->rows) * size_t(window->cols) : view_pixels * std::max<size_t>(1, views.size());
     f->n_pixels = n;
     bool ok = cudaMalloc((void **)&f->d_stats, n * 4 * sizeof(int32_t)) == cudaSuccess && cudaMalloc((void **)&f->d_flags, n) == cudaSuccess &&
               cudaMalloc((void **)&f->d_list, n * sizeof(uint32_t)) == cudaSuccess && cudaMalloc((void **)&f->d_rgb, n * 3) == cudaSuccess &&
@@ -222,6 +225,7 @@ int frame_open(RtScene *scene, const RtCamera &camera, const std::vector<ViewCam
         fp.n_views = f->n_views;
         fp.view_pixels = int32_t(view_pixels);
     }
+    if (window) set_window(fp, *window);
     fp.stats = f->d_stats;
     fp.flags = f->d_flags;
     fp.list = f->d_list;
@@ -288,7 +292,7 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
     if ((rc = check_frame_mode(opts, "rt_frame_begin")) != RT_OK) return rc;
     if ((opts->flags & RT_FLAG_NOISE) && (opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS)))
         return fail(RT_ERR_UNSUPPORTED, "rt_frame_begin: RT_FLAG_NOISE has no flow-schedule or counting kernel");
-    return frame_open(scene, *camera, {}, max_w, max_h, opts, out, progress, "rt_frame_begin");
+    return frame_open(scene, *camera, {}, nullptr, max_w, max_h, opts, out, progress, "rt_frame_begin");
 }
 
 int rt_frame_begin_views(RtScene *scene, const RtCamera *cameras, const uint64_t *seeds, int32_t n_views, int32_t max_w, int32_t max_h,
@@ -315,7 +319,22 @@ int rt_frame_begin_views(RtScene *scene, const RtCamera *cameras, const uint64_t
         table[v].k0 = uint32_t(seed);
         table[v].k1 = uint32_t(seed >> 32);
     }
-    return frame_open(scene, cameras[0], table, max_w, max_h, opts, out, progress, "rt_frame_begin_views");
+    return frame_open(scene, cameras[0], table, nullptr, max_w, max_h, opts, out, progress, "rt_frame_begin_views");
+}
+
+int rt_frame_begin_window(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_t max_h, int32_t row0, int32_t col0, int32_t rows,
+                          int32_t cols, const RtRenderOpts *opts, RtFrame **out, RtFrameProgress *progress) {
+    // rt_render_window's checks, then rt_frame_begin's
+    const FrameWindow w{row0, col0, rows, cols};
+    int rc = check_window(w, max_w, max_h, "rt_frame_begin_window");
+    if (rc != RT_OK) return rc;
+    if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin_window: out is null");
+    *out = nullptr;
+    if ((rc = check_frame_args(scene, camera, max_w, max_h, opts)) != RT_OK) return rc;
+    if ((rc = check_frame_mode(opts, "rt_frame_begin_window")) != RT_OK) return rc;
+    if (opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS))
+        return fail(RT_ERR_UNSUPPORTED, "rt_frame_begin_window: a window has no flow-schedule or counting kernel");
+    return frame_open(scene, *camera, {}, &w, max_w, max_h, opts, out, progress, "rt_frame_begin_window");
 }
 
 int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameProgress *progress) {

@@ -61,6 +61,10 @@ def _declare(lib):
         "rt_frame_begin_views": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(RtRenderOpts), C.POINTER(_vp),
                                            C.POINTER(RtFrameProgress)]),
         "rt_frame_view_noise": (C.c_int, [_vp, C.c_double, _vp]),
+        "rt_render_window": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, _i32, _i32, _i32, _i32, C.POINTER(RtRenderOpts), _vp, _vp,
+                                       C.POINTER(RtStats)]),
+        "rt_frame_begin_window": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, _i32, _i32, _i32, _i32, C.POINTER(RtRenderOpts),
+                                            C.POINTER(_vp), C.POINTER(RtFrameProgress)]),
         "rt_pixel_noise": (C.c_int, [_vp, _vp, C.c_size_t, _vp]),
         "rt_render_multi": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i32, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _vp,
                                       _vp, C.POINTER(RtStats)]),
@@ -297,6 +301,35 @@ class SceneHandle:
         frame.n_views = n
         return frame
 
+    def render_window(self, camera, max_w, max_h, window, seed=0, adaptive=True, gamma=False, flags=0, want_sums=False, rgb_out=None):
+        """The window (row0, col0, rows, cols) of render(camera, max_w, max_h, ...) without tracing the rest of the frame
+        (rt_render_window).  Returns (uint8 [rows, cols, 3], int32 [rows, cols, 4] or None, RtStats of the window);
+        window pixel (r, c) is exactly pixel (row0 + r, col0 + c) of render's frame.  RtError RT_ERR_INVALID_ARGUMENT for a
+        window that is empty or does not lie inside the (2 max_h + 1) x (2 max_w + 1) frame."""
+        row0, col0, rows, cols = (int(x) for x in window)
+        rgb = rgb_out if rgb_out is not None else _frame_buffer((max(rows, 0), max(cols, 0), 3))
+        sums = np.empty((max(rows, 0), max(cols, 0), 4), np.int32) if want_sums else None
+        opts = RtRenderOpts(seed, int(adaptive), abi.RT_MODE_MEGAKERNEL, int(gamma), flags)
+        stats = RtStats()
+        check(lib().rt_render_window(self.ptr, C.byref(camera), max_w, max_h, row0, col0, rows, cols, C.byref(opts), ptr(rgb), ptr(sums),
+                                     C.byref(stats)))
+        return rgb, sums, stats
+
+    def open_frame_window(self, camera, max_w, max_h, window, seed=0, adaptive=True, flags=0):
+        """A progressive frame of the window (row0, col0, rows, cols) of this scene's frame (rt_frame_begin_window: runs the
+        probe over the window).  A Frame whose read, noise and sums have shape [rows, cols, ...]; after any pass (and under a
+        convergence rule) it is exactly the crop of open_frame(camera, max_w, max_h, seed=seed) at the same samples_done."""
+        row0, col0, rows, cols = (int(x) for x in window)
+        opts = RtRenderOpts(seed, int(adaptive), abi.RT_MODE_MEGAKERNEL, 0, flags)
+        out = C.c_void_p()
+        progress = RtFrameProgress()
+        check(lib().rt_frame_begin_window(self.ptr, C.byref(camera), max_w, max_h, row0, col0, rows, cols, C.byref(opts), C.byref(out),
+                                          C.byref(progress)))
+        frame = Frame.__new__(Frame)
+        frame.scene, frame.ptr, frame.progress = self, out, progress
+        frame.rows, frame.cols = rows, cols
+        return frame
+
     # ---- conformance ----
     def hit_object(self, o, d, traversal=0):
         o, d = f64(o, (-1, 3)), f64(d, (-1, 3))
@@ -343,7 +376,8 @@ class Frame:
     """Owner of an RtFrame* (rt_frame_begin / rt_frame_destroy): rt_render's frame advanced in passes over windows of
     sample indices.  After every pass the frame is exactly rt_render's at samples_per_pixel = progress.samples_done.
     Holds its scene handle, so the scene outlives it.  A frame of a batch of views (SceneHandle.open_frame_views) has
-    n_views set, and its images, sums and maps carry a leading view axis."""
+    n_views set, and its images, sums and maps carry a leading view axis; a frame of a window (SceneHandle.open_frame_window)
+    has the window's rows and cols."""
 
     n_views = None  # a frame of one camera
 

@@ -9,6 +9,7 @@ reference's.  Everything that computes goes through the C ABI (native.py); nothi
   Scene.render_views    Scene.render of many cameras of one scene in one submission (rt_render_views)
   Scene.render_progressive  the same frame in sample passes, progress ticks as passes finish (native.Frame)
   Scene.render_views_progressive  Scene.render_views in sample passes, as one progressive frame of the batch
+  Scene.render_window   a window (row0, col0, rows, cols) of Scene.render's image, without tracing the rest (rt_render_window)
   Image / Image.render  RayTracing/Domain.fs:9-31
   ImageOutput.write_ppm RayTracing/ImageOutput.fs:163-197, PixelOutput.correct :11-18
 """
@@ -166,12 +167,51 @@ class Scene:
         return float(rows * n), [image(v) for v in range(n)]
 
     @staticmethod
+    def render_window(progress_increment: Callable[[float], None], print_fn: Callable[[str], None], max_width_coord: int,
+                      max_height_coord: int, camera: abi.RtCamera, s: "Scene", window, seed: Optional[int] = None, adaptive: bool = True,
+                      flags: int = 0):
+        """The window (row0, col0, rows, cols) of Scene.render's image, rendered by one GPU without the rest of the frame
+        (native.SceneHandle.render_window): a closer look at one part of a frame, or one tile of a frame split into tiles.
+        Returns (total progress, Image of rows x cols); lazy like Scene.render: the first forced row renders the window, and
+        the progress ticks total the window's rows.  With the same camera and seed, window pixel (r, c) is Scene.render's
+        pixel (row0 + r, col0 + c).  `print_fn` is ignored."""
+        if not isinstance(s._handle, native.SceneHandle):
+            raise NotImplementedError("a window runs on one GPU: make the scene with a single device")
+        row0, col0, rows, cols = (int(x) for x in window)
+        if seed is None:
+            seed = secrets.randbits(64)
+        state = {}
+
+        def frame():
+            if "rgb" not in state:
+                rgb, _, stats = s._handle.render_window(camera, max_width_coord, max_height_coord, (row0, col0, rows, cols), seed=seed,
+                                                        adaptive=adaptive, flags=flags)
+                s.last_stats = stats
+                state["rgb"] = rgb
+            return state["rgb"]
+
+        def row_thunk(r):
+            def force():
+                out = frame()[r]
+                progress_increment(1.0)
+                return out
+            return force
+
+        def all_rows():
+            out = frame()
+            for _ in range(rows):
+                progress_increment(1.0)
+            return out
+
+        return float(rows), Image([row_thunk(r) for r in range(rows)], rows, cols, all_rows)
+
+    @staticmethod
     def render_progressive(progress_increment: Callable[[float], None], print_fn: Callable[[str], None], max_width_coord: int,
                            max_height_coord: int, camera: abi.RtCamera, s: "Scene", seed: Optional[int] = None, adaptive: bool = True,
                            target_ms: float = 250.0, on_pass: Optional[Callable[[abi.RtFrameProgress, "native.Frame"], object]] = None,
                            flags: int = 0, noise_tolerance: Optional[float] = None, noise_fraction: float = 0.0,
                            converge_tolerance: Optional[float] = None, converge_min_samples: int = 64,
-                           converge_interval: int = 64) -> np.ndarray:
+                           converge_interval: int = 64, window=None) -> np.ndarray:
         """Scene.render's frame rendered in passes of about `target_ms` of device time each (native.Frame, one GPU).
         `progress_increment(1.0)` is called as passes complete, in proportion to the paths traced so far out of the frame's
         total, and exactly `rows` times in all, like the reference's one call per row (Scene.fs:232).  After every pass
@@ -186,10 +226,13 @@ class Scene:
         With `converge_tolerance` (8-bit levels) each pixel stops being sampled once its standard error is within it, checked
         at converge_min_samples + j * converge_interval samples (Frame.set_convergence): every pixel is then rt_render's pixel
         at the sample count it stopped at.  It composes with the `noise_tolerance` stop, whose summary then covers the pixels
-        still being sampled."""
+        still being sampled.
+        With `window` = (row0, col0, rows, cols) only that window of the frame is traced (native.SceneHandle.open_frame_window):
+        the progress ticks total the window's rows, and the pixels returned ([rows, cols, 3]) are exactly that crop of the
+        frame rendered without it."""
         if not isinstance(s._handle, native.SceneHandle):
             raise NotImplementedError("progressive frames run on one GPU: make the scene with a single device")
-        rows = 2 * max_height_coord + 1
+        rows = 2 * max_height_coord + 1 if window is None else int(window[2])
         if seed is None:
             seed = secrets.randbits(64)
         ticks = ProgressTicks(rows)
@@ -207,7 +250,11 @@ class Scene:
             summary, _, _ = frame.noise(noise_tolerance, want_map=False)
             return summary.pixels_above <= noise_fraction * summary.pixels
 
-        with s._handle.open_frame(camera, max_width_coord, max_height_coord, seed=seed, adaptive=adaptive, flags=flags) as frame:
+        if window is None:
+            opened = s._handle.open_frame(camera, max_width_coord, max_height_coord, seed=seed, adaptive=adaptive, flags=flags)
+        else:
+            opened = s._handle.open_frame_window(camera, max_width_coord, max_height_coord, window, seed=seed, adaptive=adaptive, flags=flags)
+        with opened as frame:
             if converge_tolerance is not None:
                 frame.set_convergence(converge_tolerance, converge_min_samples, converge_interval)
             progress = frame.progress

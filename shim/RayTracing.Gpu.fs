@@ -194,6 +194,14 @@ module internal Native =
     [<DllImport(Lib)>]
     extern int rt_frame_view_noise (nativeint frame, float tolerance, [<Out>] RtFrameNoise[] perView)
 
+    // a window of a frame, in one call or as a progressive frame (include/rtfs_b200.h, rt_render_window; ABI 6 still: detect
+    // by the symbol)
+    [<DllImport(Lib)>]
+    extern int rt_render_window (nativeint scene, RtCamera& camera, int maxWidthCoord, int maxHeightCoord, int row0, int col0, int rows, int cols, RtRenderOpts& opts, byte[] rgbOut, nativeint sumsOut, RtStats& stats)
+
+    [<DllImport(Lib)>]
+    extern int rt_frame_begin_window (nativeint scene, RtCamera& camera, int maxWidthCoord, int maxHeightCoord, int row0, int col0, int rows, int cols, RtRenderOpts& opts, nativeint& frame, RtFrameProgress& progress)
+
     [<DllImport(Lib)>]
     extern int rt_pixel_noise (int[] sums, uint64[] sq, unativeint n, float32[] seOut)
 
@@ -522,7 +530,8 @@ type FrameConvergence =
 /// After every pass it is exactly the frame rt_render gives at `SamplesDone` samples per pixel with the same seed, so
 /// `Read` shows the image sharpening; a caller stops early by not advancing any more, and `Extend` continues a finished
 /// frame to more samples.  Dispose it before its scene.  A frame of a batch of views (SceneGpu.openFrameViews) holds `Views`
-/// images of Rows * Cols pixels one after the other; the progress and convergence counts are sums over them.
+/// images of Rows * Cols pixels one after the other; the progress and convergence counts are sums over them.  A frame of a
+/// window (SceneGpu.openFrameWindow) has the window's Rows and Cols, and its counts cover the window's pixels.
 type GpuFrame internal (handle : nativeint, rows : int, cols : int, views : int, first : Native.RtFrameProgress) =
     let mutable handle = handle
     let mutable progress = first
@@ -765,6 +774,65 @@ module SceneGpu =
 
         1.0<progress> * float (rowsIter * n), Array.init n image
 
+    /// The window (row0, col0, rows, cols) of `render`'s image, traced without the rest of the frame (rt_render_window) on a
+    /// single-device scene: a closer look at one part of a frame, or one tile of a frame split between processes.  Lazy like
+    /// `render`; every row of the window reports progress once.  `seed` is the frame's: windows of one seed are crops of one
+    /// frame, bit for bit, so tiles of any grid reassemble into it.
+    let renderWindow
+        (progressIncrement : float<progress> -> unit)
+        (_print : string -> unit)
+        (maxWidthCoord : int)
+        (maxHeightCoord : int)
+        (camera : Camera)
+        (row0 : int, col0 : int, rowsIter : int, colsIter : int)
+        (seed : uint64)
+        (s : GpuScene)
+        : float<progress> * Image
+        =
+        if s.IsMulti then
+            failwith "GPU backend: a window runs on a single-device GpuScene"
+
+        let frame =
+            lazy
+                (let rgb = Array.zeroCreate<byte> (3 * rowsIter * colsIter)
+                 let mutable cam = marshalCamera camera
+                 let mutable opts = Native.RtRenderOpts ()
+                 opts.seed <- seed
+                 opts.adaptive <- 1
+                 let mutable stats = Native.RtStats ()
+
+                 Native.rt_render_window (s.Handle, &cam, maxWidthCoord, maxHeightCoord, row0, col0, rowsIter, colsIter, &opts, rgb, 0n, &stats)
+                 |> Native.check
+
+                 rgb)
+
+        let rows =
+            Seq.init
+                rowsIter
+                (fun row ->
+                    async {
+                        let rgb = frame.Force ()
+
+                        let result =
+                            Array.init
+                                colsIter
+                                (fun col ->
+                                    let i = 3 * (row * colsIter + col)
+
+                                    {
+                                        Red = rgb.[i]
+                                        Green = rgb.[i + 1]
+                                        Blue = rgb.[i + 2]
+                                    }
+                                )
+
+                        progressIncrement 1.0<progress>
+                        return result
+                    }
+                )
+
+        1.0<progress> * float rowsIter, Image.make rowsIter colsIter rows
+
     /// Opens a progressive frame with RtRenderOpts.flags `flags` (e.g. FrameFlags.Noise for GpuFrame.Noise).
     /// Single-device scenes only.
     let openFrameWith (flags : int) (maxWidthCoord : int) (maxHeightCoord : int) (camera : Camera) (seed : uint64) (s : GpuScene) : GpuFrame =
@@ -809,6 +877,27 @@ module SceneGpu =
         |> Native.check
 
         new GpuFrame (handle, 2 * maxHeightCoord + 1, 2 * maxWidthCoord + 1, cameras.Length, progress)
+
+    /// Opens a progressive frame of the window (row0, col0, rows, cols) of the frame openFrameWith gives (rt_frame_begin_window:
+    /// the probe of the window's pixels runs now) with RtRenderOpts.flags `flags`.  Its Rows and Cols are the window's, and
+    /// after every pass (under a convergence rule too) it is exactly that crop of the frame openFrameWith gives for the same
+    /// camera and seed.  Single-device scenes only.
+    let openFrameWindow (flags : int) (maxWidthCoord : int) (maxHeightCoord : int) (camera : Camera) (row0 : int, col0 : int, rows : int, cols : int) (seed : uint64) (s : GpuScene) : GpuFrame =
+        if s.IsMulti then
+            failwith "GPU backend: progressive frames run on a single-device GpuScene"
+
+        let mutable cam = marshalCamera camera
+        let mutable opts = Native.RtRenderOpts ()
+        opts.seed <- seed
+        opts.adaptive <- 1
+        opts.flags <- flags
+        let mutable handle = 0n
+        let mutable progress = Native.RtFrameProgress ()
+
+        Native.rt_frame_begin_window (s.Handle, &cam, maxWidthCoord, maxHeightCoord, row0, col0, rows, cols, &opts, &handle, &progress)
+        |> Native.check
+
+        new GpuFrame (handle, rows, cols, 1, progress)
 
     // the frame of renderWithProgressUntil and renderConverging: passes of about 250 ms with progress ticks, an optional
     // convergence rule (tolerance, minSamples, interval) and an optional stop on the noise summary (tolerance, fraction)

@@ -440,6 +440,72 @@ int rt_frame_begin_window(RtScene *scene, const RtCamera *camera, int32_t max_wi
                           int32_t row0, int32_t col0, int32_t rows, int32_t cols, const RtRenderOpts *opts,
                           RtFrame **out, RtFrameProgress *progress);
 
+/* ---- denoised previews of progressive frames (host buffers; one GPU) ----------------------------- */
+/* A clean preview of a progressive frame after its first passes, and the first-hit feature buffers it is guided by: an
+ * object-id map for selection masks, depth, normals and albedo for compositing or an external denoiser.  Both work on any
+ * RtFrame (rt_frame_begin, rt_frame_begin_views, rt_frame_begin_window); outputs have rt_frame_read's layout (the tall
+ * frame of a batch, the window's pixels of a window).
+ *
+ * These two functions were added without a change of RT_ABI_VERSION (still 6): no existing struct or prototype changed.
+ * A caller detects the feature by the presence of the symbol rt_frame_denoise.
+ *
+ * rt_frame_features: for each pixel, sample s < samples is the camera ray that the frame's path for (seed, pixel, s)
+ *   starts with (for a batch, the view's camera and seed; for a window, the frame's pixel), one closest hit (the binary
+ *   tree walk, as rt_test_hit_object with traversal 0) and one first scatter (Hittable.Reflection) of a white colour:
+ *     prim_out    the caller's Hittable index hit by sample 0; -1 for a miss;
+ *     albedo_out  per channel the integer sum over the samples of the colour the scatter leaves in the path
+ *                 (darken(albedo, combine(white, surface)) for a scattering surface, the emitted colour for an absorbing
+ *                 one, black for a miss or a scatter that fails), divided by samples with truncation (PixelStats.mean);
+ *     normal_out  the shading normal scatter computes (oriented against the ray, F10, F11), summed in float32 in sample
+ *                 order over the samples that hit and divided by their number; (0, 0, 0) if none hit;
+ *     depth_out   the hit distance t, summed and divided the same way; +inf if none hit.
+ *   The features are exact functions of (seed, pixel, samples): the same before and after any pass, under any pacing,
+ *   convergence rule or rt_frame_extend.  The frame keeps them (computed once per samples value).  Each output is optional.
+ *   RT_ERR_INVALID_ARGUMENT for a NULL frame or samples outside [1, 64].
+ *
+ * rt_frame_denoise: an edge-avoiding a-trous wavelet filter (Dammertz et al. 2010) over the frame's current means, its colour
+ *   weight scaled by each pixel's standard error E (as SVGF scales it by its variance, Schied et al. 2017) and stopped at
+ *   edges by the features of feature_samples samples.  It reads the frame and writes buffers of its own: the sums, Q,
+ *   flags, list and counters are untouched, so a frame that is denoised between passes ends as one that never was.  It
+ *   needs Q: RT_ERR_INVALID_ARGUMENT for a frame opened without RT_FLAG_NOISE, a NULL frame or opts, iterations outside
+ *   [1, 10], feature_samples outside [1, 64], or a sigma that is not > 0 and finite as a float32; the options are checked
+ *   first, before any device work.  Suggested options and where they come from: DESIGN.md section 19.
+ *   Every operation below is an IEEE float32 operation rounded to nearest, evaluated as written, left to right:
+ *     input     c_p = float(T_c) / float(n), v_p = float(E_p) * float(E_p) (E as rt_frame_noise); a pixel with n = 0 is
+ *               output black and is no pixel's neighbour;
+ *     level k   (k = 0 .. iterations - 1) out_p = sum_q w_pq c_q / sum_q w_pq over the taps q = (r + 2^k j, c + 2^k i),
+ *               j outer, i inner, both -2..2, skipping taps outside the frame, outside p's view (a batch) and pixels with
+ *               n = 0; c is the previous level's output (the input at k = 0), v always the input's;
+ *     weight    w_pq = h_j h_i * W(x_c) * W(x_n) * W(x_a) * W(x_z), h = (1, 4, 6, 4, 1) (the product h_j h_i is exact),
+ *               W(x) = 1 / (1 + x * (1 + 0.5 * x));
+ *     colour    d = |c_p - c_q|^2 = (dr*dr + dg*dg) + db*db; x_c = 0 if d == 0, else d / (s_k * s_k * (v_p + v_q)) with
+ *               s_k = float(sigma_colour) * 2^-k, the product s_k * s_k first;
+ *     normal    x_n = |n_p - n_q|^2 / (s_n * s_n), s_n = float(sigma_normal);
+ *     albedo    x_a = |a_p - a_q|^2 / (s_a * s_a), 8-bit levels, s_a = float(sigma_albedo);
+ *     depth     x_z = 0 if z_p == z_q; +inf if either is +inf; else t * t with t = (z_p - z_q) / (s_z * z_p),
+ *               s_z = float(sigma_depth).
+ *   linear_out (optional, n_pixels*3 float) is the last level; rgb_out (optional, n_pixels*3) is that value clamped to
+ *   [0, 255], truncated, and passed through PixelOutput.correct when gamma is non-zero, as rt_frame_read's gamma.
+ * Both calls return with their device work complete, like every rt_frame_* call. */
+int rt_frame_features(RtFrame *frame, int32_t samples,
+                      int32_t *prim_out,   /* n_pixels                  */
+                      uint8_t *albedo_out, /* n_pixels*3                */
+                      float *normal_out,   /* n_pixels*3                */
+                      float *depth_out);   /* n_pixels                  */
+typedef struct RtDenoiseOpts {
+    int32_t iterations;      /* a-trous levels; level k uses tap spacing 2^k; 1..10                         */
+    int32_t feature_samples; /* F of the guide features, 1..64                                              */
+    double sigma_colour;     /* > 0: scales the per-pixel standard errors in the colour weight; halved per level */
+    double sigma_normal;     /* > 0                                                                         */
+    double sigma_albedo;     /* > 0, 8-bit levels                                                           */
+    double sigma_depth;      /* > 0, relative to the centre pixel's depth                                   */
+    int32_t gamma;           /* rgb_out through PixelOutput.correct, as rt_frame_read                       */
+    int32_t _pad0;
+} RtDenoiseOpts;
+int rt_frame_denoise(RtFrame *frame, const RtDenoiseOpts *opts,
+                     uint8_t *rgb_out,   /* n_pixels*3, optional                               */
+                     float *linear_out); /* n_pixels*3 filtered means in 8-bit levels, optional */
+
 /* The same frame split over the GPUs of this process (the F# host is one process): replicated scene,
  * sample-index split (Scene.fs:191-192 shared out by sample index), probe tiles shared out by tile.
  * The devices exchange flags and sums through NVLink peer memory inside the kernels that consume them

@@ -161,3 +161,16 @@ class RtFrameConvergence(C.Structure):
         ("pixels_active", C.c_uint64),
         ("pixels_converged", C.c_uint64),
     ]
+
+
+class RtDenoiseOpts(C.Structure):
+    _fields_ = [
+        ("iterations", C.c_int32),
+        ("feature_samples", C.c_int32),
+        ("sigma_colour", C.c_double),
+        ("sigma_normal", C.c_double),
+        ("sigma_albedo", C.c_double),
+        ("sigma_depth", C.c_double),
+        ("gamma", C.c_int32),
+        ("_pad0", C.c_int32),
+    ]

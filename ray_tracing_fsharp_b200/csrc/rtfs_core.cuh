@@ -977,7 +977,8 @@ enum ScatterResult { SCATTER_CONTINUE = 0, SCATTER_ABSORBED = 1, SCATTER_ERROR =
 
 // Hittable.Reflection (Hittable.fs:8-12) -> Sphere.reflection (Sphere.fs:150-300) /
 // InfinitePlane.reflection (InfinitePlane.fs:43-99).  On SCATTER_CONTINUE the ray (o, d) and the colour
-// are updated in place; on SCATTER_ABSORBED `colour` is the emitted result.
+// are updated in place; on SCATTER_ABSORBED `colour` is the emitted result.  `inside_out` and `normal_out` (optional) receive
+// the inside flag and the shading normal, oriented against the ray (F10, F11), once they are known.
 //
 // Written so that a warp whose lanes hit different materials shares as much as possible: one normal /
 // inside computation, one colour update, ONE block of the counter RNG for whichever style draws
@@ -985,7 +986,7 @@ enum ScatterResult { SCATTER_CONTINUE = 0, SCATTER_ABSORBED = 1, SCATTER_ERROR =
 // reflection, and a common "unit(base + scale * offset)" tail; only the few style-specific lines diverge.
 template <int SMEM, class Rng>
 RTFS_HD ScatterResult scatter(const SceneAccess<SMEM> &sc, int prim, int last, float3 &o, float3 &d, float3 strike, uint32_t &colour,
-                              Rng &rng, bool *inside_out) {
+                              Rng &rng, bool *inside_out, float3 *normal_out = nullptr) {
     const Material m = load_material(sc, prim);
     const bool is_plane = (m.flags & 2u) != 0;
     const bool flipped = (m.flags & 1u) != 0;
@@ -1031,6 +1032,7 @@ RTFS_HD ScatterResult scatter(const SceneAccess<SMEM> &sc, int prim, int last, f
         }
     }
     if (inside_out) *inside_out = inside;
+    if (normal_out) *normal_out = n;
 
     // ---- emitters ----
     if (style == RT_STYLE_LIGHT_SOURCE) { // Sphere.fs:185-189, InfinitePlane.fs:52-56

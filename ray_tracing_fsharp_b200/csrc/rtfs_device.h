@@ -298,6 +298,39 @@ __device__ __forceinline__ void pixel_rgb8(int4 s, const uint8_t *lut, uint8_t *
     out[2] = lut[(s.z / n) & 255];
 }
 
+// E of a pixel from its moments: n samples, channel sums t0..t2, sum of squares q (include/rtfs_b200.h, rt_frame_noise).
+// D = n q - sum t_c^2 is exact in int64 for n <= 2^22 (each term < 3.5e18); the double arithmetic is the same, in the same
+// order, on the device and on the host (rt_pixel_noise), and IEEE division and square root round correctly on both.
+__host__ __device__ __forceinline__ double pixel_standard_error(int32_t n, int32_t t0, int32_t t1, int32_t t2, uint64_t q) {
+    if (n < 2) return HUGE_VAL;
+    // unsigned wrap-around arithmetic, then the int64 value: the same bits as the signed formula wherever that is defined
+    const uint64_t tt = uint64_t(int64_t(t0) * t0) + uint64_t(int64_t(t1) * t1) + uint64_t(int64_t(t2) * t2);
+    const int64_t d = int64_t(uint64_t(n) * q - tt);
+    const double nd = double(n);
+    return sqrt(double(d) / (3.0 * nd * nd * double(n - 1)));
+}
+
+// ---------------------------------------------------------------------------------------------------
+// denoised previews of progressive frames (rtfs_denoise.cu; rt_frame_features, rt_frame_denoise)
+// ---------------------------------------------------------------------------------------------------
+constexpr int kMaxDenoiseIterations = 10, kMaxFeatureSamples = 64;
+// per pixel, in rt_frame_features' layouts: prim n, albedo n*3, normal n*3, depth n
+struct FrameFeatures {
+    int32_t *prim;
+    uint8_t *albedo;
+    float *normal;
+    float *depth;
+};
+// the first-hit features of sample indices [0, samples) of the n_pixels pixels of the frame fp describes (one camera, a
+// batch of views or a window)
+int launch_features(const FrameParams &fp, size_t n_pixels, int samples, const FrameFeatures &out, cudaStream_t st);
+// RT_ERR_INVALID_ARGUMENT unless every option of rt_frame_denoise is in range
+int check_denoise_opts(const RtDenoiseOpts *o, const char *who);
+// the filter over a frame's sums and Q, views of view_rows rows each: buf holds 2 n_pixels float4 (the two levels); the RGB8
+// and the linear output it was asked for are left in device memory at *d_rgb and *d_linear (inside buf)
+int launch_denoise(const int32_t *stats, const unsigned long long *sq, const FrameFeatures &feat, size_t n_pixels, int view_rows, int cols,
+                   const RtDenoiseOpts &o, float4 *buf, bool want_rgb, bool want_linear, uint8_t **d_rgb, float **d_linear, cudaStream_t st);
+
 // makes sure the tree the frame will walk is on the device (the wide tree is built on first use for small scenes)
 int prepare_frame(RtScene *scene, const RtRenderOpts *opts);
 bool frame_walks_wide_tree(const DeviceScene *ds, int opt_flags, bool smem_fits);

@@ -11,6 +11,7 @@
 // and rt_frame_view_noise reduces each view as rt_frame_noise reduces a frame of its own.
 // rt_frame_begin_window opens it over a window of rt_render's frame (its kernels are in rtfs_window.cu): the frame's buffers,
 // maps and counts are the window's, and every per-pixel kernel runs over the window unchanged.
+// rt_frame_features and rt_frame_denoise (kernels in rtfs_denoise.cu) read the frame and keep buffers of their own.
 #include "rtfs_device.h"
 
 #include <algorithm>
@@ -20,18 +21,6 @@
 using namespace rtfs;
 
 namespace rtfs {
-
-// E of a pixel from its moments: n samples, channel sums t0..t2, sum of squares q (include/rtfs_b200.h, rt_frame_noise).
-// D = n q - sum t_c^2 is exact in int64 for n <= 2^22 (each term < 3.5e18); the double arithmetic is the same, in the same
-// order, on the device and on the host (rt_pixel_noise), and IEEE division and square root round correctly on both.
-__host__ __device__ __forceinline__ double pixel_standard_error(int32_t n, int32_t t0, int32_t t1, int32_t t2, uint64_t q) {
-    if (n < 2) return HUGE_VAL;
-    // unsigned wrap-around arithmetic, then the int64 value: the same bits as the signed formula wherever that is defined
-    const uint64_t tt = uint64_t(int64_t(t0) * t0) + uint64_t(int64_t(t1) * t1) + uint64_t(int64_t(t2) * t2);
-    const int64_t d = int64_t(uint64_t(n) * q - tt);
-    const double nd = double(n);
-    return sqrt(double(d) / (3.0 * nd * nd * double(n - 1)));
-}
 
 // rt_frame_noise's reduction: a fixed grid, every block a fixed contiguous range of pixels, every thread a fixed stride of
 // it, then a fixed tree in shared memory, then one block over the partials in block order: no result depends on scheduling
@@ -121,6 +110,10 @@ struct RtFrame {
     // rewrites the workspace's between two passes; null for a frame of one camera
     ViewCamera *d_views = nullptr;
     int32_t n_views = 1;
+    // rt_frame_features' buffers, allocated on first use and computed once per feature_samples (0: not computed yet)
+    FrameFeatures feat{};
+    int32_t feat_samples = 0;
+    float4 *d_denoise = nullptr; // rt_frame_denoise's two levels (2 n_pixels), allocated on first use
     unsigned long long h_counters[CN_SLOTS] = {};
     FrameEvents ev; // rt_frame_begin: ZEROED -> TRACED; a pass: BEGIN -> END
     int32_t samples_done = 0, samples_target = 0;
@@ -150,6 +143,11 @@ void frame_free(RtFrame *f) {
     cudaFree(f->d_se);
     cudaFree(f->d_partial);
     cudaFree(f->d_views);
+    cudaFree(f->feat.prim);
+    cudaFree(f->feat.albedo);
+    cudaFree(f->feat.normal);
+    cudaFree(f->feat.depth);
+    cudaFree(f->d_denoise);
     f->ev.destroy();
     delete f;
 }
@@ -270,6 +268,22 @@ void fill_noise(const NoisePartial &total, double tolerance, RtFrameNoise *out) 
     out->max_se = total.max_se;
     out->mean_se = total.pixels ? total.sum_se / double(total.pixels) : 0.0;
     out->tolerance = tolerance;
+}
+
+// the frame's features of sample indices [0, samples), computed on first use of that count (they never change with passes)
+int ensure_features(RtFrame *f, int32_t samples, cudaStream_t st) {
+    const size_t n = f->n_pixels;
+    if (!f->feat.prim) RT_CUDA(cudaMalloc((void **)&f->feat.prim, n * sizeof(int32_t)));
+    if (!f->feat.albedo) RT_CUDA(cudaMalloc((void **)&f->feat.albedo, n * 3));
+    if (!f->feat.normal) RT_CUDA(cudaMalloc((void **)&f->feat.normal, n * 3 * sizeof(float)));
+    if (!f->feat.depth) RT_CUDA(cudaMalloc((void **)&f->feat.depth, n * sizeof(float)));
+    if (f->feat_samples != samples) {
+        f->feat_samples = 0;
+        int rc = launch_features(f->fp, n, samples, f->feat, st);
+        if (rc != RT_OK) return rc;
+        f->feat_samples = samples;
+    }
+    return RT_OK;
 }
 
 // the refusals of both openers, after their own argument checks
@@ -499,6 +513,46 @@ int rt_frame_convergence(RtFrame *f, RtFrameConvergence *out) {
     out->checks = f->conv_checks;
     out->pixels_active = f->pixels_active;
     out->pixels_converged = f->pixels_flagged - f->pixels_active;
+    return RT_OK;
+}
+
+int rt_frame_features(RtFrame *f, int32_t samples, int32_t *prim_out, uint8_t *albedo_out, float *normal_out, float *depth_out) {
+    if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_features: null frame");
+    if (samples < 1 || samples > kMaxFeatureSamples) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_features: samples must be in [1, 64]");
+    auto *ds = static_cast<DeviceScene *>(f->scene->dev);
+    RT_CUDA(cudaSetDevice(ds->device));
+    cudaStream_t st = ds->ws->stream;
+    int rc = ensure_features(f, samples, st);
+    if (rc != RT_OK) return rc;
+    const size_t n = f->n_pixels;
+    if (prim_out) RT_CUDA(cudaMemcpyAsync(prim_out, f->feat.prim, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (albedo_out) RT_CUDA(cudaMemcpyAsync(albedo_out, f->feat.albedo, n * 3, cudaMemcpyDeviceToHost, st));
+    if (normal_out) RT_CUDA(cudaMemcpyAsync(normal_out, f->feat.normal, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+    if (depth_out) RT_CUDA(cudaMemcpyAsync(depth_out, f->feat.depth, n * sizeof(float), cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaStreamSynchronize(st));
+    return RT_OK;
+}
+
+int rt_frame_denoise(RtFrame *f, const RtDenoiseOpts *opts, uint8_t *rgb_out, float *linear_out) {
+    int rc = check_denoise_opts(opts, "rt_frame_denoise");
+    if (rc != RT_OK) return rc;
+    if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_denoise: null frame");
+    if (!f->d_sq) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_denoise: the frame was opened without RT_FLAG_NOISE");
+    auto *ds = static_cast<DeviceScene *>(f->scene->dev);
+    RT_CUDA(cudaSetDevice(ds->device));
+    cudaStream_t st = ds->ws->stream;
+    if ((rc = ensure_features(f, opts->feature_samples, st)) != RT_OK) return rc;
+    const size_t n = f->n_pixels;
+    if (!f->d_denoise) RT_CUDA(cudaMalloc((void **)&f->d_denoise, 2 * n * sizeof(float4)));
+    const int view_rows = f->fp.cam.rows / f->n_views; // the tall frame of a batch: taps stay inside their view
+    uint8_t *d_rgb = nullptr;
+    float *d_linear = nullptr;
+    if ((rc = launch_denoise(f->d_stats, f->d_sq, f->feat, n, view_rows, f->fp.cam.cols, *opts, f->d_denoise, rgb_out != nullptr,
+                             linear_out != nullptr, &d_rgb, &d_linear, st)) != RT_OK)
+        return rc;
+    if (rgb_out) RT_CUDA(cudaMemcpyAsync(rgb_out, d_rgb, n * 3, cudaMemcpyDeviceToHost, st));
+    if (linear_out) RT_CUDA(cudaMemcpyAsync(linear_out, d_linear, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaStreamSynchronize(st));
     return RT_OK;
 }
 

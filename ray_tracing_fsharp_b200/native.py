@@ -10,7 +10,7 @@ import os
 import numpy as np
 
 from . import abi
-from .abi import RtCamera, RtFrameConvergence, RtFrameNoise, RtFrameProgress, RtHittable, RtRenderOpts, RtStats, RtTexture
+from .abi import RtCamera, RtDenoiseOpts, RtFrameConvergence, RtFrameNoise, RtFrameProgress, RtHittable, RtRenderOpts, RtStats, RtTexture
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "librtfs_b200.so")
@@ -65,6 +65,8 @@ def _declare(lib):
                                        C.POINTER(RtStats)]),
         "rt_frame_begin_window": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, _i32, _i32, _i32, _i32, C.POINTER(RtRenderOpts),
                                             C.POINTER(_vp), C.POINTER(RtFrameProgress)]),
+        "rt_frame_features": (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp]),
+        "rt_frame_denoise": (C.c_int, [_vp, C.POINTER(RtDenoiseOpts), _vp, _vp]),
         "rt_pixel_noise": (C.c_int, [_vp, _vp, C.c_size_t, _vp]),
         "rt_render_multi": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i32, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _vp,
                                       _vp, C.POINTER(RtStats)]),
@@ -442,6 +444,31 @@ class Frame:
         out = RtFrameConvergence()
         check(lib().rt_frame_convergence(self.ptr, C.byref(out)))
         return out
+
+    def features(self, samples=4):
+        """First-hit features of sample indices 0 .. samples - 1 of every pixel (rt_frame_features): (prim int32 [rows, cols],
+        the caller's Hittable index hit by sample 0 or -1; albedo uint8 [rows, cols, 3], the truncating mean of the colour the
+        first scatter leaves in a white path; normal float32 [rows, cols, 3] and depth float32 [rows, cols], the means over the
+        samples that hit, depth +inf where none did).  Exact functions of (seed, pixel, samples): passes do not change them."""
+        prim = np.empty(self._shape(), np.int32)
+        albedo = np.empty(self._shape(3), np.uint8)
+        normal = np.empty(self._shape(3), np.float32)
+        depth = np.empty(self._shape(), np.float32)
+        check(lib().rt_frame_features(self.ptr, int(samples), ptr(prim), ptr(albedo), ptr(normal), ptr(depth)))
+        return prim, albedo, normal, depth
+
+    def denoise(self, iterations=3, feature_samples=4, sigma_colour=4.0, sigma_normal=0.1, sigma_albedo=16.0, sigma_depth=0.02, gamma=False,
+                want_linear=False):
+        """A denoised preview of the frame's current image (rt_frame_denoise: an edge-avoiding a-trous filter guided by each
+        pixel's noise estimate and by features(feature_samples)).  Only on a frame opened with abi.RT_FLAG_NOISE; the frame
+        itself is left as it was.  Returns (uint8 [rows, cols, 3], float32 [rows, cols, 3] filtered means in 8-bit levels or
+        None).  The defaults are DESIGN.md section 19's."""
+        opts = RtDenoiseOpts(int(iterations), int(feature_samples), float(sigma_colour), float(sigma_normal), float(sigma_albedo),
+                             float(sigma_depth), int(gamma), 0)
+        rgb = np.empty(self._shape(3), np.uint8)
+        linear = np.empty(self._shape(3), np.float32) if want_linear else None
+        check(lib().rt_frame_denoise(self.ptr, C.byref(opts), ptr(rgb), ptr(linear)))
+        return rgb, linear
 
     def close(self):
         if getattr(self, "ptr", None):

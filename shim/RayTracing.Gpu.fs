@@ -142,6 +142,17 @@ module internal Native =
         val mutable pixelsActive : uint64
         val mutable pixelsConverged : uint64
 
+    [<Struct ; StructLayout(LayoutKind.Sequential)>]
+    type RtDenoiseOpts =
+        val mutable iterations : int
+        val mutable featureSamples : int
+        val mutable sigmaColour : float
+        val mutable sigmaNormal : float
+        val mutable sigmaAlbedo : float
+        val mutable sigmaDepth : float
+        val mutable gamma : int
+        val mutable pad0 : int
+
 
     [<DllImport(Lib)>]
     extern nativeint rt_last_error ()
@@ -193,6 +204,14 @@ module internal Native =
 
     [<DllImport(Lib)>]
     extern int rt_frame_view_noise (nativeint frame, float tolerance, [<Out>] RtFrameNoise[] perView)
+
+    // denoised previews of progressive frames and their first-hit features (include/rtfs_b200.h, rt_frame_denoise; ABI 6
+    // still: detect by the symbol)
+    [<DllImport(Lib)>]
+    extern int rt_frame_features (nativeint frame, int samples, [<Out>] int[] primOut, [<Out>] byte[] albedoOut, [<Out>] float32[] normalOut, [<Out>] float32[] depthOut)
+
+    [<DllImport(Lib)>]
+    extern int rt_frame_denoise (nativeint frame, RtDenoiseOpts& opts, [<Out>] byte[] rgbOut, [<Out>] float32[] linearOut)
 
     // a window of a frame, in one call or as a progressive frame (include/rtfs_b200.h, rt_render_window; ABI 6 still: detect
     // by the symbol)
@@ -532,6 +551,39 @@ type FrameConvergence =
 /// frame to more samples.  Dispose it before its scene.  A frame of a batch of views (SceneGpu.openFrameViews) holds `Views`
 /// images of Rows * Cols pixels one after the other; the progress and convergence counts are sums over them.  A frame of a
 /// window (SceneGpu.openFrameWindow) has the window's Rows and Cols, and its counts cover the window's pixels.
+/// First-hit features of a progressive frame (GpuFrame.Features), row-major per view.
+type FrameFeatures =
+    {
+        Prim : int[]
+        Albedo : byte[]
+        Normal : float32[]
+        Depth : float32[]
+    }
+
+/// The options of GpuFrame.Denoise (RtDenoiseOpts; the formulas are in include/rtfs_b200.h).
+type DenoiseOptions =
+    {
+        Iterations : int
+        FeatureSamples : int
+        SigmaColour : float
+        SigmaNormal : float
+        SigmaAlbedo : float
+        SigmaDepth : float
+    }
+
+[<RequireQualifiedAccess>]
+module DenoiseOptions =
+    /// the suggested options (DESIGN.md section 19)
+    let defaults : DenoiseOptions =
+        {
+            Iterations = 3
+            FeatureSamples = 4
+            SigmaColour = 4.0
+            SigmaNormal = 0.1
+            SigmaAlbedo = 16.0
+            SigmaDepth = 0.02
+        }
+
 type GpuFrame internal (handle : nativeint, rows : int, cols : int, views : int, first : Native.RtFrameProgress) =
     let mutable handle = handle
     let mutable progress = first
@@ -596,6 +648,35 @@ type GpuFrame internal (handle : nativeint, rows : int, cols : int, views : int,
     /// its first pass.  Every pixel is then exactly rt_render's pixel at the sample count it stopped at.
     member _.SetConvergence (tolerance : float, minSamples : int, interval : int) : unit =
         Native.rt_frame_set_convergence (handle, tolerance, minSamples, interval) |> Native.check
+
+    /// First-hit features of sample indices 0 .. samples - 1 of every pixel (rt_frame_features), row-major per view: the
+    /// Hittable index hit by sample 0 (-1: a miss); the truncating mean RGB8 of the colour the first scatter leaves in a white
+    /// path; the mean shading normal (xyz) and the mean hit distance (+inf: no sample hit) over the samples that hit.  Exact
+    /// functions of (seed, pixel, samples): passes do not change them.
+    member _.Features (samples : int) : FrameFeatures =
+        let n = views * rows * cols
+        let prim = Array.zeroCreate<int> n
+        let albedo = Array.zeroCreate<byte> (3 * n)
+        let normal = Array.zeroCreate<float32> (3 * n)
+        let depth = Array.zeroCreate<float32> n
+        Native.rt_frame_features (handle, samples, prim, albedo, normal, depth) |> Native.check
+        { Prim = prim ; Albedo = albedo ; Normal = normal ; Depth = depth }
+
+    /// A denoised preview of the current image (rt_frame_denoise) as row-major RGB8 per view (PixelOutput.correct applied
+    /// when `gamma`), leaving the frame as it was.  Only on a frame opened with FrameFlags.Noise.  DenoiseOptions.defaults
+    /// holds the suggested options (DESIGN.md section 19).
+    member _.Denoise (options : DenoiseOptions, gamma : bool) : byte[] =
+        let rgb = Array.zeroCreate<byte> (3 * views * rows * cols)
+        let mutable o = Native.RtDenoiseOpts ()
+        o.iterations <- options.Iterations
+        o.featureSamples <- options.FeatureSamples
+        o.sigmaColour <- options.SigmaColour
+        o.sigmaNormal <- options.SigmaNormal
+        o.sigmaAlbedo <- options.SigmaAlbedo
+        o.sigmaDepth <- options.SigmaDepth
+        o.gamma <- (if gamma then 1 else 0)
+        Native.rt_frame_denoise (handle, &o, rgb, null) |> Native.check
+        rgb
 
     /// The rule set by SetConvergence and its state (rt_frame_convergence).
     member _.Convergence () : FrameConvergence =

@@ -219,6 +219,44 @@ size_t rt_scene_device_bytes(const RtScene *scene);
  * is too large for that and is read from global memory (L1 / L2) instead */
 size_t rt_scene_shared_memory_bytes(const RtScene *scene);
 
+/* ---- editing a scene in place ----------------------------------------------------------------- */
+/* Changes objects and textures of a scene on its device and refits its tree there: for selection and recolouring, nudging
+ * an object, or the next step of an animation, without rt_scene_create's host build and full upload.
+ *
+ * Object object_index[i] of the caller's array becomes objects[i]; texture texture_index[j] becomes textures[j].  After the
+ * call the scene is the scene rt_scene_create would make from the edited arrays, except that the SAH tree keeps its
+ * topology, its leaf order and the device primitive ids: the boxes of every node above a moved sphere are recomputed on the
+ * device, bottom-up, as the host build computes them (directed roundings of each FP32 sphere, exact unions).  So every entry
+ * point (rt_render, views, windows, progressive frames opened after the call, features and denoise; sums, RGB8, Q, stats
+ * and rays) gives bit for bit the frame of a freshly created scene of the edited arrays, wherever no closest hit is an exact
+ * tie in t between two bounded spheres (the condition under which the binary and the 8-wide trees already agree).  A tree
+ * refit over moved spheres may become slower to walk than a fresh build; DESIGN.md section 20 says when to recreate.
+ *
+ * Structure must stay: the object count, each object's shape, whether each bounded sphere's radius is >= 0, the texture
+ * count, each texture's kind, an image texture's width and height.  Anything else may change (centre, radius, normal,
+ * style, albedo, fuzz, ior, prob, colour, texture index, checker parameters, map centre and radius, image texels).  A
+ * structural change needs a new scene.
+ * Refusals (RT_ERR_INVALID_ARGUMENT, before any device work, leaving the scene as it was): a structural change, an index
+ * out of range, a duplicate index, a negative count, a NULL array with a non-zero count, and anything rt_scene_create
+ * would refuse in the edited arrays.  A scene created with device = -1: RT_ERR_UNSUPPORTED.
+ * Frames.  A progressive frame opened before the call is stale: rt_frame_advance, _extend, _set_convergence, _features
+ *   and _denoise refuse it (RT_ERR_INVALID_ARGUMENT); _read, _noise, _view_noise, _convergence and _destroy still work on
+ *   what it holds.
+ * Returns with its device work complete.  info optional.  A caller detects the feature by the symbol rt_scene_update. */
+typedef struct RtSceneUpdate {
+    int32_t objects;       /* object records that changed                                                         */
+    int32_t textures;      /* texture records that changed                                                        */
+    int32_t spheres_moved; /* bounded spheres whose device sphere (FP32 centre, radius) changed                    */
+    int32_t nodes_refit;   /* tree nodes whose child boxes were recomputed                                          */
+    uint64_t generation;   /* the scene's edit count after this call (0 = as created)                              */
+    double device_ms;      /* device time of the copy and the kernels (CUDA events)                                */
+    int32_t launches;
+    int32_t _pad0;
+} RtSceneUpdate;
+int rt_scene_update(RtScene *scene, const int32_t *object_index, const RtHittable *objects, int32_t n_objects,
+                    const int32_t *texture_index, const RtTexture *textures, int32_t n_textures,
+                    RtSceneUpdate *info /* optional */);
+
 /* ---- host buffers ----------------------------------------------------------------------------- */
 /* Page-locks a host buffer the caller owns (an output frame it renders into again and again) so that the device->host
  * copy of rt_render / rt_multi_render / rt_comm_render runs at PCIe speed and asynchronously instead of through the

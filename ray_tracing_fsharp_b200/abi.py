@@ -174,3 +174,16 @@ class RtDenoiseOpts(C.Structure):
         ("gamma", C.c_int32),
         ("_pad0", C.c_int32),
     ]
+
+
+class RtSceneUpdate(C.Structure):
+    _fields_ = [
+        ("objects", C.c_int32),
+        ("textures", C.c_int32),
+        ("spheres_moved", C.c_int32),
+        ("nodes_refit", C.c_int32),
+        ("generation", C.c_uint64),
+        ("device_ms", C.c_double),
+        ("launches", C.c_int32),
+        ("_pad0", C.c_int32),
+    ]

@@ -55,6 +55,7 @@ namespace rtfs {
 int device_scene_upload(RtScene *) { return fail(RT_ERR_NO_DEVICE, "host debug build"); }
 int device_scene_ensure_reference(RtScene *) { return RT_OK; }
 int device_scene_ensure_wide(RtScene *) { return RT_OK; }
+int device_scene_sync_layout(RtScene *) { return RT_OK; }
 void device_scene_free(RtScene *) {}
 size_t device_scene_bytes(const RtScene *) { return 0; }
 } // namespace rtfs

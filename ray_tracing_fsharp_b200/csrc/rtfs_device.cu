@@ -139,10 +139,35 @@ void device_scene_free(RtScene *scene) {
     cudaDeviceSynchronize();
     cudaFree(ds->ref_nodes);
     cudaFree(ds->wide_blob); // (the main blob lives in the workspace)
+    cudaFree(ds->edit_stage);
+    cudaFree(ds->refit);
     if (ds->ws) workspace_release(ds->ws);
     for (const PooledTexture &t : ds->images) texture_release(t);
     delete ds;
     scene->dev = nullptr;
+}
+
+DTexture device_texture_of(const RtTexture &t) {
+    DTexture o;
+    std::memset(&o, 0, sizeof o);
+    o.kind = t.kind;
+    o.rgb = (uint32_t(t.colour[0]) << 16) | (uint32_t(t.colour[1]) << 8) | uint32_t(t.colour[2]);
+    o.w = t.width;
+    o.h = t.height;
+    o.even = t.even;
+    o.odd = t.odd;
+    o.grid = float(t.grid_size);
+    o.cx = float(t.map_centre[0]);
+    o.cy = float(t.map_centre[1]);
+    o.cz = float(t.map_centre[2]);
+    o.inv_radius = float(1.0 / (t.map_radius != 0.0 ? t.map_radius : 1.0));
+    return o;
+}
+
+std::vector<uchar4> texels_of(const RtTexture &t) {
+    std::vector<uchar4> texels(size_t(t.width) * t.height);
+    for (size_t k = 0; k < texels.size(); ++k) texels[k] = make_uchar4(t.rgb8[3 * k], t.rgb8[3 * k + 1], t.rgb8[3 * k + 2], 255);
+    return texels;
 }
 
 size_t device_scene_bytes(const RtScene *scene) {
@@ -168,21 +193,9 @@ int device_scene_upload(RtScene *scene) {
     for (size_t i = 0; i < scene->textures.size(); ++i) {
         const RtTexture &t = scene->textures[i];
         DTexture &o = dt[i];
-        std::memset(&o, 0, sizeof o);
-        o.kind = t.kind;
-        o.rgb = (uint32_t(t.colour[0]) << 16) | (uint32_t(t.colour[1]) << 8) | uint32_t(t.colour[2]);
-        o.w = t.width;
-        o.h = t.height;
-        o.even = t.even;
-        o.odd = t.odd;
-        o.grid = float(t.grid_size);
-        o.cx = float(t.map_centre[0]);
-        o.cy = float(t.map_centre[1]);
-        o.cz = float(t.map_centre[2]);
-        o.inv_radius = float(1.0 / (t.map_radius != 0.0 ? t.map_radius : 1.0));
+        o = device_texture_of(t);
         if (t.kind == RT_TEX_IMAGE) {
-            std::vector<uchar4> texels(size_t(t.width) * t.height);
-            for (size_t k = 0; k < texels.size(); ++k) texels[k] = make_uchar4(t.rgb8[3 * k], t.rgb8[3 * k + 1], t.rgb8[3 * k + 2], 255);
+            const std::vector<uchar4> texels = texels_of(t);
             PooledTexture pt;
             if (!texture_acquire(ds->device, t.width, t.height, pt)) return bail(fail(RT_ERR_CUDA, "texture allocation failed for an image texture"));
             ds->images.push_back(pt);
@@ -208,14 +221,14 @@ int device_scene_upload(RtScene *scene) {
         cudaFree(ws->d_blob);
         if (ws->h_blob) cudaFreeHost(ws->h_blob);
         ws->d_blob = ws->h_blob = nullptr;
-        ws->blob_cap = 0;
+        ws->blob_cap = ws->h_blob_cap = 0;
         const size_t cap = std::max<size_t>(total + total / 2, 256 << 10);
         if (cudaMalloc(&ws->d_blob, cap) != cudaSuccess || cudaMallocHost(&ws->h_blob, cap) != cudaSuccess) {
             cudaFree(ws->d_blob);
             ws->d_blob = nullptr;
             return bail(fail(RT_ERR_CUDA, "cudaMalloc failed for the scene"));
         }
-        ws->blob_cap = cap;
+        ws->blob_cap = ws->h_blob_cap = cap;
     }
     uint8_t *host = static_cast<uint8_t *>(ws->h_blob);
     auto put = [&](size_t off, const void *src, size_t n) {
@@ -245,9 +258,9 @@ int device_scene_upload(RtScene *scene) {
     ds->g.n_tex = int32_t(scene->textures.size());
     ds->max_depth = L.max_depth;
     // lean: nothing in this scene needs the FP64 evaluation of an unbounded object or a texture lookup (SceneAccess, rtfs_core.cuh)
-    ds->lean = true;
-    for (const DUnbounded &u : L.unbounded) ds->lean = ds->lean && u.fp32 == 1;
-    for (const DMaterial &m : L.materials) ds->lean = ds->lean && m.texture < 0;
+    for (const DUnbounded &u : L.unbounded) ds->n_fp64 += u.fp32 == 1 ? 0 : 1;
+    for (const DMaterial &m : L.materials) ds->n_textured += m.texture < 0 ? 0 : 1;
+    ds->lean = ds->n_fp64 == 0 && ds->n_textured == 0;
     if (!L.wide_nodes.empty()) return device_scene_ensure_wide(scene); // built at creation for big scenes
     return RT_OK;
 }
@@ -256,6 +269,8 @@ int device_scene_upload(RtScene *scene) {
 int device_scene_ensure_wide(RtScene *scene) {
     auto *ds = static_cast<DeviceScene *>(scene->dev);
     if (!ds || ds->wide_blob || ds->g.n_bounded <= 0) return RT_OK;
+    int rc = device_scene_sync_layout(scene); // the wide tree collapses the binary one: after an edit, its refit boxes
+    if (rc != RT_OK) return rc;
     HostSceneLayout &L = scene->layout;
     build_wide_layout(L);
     if (L.wide_depth > 30) return fail(RT_ERR_UNSUPPORTED, "the wide BVH is deeper than the traversal stack");
@@ -274,6 +289,7 @@ int device_scene_ensure_wide(RtScene *scene) {
     RT_CUDA(cudaMalloc(&ds->wide_blob, total));
     RT_CUDA(cudaMemcpy(ds->wide_blob, host.data(), total, cudaMemcpyHostToDevice));
     ds->bytes += total;
+    ds->wide_bytes = total;
     uint8_t *base = static_cast<uint8_t *>(ds->wide_blob);
     ds->g.wide_nodes = reinterpret_cast<const uint4 *>(base + off_nodes);
     ds->g.wide_spheres = reinterpret_cast<const float4 *>(base + off_sph);

@@ -85,6 +85,7 @@ struct DeviceWorkspace {
     void *d_blob = nullptr;
     void *h_blob = nullptr;
     size_t blob_cap = 0;
+    size_t h_blob_cap = 0; // >= blob_cap: rt_scene_update may stage more than a blob's bytes in h_blob
     size_t views_cap = 0; // the per-view cameras and keys of rt_render_views
     ViewCamera *d_views = nullptr;
     unsigned long long *d_counters = nullptr;
@@ -116,8 +117,19 @@ struct DeviceScene {
     size_t bytes = 0;
     int32_t max_depth = 0; // depth of the tree: the walk's stack never holds more entries
     bool lean = false;     // no FP64 unbounded object, no texture index: the staged kernels have a variant without that code
+    int32_t n_fp64 = 0, n_textured = 0; // unbounded objects on the FP64 path, materials with a texture index: lean iff both are 0
+    size_t wide_bytes = 0;
     DeviceWorkspace *ws = nullptr;
+    // rt_scene_update (rtfs_edit.cu), allocated by the first edit that needs them: the landing zone of the edit records, and
+    // the refit's min / max form of the tree with its parent links and counters
+    void *edit_stage = nullptr;
+    size_t edit_stage_cap = 0;
+    void *refit = nullptr;
 };
+// an RtTexture's device record, without the texture object of an image (set by the caller)
+DTexture device_texture_of(const RtTexture &t);
+// an image texture's texels in the form its array holds
+std::vector<uchar4> texels_of(const RtTexture &t);
 
 constexpr int kTileW = 8, kTileH = 4; // a warp's 32 pixels
 constexpr int kMaxChunks = 192;

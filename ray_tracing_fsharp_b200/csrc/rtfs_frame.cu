@@ -12,6 +12,8 @@
 // rt_frame_begin_window opens it over a window of rt_render's frame (its kernels are in rtfs_window.cu): the frame's buffers,
 // maps and counts are the window's, and every per-pixel kernel runs over the window unchanged.
 // rt_frame_features and rt_frame_denoise (kernels in rtfs_denoise.cu) read the frame and keep buffers of their own.
+// A frame records its scene's edit count: once rt_scene_update has changed the scene, the calls that would trace or read the
+// scene refuse the frame, and the others keep working on what it holds.
 #include "rtfs_device.h"
 
 #include <algorithm>
@@ -125,6 +127,7 @@ struct RtFrame {
     double conv_tolerance = 0.0;
     int32_t conv_min = 0, conv_interval = 0, conv_checks = 0;
     uint64_t pixels_active = 0; // pixels still being sampled: the list's length (pixels_flagged until a check)
+    uint64_t generation = 0;    // the scene's edit count when the frame opened (rt_scene_update)
 };
 
 namespace {
@@ -194,6 +197,7 @@ int frame_open(RtScene *scene, const RtCamera &camera, const std::vector<ViewCam
     RT_CUDA(cudaSetDevice(ds->device));
     auto *f = new RtFrame();
     f->scene = scene;
+    f->generation = scene->generation;
     auto bail = [&](int code) {
         frame_free(f);
         return code;
@@ -286,6 +290,13 @@ int ensure_features(RtFrame *f, int32_t samples, cudaStream_t st) {
     return RT_OK;
 }
 
+// RT_ERR_INVALID_ARGUMENT if the scene was edited since the frame opened: its probe, flags and samples are of the old scene
+int check_current(const RtFrame *f, const char *who) {
+    if (f->generation != f->scene->generation)
+        return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": the scene changed (rt_scene_update) since the frame was opened; open a new frame");
+    return RT_OK;
+}
+
 // the refusals of both openers, after their own argument checks
 int check_frame_mode(const RtRenderOpts *opts, const char *who) {
     if (opts->mode == RT_MODE_WAVEFRONT) return fail(RT_ERR_UNSUPPORTED, std::string(who) + ": progressive frames run the megakernel only");
@@ -353,6 +364,7 @@ int rt_frame_begin_window(RtScene *scene, const RtCamera *camera, int32_t max_w,
 
 int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameProgress *progress) {
     if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_advance: null frame");
+    if (int rc = check_current(f, "rt_frame_advance"); rc != RT_OK) return rc;
     if (max_samples < 0 || !(target_ms >= 0.0)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_advance: max_samples and target_ms must be >= 0");
     const bool rule = f->conv_interval > 0;
     if (rule && f->pixels_active == 0) f->samples_done = f->samples_target; // every pixel has stopped: nothing to trace
@@ -422,6 +434,7 @@ int rt_frame_read(RtFrame *f, int32_t gamma, uint8_t *rgb_out, int32_t *sums_out
 
 int rt_frame_extend(RtFrame *f, int32_t spp) {
     if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_extend: null frame");
+    if (int rc = check_current(f, "rt_frame_extend"); rc != RT_OK) return rc;
     if (spp < 1 || spp > (1 << 22)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_extend: samples_per_pixel must be in [1, 2^22]");
     FrameParams &fp = f->fp;
     if (fp.adaptive && std::min(5, spp / 2) != fp.first_trial) // Scene.fs:172
@@ -491,6 +504,7 @@ int rt_frame_view_noise(RtFrame *f, double tolerance, RtFrameNoise *per_view) {
 
 int rt_frame_set_convergence(RtFrame *f, double tolerance, int32_t min_samples, int32_t interval) {
     if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_set_convergence: null frame");
+    if (int rc = check_current(f, "rt_frame_set_convergence"); rc != RT_OK) return rc;
     if (!f->d_sq) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_set_convergence: the frame was opened without RT_FLAG_NOISE");
     if (f->passes > 0) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_set_convergence: a pass has already run");
     if (!(tolerance >= 0.0)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_set_convergence: tolerance must be >= 0");
@@ -518,6 +532,7 @@ int rt_frame_convergence(RtFrame *f, RtFrameConvergence *out) {
 
 int rt_frame_features(RtFrame *f, int32_t samples, int32_t *prim_out, uint8_t *albedo_out, float *normal_out, float *depth_out) {
     if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_features: null frame");
+    if (int rc = check_current(f, "rt_frame_features"); rc != RT_OK) return rc;
     if (samples < 1 || samples > kMaxFeatureSamples) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_features: samples must be in [1, 64]");
     auto *ds = static_cast<DeviceScene *>(f->scene->dev);
     RT_CUDA(cudaSetDevice(ds->device));
@@ -537,6 +552,7 @@ int rt_frame_denoise(RtFrame *f, const RtDenoiseOpts *opts, uint8_t *rgb_out, fl
     int rc = check_denoise_opts(opts, "rt_frame_denoise");
     if (rc != RT_OK) return rc;
     if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_denoise: null frame");
+    if ((rc = check_current(f, "rt_frame_denoise")) != RT_OK) return rc;
     if (!f->d_sq) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_denoise: the frame was opened without RT_FLAG_NOISE");
     auto *ds = static_cast<DeviceScene *>(f->scene->dev);
     RT_CUDA(cudaSetDevice(ds->device));

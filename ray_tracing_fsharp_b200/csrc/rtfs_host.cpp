@@ -44,17 +44,6 @@ inline bool unitise(D3 v, D3 &out) {
     return true;
 }
 
-inline float round_down(double v) {
-    float f = float(v);
-    if (double(f) > v) f = std::nextafterf(f, -std::numeric_limits<float>::infinity());
-    return f;
-}
-inline float round_up(double v) {
-    float f = float(v);
-    if (double(f) < v) f = std::nextafterf(f, std::numeric_limits<float>::infinity());
-    return f;
-}
-
 } // namespace
 
 // ---------------------------------------------------------------------------------------------
@@ -358,6 +347,28 @@ struct SahBuilder {
     }
 };
 
+void export_sah(const HostSceneLayout &L, const std::vector<int32_t> &leaf_obj, int32_t ref, const float *mn, const float *mx,
+                std::vector<HostNode> &out) {
+    int32_t me = int32_t(out.size());
+    out.push_back(HostNode{});
+    for (int a = 0; a < 3; ++a) {
+        out[me].mn[a] = mn[a];
+        out[me].mx[a] = mx[a];
+    }
+    out[me].right = -1;
+    out[me].prim = -1;
+    if (ref < 0) {
+        out[me].prim = leaf_obj[~ref];
+        return;
+    }
+    const DNode nd = L.nodes[ref];
+    export_sah(L, leaf_obj, nd.left, nd.l_mn, nd.l_mx, out);
+    int32_t r = int32_t(out.size());
+    export_sah(L, leaf_obj, nd.right, nd.r_mn, nd.r_mx, out);
+    out[me].right = r;
+}
+} // namespace
+
 DMaterial make_material(const RtHittable &h, int32_t host_index) {
     DMaterial m{};
     m.albedo = h.albedo;
@@ -381,28 +392,6 @@ DMaterial make_material(const RtHittable &h, int32_t host_index) {
     m.host_index = host_index;
     return m;
 }
-
-void export_sah(const HostSceneLayout &L, const std::vector<int32_t> &leaf_obj, int32_t ref, const float *mn, const float *mx,
-                std::vector<HostNode> &out) {
-    int32_t me = int32_t(out.size());
-    out.push_back(HostNode{});
-    for (int a = 0; a < 3; ++a) {
-        out[me].mn[a] = mn[a];
-        out[me].mx[a] = mx[a];
-    }
-    out[me].right = -1;
-    out[me].prim = -1;
-    if (ref < 0) {
-        out[me].prim = leaf_obj[~ref];
-        return;
-    }
-    const DNode nd = L.nodes[ref];
-    export_sah(L, leaf_obj, nd.left, nd.l_mn, nd.l_mx, out);
-    int32_t r = int32_t(out.size());
-    export_sah(L, leaf_obj, nd.right, nd.r_mn, nd.r_mx, out);
-    out[me].right = r;
-}
-} // namespace
 
 // FP32 (expanded form) or FP64 for an unbounded object — see DUnbounded.  The expanded forms lose accuracy only through
 // the size of k next to the quantity wanted (2 r h for a ray origin at height h above a sphere, h for a plane): absolute
@@ -431,36 +420,17 @@ void classify_unbounded(DUnbounded &u) {
     }
 }
 
-// min / max boxes -> centre / half-extent boxes in the paired layout the device reads (see rtfs_internal.h), never smaller
-// than the original
-DNode device_node_of(const DNode &n) {
-    DNode d = n;
-    float c[2][3], h[2][3];
-    auto conv = [](const float *mn, const float *mx, float *c_out, float *h_out) {
-        for (int a = 0; a < 3; ++a) {
-            if (!std::isfinite(mn[a]) || !std::isfinite(mx[a])) { // the never-entered dummy box of a one-sphere tree
-                c_out[a] = 1e30f;
-                h_out[a] = 0.f;
-                continue;
-            }
-            float cf = float(0.5 * (double(mn[a]) + double(mx[a])));
-            double hd = std::max(double(mx[a]) - double(cf), double(cf) - double(mn[a]));
-            float hf = round_up(hd);
-            c_out[a] = cf;
-            h_out[a] = std::nextafterf(hf, std::numeric_limits<float>::infinity());
-        }
-    };
-    conv(n.l_mn, n.l_mx, c[0], h[0]);
-    conv(n.r_mn, n.r_mx, c[1], h[1]);
-    // {c.x l, c.x r, c.y l, c.y r | c.z l, c.z r, h.x l, h.x r | h.y l, h.y r, h.z l, h.z r}: the twelve floats of the struct in order
-    float *q = d.l_mn;
-    static_assert(offsetof(DNode, left) == 12 * sizeof(float), "the twelve box floats are contiguous");
-    for (int a = 0; a < 3; ++a)
-        for (int side = 0; side < 2; ++side) {
-            q[2 * a + side] = c[side][a];
-            q[6 + 2 * a + side] = h[side][a];
-        }
-    return d;
+DUnbounded make_unbounded(const RtHittable &h) {
+    DUnbounded u{};
+    for (int a = 0; a < 3; ++a) {
+        u.p[a] = h.p[a];
+        u.n[a] = float(h.n[a]);
+    }
+    u.r2 = h.radius * h.radius; // Sphere.make, Sphere.fs:326
+    u.r = float(h.radius);
+    u.shape = h.shape;
+    classify_unbounded(u);
+    return u;
 }
 
 void build_device_layout(const RtHittable *objs, int32_t n_objs, HostSceneLayout &L, std::vector<HostNode> &sah_tree_out) {
@@ -515,19 +485,9 @@ void build_device_layout(const RtHittable *objs, int32_t n_objs, HostSceneLayout
         device_id_of[b.leaf_obj[k]] = k;
     }
     for (int32_t i : unbounded) {
-        const RtHittable &h = objs[i];
-        DUnbounded u{};
-        for (int a = 0; a < 3; ++a) {
-            u.p[a] = h.p[a];
-            u.n[a] = float(h.n[a]);
-        }
-        u.r2 = h.radius * h.radius; // Sphere.make, Sphere.fs:326
-        u.r = float(h.radius);
-        u.shape = h.shape;
-        classify_unbounded(u);
         device_id_of[i] = L.n_bounded + int32_t(L.unbounded.size());
-        L.unbounded.push_back(u);
-        L.materials.push_back(make_material(h, i));
+        L.unbounded.push_back(make_unbounded(objs[i]));
+        L.materials.push_back(make_material(objs[i], i));
     }
     L.device_id_of = device_id_of; // bounded spheres with negative radius keep id -1: they can never be returned
     (void)sah_tree_out; // the inspection form of the tree is made on first request (scene_ensure_sah_tree)
@@ -736,6 +696,81 @@ void scene_ensure_reference(RtScene *s) {
     }
 }
 
+// Scene.make's preconditions on one object (shape, style, plane cases, texture index, finite coordinates)
+int check_object(const RtHittable &h, int32_t i, int32_t n_textures, const char *who) {
+    if (h.shape < RT_SHAPE_SPHERE || h.shape > RT_SHAPE_INFINITE_PLANE)
+        return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": object " + std::to_string(i) + " has an unknown shape");
+    if (h.style < RT_STYLE_LIGHT_SOURCE || h.style > RT_STYLE_GLASS)
+        return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": object " + std::to_string(i) + " has an unknown style");
+    if (h.shape == RT_SHAPE_INFINITE_PLANE) {
+        // InfinitePlaneStyle has four cases only (InfinitePlane.fs:3-13, F13)
+        if (h.style == RT_STYLE_LIGHT_SOURCE_CAP || h.style == RT_STYLE_DIELECTRIC || h.style == RT_STYLE_GLASS)
+            return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": object " + std::to_string(i) + ": InfinitePlaneStyle has no such case");
+        double nn = h.n[0] * h.n[0] + h.n[1] * h.n[1] + h.n[2] * h.n[2];
+        if (std::fabs(nn - 1.0) > 1e-6)
+            return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": object " + std::to_string(i) + ": plane normal must be a unit vector");
+        if (h.style != RT_STYLE_LIGHT_SOURCE && h.texture >= 0)
+            return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": object " + std::to_string(i) + ": reflecting planes carry a colour, not a texture");
+    }
+    if (h.texture >= n_textures) return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": object " + std::to_string(i) + " references a missing texture");
+    for (int a = 0; a < 3; ++a)
+        if (!std::isfinite(h.p[a])) return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": object " + std::to_string(i) + " has a non-finite coordinate");
+    if (h.shape != RT_SHAPE_INFINITE_PLANE && !std::isfinite(h.radius))
+        return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": object " + std::to_string(i) + " has a non-finite radius");
+    return RT_OK;
+}
+
+// the texture table: image sizes, checker sub-texture indices, map radii, and no checker cycle or nest deeper than the device follows
+int check_textures(const RtTexture *textures, int32_t n_textures, const char *who) {
+    for (int32_t t = 0; t < n_textures; ++t) {
+        const RtTexture &x = textures[t];
+        if (x.kind == RT_TEX_IMAGE) {
+            if (x.width <= 0 || x.height <= 0 || !x.rgb8) return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": image texture " + std::to_string(t) + " is empty");
+        } else if (x.kind == RT_TEX_CHECKERED) {
+            if (x.even < 0 || x.even >= n_textures || x.odd < 0 || x.odd >= n_textures || x.even == t || x.odd == t)
+                return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": checkered texture " + std::to_string(t) + " has bad sub-textures");
+        } else if (x.kind != RT_TEX_COLOUR) {
+            return fail(RT_ERR_UNSUPPORTED, std::string(who) + ": texture " + std::to_string(t) + " is of a kind the device cannot evaluate (closures must be baked to an image)");
+        }
+        if (x.kind != RT_TEX_COLOUR && !(std::fabs(x.map_radius) > 0.0))
+            return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": texture " + std::to_string(t) + " has map_radius 0");
+    }
+    // Checkered textures nest (Texture.fs:56-62); the device follows at most kMaxCheckerDepth levels, so deeper nests and
+    // cycles (which the reference's immutable values cannot even express) are refused here rather than rendered black
+    {
+        constexpr int kMaxCheckerDepth = 8;
+        std::vector<int> depth(size_t(n_textures), -1); // -1 unknown, -2 on the current path
+        std::vector<std::pair<int32_t, int>> stack;
+        for (int32_t root = 0; root < n_textures; ++root) {
+            if (depth[root] >= 0) continue;
+            stack.push_back({root, 0});
+            while (!stack.empty()) {
+                auto [t, phase] = stack.back();
+                const RtTexture &x = textures[t];
+                if (x.kind != RT_TEX_CHECKERED) {
+                    depth[t] = 0;
+                    stack.pop_back();
+                    continue;
+                }
+                if (phase == 0) {
+                    depth[t] = -2;
+                    stack.back().second = 1;
+                    for (int32_t c : {x.even, x.odd}) {
+                        if (depth[c] == -2) return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": checkered texture " + std::to_string(t) + " is part of a cycle");
+                        if (depth[c] == -1) stack.push_back({c, 0});
+                    }
+                } else {
+                    depth[t] = 1 + std::max(depth[x.even], depth[x.odd]);
+                    if (depth[t] > kMaxCheckerDepth)
+                        return fail(RT_ERR_UNSUPPORTED, std::string(who) + ": checkered textures nested deeper than " + std::to_string(kMaxCheckerDepth) + " levels");
+                    stack.pop_back();
+                }
+            }
+        }
+    }
+    return RT_OK;
+}
+
 } // namespace rtfs
 
 using namespace rtfs;
@@ -843,73 +878,11 @@ int rt_scene_create(const RtHittable *objects, int32_t n_objects, const RtTextur
     if (n_objects < 0 || n_textures < 0 || (n_objects > 0 && !objects) || (n_textures > 0 && !textures))
         return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_create: bad array arguments");
     for (int32_t i = 0; i < n_objects; ++i) {
-        const RtHittable &h = objects[i];
-        if (h.shape < RT_SHAPE_SPHERE || h.shape > RT_SHAPE_INFINITE_PLANE)
-            return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_create: object " + std::to_string(i) + " has an unknown shape");
-        if (h.style < RT_STYLE_LIGHT_SOURCE || h.style > RT_STYLE_GLASS)
-            return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_create: object " + std::to_string(i) + " has an unknown style");
-        if (h.shape == RT_SHAPE_INFINITE_PLANE) {
-            // InfinitePlaneStyle has four cases only (InfinitePlane.fs:3-13, F13)
-            if (h.style == RT_STYLE_LIGHT_SOURCE_CAP || h.style == RT_STYLE_DIELECTRIC || h.style == RT_STYLE_GLASS)
-                return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_create: object " + std::to_string(i) + ": InfinitePlaneStyle has no such case");
-            double nn = h.n[0] * h.n[0] + h.n[1] * h.n[1] + h.n[2] * h.n[2];
-            if (std::fabs(nn - 1.0) > 1e-6)
-                return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_create: object " + std::to_string(i) + ": plane normal must be a unit vector");
-            if (h.style != RT_STYLE_LIGHT_SOURCE && h.texture >= 0)
-                return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_create: object " + std::to_string(i) + ": reflecting planes carry a colour, not a texture");
-        }
-        if (h.texture >= n_textures) return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_create: object " + std::to_string(i) + " references a missing texture");
-        for (int a = 0; a < 3; ++a)
-            if (!std::isfinite(h.p[a])) return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_create: object " + std::to_string(i) + " has a non-finite coordinate");
-        if (h.shape != RT_SHAPE_INFINITE_PLANE && !std::isfinite(h.radius))
-            return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_create: object " + std::to_string(i) + " has a non-finite radius");
+        int rc = check_object(objects[i], i, n_textures, "rt_scene_create");
+        if (rc != RT_OK) return rc;
     }
-    for (int32_t t = 0; t < n_textures; ++t) {
-        const RtTexture &x = textures[t];
-        if (x.kind == RT_TEX_IMAGE) {
-            if (x.width <= 0 || x.height <= 0 || !x.rgb8) return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_create: image texture " + std::to_string(t) + " is empty");
-        } else if (x.kind == RT_TEX_CHECKERED) {
-            if (x.even < 0 || x.even >= n_textures || x.odd < 0 || x.odd >= n_textures || x.even == t || x.odd == t)
-                return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_create: checkered texture " + std::to_string(t) + " has bad sub-textures");
-        } else if (x.kind != RT_TEX_COLOUR) {
-            return fail(RT_ERR_UNSUPPORTED, "rt_scene_create: texture " + std::to_string(t) + " is of a kind the device cannot evaluate (closures must be baked to an image)");
-        }
-        if (x.kind != RT_TEX_COLOUR && !(std::fabs(x.map_radius) > 0.0))
-            return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_create: texture " + std::to_string(t) + " has map_radius 0");
-    }
-    // Checkered textures nest (Texture.fs:56-62); the device follows at most kMaxCheckerDepth levels, so deeper nests and
-    // cycles (which the reference's immutable values cannot even express) are refused here rather than rendered black
-    {
-        constexpr int kMaxCheckerDepth = 8;
-        std::vector<int> depth(size_t(n_textures), -1); // -1 unknown, -2 on the current path
-        std::vector<std::pair<int32_t, int>> stack;
-        for (int32_t root = 0; root < n_textures; ++root) {
-            if (depth[root] >= 0) continue;
-            stack.push_back({root, 0});
-            while (!stack.empty()) {
-                auto [t, phase] = stack.back();
-                const RtTexture &x = textures[t];
-                if (x.kind != RT_TEX_CHECKERED) {
-                    depth[t] = 0;
-                    stack.pop_back();
-                    continue;
-                }
-                if (phase == 0) {
-                    depth[t] = -2;
-                    stack.back().second = 1;
-                    for (int32_t c : {x.even, x.odd}) {
-                        if (depth[c] == -2) return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_create: checkered texture " + std::to_string(t) + " is part of a cycle");
-                        if (depth[c] == -1) stack.push_back({c, 0});
-                    }
-                } else {
-                    depth[t] = 1 + std::max(depth[x.even], depth[x.odd]);
-                    if (depth[t] > kMaxCheckerDepth)
-                        return fail(RT_ERR_UNSUPPORTED, "rt_scene_create: checkered textures nested deeper than " + std::to_string(kMaxCheckerDepth) + " levels");
-                    stack.pop_back();
-                }
-            }
-        }
-    }
+    int rc = check_textures(textures, n_textures, "rt_scene_create");
+    if (rc != RT_OK) return rc;
     auto *s = new RtScene();
     s->objects.assign(objects, objects + n_objects);
     s->textures.assign(textures, textures + n_textures);
@@ -948,12 +921,14 @@ void rt_scene_destroy(RtScene *scene) {
 
 int rt_scene_bvh_node_count(const RtScene *scene, int32_t which) {
     if (!scene) return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_bvh_node_count: null scene");
+    if (int rc = device_scene_sync_layout(const_cast<RtScene *>(scene)); rc != RT_OK) return rc;
     if (which == RT_BVH_REFERENCE) scene_ensure_reference(const_cast<RtScene *>(scene));
     else scene_ensure_sah_tree(const_cast<RtScene *>(scene));
     return int(which == RT_BVH_REFERENCE ? scene->ref_tree.size() : scene->sah_tree.size());
 }
 int rt_scene_bvh_nodes(const RtScene *scene, int32_t which, double *bounds, int32_t *right, int32_t *prim) {
     if (!scene || !bounds || !right || !prim) return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_bvh_nodes: null argument");
+    if (int rc = device_scene_sync_layout(const_cast<RtScene *>(scene)); rc != RT_OK) return rc;
     if (which == RT_BVH_REFERENCE) scene_ensure_reference(const_cast<RtScene *>(scene));
     else scene_ensure_sah_tree(const_cast<RtScene *>(scene));
     const auto &t = which == RT_BVH_REFERENCE ? scene->ref_tree : scene->sah_tree;
@@ -973,6 +948,7 @@ size_t rt_scene_device_bytes(const RtScene *scene) { return scene ? device_scene
 // slot, and the decoded box of every slot contains all the spheres below it (each plane decoded as p + q 2^e).
 int rt_scene_wide_bvh_check(RtScene *scene, int32_t *n_nodes, int32_t *depth, int32_t *n_spheres, double *mean_children) {
     if (!scene) return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_wide_bvh_check: null scene");
+    if (int rc = device_scene_sync_layout(scene); rc != RT_OK) return rc;
     HostSceneLayout &L = scene->layout;
     build_wide_layout(L);
     std::vector<int> seen(size_t(L.n_bounded), 0);
@@ -1040,10 +1016,21 @@ int rt_scene_wide_bvh_check(RtScene *scene, int32_t *n_nodes, int32_t *depth, in
 // Checks the nodes as the DEVICE will read them (device_node_of: centre / half-extent boxes, left and right child side by
 // side): every decoded box c -+ h contains the min / max box it was made from (so also every sphere below it), h >= 0, the
 // child refs are untouched, every bounded sphere is the leaf of exactly one node, and the tree is as deep as max_depth says
-// (the render kernels size their walk stacks from it).
+// (the render kernels size their walk stacks from it).  After rt_scene_update refit the tree on the device, the nodes are
+// the device's min / max boxes, and every node record the device walks must also be device_node_of of them (the device's
+// conversion is the host's).
 int rt_scene_device_bvh_check(RtScene *scene, int32_t *n_nodes, int32_t *depth, int32_t *n_spheres) {
     if (!scene) return fail(RT_ERR_INVALID_ARGUMENT, "rt_scene_device_bvh_check: null scene");
+    if (int rc = device_scene_sync_layout(scene); rc != RT_OK) return rc;
     const HostSceneLayout &L = scene->layout;
+    if (!scene->device_nodes.empty()) {
+        if (scene->device_nodes.size() != L.nodes.size()) return fail(RT_ERR_DEGENERATE, "device BVH: node count differs on the device");
+        for (size_t i = 0; i < L.nodes.size(); ++i) {
+            const DNode host = device_node_of(L.nodes[i]);
+            if (std::memcmp(&host, &scene->device_nodes[i], sizeof(DNode)) != 0)
+                return fail(RT_ERR_DEGENERATE, "device BVH: node " + std::to_string(i) + " on the device is not device_node_of its min / max boxes");
+        }
+    }
     std::vector<int> seen(size_t(L.n_bounded), 0);
     int deepest = 0;
     struct Item {

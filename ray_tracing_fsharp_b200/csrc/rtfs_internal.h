@@ -3,9 +3,19 @@
 #pragma once
 #include "../../include/rtfs_b200.h"
 
+#include <cmath>
+#include <cstddef>
 #include <cstdint>
+#include <limits>
 #include <string>
 #include <vector>
+
+// functions compiled for the host and, in the CUDA translation units, for the device too (one piece of code for both)
+#ifdef __CUDACC__
+#define RTFS_HOST_DEVICE __host__ __device__ inline
+#else
+#define RTFS_HOST_DEVICE inline
+#endif
 
 namespace rtfs {
 
@@ -51,7 +61,66 @@ static_assert(sizeof(DNode) == 64, "DNode must be 64 bytes");
 // children's values sit in adjacent, even-aligned registers after a 128-bit load, each step is ONE packed FFMA2
 // (fma.rn.f32x2, sm_100) for both boxes with the ray's constant as a broadcast operand: ten FMA-pipe instructions per visit
 // (slab_pair, rtfs_core.cuh).  device_node_of() converts, rounding the half-extent upwards so that the box never shrinks.
-DNode device_node_of(const DNode &minmax);
+
+// the FP32 value nearest v towards -inf / +inf (the directed roundings of the leaf boxes and half-extents)
+RTFS_HOST_DEVICE float round_down(double v) {
+#ifdef __CUDA_ARCH__
+    return __double2float_rd(v);
+#else
+    float f = float(v);
+    if (double(f) > v) f = std::nextafterf(f, -std::numeric_limits<float>::infinity());
+    return f;
+#endif
+}
+RTFS_HOST_DEVICE float round_up(double v) {
+#ifdef __CUDA_ARCH__
+    return __double2float_ru(v);
+#else
+    float f = float(v);
+    if (double(f) < v) f = std::nextafterf(f, std::numeric_limits<float>::infinity());
+    return f;
+#endif
+}
+
+// min / max boxes -> centre / half-extent boxes in the paired layout above, never smaller than the original.  The host
+// upload and the device refit (rtfs_edit.cu) both convert with this function, so the two give the same bytes.
+RTFS_HOST_DEVICE DNode device_node_of(const DNode &n) {
+    DNode d = n;
+    float c[2][3], h[2][3];
+    for (int side = 0; side < 2; ++side) {
+        const float *mn = side ? n.r_mn : n.l_mn, *mx = side ? n.r_mx : n.l_mx;
+        for (int a = 0; a < 3; ++a) {
+#ifdef __CUDA_ARCH__
+            const bool finite = isfinite(mn[a]) && isfinite(mx[a]);
+#else
+            const bool finite = std::isfinite(mn[a]) && std::isfinite(mx[a]);
+#endif
+            if (!finite) { // the never-entered dummy box of a one-sphere tree
+                c[side][a] = 1e30f;
+                h[side][a] = 0.f;
+                continue;
+            }
+            const float cf = float(0.5 * (double(mn[a]) + double(mx[a])));
+            const double lo = double(cf) - double(mn[a]), hi = double(mx[a]) - double(cf);
+            const float hf = round_up(hi < lo ? lo : hi);
+            c[side][a] = cf;
+#ifdef __CUDA_ARCH__
+            h[side][a] = nextafterf(hf, __int_as_float(0x7f800000));
+#else
+            h[side][a] = std::nextafterf(hf, std::numeric_limits<float>::infinity());
+#endif
+        }
+    }
+    // {c.x l, c.x r, c.y l, c.y r | c.z l, c.z r, h.x l, h.x r | h.y l, h.y r, h.z l, h.z r}: the twelve floats of the struct in order
+    float *q = d.l_mn;
+    static_assert(offsetof(DNode, left) == 12 * sizeof(float), "the twelve box floats are contiguous");
+    for (int a = 0; a < 3; ++a)
+        for (int side = 0; side < 2; ++side) {
+            q[2 * a + side] = c[side][a];
+            q[6 + 2 * a + side] = h[side][a];
+        }
+    return d;
+}
 
 // Per-primitive material record, 32 B = two 128-bit loads.  Index = device primitive id.
 struct DMaterial {
@@ -64,6 +133,8 @@ struct DMaterial {
     int32_t host_index; // index into the caller's Hittable array
 };
 static_assert(sizeof(DMaterial) == 32, "DMaterial must be 32 bytes");
+// the material record of object host_index
+DMaterial make_material(const RtHittable &h, int32_t host_index);
 
 // Unbounded objects (UnboundedSphere, InfinitePlane), tested linearly after the tree (Scene.fs:77-86).
 // These spheres are typically huge (r = 1000, 2000), and |o - c|^2 - r^2 evaluated from o - c cancels catastrophically
@@ -85,6 +156,8 @@ struct DUnbounded {
 };
 // fills fp32 / k (and n for spheres) of an object whose p, r, r2, n, shape are set
 void classify_unbounded(DUnbounded &u);
+// the device record of an unbounded object (UnboundedSphere, InfinitePlane), classified
+DUnbounded make_unbounded(const RtHittable &h);
 static_assert(sizeof(DUnbounded) == 64, "DUnbounded must be 64 bytes");
 
 struct DTexture {
@@ -152,6 +225,9 @@ struct HostSceneLayout {
 // inverted box and is never hit in the reference, F16).  Fills layout.spheres/nodes and the bounded
 // part of layout.materials; also exports the tree in HostNode form for inspection.
 void build_device_layout(const RtHittable *objs, int32_t n_objs, HostSceneLayout &layout, std::vector<HostNode> &sah_tree_out);
+// The checks rt_scene_create makes of one object and of the texture table; `who` names the caller in the message.
+int check_object(const RtHittable &h, int32_t i, int32_t n_textures, const char *who);
+int check_textures(const RtTexture *textures, int32_t n_textures, const char *who);
 // Collapses the SAH BVH2 of `layout` into the 8-wide compressed tree (fills layout.wide_*).  Idempotent.
 void build_wide_layout(HostSceneLayout &layout);
 // (built on first use: a render with RT_FLAG_WIDE_BVH, rt_test_hit_object(traversal = 2), rt_scene_wide_bvh_check)
@@ -169,6 +245,12 @@ struct RtScene {
     rtfs::HostSceneLayout layout;
     int32_t device = -1;
     void *dev = nullptr; // rtfs_device.cu: DeviceScene*
+    // rt_scene_update (rtfs_edit.cu): the edit count, which progressive frames record when they open; after a refit the
+    // tree's boxes live on the device and layout.nodes is stale until device_scene_sync_layout downloads them, together with
+    // the node records the device walks (device_nodes, which rt_scene_device_bvh_check holds to device_node_of)
+    uint64_t generation = 0;
+    bool layout_stale = false;
+    std::vector<rtfs::DNode> device_nodes;
 };
 
 // implemented in rtfs_device.cu
@@ -178,6 +260,8 @@ void scene_ensure_sah_tree(RtScene *scene);
 int device_scene_upload(RtScene *scene);
 int device_scene_ensure_reference(RtScene *scene);
 int device_scene_ensure_wide(RtScene *scene);
+// brings layout.nodes (and scene->device_nodes) up to date after rt_scene_update refit the tree (rtfs_edit.cu)
+int device_scene_sync_layout(RtScene *scene);
 void device_scene_free(RtScene *scene);
 size_t device_scene_bytes(const RtScene *scene);
 } // namespace rtfs

@@ -10,7 +10,8 @@ import os
 import numpy as np
 
 from . import abi
-from .abi import RtCamera, RtDenoiseOpts, RtFrameConvergence, RtFrameNoise, RtFrameProgress, RtHittable, RtRenderOpts, RtStats, RtTexture
+from .abi import (RtCamera, RtDenoiseOpts, RtFrameConvergence, RtFrameNoise, RtFrameProgress, RtHittable, RtRenderOpts, RtSceneUpdate, RtStats,
+                  RtTexture)
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "librtfs_b200.so")
@@ -47,6 +48,7 @@ def _declare(lib):
         "rt_scene_device_bvh_check": (C.c_int, [_vp, C.POINTER(_i32), C.POINTER(_i32), C.POINTER(_i32)]),
         "rt_scene_device_bytes": (C.c_size_t, [_vp]),
         "rt_scene_shared_memory_bytes": (C.c_size_t, [_vp]),
+        "rt_scene_update": (C.c_int, [_vp, _vp, _vp, _i32, _vp, _vp, _i32, C.POINTER(RtSceneUpdate)]),
         "rt_render": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _vp, _vp, C.POINTER(RtStats)]),
         "rt_render_views": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(RtRenderOpts), _vp, _vp, C.POINTER(RtStats)]),
         "rt_frame_begin": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), C.POINTER(_vp),
@@ -219,6 +221,23 @@ class SceneHandle:
         except Exception:
             pass
 
+    def update(self, object_index, hittables, texture_index=None, textures=None) -> RtSceneUpdate:
+        """Edits the scene on its device (rt_scene_update): object object_index[i] becomes hittables[i], texture
+        texture_index[j] becomes textures[j], and the tree is refit there.  The scene then renders bit for bit as one
+        created from the edited arrays.  Structural changes (shape, the sign of a bounded sphere's radius, a texture's kind or
+        image size), bad or repeated indices and anything creation refuses: RtError RT_ERR_INVALID_ARGUMENT, the scene left
+        as it was.  Frames opened before the call are stale (see Frame).  Returns the RtSceneUpdate."""
+        oi = np.ascontiguousarray(list(object_index), np.int32)
+        ti = np.ascontiguousarray(list(texture_index) if texture_index is not None else [], np.int32)
+        textures = list(textures) if textures is not None else []
+        if len(hittables) != len(oi) or len(textures) != len(ti):
+            raise ValueError("one record per index")
+        h = _as_array(RtHittable, hittables)
+        t = _as_array(RtTexture, textures)
+        info = RtSceneUpdate()
+        check(lib().rt_scene_update(self.ptr, ptr(oi), h, len(oi), ptr(ti), t, len(ti), C.byref(info)))
+        return info
+
     def bvh_nodes(self, which=abi.RT_BVH_SAH):
         n = lib().rt_scene_bvh_node_count(self.ptr, which)
         bounds = np.empty((n, 6))
@@ -379,7 +398,9 @@ class Frame:
     sample indices.  After every pass the frame is exactly rt_render's at samples_per_pixel = progress.samples_done.
     Holds its scene handle, so the scene outlives it.  A frame of a batch of views (SceneHandle.open_frame_views) has
     n_views set, and its images, sums and maps carry a leading view axis; a frame of a window (SceneHandle.open_frame_window)
-    has the window's rows and cols."""
+    has the window's rows and cols.  Once its scene is edited (SceneHandle.update) the frame is stale: advance, extend,
+    set_convergence, features and denoise raise RtError RT_ERR_INVALID_ARGUMENT; read, noise, view_noise and convergence
+    still return what it holds."""
 
     n_views = None  # a frame of one camera
 

@@ -5,6 +5,7 @@ reference's.  Everything that computes goes through the C ABI (native.py); nothi
 
   Camera.make_basic     RayTracing/Camera.fs:34-59
   Scene.make            RayTracing/Scene.fs:15-28
+  Scene.update          Scene.make of an edited object list, done in place on the device (rt_scene_update)
   Scene.render          RayTracing/Scene.fs:196-236
   Scene.render_views    Scene.render of many cameras of one scene in one submission (rt_render_views)
   Scene.render_progressive  the same frame in sample passes, progress ticks as passes finish (native.Frame)
@@ -13,6 +14,7 @@ reference's.  Everything that computes goes through the C ABI (native.py); nothi
   Image / Image.render  RayTracing/Domain.fs:9-31
   ImageOutput.write_ppm RayTracing/ImageOutput.fs:163-197, PixelOutput.correct :11-18
 """
+import ctypes as C
 import os
 import secrets
 from dataclasses import dataclass
@@ -81,6 +83,32 @@ class Scene:
     @property
     def handle(self):
         return self._handle
+
+    @staticmethod
+    def update(s: "Scene", objects) -> abi.RtSceneUpdate:
+        """The scene Scene.make(objects) would give, made in place: `objects` is the whole new object list (as F# holds it, an
+        immutable array).  It is marshalled and diffed against the scene's current records, and only the changed objects and
+        textures go to the device (rt_scene_update), which refits the tree there; the scene then renders bit for bit as
+        Scene.make(objects).  The structure must stay: the object count, each object's shape, the sign of each bounded
+        sphere's radius, and the texture table (its size, each texture's kind, an image's size); otherwise ValueError (make a
+        new scene).  Progressive frames opened before the call are stale.  A scene made with devices=[...] (several GPUs):
+        NotImplementedError.  Returns the RtSceneUpdate."""
+        if not isinstance(s._handle, native.SceneHandle):
+            raise NotImplementedError("Scene.update edits a scene of one device; make a scene split over devices=[...] anew")
+        hittables, textures, keep = marshal(objects)
+        if len(hittables) != len(s._hittables):
+            raise ValueError(f"Scene.update: {len(hittables)} objects for a scene of {len(s._hittables)}: make a new scene")
+        if len(textures) != len(s._textures) or any(_texture_shape(a) != _texture_shape(b) for a, b in zip(textures, s._textures)):
+            raise ValueError("Scene.update: the texture table changes its structure (count, kinds or image sizes): make a new scene")
+        size = C.sizeof(abi.RtHittable)
+        new = np.frombuffer(hittables, np.uint8).reshape(-1, size) if len(hittables) else np.zeros((0, size), np.uint8)
+        old = np.frombuffer(s._hittables, np.uint8).reshape(-1, size) if len(s._hittables) else np.zeros((0, size), np.uint8)
+        changed = np.nonzero((new != old).any(axis=1))[0].tolist()
+        tex_changed = [j for j, (a, b) in enumerate(zip(textures, s._textures)) if not _same_texture(a, b)]
+        info = s._handle.update(changed, [hittables[i] for i in changed], tex_changed, [textures[j] for j in tex_changed])
+        s._hittables, s._textures, s._keep = hittables, textures, keep
+        s._handle._h, s._handle._t, s._handle._keep = hittables, native._as_array(abi.RtTexture, textures), keep
+        return info
 
     @staticmethod
     def render(progress_increment: Callable[[float], None], print_fn: Callable[[str], None], max_width_coord: int, max_height_coord: int,
@@ -315,6 +343,25 @@ class Scene:
             rgb, _ = frame.read()
         emit(ticks.finish())
         return [rgb[v] for v in range(n)]
+
+
+def _texture_shape(t: abi.RtTexture):
+    """What rt_scene_update must keep of a texture: its kind and, for an image, its size."""
+    return (t.kind, t.width, t.height) if t.kind == abi.RT_TEX_IMAGE else (t.kind,)
+
+
+def _texels(t: abi.RtTexture) -> bytes:
+    return C.string_at(t.rgb8, t.width * t.height * 3) if t.kind == abi.RT_TEX_IMAGE else b""
+
+
+def _same_texture(a: abi.RtTexture, b: abi.RtTexture) -> bool:
+    """Every field but the texel pointer, and the texels."""
+    fields = [f for f, _ in abi.RtTexture._fields_ if f != "rgb8"]
+    return all(_plain(getattr(a, f)) == _plain(getattr(b, f)) for f in fields) and _texels(a) == _texels(b)
+
+
+def _plain(v):
+    return list(v) if isinstance(v, C.Array) else v
 
 
 class ProgressTicks:

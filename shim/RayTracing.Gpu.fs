@@ -153,6 +153,17 @@ module internal Native =
         val mutable gamma : int
         val mutable pad0 : int
 
+    [<Struct ; StructLayout(LayoutKind.Sequential)>]
+    type RtSceneUpdate =
+        val mutable objects : int
+        val mutable textures : int
+        val mutable spheresMoved : int
+        val mutable nodesRefit : int
+        val mutable generation : uint64
+        val mutable deviceMs : float
+        val mutable launches : int
+        val mutable pad0 : int
+
 
     [<DllImport(Lib)>]
     extern nativeint rt_last_error ()
@@ -165,6 +176,9 @@ module internal Native =
 
     [<DllImport(Lib)>]
     extern void rt_scene_destroy (nativeint scene)
+
+    [<DllImport(Lib)>]
+    extern int rt_scene_update (nativeint scene, int[] objectIndex, RtHittable[] objects, int nObjects, int[] textureIndex, RtTexture[] textures, int nTextures, RtSceneUpdate& info)
 
     [<DllImport(Lib)>]
     extern int rt_render (nativeint scene, RtCamera& camera, int maxWidthCoord, int maxHeightCoord, RtRenderOpts& opts, byte[] rgbOut, nativeint sumsOut, RtStats& stats)
@@ -307,6 +321,11 @@ type GpuScene =
             Handle : nativeint
             IsMulti : bool
             Pins : GCHandle list
+            /// the records the scene was made or last updated from, and each image texture's texels (null for the other
+            /// kinds): SceneGpu.update diffs the new records against them
+            mutable Hittables : Native.RtHittable[]
+            mutable Textures : Native.RtTexture[]
+            mutable Texels : byte[][]
         }
 
     interface IDisposable with
@@ -474,8 +493,9 @@ module GpuScene =
 
         h
 
-    /// Counterpart of Scene.make (Scene.fs:15-28).  `devices`: CUDA ordinals; more than one splits every frame.
-    let makeOn (devices : int[]) (objects : Hittable array) : GpuScene =
+    /// The Hittable and texture records of `objects`, each image texture's texels (null for the other kinds), and the pins
+    /// that hold the texels in place while the library copies them.
+    let internal marshal (objects : Hittable array) =
         let textures = ResizeArray<Native.RtTexture> ()
         let pins = ResizeArray<GCHandle> ()
 
@@ -488,16 +508,31 @@ module GpuScene =
                 | Hittable.InfinitePlane p -> marshalPlane textures pins p
             )
 
+        let texels =
+            textures.ToArray ()
+            |> Array.map (fun t ->
+                if t.kind = 1 then
+                    pins |> Seq.find (fun p -> p.AddrOfPinnedObject () = t.rgb8) |> fun p -> p.Target :?> byte[]
+                else
+                    null
+            )
+
+        hittables, textures.ToArray (), texels, pins
+
+    /// Counterpart of Scene.make (Scene.fs:15-28).  `devices`: CUDA ordinals; more than one splits every frame.
+    let makeOn (devices : int[]) (objects : Hittable array) : GpuScene =
+        let hittables, textures, texels, pins = marshal objects
+
         let texArr =
-            if textures.Count = 0 then Array.zeroCreate 1 else textures.ToArray ()
+            if textures.Length = 0 then Array.zeroCreate 1 else textures
 
         let mutable handle = 0n
 
         if devices.Length > 1 then
-            Native.rt_multi_create (hittables, hittables.Length, texArr, textures.Count, devices, devices.Length, &handle)
+            Native.rt_multi_create (hittables, hittables.Length, texArr, textures.Length, devices, devices.Length, &handle)
             |> Native.check
         else
-            Native.rt_scene_create (hittables, hittables.Length, texArr, textures.Count, devices.[0], &handle)
+            Native.rt_scene_create (hittables, hittables.Length, texArr, textures.Length, devices.[0], &handle)
             |> Native.check
 
         // the library copies everything it needs during create, so the pins can be released straight away
@@ -508,9 +543,29 @@ module GpuScene =
             Handle = handle
             IsMulti = devices.Length > 1
             Pins = []
+            Hittables = hittables
+            Textures = textures
+            Texels = texels
         }
 
     let make (objects : Hittable array) : GpuScene = makeOn [| 0 |] objects
+
+/// What SceneGpu.update changed (RtSceneUpdate, include/rtfs_b200.h).
+type SceneUpdate =
+    {
+        /// object records that changed
+        Objects : int
+        /// texture records that changed
+        Textures : int
+        /// bounded spheres whose device sphere (FP32 centre, radius) changed
+        SpheresMoved : int
+        /// tree nodes whose child boxes were recomputed
+        NodesRefit : int
+        /// the scene's edit count after the call (0 = as made)
+        Generation : uint64
+        /// device time of the copy and the kernels (CUDA events)
+        DeviceMs : float
+    }
 
 /// RtRenderOpts.flags bits a caller may pass to SceneGpu.openFrameWith (include/rtfs_b200.h, RT_FLAG_*).
 [<RequireQualifiedAccess>]
@@ -979,6 +1034,75 @@ module SceneGpu =
         |> Native.check
 
         new GpuFrame (handle, rows, cols, 1, progress)
+
+    /// The scene GpuScene.make would give for `objects` (the whole new object list), made in place on the device
+    /// (rt_scene_update): the list is marshalled and diffed against the scene's current records, and only the changed objects
+    /// and textures are sent; the device refits the tree.  The scene then renders bit for bit as GpuScene.make objects.  The
+    /// structure must stay (the object count, each object's shape, the sign of each bounded sphere's radius, the texture
+    /// table's size, kinds and image sizes); a structural change fails, as does a multi-GPU scene.  Frames opened before the
+    /// call are stale: GpuFrame.Advance and the calls that trace fail on them.
+    let update (s : GpuScene) (objects : Hittable array) : SceneUpdate =
+        if s.IsMulti then
+            failwith "GPU backend: SceneGpu.update edits a single-device GpuScene; make a multi-GPU scene anew"
+
+        let hittables, textures, texels, pins = GpuScene.marshal objects
+
+        try
+            let sameShape (a : Native.RtTexture) (b : Native.RtTexture) =
+                a.kind = b.kind && (a.kind <> 1 || (a.width = b.width && a.height = b.height))
+
+            if hittables.Length <> s.Hittables.Length
+               || textures.Length <> s.Textures.Length
+               || not (Array.forall2 sameShape textures s.Textures) then
+                failwith "GPU backend: SceneGpu.update keeps the scene's structure (object count, texture table); make a new scene"
+
+            let sameTexture (j : int) =
+                let a, b = textures.[j], s.Textures.[j]
+
+                a.kind = b.kind && a.colourR = b.colourR && a.colourG = b.colourG && a.colourB = b.colourB
+                && a.even = b.even && a.odd = b.odd && a.gridSize = b.gridSize && a.mapCentreX = b.mapCentreX
+                && a.mapCentreY = b.mapCentreY && a.mapCentreZ = b.mapCentreZ && a.mapRadius = b.mapRadius
+                && (a.kind <> 1 || texels.[j] = s.Texels.[j])
+
+            let objectIndex =
+                [| for i in 0 .. hittables.Length - 1 do
+                       if hittables.[i] <> s.Hittables.[i] then
+                           yield i |]
+
+            let textureIndex =
+                [| for j in 0 .. textures.Length - 1 do
+                       if not (sameTexture j) then
+                           yield j |]
+
+            let mutable info = Native.RtSceneUpdate ()
+            // the pins hold the new texels in place until the call returns (the library copies them)
+            Native.rt_scene_update (
+                s.Handle,
+                objectIndex,
+                Array.map (fun i -> hittables.[i]) objectIndex,
+                objectIndex.Length,
+                textureIndex,
+                Array.map (fun j -> textures.[j]) textureIndex,
+                textureIndex.Length,
+                &info
+            )
+            |> Native.check
+
+            s.Hittables <- hittables
+            s.Textures <- textures
+            s.Texels <- texels
+
+            {
+                Objects = info.objects
+                Textures = info.textures
+                SpheresMoved = info.spheresMoved
+                NodesRefit = info.nodesRefit
+                Generation = info.generation
+                DeviceMs = info.deviceMs
+            }
+        finally
+            for p in pins do
+                p.Free ()
 
     // the frame of renderWithProgressUntil and renderConverging: passes of about 250 ms with progress ticks, an optional
     // convergence rule (tolerance, minSamples, interval) and an optional stop on the noise summary (tolerance, fraction)

@@ -558,6 +558,35 @@ int rt_multi_render(RtMulti *multi, const RtCamera *camera, int32_t max_width_co
                     int32_t max_height_coord, const RtRenderOpts *opts, uint8_t *rgb_out,
                     int32_t *sums_out, RtStats *stats);
 void rt_multi_destroy(RtMulti *multi);
+/* A progressive frame split over the devices of an RtMulti: rt_frame_begin's frame, with its passes, noise estimate,
+ * convergence rule, features and denoised previews, at the speed of several GPUs.
+ *
+ * This function was added without a change of RT_ABI_VERSION (still 6): no struct and no existing prototype changed.  A
+ * caller detects the feature by the presence of the symbol rt_multi_frame_begin.
+ *
+ * It returns an ordinary RtFrame: rt_frame_advance, _read, _extend, _noise, _view_noise (one entry), _set_convergence,
+ * _convergence, _features, _denoise and _destroy take it unchanged.
+ *   Arguments, modes and refusals are rt_frame_begin's, checked before any device work: RT_MODE_WAVEFRONT and RT_FLAG_NOISE
+ *   with RT_FLAG_FLOW or RT_FLAG_COUNTERS are RT_ERR_UNSUPPORTED; a NULL multi or out is RT_ERR_INVALID_ARGUMENT, and *out
+ *   is NULL after any failure.  RT_FLAG_FLOW and RT_FLAG_COUNTERS without RT_FLAG_NOISE are accepted and act as in
+ *   rt_frame_begin (the split kernels of rt_multi_render).
+ * Exactness.  Device r probes the tiles t with t mod world == r and, in a pass over [s, s + k), traces the sample
+ *   indices s + r + j world (j >= 0) into buffers of its own; the sums, counts and Q are integers keyed by (seed, pixel, sample index), and the first device sums
+ *   them over the devices before anything reads them.  So after every pass, and under a convergence rule, the frame is bit
+ *   for bit rt_frame_begin's frame of the same camera, extents, opts and rule on one device of the same scene: sums,
+ *   counts, RGB8 and gamma RGB8; Q, the E map and the RtFrameNoise summary (the same fixed-order reduction, on the first
+ *   device); every field of RtFrameProgress and RtFrameConvergence except the _ms fields and passes; rt_frame_features and
+ *   rt_frame_denoise.  This holds for every device count: only the number of passes may depend on it.
+ * Pacing.  As rt_frame_begin's, with the device time per sample index of the slowest device; a paced window that neither
+ *   max_samples, a checkpoint nor the target cuts is rounded down to a multiple of the device count when it holds at least
+ *   that many indices, so that no device idles.
+ * Timing.  last_pass_ms is the largest of the devices' own spans of the pass (as rt_multi_render's kernel_ms), device_ms
+ *   the sum of those pass times and the slowest device's probe.
+ * Ownership.  The frame owns its buffers on every device (about 29 bytes per pixel on each, 25 more on the first), so
+ *   rt_multi_render and other frames may run on the same RtMulti between two passes.  Every call returns with its device
+ *   work complete on every device.  The frame must be destroyed before its RtMulti. */
+int rt_multi_frame_begin(RtMulti *multi, const RtCamera *camera, int32_t max_width_coord, int32_t max_height_coord,
+                         const RtRenderOpts *opts, RtFrame **out, RtFrameProgress *progress);
 /* create + render + destroy in one call */
 int rt_render_multi(const RtHittable *objects, int32_t n_objects, const RtTexture *textures,
                     int32_t n_textures, const int32_t *devices, int32_t n_devices,

@@ -290,6 +290,22 @@ struct ReduceTargets {
 };
 int launch_reduce_finalize(const ReduceTargets &t, int rank, size_t n_pixels, int gamma, cudaStream_t st, int *launches);
 
+// The exchange of a progressive frame split over ranks (rt_multi_frame_begin), for one rank's slice of the pixels: sum the
+// ranks' int4 sums and uint64 Q (sq null: no Q) into the totals on the first device, and at the probe (flags non-null) OR
+// the ranks' probe flags into total_flags.  Integer sums, so the totals are those of one device.  (rtfs_multi.cu)
+struct GatherTargets {
+    const int32_t *stats[kMaxDevices];
+    const unsigned long long *sq[kMaxDevices];
+    const uint8_t *flags[kMaxDevices];
+    int32_t world;
+    int32_t *total_stats;
+    unsigned long long *total_sq;
+    uint8_t *total_flags;
+};
+int launch_gather(const GatherTargets &t, int rank, size_t n_pixels, cudaStream_t st);
+// the replicas of an RtMulti's scene, in rank order (rtfs_multi.cu)
+const std::vector<RtScene *> &multi_scenes(const RtMulti *m);
+
 // PixelOutput.correct (ImageOutput.fs:11-18): the block fills `lut` with the 8-bit output of every mean, gamma or not
 __device__ __forceinline__ void fill_gamma_lut(uint8_t *lut, int gamma) {
     for (int i = threadIdx.x; i < 256; i += blockDim.x) {

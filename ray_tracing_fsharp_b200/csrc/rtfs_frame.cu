@@ -14,6 +14,9 @@
 // rt_frame_features and rt_frame_denoise (kernels in rtfs_denoise.cu) read the frame and keep buffers of their own.
 // A frame records its scene's edit count: once rt_scene_update has changed the scene, the calls that would trace or read the
 // scene refuse the frame, and the others keep working on what it holds.
+// rt_multi_frame_begin opens the same frame split over the devices of an RtMulti (FramePart, below; the exchange kernel is
+// in rtfs_multi.cu): rank r probes its tiles and traces its sample indices into buffers of its own, and the totals, the
+// shared flags and everything that reads them live on the first device.
 #include "rtfs_device.h"
 
 #include <algorithm>
@@ -92,10 +95,32 @@ __global__ void __launch_bounds__(256) converge_kernel(const int4 *stats, const 
     if (pixel_standard_error(s.w, s.x, s.y, s.z, sq[p]) <= tolerance) flags[p] = 0;
 }
 
+// One device's part of a frame split over the devices of an RtMulti (rt_multi_frame_begin): rank r of world traces the
+// tiles t with t mod world == r in the probe and, in a pass over [s, s + k), the sample indices s + r + j world, into sums, Q,
+// flags, a list and a counter block of its own on its device.
+struct FramePart {
+    RtScene *scene = nullptr; // the rank's replica; its workspace's stream carries the rank's work
+    FrameParams fp;
+    int32_t *d_stats = nullptr;
+    unsigned long long *d_sq = nullptr;
+    uint8_t *d_flags = nullptr;
+    uint32_t *d_list = nullptr;
+    unsigned long long *d_counters = nullptr;
+    unsigned long long h_counters[CN_SLOTS] = {};
+    FrameEvents ev;                 // the probe: ZEROED -> END; a pass: BEGIN -> END
+    cudaEvent_t traced = nullptr;   // the rank's samples so far are in its sums and Q
+    cudaEvent_t gathered = nullptr; // the rank's slice of the totals is written
+    cudaEvent_t listed = nullptr;   // (rank 0) the shared flags are final: the ranks may compact from them
+};
+
 } // namespace rtfs
 
 // A frame owns everything a pass writes: sums, flags, the flagged-pixel list, the image and its own counter block
 // (paths, rays, the list length and the work cursors), so rt_render and other frames can use the scene between passes.
+// A frame split over several devices (rt_multi_frame_begin) also owns one FramePart per device; its own sums and Q are then
+// the totals of the parts on the first device, its flags the flags every part compacts from, and every call that reads
+// the frame gathers the totals first.  The noise estimate, the check's converge_kernel, the features, the filter and the
+// read all run on the first device, over those buffers, exactly as on a frame of one device.
 struct RtFrame {
     RtScene *scene = nullptr;
     FrameParams fp;
@@ -128,12 +153,28 @@ struct RtFrame {
     int32_t conv_min = 0, conv_interval = 0, conv_checks = 0;
     uint64_t pixels_active = 0; // pixels still being sampled: the list's length (pixels_flagged until a check)
     uint64_t generation = 0;    // the scene's edit count when the frame opened (rt_scene_update)
+    std::vector<FramePart> parts; // rt_multi_frame_begin: one per device, in rank order (empty: a frame of one device)
+    bool gathered = true;         // the totals hold every part's samples
 };
 
 namespace {
 
 void frame_free(RtFrame *f) {
     if (!f) return;
+    for (FramePart &p : f->parts) {
+        if (!p.scene) continue; // (an opener that failed before reaching this part)
+        auto *pds = static_cast<DeviceScene *>(p.scene->dev);
+        cudaSetDevice(pds->device);
+        cudaStreamSynchronize(pds->ws->stream);
+        cudaFree(p.d_stats);
+        cudaFree(p.d_sq);
+        cudaFree(p.d_flags);
+        cudaFree(p.d_list);
+        cudaFree(p.d_counters);
+        p.ev.destroy();
+        for (cudaEvent_t e : {p.traced, p.gathered, p.listed})
+            if (e) cudaEventDestroy(e);
+    }
     auto *ds = static_cast<DeviceScene *>(f->scene->dev);
     cudaSetDevice(ds->device);
     cudaStreamSynchronize(ds->ws->stream);
@@ -255,6 +296,188 @@ int frame_open(RtScene *scene, const RtCamera &camera, const std::vector<ViewCam
     return RT_OK;
 }
 
+// ---- a frame split over the devices of an RtMulti (rt_multi_frame_begin) ----------------------------------------------
+// Devices are ordered by CUDA events only: a rank waits for the others' events on its own stream, and no kernel spins.
+
+DeviceScene *part_scene(const FramePart &p) { return static_cast<DeviceScene *>(p.scene->dev); }
+
+// The totals on the first device: once every rank's work so far is done, rank r sums its slice of the pixels of every rank
+// (launch_gather, peer loads), and at the probe also ORs the ranks' flags into the frame's flags; the first device's
+// stream then waits for every slice.
+int multi_gather(RtFrame *f, bool probe_flags) {
+    const int world = int(f->parts.size());
+    GatherTargets t{};
+    t.world = world;
+    for (int r = 0; r < world; ++r) {
+        t.stats[r] = f->parts[r].d_stats;
+        t.sq[r] = f->parts[r].d_sq;
+        t.flags[r] = f->parts[r].d_flags;
+    }
+    t.total_stats = f->d_stats;
+    t.total_sq = f->d_sq;
+    t.total_flags = probe_flags ? f->d_flags : nullptr;
+    for (FramePart &p : f->parts) {
+        RT_CUDA(cudaSetDevice(part_scene(p)->device));
+        RT_CUDA(cudaEventRecord(p.traced, part_scene(p)->ws->stream));
+    }
+    for (int r = 0; r < world; ++r) {
+        DeviceScene *ds = part_scene(f->parts[r]);
+        RT_CUDA(cudaSetDevice(ds->device));
+        for (int j = 0; j < world; ++j)
+            if (j != r) RT_CUDA(cudaStreamWaitEvent(ds->ws->stream, f->parts[j].traced, 0));
+        int rc = launch_gather(t, r, f->n_pixels, ds->ws->stream);
+        if (rc != RT_OK) return rc;
+        RT_CUDA(cudaEventRecord(f->parts[r].gathered, ds->ws->stream));
+    }
+    DeviceScene *ds0 = part_scene(f->parts[0]);
+    RT_CUDA(cudaSetDevice(ds0->device));
+    for (int j = 1; j < world; ++j) RT_CUDA(cudaStreamWaitEvent(ds0->ws->stream, f->parts[j].gathered, 0));
+    f->gathered = true;
+    return RT_OK;
+}
+
+// the totals, gathered if a pass has run since they last were (then on the first device's stream)
+int ensure_totals(RtFrame *f) { return f->parts.empty() || f->gathered ? RT_OK : multi_gather(f, false); }
+
+// After the probe (probe: the frame's flags become the OR of the ranks' probe flags) or a pass that ends on a checkpoint
+// (converge: converge_kernel clears the converged pixels' flags on the first device, as on one device): every rank compacts
+// the frame's flags into its own list, so every rank samples the same pixels.
+int multi_relist(RtFrame *f, bool probe, bool converge) {
+    int rc = multi_gather(f, probe);
+    if (rc != RT_OK) return rc;
+    cudaStream_t st0 = part_scene(f->parts[0])->ws->stream;
+    if (converge) {
+        converge_kernel<<<unsigned((f->n_pixels + 255) / 256), 256, 0, st0>>>(reinterpret_cast<const int4 *>(f->d_stats), f->d_sq, f->d_flags,
+                                                                              f->n_pixels, f->conv_tolerance);
+        RT_CUDA(cudaGetLastError());
+    }
+    RT_CUDA(cudaEventRecord(f->parts[0].listed, st0));
+    int launches = 0;
+    for (size_t r = 0; r < f->parts.size(); ++r) {
+        FramePart &p = f->parts[r];
+        DeviceScene *ds = part_scene(p);
+        RT_CUDA(cudaSetDevice(ds->device));
+        if (r) RT_CUDA(cudaStreamWaitEvent(ds->ws->stream, f->parts[0].listed, 0));
+        if ((rc = launch_compact(ds, p.fp, single_flags(f->d_flags), p.d_list, ds->ws->stream, &launches)) != RT_OK) return rc;
+    }
+    return RT_OK;
+}
+
+// Every rank: END, its counters to the host, then a synchronisation of every rank's stream.  The frame's counters are then
+// the ranks' paths summed and the shared list's length; returns the slowest rank's `from` -> END span.
+int multi_finish(RtFrame *f, FrameEvents::Which from, double *span_ms) {
+    for (FramePart &p : f->parts) {
+        DeviceScene *ds = part_scene(p);
+        RT_CUDA(cudaSetDevice(ds->device));
+        RT_CUDA(p.ev.record(FrameEvents::END, ds->ws->stream));
+        RT_CUDA(cudaMemcpyAsync(p.h_counters, p.d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ds->ws->stream));
+    }
+    *span_ms = 0.0;
+    f->h_counters[CN_PATHS] = 0;
+    for (FramePart &p : f->parts) {
+        RT_CUDA(cudaSetDevice(part_scene(p)->device));
+        RT_CUDA(cudaStreamSynchronize(part_scene(p)->ws->stream));
+        *span_ms = std::max(*span_ms, double(p.ev.ms(from, FrameEvents::END)));
+        f->h_counters[CN_PATHS] += p.h_counters[CN_PATHS];
+    }
+    f->h_counters[CN_LIST] = f->parts[0].h_counters[CN_LIST];
+    return RT_OK;
+}
+
+// rt_multi_frame_begin once its arguments are checked: the frame's totals, flags and image on the first device, one part
+// per device, the split probe and the compaction from the OR of the ranks' flags
+int multi_frame_open(RtMulti *m, const RtCamera &camera, int32_t max_w, int32_t max_h, const RtRenderOpts *opts, RtFrame **out,
+                     RtFrameProgress *progress) {
+    const std::vector<RtScene *> &scenes = multi_scenes(m);
+    const int world = int(scenes.size());
+    const bool noise = (opts->flags & RT_FLAG_NOISE) != 0;
+    int rc;
+    for (RtScene *s : scenes)
+        if ((rc = prepare_frame(s, opts)) != RT_OK) return rc;
+    auto *ds0 = static_cast<DeviceScene *>(scenes[0]->dev);
+    RT_CUDA(cudaSetDevice(ds0->device));
+    auto *f = new RtFrame();
+    f->scene = scenes[0];
+    f->generation = scenes[0]->generation;
+    auto bail = [&](int code) {
+        frame_free(f);
+        return code;
+    };
+    const size_t n = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
+    f->n_pixels = n;
+    bool ok = cudaMalloc((void **)&f->d_stats, n * 4 * sizeof(int32_t)) == cudaSuccess && cudaMalloc((void **)&f->d_flags, n) == cudaSuccess &&
+              cudaMalloc((void **)&f->d_rgb, n * 3) == cudaSuccess;
+    if (noise) ok = ok && cudaMalloc((void **)&f->d_sq, n * sizeof(unsigned long long)) == cudaSuccess;
+    f->parts.resize(size_t(world));
+    for (int r = 0; r < world && ok; ++r) {
+        FramePart &p = f->parts[size_t(r)];
+        p.scene = scenes[size_t(r)];
+        ok = cudaSetDevice(part_scene(p)->device) == cudaSuccess && cudaMalloc((void **)&p.d_stats, n * 4 * sizeof(int32_t)) == cudaSuccess &&
+             cudaMalloc((void **)&p.d_flags, n) == cudaSuccess && cudaMalloc((void **)&p.d_list, n * sizeof(uint32_t)) == cudaSuccess &&
+             cudaMalloc((void **)&p.d_counters, CN_SLOTS * sizeof(unsigned long long)) == cudaSuccess && p.ev.create() &&
+             cudaEventCreateWithFlags(&p.traced, cudaEventDisableTiming) == cudaSuccess &&
+             cudaEventCreateWithFlags(&p.gathered, cudaEventDisableTiming) == cudaSuccess &&
+             cudaEventCreateWithFlags(&p.listed, cudaEventDisableTiming) == cudaSuccess;
+        if (noise) ok = ok && cudaMalloc((void **)&p.d_sq, n * sizeof(unsigned long long)) == cudaSuccess;
+    }
+    if (!ok) return bail(fail(RT_ERR_CUDA, std::string("rt_multi_frame_begin: allocation failed: ") + cudaGetErrorString(cudaGetLastError())));
+
+    // the frame's parameters are one device's (the features, the filter and the pacing read them); each rank has its own
+    fill_frame(f->fp, ds0, camera, max_w, max_h, *opts, 0, 1);
+    f->fp.stats = f->d_stats;
+    f->fp.flags = f->d_flags;
+    f->fp.sq = f->d_sq;
+    f->samples_done = f->fp.n_probe;
+    f->samples_target = f->fp.sample_end;
+    int launches = 0;
+    for (int r = 0; r < world; ++r) {
+        FramePart &p = f->parts[size_t(r)];
+        DeviceScene *ds = part_scene(p);
+        if (cudaSetDevice(ds->device) != cudaSuccess) return bail(fail(RT_ERR_CUDA, "rt_multi_frame_begin: cudaSetDevice failed"));
+        fill_frame(p.fp, ds, camera, max_w, max_h, *opts, r, world);
+        p.fp.stats = p.d_stats;
+        p.fp.flags = p.d_flags;
+        p.fp.list = p.d_list;
+        p.fp.counters = p.d_counters;
+        p.fp.sq = p.d_sq;
+        // the tile-split probe; with its own counter block the rank keeps the raw flags of its tiles (the frame can be extended)
+        if ((rc = frame_probe(ds, p.fp, ds->ws->stream, &p.ev, &launches)) != RT_OK) return bail(rc);
+    }
+    if ((rc = multi_relist(f, true, false)) != RT_OK) return bail(rc);
+    if ((rc = multi_finish(f, FrameEvents::ZEROED, &f->device_ms)) != RT_OK) return bail(rc);
+    f->pixels_flagged = f->pixels_active = f->h_counters[CN_LIST];
+    // rt_frame_begin's rate: the slowest rank probed 1 / world of the pixels and a pass gives it 1 / world of the indices
+    if (f->fp.adaptive) f->ms_per_sample = f->device_ms * double(f->pixels_flagged) / (double(n) * double(f->fp.n_probe));
+    *out = f;
+    frame_progress(f, progress);
+    return RT_OK;
+}
+
+// one pass of every rank over [s, s + k) with s = samples_done (rank r: the indices s + r + j world) and, when it
+// ends on a checkpoint, the check; *span_ms is the slowest rank's BEGIN -> END
+int multi_pass(RtFrame *f, int k, bool check, double *span_ms) {
+    int launches = 0;
+    for (FramePart &p : f->parts) {
+        DeviceScene *ds = part_scene(p);
+        RT_CUDA(cudaSetDevice(ds->device));
+        cudaStream_t st = ds->ws->stream;
+        FrameParams fp = p.fp;
+        fp.cam.spp = f->fp.cam.spp; // (rt_frame_extend changes the frame's parameters only)
+        fp.sample_begin = f->samples_done;
+        fp.sample_end = f->samples_done + k;
+        RT_CUDA(cudaMemsetAsync(p.d_counters + CN_WORK_MAIN, 0, sizeof(unsigned long long), st));
+        RT_CUDA(p.ev.record(FrameEvents::BEGIN, st));
+        int rc = launch_samples(ds, fp, st, &launches);
+        if (rc != RT_OK) return rc;
+    }
+    f->gathered = false;
+    if (check) {
+        int rc = multi_relist(f, false, true);
+        if (rc != RT_OK) return rc;
+    }
+    return multi_finish(f, FrameEvents::BEGIN, span_ms);
+}
+
 // rt_frame_view_noise reduces at most this many views per launch: the grid's y extent stays far below its limit (65535),
 // and the partials stay at most 16.8 MB however many views a batch of small extents has
 constexpr int32_t kNoiseViewChunk = 1024;
@@ -362,6 +585,20 @@ int rt_frame_begin_window(RtScene *scene, const RtCamera *camera, int32_t max_w,
     return frame_open(scene, *camera, {}, &w, max_w, max_h, opts, out, progress, "rt_frame_begin_window");
 }
 
+int rt_multi_frame_begin(RtMulti *multi, const RtCamera *camera, int32_t max_w, int32_t max_h, const RtRenderOpts *opts, RtFrame **out,
+                         RtFrameProgress *progress) {
+    if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_multi_frame_begin: out is null");
+    *out = nullptr;
+    if (!multi || multi_scenes(multi).empty()) return fail(RT_ERR_INVALID_ARGUMENT, "rt_multi_frame_begin: null handle");
+    // rt_frame_begin's checks and refusals, on the first device's replica
+    int rc = check_frame_args(multi_scenes(multi)[0], camera, max_w, max_h, opts);
+    if (rc != RT_OK) return rc;
+    if ((rc = check_frame_mode(opts, "rt_multi_frame_begin")) != RT_OK) return rc;
+    if ((opts->flags & RT_FLAG_NOISE) && (opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS)))
+        return fail(RT_ERR_UNSUPPORTED, "rt_multi_frame_begin: RT_FLAG_NOISE has no flow-schedule or counting kernel");
+    return multi_frame_open(multi, *camera, max_w, max_h, opts, out, progress);
+}
+
 int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameProgress *progress) {
     if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_advance: null frame");
     if (int rc = check_current(f, "rt_frame_advance"); rc != RT_OK) return rc;
@@ -376,32 +613,41 @@ int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameP
             int paced = 1; // no rate known yet (no probe without the early-out): one sample index
             if (f->ms_per_sample == 0.0) paced = left; // nothing to trace (no pixel is flagged)
             else if (f->ms_per_sample > 0.0) paced = int(std::min(double(left), std::floor(target_ms / f->ms_per_sample)));
+            // over several devices a paced window that the end does not cut is a multiple of the device count: no rank idles
+            const int world = int(f->parts.size());
+            if (world > 1 && paced < left && paced >= world) paced -= paced % world;
             k = std::min(k, std::max(1, paced));
         }
         if (rule) k = int(std::min<int64_t>(k, next_checkpoint(f) - f->samples_done)); // a pass never crosses a checkpoint
         const bool check = rule && f->samples_done + k == next_checkpoint(f);
-        auto *ds = static_cast<DeviceScene *>(f->scene->dev);
-        RT_CUDA(cudaSetDevice(ds->device));
-        cudaStream_t st = ds->ws->stream;
-        FrameParams fp = f->fp;
-        fp.sample_begin = f->samples_done;
-        fp.sample_end = f->samples_done + k;
-        int launches = 0;
-        RT_CUDA(cudaMemsetAsync(f->d_counters + CN_WORK_MAIN, 0, sizeof(unsigned long long), st));
-        RT_CUDA(f->ev.record(FrameEvents::BEGIN, st));
-        int rc = launch_samples(ds, fp, st, &launches);
-        if (rc != RT_OK) return rc;
-        if (check) { // the pass ends on a checkpoint: stop the converged pixels and list the others
-            converge_kernel<<<unsigned((f->n_pixels + 255) / 256), 256, 0, st>>>(reinterpret_cast<const int4 *>(f->d_stats), f->d_sq, f->d_flags,
-                                                                                 f->n_pixels, f->conv_tolerance);
-            RT_CUDA(cudaGetLastError());
-            if ((rc = launch_compact(ds, fp, single_flags(f->d_flags), f->d_list, st, &launches)) != RT_OK) return rc;
+        double span_ms = 0.0;
+        if (f->parts.empty()) {
+            auto *ds = static_cast<DeviceScene *>(f->scene->dev);
+            RT_CUDA(cudaSetDevice(ds->device));
+            cudaStream_t st = ds->ws->stream;
+            FrameParams fp = f->fp;
+            fp.sample_begin = f->samples_done;
+            fp.sample_end = f->samples_done + k;
+            int launches = 0;
+            RT_CUDA(cudaMemsetAsync(f->d_counters + CN_WORK_MAIN, 0, sizeof(unsigned long long), st));
+            RT_CUDA(f->ev.record(FrameEvents::BEGIN, st));
+            int rc = launch_samples(ds, fp, st, &launches);
+            if (rc != RT_OK) return rc;
+            if (check) { // the pass ends on a checkpoint: stop the converged pixels and list the others
+                converge_kernel<<<unsigned((f->n_pixels + 255) / 256), 256, 0, st>>>(reinterpret_cast<const int4 *>(f->d_stats), f->d_sq,
+                                                                                     f->d_flags, f->n_pixels, f->conv_tolerance);
+                RT_CUDA(cudaGetLastError());
+                if ((rc = launch_compact(ds, fp, single_flags(f->d_flags), f->d_list, st, &launches)) != RT_OK) return rc;
+            }
+            RT_CUDA(f->ev.record(FrameEvents::END, st));
+            if ((rc = frame_sync(f, st)) != RT_OK) return rc;
+            span_ms = f->ev.ms(FrameEvents::BEGIN, FrameEvents::END);
+        } else if (int rc = multi_pass(f, k, check, &span_ms); rc != RT_OK) {
+            return rc;
         }
-        RT_CUDA(f->ev.record(FrameEvents::END, st));
-        if ((rc = frame_sync(f, st)) != RT_OK) return rc;
         f->samples_done += k;
         f->passes += 1;
-        f->last_pass_ms = f->ev.ms(FrameEvents::BEGIN, FrameEvents::END);
+        f->last_pass_ms = span_ms;
         f->device_ms += f->last_pass_ms;
         const uint64_t before = f->pixels_active;
         if (check) {
@@ -418,6 +664,7 @@ int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameP
 
 int rt_frame_read(RtFrame *f, int32_t gamma, uint8_t *rgb_out, int32_t *sums_out) {
     if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_read: null frame");
+    if (int rc = ensure_totals(f); rc != RT_OK) return rc;
     auto *ds = static_cast<DeviceScene *>(f->scene->dev);
     RT_CUDA(cudaSetDevice(ds->device));
     cudaStream_t st = ds->ws->stream;
@@ -453,10 +700,12 @@ int rt_frame_noise(RtFrame *f, double tolerance, float *se_out, uint64_t *sq_out
     if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_noise: null frame");
     if (!f->d_sq) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_noise: the frame was opened without RT_FLAG_NOISE");
     if (!(tolerance >= 0.0)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_noise: tolerance must be >= 0");
+    int rc = ensure_totals(f);
+    if (rc != RT_OK) return rc;
     auto *ds = static_cast<DeviceScene *>(f->scene->dev);
     RT_CUDA(cudaSetDevice(ds->device));
     cudaStream_t st = ds->ws->stream;
-    int rc = ensure_partials(f);
+    rc = ensure_partials(f);
     if (rc != RT_OK) return rc;
     if (se_out && !f->d_se) RT_CUDA(cudaMalloc((void **)&f->d_se, f->n_pixels * sizeof(float)));
     noise_kernel<<<kNoiseBlocks, kNoiseThreads, 0, st>>>(reinterpret_cast<const int4 *>(f->d_stats), f->d_sq, f->d_flags, f->n_pixels, tolerance,
@@ -477,10 +726,12 @@ int rt_frame_view_noise(RtFrame *f, double tolerance, RtFrameNoise *per_view) {
     if (!f || !per_view) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_view_noise: null frame or output");
     if (!f->d_sq) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_view_noise: the frame was opened without RT_FLAG_NOISE");
     if (!(tolerance >= 0.0)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_view_noise: tolerance must be >= 0");
+    int rc = ensure_totals(f);
+    if (rc != RT_OK) return rc;
     auto *ds = static_cast<DeviceScene *>(f->scene->dev);
     RT_CUDA(cudaSetDevice(ds->device));
     cudaStream_t st = ds->ws->stream;
-    int rc = ensure_partials(f);
+    rc = ensure_partials(f);
     if (rc != RT_OK) return rc;
     // every view reduced as rt_frame_noise reduces a frame of its pixels: the same 512 ranges, tree and block order
     const size_t view_pixels = f->n_pixels / size_t(f->n_views);
@@ -554,6 +805,7 @@ int rt_frame_denoise(RtFrame *f, const RtDenoiseOpts *opts, uint8_t *rgb_out, fl
     if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_denoise: null frame");
     if ((rc = check_current(f, "rt_frame_denoise")) != RT_OK) return rc;
     if (!f->d_sq) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_denoise: the frame was opened without RT_FLAG_NOISE");
+    if ((rc = ensure_totals(f)) != RT_OK) return rc;
     auto *ds = static_cast<DeviceScene *>(f->scene->dev);
     RT_CUDA(cudaSetDevice(ds->device));
     cudaStream_t st = ds->ws->stream;

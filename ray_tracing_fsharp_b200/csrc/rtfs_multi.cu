@@ -17,6 +17,7 @@
 #include "rtfs_device.h"
 
 #include <chrono>
+#include <cstdlib>
 #include <cstring>
 #include <memory>
 
@@ -66,6 +67,62 @@ __global__ void reduce_finalize_kernel(const ReduceTargets t, int n_pixels, int 
         } else {
             for (int k = 0; k < 3 * n_valid; ++k) t.rgb[r][12 * size_t(quad) + k] = out[k];
         }
+    }
+}
+
+// A progressive frame's exchange (launch_gather): four pixels per thread, so that every rank's sums are four 128-bit peer
+// loads, its Q two, and its four probe flags one 32-bit load (flags are 0 or 1 bytes, so OR-ing the words ORs the pixels).
+__global__ void gather_kernel(const GatherTargets t, size_t n_pixels, size_t quad_begin, size_t quad_end) {
+    const size_t quad = quad_begin + size_t(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (quad >= quad_end) return;
+    const size_t p0 = 4 * quad;
+    if (p0 + 4 <= n_pixels) {
+        int4 s[4];
+        ulonglong2 q[2];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) s[k] = make_int4(0, 0, 0, 0);
+        q[0] = q[1] = make_ulonglong2(0ull, 0ull);
+        uint32_t f = 0;
+        for (int r = 0; r < t.world; ++r) {
+            const int4 *src = reinterpret_cast<const int4 *>(t.stats[r]) + p0;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const int4 v = src[k];
+                s[k].x += v.x; s[k].y += v.y; s[k].z += v.z; s[k].w += v.w;
+            }
+            if (t.total_sq) {
+                const ulonglong2 *qs = reinterpret_cast<const ulonglong2 *>(t.sq[r] + p0);
+#pragma unroll
+                for (int k = 0; k < 2; ++k) {
+                    const ulonglong2 v = qs[k];
+                    q[k].x += v.x; q[k].y += v.y;
+                }
+            }
+            if (t.total_flags) f |= *reinterpret_cast<const uint32_t *>(t.flags[r] + p0);
+        }
+        int4 *dst = reinterpret_cast<int4 *>(t.total_stats) + p0;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) dst[k] = s[k];
+        if (t.total_sq) {
+            reinterpret_cast<ulonglong2 *>(t.total_sq + p0)[0] = q[0];
+            reinterpret_cast<ulonglong2 *>(t.total_sq + p0)[1] = q[1];
+        }
+        if (t.total_flags) *reinterpret_cast<uint32_t *>(t.total_flags + p0) = f;
+        return;
+    }
+    for (size_t p = p0; p < n_pixels; ++p) { // the last quad of a frame whose size is not a multiple of four
+        int4 s = make_int4(0, 0, 0, 0);
+        unsigned long long q = 0;
+        uint8_t f = 0;
+        for (int r = 0; r < t.world; ++r) {
+            const int4 v = reinterpret_cast<const int4 *>(t.stats[r])[p];
+            s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+            if (t.total_sq) q += t.sq[r][p];
+            if (t.total_flags) f |= t.flags[r][p];
+        }
+        reinterpret_cast<int4 *>(t.total_stats)[p] = s;
+        if (t.total_sq) t.total_sq[p] = q;
+        if (t.total_flags) t.total_flags[p] = f;
     }
 }
 
@@ -130,6 +187,17 @@ int launch_reduce_finalize(const ReduceTargets &t, int rank, size_t n_pixels, in
     return RT_OK;
 }
 
+int launch_gather(const GatherTargets &t, int rank, size_t n_pixels, cudaStream_t st) {
+    const size_t n_quads = (n_pixels + 3) / 4;
+    const size_t quad_begin = n_quads * size_t(rank) / size_t(t.world), quad_end = n_quads * size_t(rank + 1) / size_t(t.world);
+    if (quad_end <= quad_begin) return RT_OK;
+    gather_kernel<<<unsigned((quad_end - quad_begin + 255) / 256), 256, 0, st>>>(t, n_pixels, quad_begin, quad_end);
+    RT_CUDA(cudaGetLastError());
+    return RT_OK;
+}
+
+const std::vector<RtScene *> &multi_scenes(const RtMulti *m) { return m->scenes; }
+
 } // namespace rtfs
 
 using namespace rtfs;
@@ -143,16 +211,19 @@ int rt_multi_create(const RtHittable *objects, int32_t n_objects, const RtTextur
     if (!devices || n_devices < 1 || n_devices > kMaxDevices) return fail(RT_ERR_INVALID_ARGUMENT, "rt_multi_create: 1..16 devices");
     int visible = rt_device_count();
     if (visible <= 0) return fail(RT_ERR_NO_DEVICE, "no CUDA device is visible: librtfs_b200 has no CPU fallback");
+    // RTFS_MULTI_SHARE_DEVICES (tests): ranks may share a device, so that the split, its exchange and its cross-stream
+    // ordering run on a machine with fewer GPUs than ranks; each rank still has its own replica, workspace and stream
+    const bool share = std::getenv("RTFS_MULTI_SHARE_DEVICES") != nullptr;
     for (int i = 0; i < n_devices; ++i) {
         if (devices[i] < 0 || devices[i] >= visible) return fail(RT_ERR_INVALID_ARGUMENT, "rt_multi_create: device ordinal out of range");
         for (int j = 0; j < i; ++j)
-            if (devices[j] == devices[i]) return fail(RT_ERR_INVALID_ARGUMENT, "rt_multi_create: duplicate device");
+            if (devices[j] == devices[i] && !share) return fail(RT_ERR_INVALID_ARGUMENT, "rt_multi_create: duplicate device");
     }
     // every device must be able to read every other device's buffers (NVLink / NVSwitch peer access)
     for (int i = 0; i < n_devices; ++i) {
         RT_CUDA(cudaSetDevice(devices[i]));
         for (int j = 0; j < n_devices; ++j) {
-            if (i == j) continue;
+            if (devices[i] == devices[j]) continue;
             int can = 0;
             RT_CUDA(cudaDeviceCanAccessPeer(&can, devices[i], devices[j]));
             if (!can) return fail(RT_ERR_UNSUPPORTED, "rt_multi_create: devices without peer access cannot share a frame");

@@ -75,6 +75,8 @@ def _declare(lib):
         "rt_multi_create": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i32, C.POINTER(_vp)]),
         "rt_multi_render": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _vp, _vp, C.POINTER(RtStats)]),
         "rt_multi_destroy": (None, [_vp]),
+        "rt_multi_frame_begin": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), C.POINTER(_vp),
+                                           C.POINTER(RtFrameProgress)]),
         "rt_device_probe": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _i32, _i32, _vp, _vp, _vp,
                                       C.POINTER(RtStats)]),
         "rt_device_main": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _i32, _i32, _vp, _vp, _vp,
@@ -541,6 +543,19 @@ class MultiHandle:
         stats = RtStats()
         check(lib().rt_multi_render(self.ptr, C.byref(camera), max_w, max_h, C.byref(opts), ptr(rgb), ptr(sums), C.byref(stats)))
         return rgb, sums, stats
+
+    def open_frame(self, camera, max_w, max_h, seed=0, adaptive=True, flags=0, mode=abi.RT_MODE_MEGAKERNEL):
+        """A progressive frame split over this handle's devices (rt_multi_frame_begin: runs the probe).  A Frame that is bit
+        for bit SceneHandle.open_frame's frame of one device after every pass; it holds this handle, so the handle outlives
+        it."""
+        opts = RtRenderOpts(seed, int(adaptive), mode, 0, flags)
+        out = C.c_void_p()
+        progress = RtFrameProgress()
+        check(lib().rt_multi_frame_begin(self.ptr, C.byref(camera), max_w, max_h, C.byref(opts), C.byref(out), C.byref(progress)))
+        frame = Frame.__new__(Frame)
+        frame.scene, frame.ptr, frame.progress = self, out, progress
+        frame.rows, frame.cols = 2 * max_h + 1, 2 * max_w + 1
+        return frame
 
 
 class CommHandle:

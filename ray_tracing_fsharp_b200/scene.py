@@ -8,7 +8,7 @@ reference's.  Everything that computes goes through the C ABI (native.py); nothi
   Scene.update          Scene.make of an edited object list, done in place on the device (rt_scene_update)
   Scene.render          RayTracing/Scene.fs:196-236
   Scene.render_views    Scene.render of many cameras of one scene in one submission (rt_render_views)
-  Scene.render_progressive  the same frame in sample passes, progress ticks as passes finish (native.Frame)
+  Scene.render_progressive  the same frame in sample passes, progress ticks as passes finish (native.Frame, one GPU or several)
   Scene.render_views_progressive  Scene.render_views in sample passes, as one progressive frame of the batch
   Scene.render_window   a window (row0, col0, rows, cols) of Scene.render's image, without tracing the rest (rt_render_window)
   Image / Image.render  RayTracing/Domain.fs:9-31
@@ -240,7 +240,8 @@ class Scene:
                            flags: int = 0, noise_tolerance: Optional[float] = None, noise_fraction: float = 0.0,
                            converge_tolerance: Optional[float] = None, converge_min_samples: int = 64,
                            converge_interval: int = 64, window=None) -> np.ndarray:
-        """Scene.render's frame rendered in passes of about `target_ms` of device time each (native.Frame, one GPU).
+        """Scene.render's frame rendered in passes of about `target_ms` of device time each (native.Frame; on a scene made
+        with devices=[...], one frame split over those GPUs, bit for bit the frame of one GPU).
         `progress_increment(1.0)` is called as passes complete, in proportion to the paths traced so far out of the frame's
         total, and exactly `rows` times in all, like the reference's one call per row (Scene.fs:232).  After every pass
         `on_pass(progress, frame)` is called, if given: it may read the current image (`frame.read()`, exactly the frame of
@@ -257,9 +258,9 @@ class Scene:
         still being sampled.
         With `window` = (row0, col0, rows, cols) only that window of the frame is traced (native.SceneHandle.open_frame_window):
         the progress ticks total the window's rows, and the pixels returned ([rows, cols, 3]) are exactly that crop of the
-        frame rendered without it."""
-        if not isinstance(s._handle, native.SceneHandle):
-            raise NotImplementedError("progressive frames run on one GPU: make the scene with a single device")
+        frame rendered without it; a window runs on one GPU (NotImplementedError on a scene made with devices=[...])."""
+        if window is not None and not isinstance(s._handle, native.SceneHandle):
+            raise NotImplementedError("a window runs on one GPU: make the scene with a single device")
         rows = 2 * max_height_coord + 1 if window is None else int(window[2])
         if seed is None:
             seed = secrets.randbits(64)

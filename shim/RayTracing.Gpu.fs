@@ -247,6 +247,9 @@ module internal Native =
     [<DllImport(Lib)>]
     extern void rt_multi_destroy (nativeint multi)
 
+    [<DllImport(Lib)>]
+    extern int rt_multi_frame_begin (nativeint multi, RtCamera& camera, int maxWidthCoord, int maxHeightCoord, RtRenderOpts& opts, nativeint& frame, RtFrameProgress& progress)
+
     // one rank of a one-process-per-GPU job: the library issues the NCCL collectives itself (include/rtfs_b200.h, rt_comm_*)
     [<DllImport(Lib)>]
     extern int rt_comm_unique_id (byte[] idOut)
@@ -600,7 +603,8 @@ type FrameConvergence =
         PixelsConverged : uint64
     }
 
-/// A frame in progress on a single-device GpuScene (rt_frame_*): advanced in passes over windows of sample indices.
+/// A frame in progress on a GpuScene (rt_frame_*; on a multi-GPU scene split over its devices, bit for bit the frame of one
+/// GPU): advanced in passes over windows of sample indices.
 /// After every pass it is exactly the frame rt_render gives at `SamplesDone` samples per pixel with the same seed, so
 /// `Read` shows the image sharpening; a caller stops early by not advancing any more, and `Extend` continues a finished
 /// frame to more samples.  Dispose it before its scene.  A frame of a batch of views (SceneGpu.openFrameViews) holds `Views`
@@ -969,12 +973,9 @@ module SceneGpu =
 
         1.0<progress> * float rowsIter, Image.make rowsIter colsIter rows
 
-    /// Opens a progressive frame with RtRenderOpts.flags `flags` (e.g. FrameFlags.Noise for GpuFrame.Noise).
-    /// Single-device scenes only.
+    /// Opens a progressive frame with RtRenderOpts.flags `flags` (e.g. FrameFlags.Noise for GpuFrame.Noise).  On a
+    /// multi-GPU scene the frame is split over its devices (rt_multi_frame_begin) and is bit for bit the frame of one GPU.
     let openFrameWith (flags : int) (maxWidthCoord : int) (maxHeightCoord : int) (camera : Camera) (seed : uint64) (s : GpuScene) : GpuFrame =
-        if s.IsMulti then
-            failwith "GPU backend: progressive frames run on a single-device GpuScene"
-
         let mutable cam = marshalCamera camera
         let mutable opts = Native.RtRenderOpts ()
         opts.seed <- seed
@@ -983,12 +984,17 @@ module SceneGpu =
         let mutable handle = 0n
         let mutable progress = Native.RtFrameProgress ()
 
-        Native.rt_frame_begin (s.Handle, &cam, maxWidthCoord, maxHeightCoord, &opts, &handle, &progress)
-        |> Native.check
+        let rc =
+            if s.IsMulti then
+                Native.rt_multi_frame_begin (s.Handle, &cam, maxWidthCoord, maxHeightCoord, &opts, &handle, &progress)
+            else
+                Native.rt_frame_begin (s.Handle, &cam, maxWidthCoord, maxHeightCoord, &opts, &handle, &progress)
+
+        Native.check rc
 
         new GpuFrame (handle, 2 * maxHeightCoord + 1, 2 * maxWidthCoord + 1, 1, progress)
 
-    /// Opens a progressive frame (rt_frame_begin: the probe runs now).  Single-device scenes only.
+    /// Opens a progressive frame (rt_frame_begin, or rt_multi_frame_begin on a multi-GPU scene: the probe runs now).
     let openFrame (maxWidthCoord : int) (maxHeightCoord : int) (camera : Camera) (seed : uint64) (s : GpuScene) : GpuFrame =
         openFrameWith 0 maxWidthCoord maxHeightCoord camera seed s
 
@@ -997,7 +1003,7 @@ module SceneGpu =
     /// exactly the frame openFrameWith gives for cameras.[v] and seeds.[v].  Single-device scenes only.
     let openFrameViews (flags : int) (maxWidthCoord : int) (maxHeightCoord : int) (cameras : Camera array) (seeds : uint64 array) (s : GpuScene) : GpuFrame =
         if s.IsMulti then
-            failwith "GPU backend: progressive frames run on a single-device GpuScene"
+            failwith "GPU backend: a progressive frame of a batch of views runs on a single-device GpuScene"
 
         if seeds.Length <> cameras.Length then
             invalidArg "seeds" "one seed per camera"
@@ -1020,7 +1026,7 @@ module SceneGpu =
     /// camera and seed.  Single-device scenes only.
     let openFrameWindow (flags : int) (maxWidthCoord : int) (maxHeightCoord : int) (camera : Camera) (row0 : int, col0 : int, rows : int, cols : int) (seed : uint64) (s : GpuScene) : GpuFrame =
         if s.IsMulti then
-            failwith "GPU backend: progressive frames run on a single-device GpuScene"
+            failwith "GPU backend: a progressive frame of a window runs on a single-device GpuScene"
 
         let mutable cam = marshalCamera camera
         let mutable opts = Native.RtRenderOpts ()
@@ -1225,7 +1231,7 @@ module SceneGpu =
 
     /// `render`'s signature and laziness, but the frame is traced in passes of about 250 ms of device time and
     /// `progressIncrement 1.0<progress>` is called as passes finish, in proportion to the paths traced out of the frame's
-    /// total: `rows` calls in all, as the reference makes (Scene.fs:232).  Single-device scenes only.
+    /// total: `rows` calls in all, as the reference makes (Scene.fs:232).  A multi-GPU scene splits every pass over its devices.
     let renderWithProgress
         (progressIncrement : float<progress> -> unit)
         (print : string -> unit)

@@ -409,6 +409,14 @@ int check_frame_args(const RtScene *scene, const RtCamera *camera, int max_w, in
     return RT_OK;
 }
 
+int check_frame_mode(const RtRenderOpts *opts, const char *who, bool batch_or_window) {
+    if (opts->mode == RT_MODE_WAVEFRONT) return fail(RT_ERR_UNSUPPORTED, std::string(who) + ": RT_MODE_WAVEFRONT is not supported (megakernel only)");
+    if (opts->mode != RT_MODE_MEGAKERNEL) return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": unknown mode");
+    if ((opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS)) && (batch_or_window || (opts->flags & RT_FLAG_NOISE)))
+        return fail(RT_ERR_UNSUPPORTED, std::string(who) + ": batches of views, windows and RT_FLAG_NOISE have no flow-schedule or counting kernel");
+    return RT_OK;
+}
+
 struct LaunchPlan {
     bool smem;
     size_t smem_bytes;

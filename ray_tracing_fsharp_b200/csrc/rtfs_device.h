@@ -224,6 +224,21 @@ int check_window(const FrameWindow &w, int max_w, int max_h, const char *who);
 // narrows a frame filled by fill_frame to the window: probe tiles, flags, list, sums and the output tail run over its pixels
 void set_window(FrameParams &fp, const FrameWindow &w);
 
+// a batch of views (rtfs_views.cu).  check_views: RT_ERR_INVALID_ARGUMENT unless n_views >= 1 and cameras is non-null, then
+// check_frame_args on the first camera, then every camera must have the first one's samples_per_pixel and bounce_depth and
+// the tall frame fewer than 2^31 pixels
+int check_views(const RtScene *scene, const RtCamera *cameras, int32_t n_views, int max_w, int max_h, const RtRenderOpts *opts, const char *who);
+// every view's camera and Philox key (seeds null: every view has `seed`)
+std::vector<ViewCamera> view_table(const RtCamera *cameras, const uint64_t *seeds, int32_t n_views, int max_w, int max_h, uint64_t seed);
+// stacks a frame filled by fill_frame into the tall frame of n_views views of view_pixels pixels: probe tiles, flags, list,
+// sums and Q run over it as over one frame, and the render kernels find each view's camera and key in d_views
+void set_views(FrameParams &fp, const ViewCamera *d_views, int32_t n_views, int32_t view_pixels);
+
+// the mode and flag refusals of rt_render_views, rt_render_window and the openers of progressive frames: RT_MODE_WAVEFRONT
+// (RT_ERR_UNSUPPORTED), an unknown mode (RT_ERR_INVALID_ARGUMENT), and RT_FLAG_FLOW or RT_FLAG_COUNTERS (RT_ERR_UNSUPPORTED)
+// for a batch of views or a window, and for any frame with RT_FLAG_NOISE: they have no flow-schedule or counting kernel
+int check_frame_mode(const RtRenderOpts *opts, const char *who, bool batch_or_window);
+
 
 constexpr int kMaxDevices = 16;
 // where the main phase finds the probe flags: one buffer (single device, or already combined by the

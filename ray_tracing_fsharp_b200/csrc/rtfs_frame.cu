@@ -1,6 +1,6 @@
-// rtfs_frame.cu — progressive frames (rt_frame_*): rt_render's frame on one device, cut into passes over windows of
-// sample indices.  The probe and the compaction run once, in rt_frame_begin; every rt_frame_advance is one
-// launch_samples over [samples_done, samples_done + k), i.e. the same render_kernel<PROBE = false> that rt_render's main
+// rtfs_frame.cu — progressive frames (rt_frame_*): rt_render's frame, cut into passes over windows of sample indices.
+// The probe and the compaction run once, in the opener; every rt_frame_advance is one launch_samples per part over
+// [samples_done, samples_done + k), i.e. the same render_kernel<PROBE = false> that rt_render's main
 // phase launches, with the same chunking.  Sums are integers keyed by (seed, pixel, sample index), so a frame that has
 // reached samples_done is bit for bit rt_render's frame at samples_per_pixel = samples_done (include/rtfs_b200.h).
 // A frame opened with RT_FLAG_NOISE also holds per pixel the sum of squares Q (render_kernel<NOISE = true>), from which
@@ -14,9 +14,11 @@
 // rt_frame_features and rt_frame_denoise (kernels in rtfs_denoise.cu) read the frame and keep buffers of their own.
 // A frame records its scene's edit count: once rt_scene_update has changed the scene, the calls that would trace or read the
 // scene refuse the frame, and the others keep working on what it holds.
-// rt_multi_frame_begin opens the same frame split over the devices of an RtMulti (FramePart, below; the exchange kernel is
-// in rtfs_multi.cu): rank r probes its tiles and traces its sample indices into buffers of its own, and the totals, the
-// shared flags and everything that reads them live on the first device.
+// Every frame is split into parts (FramePart, below), one per device: rt_frame_begin* open one, and rt_multi_frame_begin
+// one per device of an RtMulti.  Part r probes its tiles and traces its sample indices, and every part runs the same
+// opener, pass and end of step.  The totals, the shared flags and everything that reads them live on the first device: the
+// only part of a frame of one device traces into them directly, and over several devices the parts trace into buffers of
+// their own that the exchange kernel (rtfs_multi.cu) sums into the totals.
 #include "rtfs_device.h"
 
 #include <algorithm>
@@ -95,9 +97,10 @@ __global__ void __launch_bounds__(256) converge_kernel(const int4 *stats, const 
     if (pixel_standard_error(s.w, s.x, s.y, s.z, sq[p]) <= tolerance) flags[p] = 0;
 }
 
-// One device's part of a frame split over the devices of an RtMulti (rt_multi_frame_begin): rank r of world traces the
-// tiles t with t mod world == r in the probe and, in a pass over [s, s + k), the sample indices s + r + j world, into sums, Q,
-// flags, a list and a counter block of its own on its device.
+// One device's part of a frame: rank r of world traces the tiles t with t mod world == r in the probe and, in a pass over
+// [s, s + k), the sample indices s + r + j world, into sums, Q and flags on its device, and compacts the frame's flags into
+// a list and a counter block of its own.  The only part of a frame of one device traces into the frame's own sums, Q and
+// flags; over several devices every part has its own.
 struct FramePart {
     RtScene *scene = nullptr; // the rank's replica; its workspace's stream carries the rank's work
     FrameParams fp;
@@ -115,21 +118,19 @@ struct FramePart {
 
 } // namespace rtfs
 
-// A frame owns everything a pass writes: sums, flags, the flagged-pixel list, the image and its own counter block
-// (paths, rays, the list length and the work cursors), so rt_render and other frames can use the scene between passes.
-// A frame split over several devices (rt_multi_frame_begin) also owns one FramePart per device; its own sums and Q are then
-// the totals of the parts on the first device, its flags the flags every part compacts from, and every call that reads
-// the frame gathers the totals first.  The noise estimate, the check's converge_kernel, the features, the filter and the
-// read all run on the first device, over those buffers, exactly as on a frame of one device.
+// A frame owns everything a pass writes: sums, flags, the image and, in its parts, the flagged-pixel lists and counter
+// blocks (paths, rays, the list length and the work cursors), so rt_render and other frames can use the scene between
+// passes.  It has one part per device, in rank order: one for rt_frame_begin*, one per device of the RtMulti for
+// rt_multi_frame_begin.  Its own sums and Q are the totals of the parts on the first device, and its flags the flags every
+// part compacts from; over several devices every call that reads the frame gathers the totals first.  The noise estimate,
+// the check's converge_kernel, the features, the filter and the read all run on the first device, over those buffers.
 struct RtFrame {
-    RtScene *scene = nullptr;
+    RtScene *scene = nullptr; // the first device's
     FrameParams fp;
     size_t n_pixels = 0;
     int32_t *d_stats = nullptr;
     uint8_t *d_flags = nullptr;
-    uint32_t *d_list = nullptr;
     uint8_t *d_rgb = nullptr;
-    unsigned long long *d_counters = nullptr;
     unsigned long long *d_sq = nullptr; // RT_FLAG_NOISE: per pixel the sum of r^2 + g^2 + b^2 (null otherwise)
     float *d_se = nullptr;              // rt_frame_noise's map, allocated on first use
     NoisePartial *d_partial = nullptr;  // and its per-block partial summaries, then the summary (kNoiseBlocks + 1 per view)
@@ -141,8 +142,8 @@ struct RtFrame {
     FrameFeatures feat{};
     int32_t feat_samples = 0;
     float4 *d_denoise = nullptr; // rt_frame_denoise's two levels (2 n_pixels), allocated on first use
-    unsigned long long h_counters[CN_SLOTS] = {};
-    FrameEvents ev; // rt_frame_begin: ZEROED -> TRACED; a pass: BEGIN -> END
+    uint64_t paths_done = 0;     // the parts' paths, summed at the end of every step
+    uint64_t pixels_listed = 0;  // the length of the list every part compacted last
     int32_t samples_done = 0, samples_target = 0;
     uint64_t pixels_flagged = 0;
     double ms_per_sample = -1.0; // measured device time of one sample index of every flagged pixel (< 0: not known yet)
@@ -153,36 +154,35 @@ struct RtFrame {
     int32_t conv_min = 0, conv_interval = 0, conv_checks = 0;
     uint64_t pixels_active = 0; // pixels still being sampled: the list's length (pixels_flagged until a check)
     uint64_t generation = 0;    // the scene's edit count when the frame opened (rt_scene_update)
-    std::vector<FramePart> parts; // rt_multi_frame_begin: one per device, in rank order (empty: a frame of one device)
-    bool gathered = true;         // the totals hold every part's samples
+    std::vector<FramePart> parts;
+    bool gathered = true; // the totals hold every part's samples (always, with one part)
 };
 
 namespace {
+
+DeviceScene *part_scene(const FramePart &p) { return static_cast<DeviceScene *>(p.scene->dev); }
 
 void frame_free(RtFrame *f) {
     if (!f) return;
     for (FramePart &p : f->parts) {
         if (!p.scene) continue; // (an opener that failed before reaching this part)
-        auto *pds = static_cast<DeviceScene *>(p.scene->dev);
-        cudaSetDevice(pds->device);
-        cudaStreamSynchronize(pds->ws->stream);
-        cudaFree(p.d_stats);
-        cudaFree(p.d_sq);
-        cudaFree(p.d_flags);
+        cudaSetDevice(part_scene(p)->device);
+        cudaStreamSynchronize(part_scene(p)->ws->stream);
+        if (f->parts.size() > 1) { // (the only part of a frame traces into the frame's own buffers, freed below)
+            cudaFree(p.d_stats);
+            cudaFree(p.d_sq);
+            cudaFree(p.d_flags);
+        }
         cudaFree(p.d_list);
         cudaFree(p.d_counters);
         p.ev.destroy();
         for (cudaEvent_t e : {p.traced, p.gathered, p.listed})
             if (e) cudaEventDestroy(e);
     }
-    auto *ds = static_cast<DeviceScene *>(f->scene->dev);
-    cudaSetDevice(ds->device);
-    cudaStreamSynchronize(ds->ws->stream);
+    cudaSetDevice(static_cast<DeviceScene *>(f->scene->dev)->device); // (its stream, the first part's, is synchronised above)
     cudaFree(f->d_stats);
     cudaFree(f->d_flags);
-    cudaFree(f->d_list);
     cudaFree(f->d_rgb);
-    cudaFree(f->d_counters);
     cudaFree(f->d_sq);
     cudaFree(f->d_se);
     cudaFree(f->d_partial);
@@ -192,15 +192,7 @@ void frame_free(RtFrame *f) {
     cudaFree(f->feat.normal);
     cudaFree(f->feat.depth);
     cudaFree(f->d_denoise);
-    f->ev.destroy();
     delete f;
-}
-
-// one small device->host copy of the frame's counters and a synchronisation of the scene's stream
-int frame_sync(RtFrame *f, cudaStream_t st) {
-    RT_CUDA(cudaMemcpyAsync(f->h_counters, f->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    RT_CUDA(cudaStreamSynchronize(st));
-    return RT_OK;
 }
 
 // the first checkpoint of the frame's rule above samples_done (int64: m + j k may pass INT32_MAX)
@@ -215,7 +207,7 @@ void frame_progress(const RtFrame *f, RtFrameProgress *p) {
     const uint64_t n_probe = uint64_t(f->fp.n_probe);
     p->samples_done = f->samples_done;
     p->samples_target = f->samples_target;
-    p->paths_done = f->h_counters[CN_PATHS];
+    p->paths_done = f->paths_done;
     p->paths_target = uint64_t(f->n_pixels) * n_probe + f->pixels_flagged * (uint64_t(f->samples_target) - n_probe);
     // with a rule: exact if nothing more converges, so it only shrinks at a check
     if (f->conv_interval) p->paths_target = p->paths_done + f->pixels_active * uint64_t(f->samples_target - f->samples_done);
@@ -226,85 +218,13 @@ void frame_progress(const RtFrame *f, RtFrameProgress *p) {
     p->done = f->samples_done == f->samples_target ? 1 : 0;
 }
 
-// rt_frame_begin (views empty, no window), rt_frame_begin_views and rt_frame_begin_window, once their arguments are checked:
-// allocates the frame, and runs the probe and the compaction.  A batch's frame is the tall frame of rt_render_views
-// (rtfs_views.cu) with its own table; a window's frame holds the window's pixels only (rtfs_window.cu).
-int frame_open(RtScene *scene, const RtCamera &camera, const std::vector<ViewCamera> &views, const FrameWindow *window, int32_t max_w,
-               int32_t max_h, const RtRenderOpts *opts, RtFrame **out, RtFrameProgress *progress, const char *who) {
-    const bool noise = (opts->flags & RT_FLAG_NOISE) != 0;
-    int rc = prepare_frame(scene, opts);
-    if (rc != RT_OK) return rc;
-    auto *ds = static_cast<DeviceScene *>(scene->dev);
-    RT_CUDA(cudaSetDevice(ds->device));
-    auto *f = new RtFrame();
-    f->scene = scene;
-    f->generation = scene->generation;
-    auto bail = [&](int code) {
-        frame_free(f);
-        return code;
-    };
-    const size_t view_pixels = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
-    const size_t n = window ? size_t(window->rows) * size_t(window->cols) : view_pixels * std::max<size_t>(1, views.size());
-    f->n_pixels = n;
-    bool ok = cudaMalloc((void **)&f->d_stats, n * 4 * sizeof(int32_t)) == cudaSuccess && cudaMalloc((void **)&f->d_flags, n) == cudaSuccess &&
-              cudaMalloc((void **)&f->d_list, n * sizeof(uint32_t)) == cudaSuccess && cudaMalloc((void **)&f->d_rgb, n * 3) == cudaSuccess &&
-              cudaMalloc((void **)&f->d_counters, CN_SLOTS * sizeof(unsigned long long)) == cudaSuccess;
-    if (noise) ok = ok && cudaMalloc((void **)&f->d_sq, n * sizeof(unsigned long long)) == cudaSuccess;
-    if (!views.empty()) ok = ok && cudaMalloc((void **)&f->d_views, views.size() * sizeof(ViewCamera)) == cudaSuccess;
-    ok = ok && f->ev.create();
-    if (!ok) return bail(fail(RT_ERR_CUDA, std::string(who) + ": allocation failed: " + cudaGetErrorString(cudaGetLastError())));
-
-    cudaStream_t st = ds->ws->stream;
-    FrameParams &fp = f->fp;
-    fill_frame(fp, ds, camera, max_w, max_h, *opts, 0, 1);
-    if (!views.empty()) {
-        // (from pageable memory: staged before the call returns; the probe below follows it on the stream)
-        if (cudaMemcpyAsync(f->d_views, views.data(), views.size() * sizeof(ViewCamera), cudaMemcpyHostToDevice, st) != cudaSuccess)
-            return bail(fail(RT_ERR_CUDA, std::string(who) + ": view table upload failed: " + cudaGetErrorString(cudaGetLastError())));
-        f->n_views = int32_t(views.size());
-        fp.cam.rows *= f->n_views; // the tall frame: probe tiles, flags, list, sums and Q run over it as over one frame
-        fp.tiles_y = (fp.cam.rows + kTileH - 1) / kTileH;
-        fp.views = f->d_views;
-        fp.n_views = f->n_views;
-        fp.view_pixels = int32_t(view_pixels);
-    }
-    if (window) set_window(fp, *window);
-    fp.stats = f->d_stats;
-    fp.flags = f->d_flags;
-    fp.list = f->d_list;
-    fp.counters = f->d_counters;
-    fp.sq = f->d_sq; // non-null: plan_launch picks the kernels that also sum the squares
-    f->samples_done = fp.n_probe; // 0 without the early-out
-    f->samples_target = fp.sample_end;
-    int launches = 0;
-    // with its own counter block, the frame's probe keeps the raw "means differ" flags, also where this target has no main
-    // phase: the frame can be extended
-    auto enqueue = [&]() -> int {
-        int rc2 = frame_probe(ds, fp, st, &f->ev, &launches);
-        if (rc2 != RT_OK) return rc2;
-        if ((rc2 = launch_compact(ds, fp, single_flags(f->d_flags), f->d_list, st, &launches)) != RT_OK) return rc2;
-        RT_CUDA(f->ev.record(FrameEvents::TRACED, st));
-        return frame_sync(f, st);
-    };
-    if ((rc = enqueue()) != RT_OK) return bail(rc);
-    f->pixels_flagged = f->pixels_active = f->h_counters[CN_LIST];
-    f->device_ms = f->ev.ms(FrameEvents::ZEROED, FrameEvents::TRACED);
-    // the probe traced n_probe samples of every pixel; a pass traces samples of the flagged pixels only
-    if (fp.adaptive) f->ms_per_sample = f->device_ms * double(f->pixels_flagged) / (double(n) * double(fp.n_probe));
-    *out = f;
-    frame_progress(f, progress);
-    return RT_OK;
-}
-
-// ---- a frame split over the devices of an RtMulti (rt_multi_frame_begin) ----------------------------------------------
+// ---- the parts of a frame ------------------------------------------------------------------------------------------------
 // Devices are ordered by CUDA events only: a rank waits for the others' events on its own stream, and no kernel spins.
 
-DeviceScene *part_scene(const FramePart &p) { return static_cast<DeviceScene *>(p.scene->dev); }
-
-// The totals on the first device: once every rank's work so far is done, rank r sums its slice of the pixels of every rank
-// (launch_gather, peer loads), and at the probe also ORs the ranks' flags into the frame's flags; the first device's
-// stream then waits for every slice.
-int multi_gather(RtFrame *f, bool probe_flags) {
+// The totals on the first device, over several parts: once every rank's work so far is done, rank r sums its slice of the
+// pixels of every rank (launch_gather, peer loads), and at the probe also ORs the ranks' flags into the frame's flags; the
+// first device's stream then waits for every slice.
+int frame_gather(RtFrame *f, bool probe_flags) {
     const int world = int(f->parts.size());
     GatherTargets t{};
     t.world = world;
@@ -337,23 +257,25 @@ int multi_gather(RtFrame *f, bool probe_flags) {
 }
 
 // the totals, gathered if a pass has run since they last were (then on the first device's stream)
-int ensure_totals(RtFrame *f) { return f->parts.empty() || f->gathered ? RT_OK : multi_gather(f, false); }
+int ensure_totals(RtFrame *f) { return f->gathered ? RT_OK : frame_gather(f, false); }
 
-// After the probe (probe: the frame's flags become the OR of the ranks' probe flags) or a pass that ends on a checkpoint
-// (converge: converge_kernel clears the converged pixels' flags on the first device, as on one device): every rank compacts
-// the frame's flags into its own list, so every rank samples the same pixels.
-int multi_relist(RtFrame *f, bool probe, bool converge) {
-    int rc = multi_gather(f, probe);
-    if (rc != RT_OK) return rc;
+// After the probe (probe: over several parts, the frame's flags become the OR of the ranks' probe flags) or a pass that
+// ends on a checkpoint (converge: converge_kernel clears the converged pixels' flags on the first device): every rank
+// compacts the frame's flags into its own list, so every rank samples the same pixels.  With one part nothing is gathered
+// and no stream waits for another.
+int frame_relist(RtFrame *f, bool probe, bool converge) {
+    const size_t world = f->parts.size();
+    int rc;
+    if (world > 1 && (rc = frame_gather(f, probe)) != RT_OK) return rc;
     cudaStream_t st0 = part_scene(f->parts[0])->ws->stream;
     if (converge) {
         converge_kernel<<<unsigned((f->n_pixels + 255) / 256), 256, 0, st0>>>(reinterpret_cast<const int4 *>(f->d_stats), f->d_sq, f->d_flags,
                                                                               f->n_pixels, f->conv_tolerance);
         RT_CUDA(cudaGetLastError());
     }
-    RT_CUDA(cudaEventRecord(f->parts[0].listed, st0));
+    if (world > 1) RT_CUDA(cudaEventRecord(f->parts[0].listed, st0));
     int launches = 0;
-    for (size_t r = 0; r < f->parts.size(); ++r) {
+    for (size_t r = 0; r < world; ++r) {
         FramePart &p = f->parts[r];
         DeviceScene *ds = part_scene(p);
         RT_CUDA(cudaSetDevice(ds->device));
@@ -363,9 +285,10 @@ int multi_relist(RtFrame *f, bool probe, bool converge) {
     return RT_OK;
 }
 
-// Every rank: END, its counters to the host, then a synchronisation of every rank's stream.  The frame's counters are then
-// the ranks' paths summed and the shared list's length; returns the slowest rank's `from` -> END span.
-int multi_finish(RtFrame *f, FrameEvents::Which from, double *span_ms) {
+// The end of a step (the opener's or a pass), on every rank: END, its counters to the host, then a synchronisation of every
+// rank's stream.  The frame's paths are then the ranks' paths summed, and its list length the shared list's; returns the
+// slowest rank's `from` -> END span.
+int frame_sync(RtFrame *f, FrameEvents::Which from, double *span_ms) {
     for (FramePart &p : f->parts) {
         DeviceScene *ds = part_scene(p);
         RT_CUDA(cudaSetDevice(ds->device));
@@ -373,22 +296,23 @@ int multi_finish(RtFrame *f, FrameEvents::Which from, double *span_ms) {
         RT_CUDA(cudaMemcpyAsync(p.h_counters, p.d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ds->ws->stream));
     }
     *span_ms = 0.0;
-    f->h_counters[CN_PATHS] = 0;
+    f->paths_done = 0;
     for (FramePart &p : f->parts) {
         RT_CUDA(cudaSetDevice(part_scene(p)->device));
         RT_CUDA(cudaStreamSynchronize(part_scene(p)->ws->stream));
         *span_ms = std::max(*span_ms, double(p.ev.ms(from, FrameEvents::END)));
-        f->h_counters[CN_PATHS] += p.h_counters[CN_PATHS];
+        f->paths_done += p.h_counters[CN_PATHS];
     }
-    f->h_counters[CN_LIST] = f->parts[0].h_counters[CN_LIST];
+    f->pixels_listed = f->parts[0].h_counters[CN_LIST];
     return RT_OK;
 }
 
-// rt_multi_frame_begin once its arguments are checked: the frame's totals, flags and image on the first device, one part
-// per device, the split probe and the compaction from the OR of the ranks' flags
-int multi_frame_open(RtMulti *m, const RtCamera &camera, int32_t max_w, int32_t max_h, const RtRenderOpts *opts, RtFrame **out,
-                     RtFrameProgress *progress) {
-    const std::vector<RtScene *> &scenes = multi_scenes(m);
+// Every opener, once its arguments are checked: the frame's sums, Q, flags and image on the first device, one part per
+// scene (the scene of rt_frame_begin*, or the replicas of an RtMulti in rank order), the split probe and the compaction.  A
+// batch's frame is the tall frame of rt_render_views (rtfs_views.cu) with its own table; a window's frame holds the
+// window's pixels only (rtfs_window.cu).
+int frame_open(const std::vector<RtScene *> &scenes, const RtCamera &camera, const std::vector<ViewCamera> &views, const FrameWindow *window,
+               int32_t max_w, int32_t max_h, const RtRenderOpts *opts, RtFrame **out, RtFrameProgress *progress, const char *who) {
     const int world = int(scenes.size());
     const bool noise = (opts->flags & RT_FLAG_NOISE) != 0;
     int rc;
@@ -403,50 +327,69 @@ int multi_frame_open(RtMulti *m, const RtCamera &camera, int32_t max_w, int32_t 
         frame_free(f);
         return code;
     };
-    const size_t n = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
+    const size_t view_pixels = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
+    const size_t n = window ? size_t(window->rows) * size_t(window->cols) : view_pixels * std::max<size_t>(1, views.size());
     f->n_pixels = n;
+    f->n_views = std::max(1, int32_t(views.size()));
     bool ok = cudaMalloc((void **)&f->d_stats, n * 4 * sizeof(int32_t)) == cudaSuccess && cudaMalloc((void **)&f->d_flags, n) == cudaSuccess &&
               cudaMalloc((void **)&f->d_rgb, n * 3) == cudaSuccess;
     if (noise) ok = ok && cudaMalloc((void **)&f->d_sq, n * sizeof(unsigned long long)) == cudaSuccess;
+    if (!views.empty()) ok = ok && cudaMalloc((void **)&f->d_views, views.size() * sizeof(ViewCamera)) == cudaSuccess;
     f->parts.resize(size_t(world));
     for (int r = 0; r < world && ok; ++r) {
         FramePart &p = f->parts[size_t(r)];
         p.scene = scenes[size_t(r)];
-        ok = cudaSetDevice(part_scene(p)->device) == cudaSuccess && cudaMalloc((void **)&p.d_stats, n * 4 * sizeof(int32_t)) == cudaSuccess &&
-             cudaMalloc((void **)&p.d_flags, n) == cudaSuccess && cudaMalloc((void **)&p.d_list, n * sizeof(uint32_t)) == cudaSuccess &&
+        ok = cudaSetDevice(part_scene(p)->device) == cudaSuccess && cudaMalloc((void **)&p.d_list, n * sizeof(uint32_t)) == cudaSuccess &&
              cudaMalloc((void **)&p.d_counters, CN_SLOTS * sizeof(unsigned long long)) == cudaSuccess && p.ev.create() &&
              cudaEventCreateWithFlags(&p.traced, cudaEventDisableTiming) == cudaSuccess &&
              cudaEventCreateWithFlags(&p.gathered, cudaEventDisableTiming) == cudaSuccess &&
              cudaEventCreateWithFlags(&p.listed, cudaEventDisableTiming) == cudaSuccess;
+        if (world == 1) { // the only part traces into the frame's own buffers: its totals need no gather
+            p.d_stats = f->d_stats;
+            p.d_flags = f->d_flags;
+            p.d_sq = f->d_sq;
+            continue;
+        }
+        ok = ok && cudaMalloc((void **)&p.d_stats, n * 4 * sizeof(int32_t)) == cudaSuccess && cudaMalloc((void **)&p.d_flags, n) == cudaSuccess;
         if (noise) ok = ok && cudaMalloc((void **)&p.d_sq, n * sizeof(unsigned long long)) == cudaSuccess;
     }
-    if (!ok) return bail(fail(RT_ERR_CUDA, std::string("rt_multi_frame_begin: allocation failed: ") + cudaGetErrorString(cudaGetLastError())));
+    if (!ok) return bail(fail(RT_ERR_CUDA, std::string(who) + ": allocation failed: " + cudaGetErrorString(cudaGetLastError())));
 
-    // the frame's parameters are one device's (the features, the filter and the pacing read them); each rank has its own
-    fill_frame(f->fp, ds0, camera, max_w, max_h, *opts, 0, 1);
-    f->fp.stats = f->d_stats;
-    f->fp.flags = f->d_flags;
-    f->fp.sq = f->d_sq;
-    f->samples_done = f->fp.n_probe;
+    // the frame's parameters are one device's (the features, the filter, the pacing and rt_frame_extend read them); each
+    // part has its own, of rank r of world
+    auto fill = [&](FrameParams &fp, DeviceScene *ds, int r, int w) {
+        fill_frame(fp, ds, camera, max_w, max_h, *opts, r, w);
+        if (!views.empty()) set_views(fp, f->d_views, f->n_views, int32_t(view_pixels));
+        if (window) set_window(fp, *window);
+    };
+    fill(f->fp, ds0, 0, 1);
+    f->samples_done = f->fp.n_probe; // 0 without the early-out
     f->samples_target = f->fp.sample_end;
+    // (a batch has one part, on the current device; from pageable memory: staged before the call returns, and the probe
+    // follows it on the stream)
+    if (!views.empty() &&
+        cudaMemcpyAsync(f->d_views, views.data(), views.size() * sizeof(ViewCamera), cudaMemcpyHostToDevice, ds0->ws->stream) != cudaSuccess)
+        return bail(fail(RT_ERR_CUDA, std::string(who) + ": view table upload failed: " + cudaGetErrorString(cudaGetLastError())));
     int launches = 0;
     for (int r = 0; r < world; ++r) {
         FramePart &p = f->parts[size_t(r)];
         DeviceScene *ds = part_scene(p);
-        if (cudaSetDevice(ds->device) != cudaSuccess) return bail(fail(RT_ERR_CUDA, "rt_multi_frame_begin: cudaSetDevice failed"));
-        fill_frame(p.fp, ds, camera, max_w, max_h, *opts, r, world);
+        if (cudaSetDevice(ds->device) != cudaSuccess) return bail(fail(RT_ERR_CUDA, std::string(who) + ": cudaSetDevice failed"));
+        fill(p.fp, ds, r, world);
         p.fp.stats = p.d_stats;
         p.fp.flags = p.d_flags;
         p.fp.list = p.d_list;
         p.fp.counters = p.d_counters;
-        p.fp.sq = p.d_sq;
-        // the tile-split probe; with its own counter block the rank keeps the raw flags of its tiles (the frame can be extended)
+        p.fp.sq = p.d_sq; // non-null: plan_launch picks the kernels that also sum the squares
+        // the probe of the rank's tiles; with its own counter block the rank keeps the raw "means differ" flags, also where
+        // this target has no main phase: the frame can be extended
         if ((rc = frame_probe(ds, p.fp, ds->ws->stream, &p.ev, &launches)) != RT_OK) return bail(rc);
     }
-    if ((rc = multi_relist(f, true, false)) != RT_OK) return bail(rc);
-    if ((rc = multi_finish(f, FrameEvents::ZEROED, &f->device_ms)) != RT_OK) return bail(rc);
-    f->pixels_flagged = f->pixels_active = f->h_counters[CN_LIST];
-    // rt_frame_begin's rate: the slowest rank probed 1 / world of the pixels and a pass gives it 1 / world of the indices
+    if ((rc = frame_relist(f, true, false)) != RT_OK) return bail(rc);
+    if ((rc = frame_sync(f, FrameEvents::ZEROED, &f->device_ms)) != RT_OK) return bail(rc);
+    f->pixels_flagged = f->pixels_active = f->pixels_listed;
+    // the probe traced n_probe samples of every pixel, a pass traces samples of the flagged pixels only; over several
+    // devices the slowest rank probed 1 / world of the pixels and a pass gives it 1 / world of the indices
     if (f->fp.adaptive) f->ms_per_sample = f->device_ms * double(f->pixels_flagged) / (double(n) * double(f->fp.n_probe));
     *out = f;
     frame_progress(f, progress);
@@ -455,7 +398,7 @@ int multi_frame_open(RtMulti *m, const RtCamera &camera, int32_t max_w, int32_t 
 
 // one pass of every rank over [s, s + k) with s = samples_done (rank r: the indices s + r + j world) and, when it
 // ends on a checkpoint, the check; *span_ms is the slowest rank's BEGIN -> END
-int multi_pass(RtFrame *f, int k, bool check, double *span_ms) {
+int frame_pass(RtFrame *f, int k, bool check, double *span_ms) {
     int launches = 0;
     for (FramePart &p : f->parts) {
         DeviceScene *ds = part_scene(p);
@@ -470,22 +413,43 @@ int multi_pass(RtFrame *f, int k, bool check, double *span_ms) {
         int rc = launch_samples(ds, fp, st, &launches);
         if (rc != RT_OK) return rc;
     }
-    f->gathered = false;
+    f->gathered = f->parts.size() == 1;
     if (check) {
-        int rc = multi_relist(f, false, true);
+        int rc = frame_relist(f, false, true);
         if (rc != RT_OK) return rc;
     }
-    return multi_finish(f, FrameEvents::BEGIN, span_ms);
+    return frame_sync(f, FrameEvents::BEGIN, span_ms);
 }
 
 // rt_frame_view_noise reduces at most this many views per launch: the grid's y extent stays far below its limit (65535),
 // and the partials stay at most 16.8 MB however many views a batch of small extents has
 constexpr int32_t kNoiseViewChunk = 1024;
 
-// the noise reductions' partial summaries, kNoiseBlocks + 1 per view of one chunk of views, allocated on first use
-int ensure_partials(RtFrame *f) {
+// What rt_frame_noise and rt_frame_view_noise share before they reduce: their checks, the totals, and the partial summaries
+// (kNoiseBlocks + 1 per view of one chunk of views, allocated on first use); *st is the first device's stream.
+int noise_begin(RtFrame *f, double tolerance, const char *who, cudaStream_t *st) {
+    if (!f->d_sq) return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": the frame was opened without RT_FLAG_NOISE");
+    if (!(tolerance >= 0.0)) return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": tolerance must be >= 0");
+    int rc = ensure_totals(f);
+    if (rc != RT_OK) return rc;
+    auto *ds = static_cast<DeviceScene *>(f->scene->dev);
+    RT_CUDA(cudaSetDevice(ds->device));
+    *st = ds->ws->stream;
     const size_t views = size_t(std::min(f->n_views, kNoiseViewChunk));
     if (!f->d_partial) RT_CUDA(cudaMalloc((void **)&f->d_partial, views * (kNoiseBlocks + 1) * sizeof(NoisePartial)));
+    return RT_OK;
+}
+
+// The reduction of views [v0, v0 + nv) of view_pixels pixels each, every view as rt_frame_noise reduces a frame of its
+// pixels (the same 512 ranges, tree and block order): view v0 + i's summary is then at d_partial + i (kNoiseBlocks + 1) +
+// kNoiseBlocks.  se (or null) receives E of every pixel of those views.
+int launch_noise(RtFrame *f, int32_t v0, int32_t nv, size_t view_pixels, double tolerance, float *se, cudaStream_t st) {
+    const size_t at = size_t(v0) * view_pixels;
+    noise_kernel<<<dim3(kNoiseBlocks, unsigned(nv)), kNoiseThreads, 0, st>>>(reinterpret_cast<const int4 *>(f->d_stats) + at, f->d_sq + at,
+                                                                              f->d_flags + at, view_pixels, tolerance, se, f->d_partial);
+    RT_CUDA(cudaGetLastError());
+    noise_summary_kernel<<<unsigned(nv), kNoiseThreads, 0, st>>>(f->d_partial);
+    RT_CUDA(cudaGetLastError());
     return RT_OK;
 }
 
@@ -520,13 +484,6 @@ int check_current(const RtFrame *f, const char *who) {
     return RT_OK;
 }
 
-// the refusals of both openers, after their own argument checks
-int check_frame_mode(const RtRenderOpts *opts, const char *who) {
-    if (opts->mode == RT_MODE_WAVEFRONT) return fail(RT_ERR_UNSUPPORTED, std::string(who) + ": progressive frames run the megakernel only");
-    if (opts->mode != RT_MODE_MEGAKERNEL) return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": unknown mode");
-    return RT_OK;
-}
-
 } // namespace
 
 extern "C" {
@@ -537,37 +494,20 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
     if (rc != RT_OK) return rc;
     if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin: out is null");
     *out = nullptr;
-    if ((rc = check_frame_mode(opts, "rt_frame_begin")) != RT_OK) return rc;
-    if ((opts->flags & RT_FLAG_NOISE) && (opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS)))
-        return fail(RT_ERR_UNSUPPORTED, "rt_frame_begin: RT_FLAG_NOISE has no flow-schedule or counting kernel");
-    return frame_open(scene, *camera, {}, nullptr, max_w, max_h, opts, out, progress, "rt_frame_begin");
+    if ((rc = check_frame_mode(opts, "rt_frame_begin", false)) != RT_OK) return rc;
+    return frame_open({scene}, *camera, {}, nullptr, max_w, max_h, opts, out, progress, "rt_frame_begin");
 }
 
 int rt_frame_begin_views(RtScene *scene, const RtCamera *cameras, const uint64_t *seeds, int32_t n_views, int32_t max_w, int32_t max_h,
                          const RtRenderOpts *opts, RtFrame **out, RtFrameProgress *progress) {
     // rt_render_views' checks, then rt_frame_begin's
-    if (n_views < 1) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin_views: n_views must be >= 1");
-    if (!cameras) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin_views: cameras is null");
-    int rc = check_frame_args(scene, &cameras[0], max_w, max_h, opts);
+    int rc = check_views(scene, cameras, n_views, max_w, max_h, opts, "rt_frame_begin_views");
     if (rc != RT_OK) return rc;
-    for (int32_t v = 1; v < n_views; ++v)
-        if (cameras[v].samples_per_pixel != cameras[0].samples_per_pixel || cameras[v].bounce_depth != cameras[0].bounce_depth)
-            return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin_views: every camera must have the same samples_per_pixel and bounce_depth");
-    if (size_t(2 * max_w + 1) * size_t(2 * max_h + 1) * size_t(n_views) >= (size_t(1) << 31))
-        return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin_views: n_views x rows x cols must be below 2^31");
     if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin_views: out is null");
     *out = nullptr;
-    if ((rc = check_frame_mode(opts, "rt_frame_begin_views")) != RT_OK) return rc;
-    if (opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS))
-        return fail(RT_ERR_UNSUPPORTED, "rt_frame_begin_views: a batch of views has no flow-schedule or counting kernel");
-    std::vector<ViewCamera> table(n_views);
-    for (int32_t v = 0; v < n_views; ++v) {
-        const uint64_t seed = seeds ? seeds[v] : opts->seed;
-        table[v].cam = make_dev_camera(cameras[v], max_w, max_h);
-        table[v].k0 = uint32_t(seed);
-        table[v].k1 = uint32_t(seed >> 32);
-    }
-    return frame_open(scene, cameras[0], table, nullptr, max_w, max_h, opts, out, progress, "rt_frame_begin_views");
+    if ((rc = check_frame_mode(opts, "rt_frame_begin_views", true)) != RT_OK) return rc;
+    return frame_open({scene}, cameras[0], view_table(cameras, seeds, n_views, max_w, max_h, opts->seed), nullptr, max_w, max_h, opts, out,
+                      progress, "rt_frame_begin_views");
 }
 
 int rt_frame_begin_window(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_t max_h, int32_t row0, int32_t col0, int32_t rows,
@@ -579,10 +519,8 @@ int rt_frame_begin_window(RtScene *scene, const RtCamera *camera, int32_t max_w,
     if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin_window: out is null");
     *out = nullptr;
     if ((rc = check_frame_args(scene, camera, max_w, max_h, opts)) != RT_OK) return rc;
-    if ((rc = check_frame_mode(opts, "rt_frame_begin_window")) != RT_OK) return rc;
-    if (opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS))
-        return fail(RT_ERR_UNSUPPORTED, "rt_frame_begin_window: a window has no flow-schedule or counting kernel");
-    return frame_open(scene, *camera, {}, &w, max_w, max_h, opts, out, progress, "rt_frame_begin_window");
+    if ((rc = check_frame_mode(opts, "rt_frame_begin_window", true)) != RT_OK) return rc;
+    return frame_open({scene}, *camera, {}, &w, max_w, max_h, opts, out, progress, "rt_frame_begin_window");
 }
 
 int rt_multi_frame_begin(RtMulti *multi, const RtCamera *camera, int32_t max_w, int32_t max_h, const RtRenderOpts *opts, RtFrame **out,
@@ -593,10 +531,8 @@ int rt_multi_frame_begin(RtMulti *multi, const RtCamera *camera, int32_t max_w, 
     // rt_frame_begin's checks and refusals, on the first device's replica
     int rc = check_frame_args(multi_scenes(multi)[0], camera, max_w, max_h, opts);
     if (rc != RT_OK) return rc;
-    if ((rc = check_frame_mode(opts, "rt_multi_frame_begin")) != RT_OK) return rc;
-    if ((opts->flags & RT_FLAG_NOISE) && (opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS)))
-        return fail(RT_ERR_UNSUPPORTED, "rt_multi_frame_begin: RT_FLAG_NOISE has no flow-schedule or counting kernel");
-    return multi_frame_open(multi, *camera, max_w, max_h, opts, out, progress);
+    if ((rc = check_frame_mode(opts, "rt_multi_frame_begin", false)) != RT_OK) return rc;
+    return frame_open(multi_scenes(multi), *camera, {}, nullptr, max_w, max_h, opts, out, progress, "rt_multi_frame_begin");
 }
 
 int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameProgress *progress) {
@@ -621,37 +557,14 @@ int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameP
         if (rule) k = int(std::min<int64_t>(k, next_checkpoint(f) - f->samples_done)); // a pass never crosses a checkpoint
         const bool check = rule && f->samples_done + k == next_checkpoint(f);
         double span_ms = 0.0;
-        if (f->parts.empty()) {
-            auto *ds = static_cast<DeviceScene *>(f->scene->dev);
-            RT_CUDA(cudaSetDevice(ds->device));
-            cudaStream_t st = ds->ws->stream;
-            FrameParams fp = f->fp;
-            fp.sample_begin = f->samples_done;
-            fp.sample_end = f->samples_done + k;
-            int launches = 0;
-            RT_CUDA(cudaMemsetAsync(f->d_counters + CN_WORK_MAIN, 0, sizeof(unsigned long long), st));
-            RT_CUDA(f->ev.record(FrameEvents::BEGIN, st));
-            int rc = launch_samples(ds, fp, st, &launches);
-            if (rc != RT_OK) return rc;
-            if (check) { // the pass ends on a checkpoint: stop the converged pixels and list the others
-                converge_kernel<<<unsigned((f->n_pixels + 255) / 256), 256, 0, st>>>(reinterpret_cast<const int4 *>(f->d_stats), f->d_sq,
-                                                                                     f->d_flags, f->n_pixels, f->conv_tolerance);
-                RT_CUDA(cudaGetLastError());
-                if ((rc = launch_compact(ds, fp, single_flags(f->d_flags), f->d_list, st, &launches)) != RT_OK) return rc;
-            }
-            RT_CUDA(f->ev.record(FrameEvents::END, st));
-            if ((rc = frame_sync(f, st)) != RT_OK) return rc;
-            span_ms = f->ev.ms(FrameEvents::BEGIN, FrameEvents::END);
-        } else if (int rc = multi_pass(f, k, check, &span_ms); rc != RT_OK) {
-            return rc;
-        }
+        if (int rc = frame_pass(f, k, check, &span_ms); rc != RT_OK) return rc;
         f->samples_done += k;
         f->passes += 1;
         f->last_pass_ms = span_ms;
         f->device_ms += f->last_pass_ms;
         const uint64_t before = f->pixels_active;
         if (check) {
-            f->pixels_active = f->h_counters[CN_LIST];
+            f->pixels_active = f->pixels_listed;
             f->conv_checks += 1;
             if (f->pixels_active == 0) f->samples_done = f->samples_target; // done, without a launch
         }
@@ -698,21 +611,11 @@ void rt_frame_destroy(RtFrame *f) { frame_free(f); }
 
 int rt_frame_noise(RtFrame *f, double tolerance, float *se_out, uint64_t *sq_out, RtFrameNoise *summary) {
     if (!f) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_noise: null frame");
-    if (!f->d_sq) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_noise: the frame was opened without RT_FLAG_NOISE");
-    if (!(tolerance >= 0.0)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_noise: tolerance must be >= 0");
-    int rc = ensure_totals(f);
-    if (rc != RT_OK) return rc;
-    auto *ds = static_cast<DeviceScene *>(f->scene->dev);
-    RT_CUDA(cudaSetDevice(ds->device));
-    cudaStream_t st = ds->ws->stream;
-    rc = ensure_partials(f);
+    cudaStream_t st;
+    int rc = noise_begin(f, tolerance, "rt_frame_noise", &st);
     if (rc != RT_OK) return rc;
     if (se_out && !f->d_se) RT_CUDA(cudaMalloc((void **)&f->d_se, f->n_pixels * sizeof(float)));
-    noise_kernel<<<kNoiseBlocks, kNoiseThreads, 0, st>>>(reinterpret_cast<const int4 *>(f->d_stats), f->d_sq, f->d_flags, f->n_pixels, tolerance,
-                                                         se_out ? f->d_se : nullptr, f->d_partial);
-    RT_CUDA(cudaGetLastError());
-    noise_summary_kernel<<<1, kNoiseThreads, 0, st>>>(f->d_partial);
-    RT_CUDA(cudaGetLastError());
+    if ((rc = launch_noise(f, 0, 1, f->n_pixels, tolerance, se_out ? f->d_se : nullptr, st)) != RT_OK) return rc;
     NoisePartial total;
     RT_CUDA(cudaMemcpyAsync(&total, f->d_partial + kNoiseBlocks, sizeof total, cudaMemcpyDeviceToHost, st));
     if (se_out) RT_CUDA(cudaMemcpyAsync(se_out, f->d_se, f->n_pixels * sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -724,27 +627,15 @@ int rt_frame_noise(RtFrame *f, double tolerance, float *se_out, uint64_t *sq_out
 
 int rt_frame_view_noise(RtFrame *f, double tolerance, RtFrameNoise *per_view) {
     if (!f || !per_view) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_view_noise: null frame or output");
-    if (!f->d_sq) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_view_noise: the frame was opened without RT_FLAG_NOISE");
-    if (!(tolerance >= 0.0)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_view_noise: tolerance must be >= 0");
-    int rc = ensure_totals(f);
+    cudaStream_t st;
+    int rc = noise_begin(f, tolerance, "rt_frame_view_noise", &st);
     if (rc != RT_OK) return rc;
-    auto *ds = static_cast<DeviceScene *>(f->scene->dev);
-    RT_CUDA(cudaSetDevice(ds->device));
-    cudaStream_t st = ds->ws->stream;
-    rc = ensure_partials(f);
-    if (rc != RT_OK) return rc;
-    // every view reduced as rt_frame_noise reduces a frame of its pixels: the same 512 ranges, tree and block order
     const size_t view_pixels = f->n_pixels / size_t(f->n_views);
     std::vector<NoisePartial> totals(size_t(f->n_views));
     for (int32_t v0 = 0; v0 < f->n_views; v0 += kNoiseViewChunk) {
         const int32_t nv = std::min(kNoiseViewChunk, f->n_views - v0);
-        const size_t at = size_t(v0) * view_pixels;
-        noise_kernel<<<dim3(kNoiseBlocks, unsigned(nv)), kNoiseThreads, 0, st>>>(reinterpret_cast<const int4 *>(f->d_stats) + at, f->d_sq + at,
-                                                                                  f->d_flags + at, view_pixels, tolerance, nullptr, f->d_partial);
-        RT_CUDA(cudaGetLastError());
-        noise_summary_kernel<<<unsigned(nv), kNoiseThreads, 0, st>>>(f->d_partial);
-        RT_CUDA(cudaGetLastError());
-        // (the next chunk's kernels follow this copy on the stream before they overwrite the partials)
+        if ((rc = launch_noise(f, v0, nv, view_pixels, tolerance, nullptr, st)) != RT_OK) return rc;
+    // (the next chunk's kernels follow this copy on the stream before they overwrite the partials)
         RT_CUDA(cudaMemcpy2DAsync(totals.data() + v0, sizeof(NoisePartial), f->d_partial + kNoiseBlocks, (kNoiseBlocks + 1) * sizeof(NoisePartial),
                                   sizeof(NoisePartial), size_t(nv), cudaMemcpyDeviceToHost, st));
     }

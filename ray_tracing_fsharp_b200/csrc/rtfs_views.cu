@@ -84,6 +84,39 @@ static int ensure_views(DeviceWorkspace *ws, size_t n_views) {
     return RT_OK;
 }
 
+int check_views(const RtScene *scene, const RtCamera *cameras, int32_t n_views, int max_w, int max_h, const RtRenderOpts *opts, const char *who) {
+    if (n_views < 1) return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": n_views must be >= 1");
+    if (!cameras) return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": cameras is null");
+    int rc = check_frame_args(scene, &cameras[0], max_w, max_h, opts);
+    if (rc != RT_OK) return rc;
+    // the probe's firstTrial, the chunk table and the bounce budget are the batch's
+    for (int32_t v = 1; v < n_views; ++v)
+        if (cameras[v].samples_per_pixel != cameras[0].samples_per_pixel || cameras[v].bounce_depth != cameras[0].bounce_depth)
+            return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": every camera must have the same samples_per_pixel and bounce_depth");
+    if (size_t(2 * max_w + 1) * size_t(2 * max_h + 1) * size_t(n_views) >= (size_t(1) << 31))
+        return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": n_views x rows x cols must be below 2^31");
+    return RT_OK;
+}
+
+std::vector<ViewCamera> view_table(const RtCamera *cameras, const uint64_t *seeds, int32_t n_views, int max_w, int max_h, uint64_t seed) {
+    std::vector<ViewCamera> table(n_views);
+    for (int32_t v = 0; v < n_views; ++v) {
+        const uint64_t s = seeds ? seeds[v] : seed;
+        table[v].cam = make_dev_camera(cameras[v], max_w, max_h);
+        table[v].k0 = uint32_t(s);
+        table[v].k1 = uint32_t(s >> 32);
+    }
+    return table;
+}
+
+void set_views(FrameParams &fp, const ViewCamera *d_views, int32_t n_views, int32_t view_pixels) {
+    fp.cam.rows *= n_views;
+    fp.tiles_y = (fp.cam.rows + kTileH - 1) / kTileH;
+    fp.views = d_views;
+    fp.n_views = n_views;
+    fp.view_pixels = view_pixels;
+}
+
 } // namespace rtfs
 
 using namespace rtfs;
@@ -92,21 +125,12 @@ extern "C" {
 
 int rt_render_views(RtScene *scene, const RtCamera *cameras, const uint64_t *seeds, int32_t n_views, int32_t max_w, int32_t max_h,
                     const RtRenderOpts *opts, uint8_t *rgb_out, int32_t *sums_out, RtStats *stats) {
-    if (n_views < 1) return fail(RT_ERR_INVALID_ARGUMENT, "rt_render_views: n_views must be >= 1");
-    if (!cameras || !rgb_out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_render_views: cameras or rgb_out is null");
-    int rc = check_frame_args(scene, &cameras[0], max_w, max_h, opts);
+    if (!rgb_out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_render_views: rgb_out is null");
+    int rc = check_views(scene, cameras, n_views, max_w, max_h, opts, "rt_render_views");
     if (rc != RT_OK) return rc;
-    // the probe's firstTrial, the chunk table and the bounce budget are the batch's
-    for (int32_t v = 1; v < n_views; ++v)
-        if (cameras[v].samples_per_pixel != cameras[0].samples_per_pixel || cameras[v].bounce_depth != cameras[0].bounce_depth)
-            return fail(RT_ERR_INVALID_ARGUMENT, "rt_render_views: every camera must have the same samples_per_pixel and bounce_depth");
+    if ((rc = check_frame_mode(opts, "rt_render_views", true)) != RT_OK) return rc;
     const size_t view_pixels = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
     const size_t n_pixels = view_pixels * size_t(n_views);
-    if (n_pixels >= (size_t(1) << 31)) return fail(RT_ERR_INVALID_ARGUMENT, "rt_render_views: n_views x rows x cols must be below 2^31");
-    if (opts->mode == RT_MODE_WAVEFRONT) return fail(RT_ERR_UNSUPPORTED, "rt_render_views: a batch of views runs the megakernel only");
-    if (opts->mode != RT_MODE_MEGAKERNEL) return fail(RT_ERR_INVALID_ARGUMENT, "rt_render_views: unknown mode");
-    if (opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS))
-        return fail(RT_ERR_UNSUPPORTED, "rt_render_views: a batch of views has no flow-schedule or counting kernel");
     if ((rc = prepare_frame(scene, opts)) != RT_OK) return rc;
     auto *ds = static_cast<DeviceScene *>(scene->dev);
     RT_CUDA(cudaSetDevice(ds->device));
@@ -114,22 +138,12 @@ int rt_render_views(RtScene *scene, const RtCamera *cameras, const uint64_t *see
     if ((rc = ensure_frame_buffers(ws, n_pixels)) != RT_OK) return rc;
     if ((rc = ensure_views(ws, size_t(n_views))) != RT_OK) return rc;
     cudaStream_t st = ws->stream;
-    std::vector<ViewCamera> table(n_views);
-    for (int32_t v = 0; v < n_views; ++v) {
-        const uint64_t seed = seeds ? seeds[v] : opts->seed;
-        table[v].cam = make_dev_camera(cameras[v], max_w, max_h);
-        table[v].k0 = uint32_t(seed);
-        table[v].k1 = uint32_t(seed >> 32);
-    }
+    const std::vector<ViewCamera> table = view_table(cameras, seeds, n_views, max_w, max_h, opts->seed);
     // (from pageable memory: the call returns once the table is staged, so it may go out of scope)
     RT_CUDA(cudaMemcpyAsync(ws->d_views, table.data(), table.size() * sizeof(ViewCamera), cudaMemcpyHostToDevice, st));
     FrameParams fp;
     fill_frame(fp, ds, cameras[0], max_w, max_h, *opts, 0, 1);
-    fp.cam.rows *= n_views; // the tall frame: probe tiles, flags, list and sums run over it as over one frame
-    fp.tiles_y = (fp.cam.rows + kTileH - 1) / kTileH;
-    fp.views = ws->d_views;
-    fp.n_views = n_views;
-    fp.view_pixels = int32_t(view_pixels);
+    set_views(fp, ws->d_views, n_views, int32_t(view_pixels));
     fp.stats = ws->d_stats;
     fp.flags = ws->d_flags;
     int launches = 0;

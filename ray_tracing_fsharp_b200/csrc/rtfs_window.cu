@@ -89,10 +89,7 @@ int rt_render_window(RtScene *scene, const RtCamera *camera, int32_t max_w, int3
     if (rc != RT_OK) return rc;
     if (!rgb_out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_render_window: rgb_out is null");
     if ((rc = check_frame_args(scene, camera, max_w, max_h, opts)) != RT_OK) return rc;
-    if (opts->mode == RT_MODE_WAVEFRONT) return fail(RT_ERR_UNSUPPORTED, "rt_render_window: a window runs the megakernel only");
-    if (opts->mode != RT_MODE_MEGAKERNEL) return fail(RT_ERR_INVALID_ARGUMENT, "rt_render_window: unknown mode");
-    if (opts->flags & (RT_FLAG_FLOW | RT_FLAG_COUNTERS))
-        return fail(RT_ERR_UNSUPPORTED, "rt_render_window: a window has no flow-schedule or counting kernel");
+    if ((rc = check_frame_mode(opts, "rt_render_window", true)) != RT_OK) return rc;
     if ((rc = prepare_frame(scene, opts)) != RT_OK) return rc;
     auto *ds = static_cast<DeviceScene *>(scene->dev);
     RT_CUDA(cudaSetDevice(ds->device));

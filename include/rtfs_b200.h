@@ -257,6 +257,41 @@ int rt_scene_update(RtScene *scene, const int32_t *object_index, const RtHittabl
                     const int32_t *texture_index, const RtTexture *textures, int32_t n_textures,
                     RtSceneUpdate *info /* optional */);
 
+/* Removes and appends objects of a scene and builds its tree anew on the device: for adding or deleting an object of a live
+ * scene, and for renewing a tree that rt_scene_update's refits have left slow to walk, without rt_scene_create's host build
+ * and full upload, and without closing the scene's handle.
+ *
+ * The objects remove[0..n_remove) (indices into the caller's array) are taken out; the others keep their order and are
+ * renumbered densely; then append[0..n_append) are added at the end.  After the call the scene is rt_scene_create(new array,
+ * the same textures), except that its tree comes from the device builder (PLOC over the FP32 sphere boxes, DESIGN.md section
+ * 22): every entry point (rt_render, views, windows, progressive frames opened after the call, features with the new object
+ * indices, denoise; sums, RGB8, Q, stats, rays, every flag) gives bit for bit the frame of a freshly created scene of the new
+ * array, wherever no closest hit is an exact tie in t between two bounded spheres (rt_scene_update's condition).  With
+ * n_remove = n_append = 0 the call rebuilds the tree of the current objects.
+ * Determinism.  The tree is a pure function of the object array after the call: two scenes that reach the same array by any
+ *   edit sequences hold identical trees, byte for byte.
+ * Fallback.  A device tree deeper than the walk stacks allow (60) is replaced by the host SAH tree rt_scene_create builds
+ *   (on_device = 0); the call does not fail for that reason.
+ * Refusals (RT_ERR_INVALID_ARGUMENT, before any change or device work, leaving the scene as it was): a remove index out of
+ * range or repeated, a negative count, a NULL array with a non-zero count, and anything rt_scene_create would refuse in an
+ * appended object (such as a texture index out of range).  Textures cannot be added or removed here (rt_scene_update
+ * replaces a texture's content).  A scene created with device = -1: RT_ERR_UNSUPPORTED.
+ * Frames opened before the call are stale, as after rt_scene_update; rt_scene_update refits the new tree.
+ * Returns with its device work complete.  info optional.  A caller detects the feature by the symbol rt_scene_rebuild. */
+typedef struct RtSceneRebuild {
+    int32_t objects_removed, objects_appended;
+    int32_t n_objects; /* the caller's array after the call                                                       */
+    int32_t n_bounded; /* spheres in the tree                                                                     */
+    int32_t nodes;     /* of the new tree                                                                         */
+    int32_t depth;     /* of the new tree: internal nodes on its longest root-to-leaf path                        */
+    int32_t on_device; /* 1: the device build; 0: the host SAH build (the device tree was deeper than 60)         */
+    int32_t launches;
+    uint64_t generation; /* the scene's edit count after the call                                                 */
+    double device_ms;    /* CUDA events around the device work                                                   */
+} RtSceneRebuild;
+int rt_scene_rebuild(RtScene *scene, const int32_t *remove, int32_t n_remove, const RtHittable *append, int32_t n_append,
+                     RtSceneRebuild *info /* optional */);
+
 /* ---- host buffers ----------------------------------------------------------------------------- */
 /* Page-locks a host buffer the caller owns (an output frame it renders into again and again) so that the device->host
  * copy of rt_render / rt_multi_render / rt_comm_render runs at PCIe speed and asynchronously instead of through the

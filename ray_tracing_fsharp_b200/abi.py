@@ -176,6 +176,21 @@ class RtDenoiseOpts(C.Structure):
     ]
 
 
+class RtSceneRebuild(C.Structure):
+    _fields_ = [
+        ("objects_removed", C.c_int32),
+        ("objects_appended", C.c_int32),
+        ("n_objects", C.c_int32),
+        ("n_bounded", C.c_int32),
+        ("nodes", C.c_int32),
+        ("depth", C.c_int32),
+        ("on_device", C.c_int32),
+        ("launches", C.c_int32),
+        ("generation", C.c_uint64),
+        ("device_ms", C.c_double),
+    ]
+
+
 class RtSceneUpdate(C.Structure):
     _fields_ = [
         ("objects", C.c_int32),

@@ -220,7 +220,7 @@ int scene_device(RtScene *scene, DeviceScene **out) {
     if (!scene->dev) return fail(RT_ERR_NO_DEVICE, "the scene was created without a device (device = -1); there is no CPU fallback");
     *out = static_cast<DeviceScene *>(scene->dev);
     RT_CUDA(cudaSetDevice((*out)->device));
-    return RT_OK;
+    return device_scene_sync_layout(scene); // after a rebuild: the device ids the primitive indices map to
 }
 
 int map_prims(const RtScene *scene, int n, const int32_t *prim, std::vector<int32_t> &out) {

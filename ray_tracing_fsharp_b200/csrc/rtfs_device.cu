@@ -141,6 +141,8 @@ void device_scene_free(RtScene *scene) {
     cudaFree(ds->wide_blob); // (the main blob lives in the workspace)
     cudaFree(ds->edit_stage);
     cudaFree(ds->refit);
+    cudaFree(ds->build_scratch);
+    cudaFree(ds->dev_of);
     if (ds->ws) workspace_release(ds->ws);
     for (const PooledTexture &t : ds->images) texture_release(t);
     delete ds;
@@ -208,16 +210,10 @@ int device_scene_upload(RtScene *scene) {
     }
 
     // everything else travels as one blob: one allocation, one host->device copy
-    auto align = [](size_t x) { return (x + 255) & ~size_t(255); };
-    const size_t off_nodes = 0;
-    const size_t off_spheres = align(off_nodes + L.nodes.size() * sizeof(DNode));
-    const size_t off_mats = align(off_spheres + L.spheres.size() * sizeof(DSphere));
-    const size_t off_unb = align(off_mats + L.materials.size() * sizeof(DMaterial));
-    const size_t off_ref = align(off_unb + L.unbounded.size() * sizeof(DUnbounded));
-    const size_t off_tex = off_ref;
-    const size_t total = align(off_tex + dt.size() * sizeof(DTexture)) + 256;
+    const BlobLayout B = blob_layout(L.nodes.size(), L.spheres.size(), L.unbounded.size(), dt.size());
+    const size_t off_nodes = B.nodes, off_spheres = B.spheres, off_mats = B.mats, off_unb = B.unb, off_tex = B.tex, total = B.total;
     DeviceWorkspace *ws = ds->ws;
-    if (ws->blob_cap < total) { // grow the pooled blob and its pinned staging copy
+    if (ws->blob_cap < total || ws->h_blob_cap < total) { // grow the pooled blob and its pinned staging copy (rt_scene_rebuild grows the blob alone)
         cudaFree(ws->d_blob);
         if (ws->h_blob) cudaFreeHost(ws->h_blob);
         ws->d_blob = ws->h_blob = nullptr;
@@ -317,6 +313,7 @@ int prepare_frame(RtScene *scene, const RtRenderOpts *opts) {
 int device_scene_ensure_reference(RtScene *scene) {
     auto *ds = static_cast<DeviceScene *>(scene->dev);
     if (!ds || ds->ref_nodes) return RT_OK;
+    if (int rc = device_scene_sync_layout(scene); rc != RT_OK) return rc; // after a rebuild: the device ids of its leaves
     scene_ensure_reference(scene);
     const auto &nodes = scene->layout.ref_nodes;
     RT_CUDA(cudaSetDevice(ds->device));

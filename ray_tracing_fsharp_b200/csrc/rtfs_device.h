@@ -125,7 +125,53 @@ struct DeviceScene {
     void *edit_stage = nullptr;
     size_t edit_stage_cap = 0;
     void *refit = nullptr;
+    // rt_scene_rebuild (rtfs_build.cu): the builder's scratch (grow-only), and the caller's index -> device primitive id map
+    // on the device (dev_of_valid: it matches the scene; else the next rebuild uploads layout.device_id_of)
+    void *build_scratch = nullptr;
+    size_t build_scratch_cap = 0;
+    int32_t *dev_of = nullptr;
+    size_t dev_of_cap = 0;
+    bool dev_of_valid = false;
 };
+
+// Where the scene blob holds each section: nodes | spheres | materials | unbounded | textures, each 256-byte aligned
+// (device_scene_upload, rt_scene_rebuild)
+struct BlobLayout {
+    size_t nodes, spheres, mats, unb, tex, total;
+};
+inline BlobLayout blob_layout(size_t n_nodes, size_t n_bounded, size_t n_unbounded, size_t n_tex) {
+    auto align = [](size_t x) { return (x + 255) & ~size_t(255); };
+    BlobLayout b;
+    b.nodes = 0;
+    b.spheres = align(b.nodes + n_nodes * sizeof(DNode));
+    b.mats = align(b.spheres + n_bounded * sizeof(DSphere));
+    b.unb = align(b.mats + (n_bounded + n_unbounded) * sizeof(DMaterial));
+    b.tex = align(b.unb + n_unbounded * sizeof(DUnbounded));
+    b.total = align(b.tex + n_tex * sizeof(DTexture)) + 256;
+    return b;
+}
+
+// The refit's state on the device (rtfs_edit.cu), one allocation: the tree's min / max form, the parent link
+// (node << 1 | side; -1 for the root) of every node and every leaf, per node the number of dirty children and the arrivals
+// so far (both back to 0 once a node is refit), and the count of nodes refit by a call.  rt_scene_rebuild writes it for
+// the tree it builds.
+struct RefitView {
+    DNode *minmax;
+    int32_t *node_parent;
+    int32_t *leaf_parent;
+    uint32_t *dirty;
+    uint32_t *arrive;
+    uint32_t *refit_nodes;
+};
+// the view of the refit state of a tree of n_nodes nodes over n_bounded spheres at `base` (null: offsets only); *total its
+// bytes, *zeroed_from the offset from which it starts as zeros (dirty, arrive, count)
+RefitView refit_view(void *base, size_t n_nodes, size_t n_bounded, size_t *total, size_t *zeroed_from);
+// RT_ERR_INVALID_ARGUMENT unless every index lies in [0, count) and none repeats; `what` names the indices, `who` the caller
+int check_indices(const int32_t *index, int32_t n, int32_t count, const char *what, const char *who);
+// after the tree changed (rtfs_edit.cu): the trees derived from it are rebuilt on first use, the 8-wide one after its boxes
+// changed, the reference-topology one after a sphere's centre or radius or the object array did
+void invalidate_wide(RtScene *scene, DeviceScene *ds);
+void invalidate_reference(RtScene *scene, DeviceScene *ds);
 // an RtTexture's device record, without the texture object of an image (set by the caller)
 DTexture device_texture_of(const RtTexture &t);
 // an image texture's texels in the form its array holds

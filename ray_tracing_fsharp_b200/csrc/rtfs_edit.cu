@@ -23,18 +23,6 @@ using namespace rtfs;
 
 namespace rtfs {
 
-// the refit's state on the device: the tree's min / max form, the parent link (node << 1 | side; -1 for the root) of every
-// node and every leaf, per node the number of dirty children and the arrivals so far (both back to 0 once a node is
-// refit), and the count of nodes refit by this call
-struct RefitView {
-    DNode *minmax;
-    int32_t *node_parent;
-    int32_t *leaf_parent;
-    uint32_t *dirty;
-    uint32_t *arrive;
-    uint32_t *refit_nodes;
-};
-
 constexpr int kEditThreads = 256;
 
 __global__ void __launch_bounds__(kEditThreads) edit_scatter_kernel(const uint4 *words, const uint32_t *dst, int32_t n, uint4 *blob) {
@@ -115,21 +103,18 @@ namespace {
 size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
 
 // The refit's state, allocated and uploaded from the host layout by the first edit that moves a sphere (scenes that are
-// never edited pay nothing).  The one-sphere tree's root holds the leaf on the left and the never-entered {+inf} box on
-// the right, which no edit touches.
+// never edited pay nothing; rt_scene_rebuild leaves it written for the tree it built).  The one-sphere tree's root holds
+// the leaf on the left and the never-entered {+inf} box on the right, which no edit touches.
 int ensure_refit(RtScene *scene, DeviceScene *ds, RefitView &r) {
     const HostSceneLayout &L = scene->layout;
     const size_t nn = L.nodes.size(), nb = size_t(L.n_bounded);
-    const size_t off_np = align256(nn * sizeof(DNode));
-    const size_t off_lp = align256(off_np + nn * sizeof(int32_t));
-    const size_t off_dirty = align256(off_lp + nb * sizeof(int32_t));
-    const size_t off_arrive = align256(off_dirty + nn * sizeof(uint32_t));
-    const size_t off_count = align256(off_arrive + nn * sizeof(uint32_t));
-    const size_t total = off_count + 256;
+    size_t total = 0, off_dirty = 0;
+    const RefitView offsets = refit_view(nullptr, nn, nb, &total, &off_dirty);
     if (!ds->refit) {
         std::vector<uint8_t> host(off_dirty, 0);
         std::memcpy(host.data(), L.nodes.data(), nn * sizeof(DNode));
-        int32_t *np = reinterpret_cast<int32_t *>(host.data() + off_np), *lp = reinterpret_cast<int32_t *>(host.data() + off_lp);
+        int32_t *np = reinterpret_cast<int32_t *>(host.data() + size_t(offsets.node_parent)),
+                *lp = reinterpret_cast<int32_t *>(host.data() + size_t(offsets.leaf_parent));
         np[0] = -1;
         for (size_t i = 0; i < nn; ++i) {
             const DNode &nd = L.nodes[i];
@@ -145,28 +130,39 @@ int ensure_refit(RtScene *scene, DeviceScene *ds, RefitView &r) {
         RT_CUDA(cudaMemset(static_cast<uint8_t *>(ds->refit) + off_dirty, 0, total - off_dirty));
         ds->bytes += total;
     }
-    uint8_t *base = static_cast<uint8_t *>(ds->refit);
-    r.minmax = reinterpret_cast<DNode *>(base);
-    r.node_parent = reinterpret_cast<int32_t *>(base + off_np);
-    r.leaf_parent = reinterpret_cast<int32_t *>(base + off_lp);
-    r.dirty = reinterpret_cast<uint32_t *>(base + off_dirty);
-    r.arrive = reinterpret_cast<uint32_t *>(base + off_arrive);
-    r.refit_nodes = reinterpret_cast<uint32_t *>(base + off_count);
+    r = refit_view(ds->refit, nn, nb, &total, &off_dirty);
     return RT_OK;
 }
 
-// RT_ERR_INVALID_ARGUMENT unless every index lies in [0, count) and none repeats
-int check_indices(const int32_t *index, int32_t n, int32_t count, const char *what) {
+} // namespace
+
+RefitView refit_view(void *base, size_t nn, size_t nb, size_t *total, size_t *zeroed_from) {
+    const size_t off_np = align256(nn * sizeof(DNode));
+    const size_t off_lp = align256(off_np + nn * sizeof(int32_t));
+    const size_t off_dirty = align256(off_lp + nb * sizeof(int32_t));
+    const size_t off_arrive = align256(off_dirty + nn * sizeof(uint32_t));
+    const size_t off_count = align256(off_arrive + nn * sizeof(uint32_t));
+    *total = off_count + 256;
+    *zeroed_from = off_dirty;
+    uint8_t *b = static_cast<uint8_t *>(base);
+    return RefitView{reinterpret_cast<DNode *>(b), reinterpret_cast<int32_t *>(b + off_np), reinterpret_cast<int32_t *>(b + off_lp),
+                     reinterpret_cast<uint32_t *>(b + off_dirty), reinterpret_cast<uint32_t *>(b + off_arrive),
+                     reinterpret_cast<uint32_t *>(b + off_count)};
+}
+
+int check_indices(const int32_t *index, int32_t n, int32_t count, const char *what, const char *who) {
     std::vector<int32_t> sorted(index, index + n);
     std::sort(sorted.begin(), sorted.end());
     for (int32_t i = 0; i < n; ++i) {
         if (sorted[i] < 0 || sorted[i] >= count)
-            return fail(RT_ERR_INVALID_ARGUMENT, std::string("rt_scene_update: ") + what + " index " + std::to_string(sorted[i]) + " is out of range");
+            return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": " + what + " index " + std::to_string(sorted[i]) + " is out of range");
         if (i > 0 && sorted[i] == sorted[i - 1])
-            return fail(RT_ERR_INVALID_ARGUMENT, std::string("rt_scene_update: ") + what + " index " + std::to_string(sorted[i]) + " appears twice");
+            return fail(RT_ERR_INVALID_ARGUMENT, std::string(who) + ": " + what + " index " + std::to_string(sorted[i]) + " appears twice");
     }
     return RT_OK;
 }
+
+namespace {
 
 bool same_texture(const RtTexture &a, const RtTexture &b) { // every field but the texel pointer, and the texels
     if (a.kind != b.kind || std::memcmp(a.colour, b.colour, 3) != 0 || a.width != b.width || a.height != b.height || a.even != b.even ||
@@ -177,7 +173,8 @@ bool same_texture(const RtTexture &a, const RtTexture &b) { // every field but t
     return a.kind != RT_TEX_IMAGE || std::memcmp(a.rgb8, b.rgb8, size_t(a.width) * a.height * 3) == 0;
 }
 
-// after the tree's boxes changed: the trees derived from it are rebuilt on first use
+} // namespace
+
 void invalidate_wide(RtScene *scene, DeviceScene *ds) {
     HostSceneLayout &L = scene->layout;
     L.wide_nodes.clear();
@@ -205,17 +202,29 @@ void invalidate_reference(RtScene *scene, DeviceScene *ds) {
     ds->n_ref_nodes = 0;
 }
 
-} // namespace
-
 int device_scene_sync_layout(RtScene *scene) {
-    if (!scene->layout_stale) return RT_OK;
+    if (!scene->layout_stale && !scene->records_stale) return RT_OK;
     auto *ds = static_cast<DeviceScene *>(scene->dev);
     HostSceneLayout &L = scene->layout;
     RT_CUDA(cudaSetDevice(ds->device));
-    scene->device_nodes.resize(L.nodes.size());
-    RT_CUDA(cudaMemcpy(L.nodes.data(), ds->refit, L.nodes.size() * sizeof(DNode), cudaMemcpyDeviceToHost));
-    RT_CUDA(cudaMemcpy(scene->device_nodes.data(), ds->g.nodes, L.nodes.size() * sizeof(DNode), cudaMemcpyDeviceToHost));
-    scene->layout_stale = false;
+    if (scene->records_stale) { // after rt_scene_rebuild: the records in leaf order, and the caller's index -> device id map
+        const size_t nb = size_t(L.n_bounded), nu = size_t(ds->g.n_unbounded);
+        L.spheres.resize(nb);
+        L.materials.resize(nb + nu);
+        L.unbounded.resize(nu);
+        L.device_id_of.resize(scene->objects.size());
+        RT_CUDA(cudaMemcpy(L.spheres.data(), ds->g.spheres, nb * sizeof(DSphere), cudaMemcpyDeviceToHost));
+        RT_CUDA(cudaMemcpy(L.materials.data(), ds->g.mats, (nb + nu) * sizeof(DMaterial), cudaMemcpyDeviceToHost));
+        RT_CUDA(cudaMemcpy(L.unbounded.data(), ds->g.unb, nu * sizeof(DUnbounded), cudaMemcpyDeviceToHost));
+        RT_CUDA(cudaMemcpy(L.device_id_of.data(), ds->dev_of, L.device_id_of.size() * sizeof(int32_t), cudaMemcpyDeviceToHost));
+        scene->records_stale = false;
+    }
+    if (scene->layout_stale) {
+        scene->device_nodes.resize(L.nodes.size());
+        RT_CUDA(cudaMemcpy(L.nodes.data(), ds->refit, L.nodes.size() * sizeof(DNode), cudaMemcpyDeviceToHost));
+        RT_CUDA(cudaMemcpy(scene->device_nodes.data(), ds->g.nodes, L.nodes.size() * sizeof(DNode), cudaMemcpyDeviceToHost));
+        scene->layout_stale = false;
+    }
     return RT_OK;
 }
 
@@ -232,8 +241,8 @@ int rt_scene_update(RtScene *scene, const int32_t *object_index, const RtHittabl
     if (scene->device < 0 || !scene->dev)
         return fail(RT_ERR_UNSUPPORTED, "rt_scene_update: the scene was created without a device (device = -1)");
     const int32_t n_obj_all = int32_t(scene->objects.size()), n_tex_all = int32_t(scene->textures.size());
-    int rc = check_indices(object_index, n_objects, n_obj_all, "object");
-    if (rc == RT_OK) rc = check_indices(texture_index, n_textures, n_tex_all, "texture");
+    int rc = check_indices(object_index, n_objects, n_obj_all, "object", who);
+    if (rc == RT_OK) rc = check_indices(texture_index, n_textures, n_tex_all, "texture", who);
     if (rc != RT_OK) return rc;
 
     // ---- every check before any change: structure, then what rt_scene_create checks in the edited arrays
@@ -261,6 +270,7 @@ int rt_scene_update(RtScene *scene, const int32_t *object_index, const RtHittabl
         if ((rc = check_textures(table.data(), n_tex_all, who)) != RT_OK) return fail(RT_ERR_INVALID_ARGUMENT, rt_last_error());
     }
     if ((rc = require_device(scene->device)) != RT_OK) return rc;
+    if (scene->records_stale && (rc = device_scene_sync_layout(scene)) != RT_OK) return rc; // after a rebuild: the records it placed
 
     // ---- the changed device records, as 16-byte words with their destination word in the scene blob
     auto *ds = static_cast<DeviceScene *>(scene->dev);

@@ -251,6 +251,9 @@ struct RtScene {
     uint64_t generation = 0;
     bool layout_stale = false;
     std::vector<rtfs::DNode> device_nodes;
+    // rt_scene_rebuild (rtfs_build.cu) builds the tree on the device and places the records there: layout.spheres,
+    // materials, unbounded and device_id_of are stale until device_scene_sync_layout downloads them
+    bool records_stale = false;
 };
 
 // implemented in rtfs_device.cu
@@ -260,7 +263,8 @@ void scene_ensure_sah_tree(RtScene *scene);
 int device_scene_upload(RtScene *scene);
 int device_scene_ensure_reference(RtScene *scene);
 int device_scene_ensure_wide(RtScene *scene);
-// brings layout.nodes (and scene->device_nodes) up to date after rt_scene_update refit the tree (rtfs_edit.cu)
+// brings layout.nodes (and scene->device_nodes) up to date after rt_scene_update refit the tree, and the records of the
+// layout after rt_scene_rebuild placed them on the device (rtfs_edit.cu)
 int device_scene_sync_layout(RtScene *scene);
 void device_scene_free(RtScene *scene);
 size_t device_scene_bytes(const RtScene *scene);

@@ -10,7 +10,7 @@ import os
 import numpy as np
 
 from . import abi
-from .abi import (RtCamera, RtDenoiseOpts, RtFrameConvergence, RtFrameNoise, RtFrameProgress, RtHittable, RtRenderOpts, RtSceneUpdate, RtStats,
+from .abi import (RtCamera, RtDenoiseOpts, RtFrameConvergence, RtFrameNoise, RtFrameProgress, RtHittable, RtRenderOpts, RtSceneRebuild, RtSceneUpdate, RtStats,
                   RtTexture)
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -49,6 +49,7 @@ def _declare(lib):
         "rt_scene_device_bytes": (C.c_size_t, [_vp]),
         "rt_scene_shared_memory_bytes": (C.c_size_t, [_vp]),
         "rt_scene_update": (C.c_int, [_vp, _vp, _vp, _i32, _vp, _vp, _i32, C.POINTER(RtSceneUpdate)]),
+        "rt_scene_rebuild": (C.c_int, [_vp, _vp, _i32, _vp, _i32, C.POINTER(RtSceneRebuild)]),
         "rt_render": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _vp, _vp, C.POINTER(RtStats)]),
         "rt_render_views": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(RtRenderOpts), _vp, _vp, C.POINTER(RtStats)]),
         "rt_frame_begin": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), C.POINTER(_vp),
@@ -238,6 +239,21 @@ class SceneHandle:
         t = _as_array(RtTexture, textures)
         info = RtSceneUpdate()
         check(lib().rt_scene_update(self.ptr, ptr(oi), h, len(oi), ptr(ti), t, len(ti), C.byref(info)))
+        return info
+
+    def rebuild(self, remove=(), append=()) -> RtSceneRebuild:
+        """Removes and appends objects and builds the tree anew on the device (rt_scene_rebuild): the objects `remove`
+        (indices) are taken out, the others keep their order, and `append` (RtHittable records) are added at the end.  The
+        scene then renders bit for bit as one created from the new array.  With neither, the tree of the current objects is
+        rebuilt.  Bad or repeated indices and anything creation refuses in an appended object: RtError
+        RT_ERR_INVALID_ARGUMENT, the scene left as it was.  Frames opened before the call are stale (see Frame).  Returns the
+        RtSceneRebuild."""
+        rm = np.ascontiguousarray(list(remove), np.int32)
+        append = list(append)
+        a = _as_array(RtHittable, append)
+        info = RtSceneRebuild()
+        check(lib().rt_scene_rebuild(self.ptr, ptr(rm), len(rm), a, len(append), C.byref(info)))
+        self.n_objects = info.n_objects
         return info
 
     def bvh_nodes(self, which=abi.RT_BVH_SAH):

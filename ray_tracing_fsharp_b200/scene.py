@@ -111,6 +111,56 @@ class Scene:
         return info
 
     @staticmethod
+    def add(s: "Scene", objects) -> abi.RtSceneRebuild:
+        """Appends `objects` to the scene, in place (rt_scene_rebuild): the scene then renders bit for bit as Scene.make of its
+        objects followed by these, and the new objects take the next indices.  Their textures must be textures the scene
+        already holds (a texture table cannot grow here; otherwise ValueError: make a new scene).  Progressive frames opened
+        before the call are stale.  A scene made with devices=[...] (several GPUs): NotImplementedError."""
+        hittables, textures, keep = marshal(objects)
+        remap = []
+        for t in textures:
+            same = [j for j, u in enumerate(s._textures) if _same_texture(t, u)]
+            if not same:
+                raise ValueError("Scene.add: an object brings a texture the scene does not hold: make a new scene")
+            remap.append(same[0])
+        for h in hittables:
+            if h.texture >= 0:
+                h.texture = remap[h.texture]
+        return Scene._restructure(s, [], list(hittables), keep)
+
+    @staticmethod
+    def remove(s: "Scene", indices) -> abi.RtSceneRebuild:
+        """Removes the objects at `indices`, in place (rt_scene_rebuild): the others keep their order and are renumbered
+        densely, and the scene renders bit for bit as Scene.make of them.  Bad or repeated indices: RtError
+        RT_ERR_INVALID_ARGUMENT.  Progressive frames opened before the call are stale.  A scene made with devices=[...]:
+        NotImplementedError."""
+        return Scene._restructure(s, list(indices), [], None)
+
+    @staticmethod
+    def rebuild(s: "Scene") -> abi.RtSceneRebuild:
+        """Builds the scene's tree anew on the device from its current objects: the remedy for a tree that Scene.update's
+        refits have left slow to walk (DESIGN.md section 20).  Frames are unchanged bit for bit; progressive frames opened
+        before the call are stale.  A scene made with devices=[...]: NotImplementedError."""
+        return Scene._restructure(s, [], [], None)
+
+    @staticmethod
+    def _restructure(s: "Scene", remove, append, keep) -> abi.RtSceneRebuild:
+        if not isinstance(s._handle, native.SceneHandle):
+            raise NotImplementedError("structural edits change a scene of one device; make a scene split over devices=[...] anew")
+        info = s._handle.rebuild(remove, append)
+        size = C.sizeof(abi.RtHittable)
+        old = np.frombuffer(s._hittables, np.uint8).reshape(-1, size) if len(s._hittables) else np.zeros((0, size), np.uint8)
+        kept = np.ones(len(old), bool)
+        kept[np.asarray(remove, np.int64)] = False
+        buf = bytearray(old[kept].tobytes() + b"".join(bytes(h) for h in append))
+        n = len(buf) // size
+        hittables = (abi.RtHittable * n).from_buffer(buf) if n else (abi.RtHittable * 0)()
+        s._hittables = hittables
+        s._keep = (s._keep, keep) if keep is not None else s._keep
+        s._handle._h, s._handle._keep = hittables, s._keep
+        return info
+
+    @staticmethod
     def render(progress_increment: Callable[[float], None], print_fn: Callable[[str], None], max_width_coord: int, max_height_coord: int,
                camera: abi.RtCamera, s: "Scene", seed: Optional[int] = None, adaptive: bool = True, mode: int = abi.RT_MODE_MEGAKERNEL,
                flags: int = 0, frames: Optional["native.FrameRing"] = None):

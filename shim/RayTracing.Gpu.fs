@@ -164,6 +164,19 @@ module internal Native =
         val mutable launches : int
         val mutable pad0 : int
 
+    [<Struct ; StructLayout(LayoutKind.Sequential)>]
+    type RtSceneRebuild =
+        val mutable objectsRemoved : int
+        val mutable objectsAppended : int
+        val mutable nObjects : int
+        val mutable nBounded : int
+        val mutable nodes : int
+        val mutable depth : int
+        val mutable onDevice : int
+        val mutable launches : int
+        val mutable generation : uint64
+        val mutable deviceMs : float
+
 
     [<DllImport(Lib)>]
     extern nativeint rt_last_error ()
@@ -179,6 +192,9 @@ module internal Native =
 
     [<DllImport(Lib)>]
     extern int rt_scene_update (nativeint scene, int[] objectIndex, RtHittable[] objects, int nObjects, int[] textureIndex, RtTexture[] textures, int nTextures, RtSceneUpdate& info)
+
+    [<DllImport(Lib)>]
+    extern int rt_scene_rebuild (nativeint scene, int[] remove, int nRemove, RtHittable[] append, int nAppend, RtSceneRebuild& info)
 
     [<DllImport(Lib)>]
     extern int rt_render (nativeint scene, RtCamera& camera, int maxWidthCoord, int maxHeightCoord, RtRenderOpts& opts, byte[] rgbOut, nativeint sumsOut, RtStats& stats)
@@ -567,6 +583,26 @@ type SceneUpdate =
         /// the scene's edit count after the call (0 = as made)
         Generation : uint64
         /// device time of the copy and the kernels (CUDA events)
+        DeviceMs : float
+    }
+
+/// What SceneGpu.addObjects, removeObjects and rebuild did (RtSceneRebuild, include/rtfs_b200.h).
+type SceneRebuild =
+    {
+        /// objects taken out and added at the end
+        ObjectsRemoved : int
+        ObjectsAppended : int
+        /// the scene's objects after the call, and the spheres in its tree
+        Objects : int
+        Bounded : int
+        /// nodes and depth (internal nodes on the longest path) of the new tree
+        Nodes : int
+        Depth : int
+        /// true: built on the device; false: the host SAH tree (the device tree was deeper than the walk stacks allow)
+        OnDevice : bool
+        /// the scene's edit count after the call
+        Generation : uint64
+        /// device time of the build (CUDA events)
         DeviceMs : float
     }
 
@@ -1109,6 +1145,80 @@ module SceneGpu =
         finally
             for p in pins do
                 p.Free ()
+
+    let private restructure (s : GpuScene) (remove : int array) (append : Native.RtHittable array) : SceneRebuild =
+        if s.IsMulti then
+            failwith "GPU backend: structural edits change a single-device GpuScene; make a multi-GPU scene anew"
+
+        let mutable info = Native.RtSceneRebuild ()
+
+        Native.rt_scene_rebuild (s.Handle, remove, remove.Length, append, append.Length, &info)
+        |> Native.check
+
+        let gone = Set.ofArray remove
+
+        s.Hittables <-
+            Array.append
+                [| for i in 0 .. s.Hittables.Length - 1 do
+                       if not (gone.Contains i) then
+                           yield s.Hittables.[i] |]
+                append
+
+        {
+            ObjectsRemoved = info.objectsRemoved
+            ObjectsAppended = info.objectsAppended
+            Objects = info.nObjects
+            Bounded = info.nBounded
+            Nodes = info.nodes
+            Depth = info.depth
+            OnDevice = info.onDevice <> 0
+            Generation = info.generation
+            DeviceMs = info.deviceMs
+        }
+
+    /// Appends `objects` to the scene in place (rt_scene_rebuild): the device builds the tree anew, and the scene then renders
+    /// bit for bit as GpuScene.make of its objects followed by these.  Their textures must be textures the scene already
+    /// holds (the texture table cannot grow here); otherwise, and on a multi-GPU scene, the call fails.  Frames opened before
+    /// the call are stale.
+    let addObjects (s : GpuScene) (objects : Hittable array) : SceneRebuild =
+        let hittables, textures, texels, pins = GpuScene.marshal objects
+
+        try
+            let find (j : int) =
+                let a = textures.[j]
+
+                s.Textures
+                |> Array.tryFindIndex (fun b ->
+                    a.kind = b.kind && a.colourR = b.colourR && a.colourG = b.colourG && a.colourB = b.colourB
+                    && a.even = b.even && a.odd = b.odd && a.gridSize = b.gridSize && a.mapCentreX = b.mapCentreX
+                    && a.mapCentreY = b.mapCentreY && a.mapCentreZ = b.mapCentreZ && a.mapRadius = b.mapRadius
+                    && a.width = b.width && a.height = b.height)
+                |> Option.filter (fun k -> a.kind <> 1 || texels.[j] = s.Texels.[k])
+                |> Option.defaultWith (fun () ->
+                    failwith "GPU backend: SceneGpu.addObjects: an object brings a texture the scene does not hold; make a new scene")
+
+            let remap = Array.init textures.Length find
+
+            let appended =
+                hittables
+                |> Array.map (fun h ->
+                    let mutable h = h
+                    if h.texture >= 0 then h.texture <- remap.[h.texture]
+                    h)
+
+            restructure s [||] appended
+        finally
+            for p in pins do
+                p.Free ()
+
+    /// Removes the objects at `indices` in place (rt_scene_rebuild): the others keep their order and are renumbered densely,
+    /// and the scene renders bit for bit as GpuScene.make of them.  Bad or repeated indices, or a multi-GPU scene, fail.
+    /// Frames opened before the call are stale.
+    let removeObjects (s : GpuScene) (indices : int array) : SceneRebuild = restructure s indices [||]
+
+    /// Builds the scene's tree anew on the device from its current objects: the remedy for a tree that update's refits have
+    /// left slow to walk (DESIGN.md section 20).  Frames are unchanged bit for bit; frames opened before the call are stale.
+    let rebuild (s : GpuScene) : SceneRebuild = restructure s [||] [||]
 
     // the frame of renderWithProgressUntil and renderConverging: passes of about 250 ms with progress ticks, an optional
     // convergence rule (tolerance, minSamples, interval) and an optional stop on the noise summary (tolerance, fraction)

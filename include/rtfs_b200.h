@@ -622,6 +622,36 @@ void rt_multi_destroy(RtMulti *multi);
  *   work complete on every device.  The frame must be destroyed before its RtMulti. */
 int rt_multi_frame_begin(RtMulti *multi, const RtCamera *camera, int32_t max_width_coord, int32_t max_height_coord,
                          const RtRenderOpts *opts, RtFrame **out, RtFrameProgress *progress);
+/* A batch of views split over the devices of an RtMulti, in one call or as a progressive frame: rt_render_views' and
+ * rt_frame_begin_views' tall frame (n_views * rows rows, view v at rows [v rows, (v + 1) rows)), split by sample index as
+ * rt_multi_render splits one frame.  A batch of small views makes each device's share of the work large again, where one
+ * rt_multi_render per view would give each device 1 / world of a frame already too small to hide its fixed costs.
+ *
+ * These two functions were added without a change of RT_ABI_VERSION (still 6): no struct and no existing prototype
+ * changed.  A caller detects the feature by the presence of the symbol rt_multi_render_views.
+ *
+ *   Arguments are the union of rt_render_views' and rt_multi_render's (rt_frame_begin_views' and rt_multi_frame_begin's),
+ *   checked before any device work: a NULL multi, out or rgb_out, n_views < 1, NULL cameras, cameras with differing
+ *   samples_per_pixel or bounce_depth, and n_views * rows * cols >= 2^31 are RT_ERR_INVALID_ARGUMENT; RT_MODE_WAVEFRONT,
+ *   RT_FLAG_FLOW and RT_FLAG_COUNTERS are RT_ERR_UNSUPPORTED (the kernels of a batch have no such variant).  *out is NULL
+ *   after any failure.  seeds may be NULL (every view then has opts->seed).
+ * Exactness.  Device r probes the tiles t with t mod world == r of the tall frame (a tile may straddle two views) and traces
+ *   the sample indices s + r + j world; every device holds its own copy of the table of view cameras and keys.  So
+ *   rt_multi_render_views equals rt_render_views on one device of the same arrays bit for bit, for every device count: RGB8
+ *   with and without gamma, the sums, and the RtStats paths, rays, degenerate_paths and pixels_early_out (box_tests and
+ *   prim_tests are 0; the _ms fields describe the slowest device, as in rt_multi_render).  rt_multi_frame_begin_views
+ *   returns an ordinary RtFrame, and after every pass, under a convergence rule too, it is rt_frame_begin_views' frame on
+ *   one device in everything rt_multi_frame_begin's frame equals rt_frame_begin's, and in every entry of
+ *   rt_frame_view_noise; only the number of passes may depend on the device count, and rt_multi_frame_begin's pacing
+ *   applies.
+ * Ownership.  As rt_multi_frame_begin's frame, plus its table of views on every device; the frame must be destroyed before
+ *   its RtMulti. */
+int rt_multi_render_views(RtMulti *multi, const RtCamera *cameras, const uint64_t *seeds, int32_t n_views,
+                          int32_t max_width_coord, int32_t max_height_coord, const RtRenderOpts *opts,
+                          uint8_t *rgb_out, int32_t *sums_out, RtStats *stats);
+int rt_multi_frame_begin_views(RtMulti *multi, const RtCamera *cameras, const uint64_t *seeds, int32_t n_views,
+                               int32_t max_width_coord, int32_t max_height_coord, const RtRenderOpts *opts,
+                               RtFrame **out, RtFrameProgress *progress);
 /* create + render + destroy in one call */
 int rt_render_multi(const RtHittable *objects, int32_t n_objects, const RtTexture *textures,
                     int32_t n_textures, const int32_t *devices, int32_t n_devices,

@@ -276,6 +276,9 @@ void set_window(FrameParams &fp, const FrameWindow &w);
 int check_views(const RtScene *scene, const RtCamera *cameras, int32_t n_views, int max_w, int max_h, const RtRenderOpts *opts, const char *who);
 // every view's camera and Philox key (seeds null: every view has `seed`)
 std::vector<ViewCamera> view_table(const RtCamera *cameras, const uint64_t *seeds, int32_t n_views, int max_w, int max_h, uint64_t seed);
+// grow-only: room for n_views entries in ws->d_views, the table of the one-call batches (rt_render_views,
+// rt_multi_render_views) on the workspace's device
+int ensure_views(DeviceWorkspace *ws, size_t n_views);
 // stacks a frame filled by fill_frame into the tall frame of n_views views of view_pixels pixels: probe tiles, flags, list,
 // sums and Q run over it as over one frame, and the render kernels find each view's camera and key in d_views
 void set_views(FrameParams &fp, const ViewCamera *d_views, int32_t n_views, int32_t view_pixels);

@@ -8,7 +8,8 @@
 // (rt_frame_set_convergence) stops sampling each pixel once its estimate is within a tolerance.
 // rt_frame_begin_views opens the same frame over rt_render_views' tall frame of a batch of views (its kernels are in
 // rtfs_views.cu); the probe flags, the compaction, the checks and the output tail work per pixel and need no change for it,
-// and rt_frame_view_noise reduces each view as rt_frame_noise reduces a frame of its own.
+// and rt_frame_view_noise reduces each view as rt_frame_noise reduces a frame of its own.  rt_multi_frame_begin_views splits
+// that frame over an RtMulti: every part holds a copy of the table of view cameras and keys on its own device.
 // rt_frame_begin_window opens it over a window of rt_render's frame (its kernels are in rtfs_window.cu): the frame's buffers,
 // maps and counts are the window's, and every per-pixel kernel runs over the window unchanged.
 // rt_frame_features and rt_frame_denoise (kernels in rtfs_denoise.cu) read the frame and keep buffers of their own.
@@ -110,6 +111,9 @@ struct FramePart {
     uint32_t *d_list = nullptr;
     unsigned long long *d_counters = nullptr;
     unsigned long long h_counters[CN_SLOTS] = {};
+    // a batch of views: the table of view cameras and keys the rank's render kernels read, on the rank's device (every
+    // path start and every draw reads it); the first part's is the frame's own
+    ViewCamera *d_views = nullptr;
     FrameEvents ev;                 // the probe: ZEROED -> END; a pass: BEGIN -> END
     cudaEvent_t traced = nullptr;   // the rank's samples so far are in its sums and Q
     cudaEvent_t gathered = nullptr; // the rank's slice of the totals is written
@@ -172,6 +176,7 @@ void frame_free(RtFrame *f) {
             cudaFree(p.d_stats);
             cudaFree(p.d_sq);
             cudaFree(p.d_flags);
+            if (p.d_views != f->d_views) cudaFree(p.d_views);
         }
         cudaFree(p.d_list);
         cudaFree(p.d_counters);
@@ -344,6 +349,7 @@ int frame_open(const std::vector<RtScene *> &scenes, const RtCamera &camera, con
              cudaEventCreateWithFlags(&p.traced, cudaEventDisableTiming) == cudaSuccess &&
              cudaEventCreateWithFlags(&p.gathered, cudaEventDisableTiming) == cudaSuccess &&
              cudaEventCreateWithFlags(&p.listed, cudaEventDisableTiming) == cudaSuccess;
+        p.d_views = f->d_views;
         if (world == 1) { // the only part traces into the frame's own buffers: its totals need no gather
             p.d_stats = f->d_stats;
             p.d_flags = f->d_flags;
@@ -352,30 +358,34 @@ int frame_open(const std::vector<RtScene *> &scenes, const RtCamera &camera, con
         }
         ok = ok && cudaMalloc((void **)&p.d_stats, n * 4 * sizeof(int32_t)) == cudaSuccess && cudaMalloc((void **)&p.d_flags, n) == cudaSuccess;
         if (noise) ok = ok && cudaMalloc((void **)&p.d_sq, n * sizeof(unsigned long long)) == cudaSuccess;
+        if (r > 0 && !views.empty()) {
+            p.d_views = nullptr;
+            ok = ok && cudaMalloc((void **)&p.d_views, views.size() * sizeof(ViewCamera)) == cudaSuccess;
+        }
     }
     if (!ok) return bail(fail(RT_ERR_CUDA, std::string(who) + ": allocation failed: " + cudaGetErrorString(cudaGetLastError())));
 
     // the frame's parameters are one device's (the features, the filter, the pacing and rt_frame_extend read them); each
     // part has its own, of rank r of world
-    auto fill = [&](FrameParams &fp, DeviceScene *ds, int r, int w) {
+    auto fill = [&](FrameParams &fp, DeviceScene *ds, const ViewCamera *d_views, int r, int w) {
         fill_frame(fp, ds, camera, max_w, max_h, *opts, r, w);
-        if (!views.empty()) set_views(fp, f->d_views, f->n_views, int32_t(view_pixels));
+        if (!views.empty()) set_views(fp, d_views, f->n_views, int32_t(view_pixels));
         if (window) set_window(fp, *window);
     };
-    fill(f->fp, ds0, 0, 1);
+    fill(f->fp, ds0, f->d_views, 0, 1);
     f->samples_done = f->fp.n_probe; // 0 without the early-out
     f->samples_target = f->fp.sample_end;
-    // (a batch has one part, on the current device; from pageable memory: staged before the call returns, and the probe
-    // follows it on the stream)
-    if (!views.empty() &&
-        cudaMemcpyAsync(f->d_views, views.data(), views.size() * sizeof(ViewCamera), cudaMemcpyHostToDevice, ds0->ws->stream) != cudaSuccess)
-        return bail(fail(RT_ERR_CUDA, std::string(who) + ": view table upload failed: " + cudaGetErrorString(cudaGetLastError())));
     int launches = 0;
     for (int r = 0; r < world; ++r) {
         FramePart &p = f->parts[size_t(r)];
         DeviceScene *ds = part_scene(p);
         if (cudaSetDevice(ds->device) != cudaSuccess) return bail(fail(RT_ERR_CUDA, std::string(who) + ": cudaSetDevice failed"));
-        fill(p.fp, ds, r, world);
+        // a batch: the rank's table on its device (from pageable memory: staged before the call returns, and the probe
+        // follows it on the stream)
+        if (!views.empty() &&
+            cudaMemcpyAsync(p.d_views, views.data(), views.size() * sizeof(ViewCamera), cudaMemcpyHostToDevice, ds->ws->stream) != cudaSuccess)
+            return bail(fail(RT_ERR_CUDA, std::string(who) + ": view table upload failed: " + cudaGetErrorString(cudaGetLastError())));
+        fill(p.fp, ds, p.d_views, r, world);
         p.fp.stats = p.d_stats;
         p.fp.flags = p.d_flags;
         p.fp.list = p.d_list;
@@ -533,6 +543,19 @@ int rt_multi_frame_begin(RtMulti *multi, const RtCamera *camera, int32_t max_w, 
     if (rc != RT_OK) return rc;
     if ((rc = check_frame_mode(opts, "rt_multi_frame_begin", false)) != RT_OK) return rc;
     return frame_open(multi_scenes(multi), *camera, {}, nullptr, max_w, max_h, opts, out, progress, "rt_multi_frame_begin");
+}
+
+int rt_multi_frame_begin_views(RtMulti *multi, const RtCamera *cameras, const uint64_t *seeds, int32_t n_views, int32_t max_w, int32_t max_h,
+                               const RtRenderOpts *opts, RtFrame **out, RtFrameProgress *progress) {
+    if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_multi_frame_begin_views: out is null");
+    *out = nullptr;
+    if (!multi || multi_scenes(multi).empty()) return fail(RT_ERR_INVALID_ARGUMENT, "rt_multi_frame_begin_views: null handle");
+    // rt_frame_begin_views' checks and refusals, on the first device's replica
+    int rc = check_views(multi_scenes(multi)[0], cameras, n_views, max_w, max_h, opts, "rt_multi_frame_begin_views");
+    if (rc != RT_OK) return rc;
+    if ((rc = check_frame_mode(opts, "rt_multi_frame_begin_views", true)) != RT_OK) return rc;
+    return frame_open(multi_scenes(multi), cameras[0], view_table(cameras, seeds, n_views, max_w, max_h, opts->seed), nullptr, max_w, max_h,
+                      opts, out, progress, "rt_multi_frame_begin_views");
 }
 
 int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameProgress *progress) {

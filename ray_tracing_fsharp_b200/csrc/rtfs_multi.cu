@@ -1,4 +1,4 @@
-// rtfs_multi.cu — one frame split over several GPUs of this process (rt_multi_*, rt_render_multi).
+// rtfs_multi.cu — one frame or one batch of views split over several GPUs of this process (rt_multi_*, rt_render_multi).
 //
 // Replicated scene, sample-index split (SURVEY.md §8e).  The devices exchange data only through NVLink
 // peer memory, inside the kernels that need it:
@@ -12,6 +12,8 @@
 //              128-bit peer loads, divides (PixelStats.mean, Pixel.fs:103-108), applies the optional
 //              gamma (ImageOutput.fs:11-18) and stores RGB8 straight into pinned host memory.
 // Integer sums keyed by sample index make the image bit-identical for every device count.
+// rt_multi_render_views runs the same sequence over rt_render_views' tall frame of a batch of views: the split, the
+// exchange and the reduce work per pixel, and every rank reads the table of view cameras and keys from its own device.
 // (The one-process-per-GPU form of the same split, with NCCL all-reduces between rt_device_probe /
 // rt_device_main / rt_device_finalize, is driven from bench.py through torch.distributed.)
 #include "rtfs_device.h"
@@ -175,6 +177,96 @@ int multi_workspace(RtMulti *m, size_t n_pixels, bool want_sums) {
     return RT_OK;
 }
 
+// rt_multi_render's body, once its arguments are checked: one frame (views empty), or rt_render_views' tall frame of a
+// batch (views: the table of every view's camera and key).  Every rank uploads the table into its replica's workspace
+// (ws->d_views, on its own device), so the render kernels read every view's camera and key from local memory; the probe,
+// the compaction, the main phase and the reduce then run over the tall frame as over one frame.
+int multi_render(RtMulti *m, const RtCamera &camera, const std::vector<ViewCamera> &views, int32_t max_w, int32_t max_h,
+                 const RtRenderOpts *opts, uint8_t *rgb_out, int32_t *sums_out, RtStats *stats) {
+    const auto t0 = std::chrono::steady_clock::now();
+    const int world = int(m->devices.size());
+    const size_t view_pixels = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
+    const size_t n_pixels = view_pixels * std::max<size_t>(1, views.size());
+    int rc = multi_workspace(m, n_pixels, sums_out != nullptr);
+    if (rc != RT_OK) return rc;
+    for (RtScene *s : m->scenes)
+        if ((rc = prepare_frame(s, opts)) != RT_OK) return rc;
+    std::vector<int> launches(world, 0);
+    std::vector<FrameParams> fps(world);
+    FlagsView flags{};
+    flags.world = world;
+    for (int i = 0; i < world; ++i) flags.by_rank[i] = m->d_flags[i];
+
+    // phase 1 on every device
+    for (int i = 0; i < world; ++i) {
+        auto *ds = static_cast<DeviceScene *>(m->scenes[i]->dev);
+        RT_CUDA(cudaSetDevice(m->devices[i]));
+        cudaStream_t st = m->streams[i];
+        fill_frame(fps[i], ds, camera, max_w, max_h, *opts, i, world);
+        if (!views.empty()) { // (from pageable memory: staged before the call returns, and the probe follows it on the stream)
+            if ((rc = ensure_views(ds->ws, views.size())) != RT_OK) return rc;
+            RT_CUDA(cudaMemcpyAsync(ds->ws->d_views, views.data(), views.size() * sizeof(ViewCamera), cudaMemcpyHostToDevice, st));
+            set_views(fps[i], ds->ws->d_views, int32_t(views.size()), int32_t(view_pixels));
+        }
+        fps[i].stats = m->d_stats[i];
+        fps[i].flags = m->d_flags[i];
+        RT_CUDA(cudaEventRecord(m->ev_begin[i], st));
+        if ((rc = frame_probe(ds, fps[i], st, nullptr, &launches[i])) != RT_OK) return rc;
+        RT_CUDA(cudaEventRecord(m->ev_probe[i], st));
+    }
+    // phase 2: needs everyone's flags
+    for (int i = 0; i < world; ++i) {
+        auto *ds = static_cast<DeviceScene *>(m->scenes[i]->dev);
+        RT_CUDA(cudaSetDevice(m->devices[i]));
+        cudaStream_t st = m->streams[i];
+        for (int j = 0; j < world; ++j)
+            if (j != i) RT_CUDA(cudaStreamWaitEvent(st, m->ev_probe[j], 0));
+        if ((rc = launch_main(ds, fps[i], flags, st, &launches[i])) != RT_OK) return rc;
+        RT_CUDA(cudaMemcpyAsync(ds->ws->h_counters, ds->ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        RT_CUDA(cudaEventRecord(m->ev_main[i], st));
+    }
+    // reduce + finalize: needs everyone's sums; each device owns a slice of the pixels
+    ReduceTargets t{};
+    for (int j = 0; j < world; ++j) t.stats[j] = m->d_stats[j];
+    t.world = world;
+    t.n_rgb = 1;
+    for (int i = 0; i < world; ++i) {
+        RT_CUDA(cudaSetDevice(m->devices[i]));
+        cudaStream_t st = m->streams[i];
+        for (int j = 0; j < world; ++j)
+            if (j != i) RT_CUDA(cudaStreamWaitEvent(st, m->ev_main[j], 0));
+        RT_CUDA(cudaHostGetDevicePointer((void **)&t.rgb[0], m->h_rgb, 0));
+        if (sums_out) RT_CUDA(cudaHostGetDevicePointer((void **)&t.sums, m->h_sums, 0));
+        if ((rc = launch_reduce_finalize(t, i, n_pixels, opts->gamma, st, &launches[i])) != RT_OK) return rc;
+        RT_CUDA(cudaEventRecord(m->ev_end[i], st));
+    }
+    for (int i = 0; i < world; ++i) {
+        RT_CUDA(cudaSetDevice(m->devices[i]));
+        RT_CUDA(cudaStreamSynchronize(m->streams[i]));
+    }
+    std::memcpy(rgb_out, m->h_rgb, n_pixels * 3);
+    if (sums_out) std::memcpy(sums_out, m->h_sums, n_pixels * 4 * sizeof(int32_t));
+    if (stats) {
+        std::memset(stats, 0, sizeof *stats);
+        for (int i = 0; i < world; ++i) {
+            RtStats d;
+            read_stats(static_cast<DeviceScene *>(m->scenes[i]->dev), n_pixels, opts->adaptive != 0, launches[i], nullptr, &d);
+            stats->paths += d.paths;
+            stats->rays += d.rays;
+            stats->box_tests += d.box_tests;
+            stats->prim_tests += d.prim_tests;
+            stats->degenerate_paths += d.degenerate_paths;
+            stats->launches += d.launches;
+            stats->pixels_early_out = d.pixels_early_out; // every device compacted the same flags
+            float ms = 0.f;
+            cudaEventElapsedTime(&ms, m->ev_begin[i], m->ev_end[i]);
+            stats->kernel_ms = std::max(stats->kernel_ms, double(ms)); // device time of the slowest GPU, probe -> reduce
+        }
+        stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    }
+    return RT_OK;
+}
+
 } // namespace
 
 int launch_reduce_finalize(const ReduceTargets &t, int rank, size_t n_pixels, int gamma, cudaStream_t st, int *launches) {
@@ -269,82 +361,19 @@ int rt_multi_render(RtMulti *m, const RtCamera *camera, int32_t max_w, int32_t m
     if (rc != RT_OK) return rc;
     if (!rgb_out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_multi_render: rgb_out is null");
     if (opts->mode != RT_MODE_MEGAKERNEL) return fail(RT_ERR_UNSUPPORTED, "rt_multi_render: only RT_MODE_MEGAKERNEL is split over devices");
-    const auto t0 = std::chrono::steady_clock::now();
-    const int world = int(m->devices.size());
-    const size_t n_pixels = size_t(2 * max_w + 1) * size_t(2 * max_h + 1);
-    rc = multi_workspace(m, n_pixels, sums_out != nullptr);
-    if (rc != RT_OK) return rc;
-    for (RtScene *s : m->scenes)
-        if ((rc = prepare_frame(s, opts)) != RT_OK) return rc;
-    std::vector<int> launches(world, 0);
-    std::vector<FrameParams> fps(world);
-    FlagsView flags{};
-    flags.world = world;
-    for (int i = 0; i < world; ++i) flags.by_rank[i] = m->d_flags[i];
+    return multi_render(m, *camera, {}, max_w, max_h, opts, rgb_out, sums_out, stats);
+}
 
-    // phase 1 on every device
-    for (int i = 0; i < world; ++i) {
-        auto *ds = static_cast<DeviceScene *>(m->scenes[i]->dev);
-        RT_CUDA(cudaSetDevice(m->devices[i]));
-        cudaStream_t st = m->streams[i];
-        fill_frame(fps[i], ds, *camera, max_w, max_h, *opts, i, world);
-        fps[i].stats = m->d_stats[i];
-        fps[i].flags = m->d_flags[i];
-        RT_CUDA(cudaEventRecord(m->ev_begin[i], st));
-        if ((rc = frame_probe(ds, fps[i], st, nullptr, &launches[i])) != RT_OK) return rc;
-        RT_CUDA(cudaEventRecord(m->ev_probe[i], st));
-    }
-    // phase 2: needs everyone's flags
-    for (int i = 0; i < world; ++i) {
-        auto *ds = static_cast<DeviceScene *>(m->scenes[i]->dev);
-        RT_CUDA(cudaSetDevice(m->devices[i]));
-        cudaStream_t st = m->streams[i];
-        for (int j = 0; j < world; ++j)
-            if (j != i) RT_CUDA(cudaStreamWaitEvent(st, m->ev_probe[j], 0));
-        if ((rc = launch_main(ds, fps[i], flags, st, &launches[i])) != RT_OK) return rc;
-        RT_CUDA(cudaMemcpyAsync(ds->ws->h_counters, ds->ws->d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-        RT_CUDA(cudaEventRecord(m->ev_main[i], st));
-    }
-    // reduce + finalize: needs everyone's sums; each device owns a slice of the pixels
-    ReduceTargets t{};
-    for (int j = 0; j < world; ++j) t.stats[j] = m->d_stats[j];
-    t.world = world;
-    t.n_rgb = 1;
-    for (int i = 0; i < world; ++i) {
-        RT_CUDA(cudaSetDevice(m->devices[i]));
-        cudaStream_t st = m->streams[i];
-        for (int j = 0; j < world; ++j)
-            if (j != i) RT_CUDA(cudaStreamWaitEvent(st, m->ev_main[j], 0));
-        RT_CUDA(cudaHostGetDevicePointer((void **)&t.rgb[0], m->h_rgb, 0));
-        if (sums_out) RT_CUDA(cudaHostGetDevicePointer((void **)&t.sums, m->h_sums, 0));
-        if ((rc = launch_reduce_finalize(t, i, n_pixels, opts->gamma, st, &launches[i])) != RT_OK) return rc;
-        RT_CUDA(cudaEventRecord(m->ev_end[i], st));
-    }
-    for (int i = 0; i < world; ++i) {
-        RT_CUDA(cudaSetDevice(m->devices[i]));
-        RT_CUDA(cudaStreamSynchronize(m->streams[i]));
-    }
-    std::memcpy(rgb_out, m->h_rgb, n_pixels * 3);
-    if (sums_out) std::memcpy(sums_out, m->h_sums, n_pixels * 4 * sizeof(int32_t));
-    if (stats) {
-        std::memset(stats, 0, sizeof *stats);
-        for (int i = 0; i < world; ++i) {
-            RtStats d;
-            read_stats(static_cast<DeviceScene *>(m->scenes[i]->dev), n_pixels, opts->adaptive != 0, launches[i], nullptr, &d);
-            stats->paths += d.paths;
-            stats->rays += d.rays;
-            stats->box_tests += d.box_tests;
-            stats->prim_tests += d.prim_tests;
-            stats->degenerate_paths += d.degenerate_paths;
-            stats->launches += d.launches;
-            stats->pixels_early_out = d.pixels_early_out; // every device compacted the same flags
-            float ms = 0.f;
-            cudaEventElapsedTime(&ms, m->ev_begin[i], m->ev_end[i]);
-            stats->kernel_ms = std::max(stats->kernel_ms, double(ms)); // device time of the slowest GPU, probe -> reduce
-        }
-        stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    }
-    return RT_OK;
+int rt_multi_render_views(RtMulti *m, const RtCamera *cameras, const uint64_t *seeds, int32_t n_views, int32_t max_w, int32_t max_h,
+                          const RtRenderOpts *opts, uint8_t *rgb_out, int32_t *sums_out, RtStats *stats) {
+    // the union of rt_multi_render's and rt_render_views' checks, before any device work
+    if (!m || m->scenes.empty()) return fail(RT_ERR_INVALID_ARGUMENT, "rt_multi_render_views: null handle");
+    if (!rgb_out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_multi_render_views: rgb_out is null");
+    int rc = check_views(m->scenes[0], cameras, n_views, max_w, max_h, opts, "rt_multi_render_views");
+    if (rc != RT_OK) return rc;
+    if ((rc = check_frame_mode(opts, "rt_multi_render_views", true)) != RT_OK) return rc;
+    return multi_render(m, cameras[0], view_table(cameras, seeds, n_views, max_w, max_h, opts->seed), max_w, max_h, opts, rgb_out, sums_out,
+                        stats);
 }
 
 int rt_render_multi(const RtHittable *objects, int32_t n_objects, const RtTexture *textures, int32_t n_textures, const int32_t *devices,

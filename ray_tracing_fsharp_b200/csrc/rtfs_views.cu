@@ -74,7 +74,7 @@ RenderKernelFn pick_views_kernel(bool probe, bool smem, bool lean, bool sstack, 
 }
 
 // grow-only, like the frame buffers
-static int ensure_views(DeviceWorkspace *ws, size_t n_views) {
+int ensure_views(DeviceWorkspace *ws, size_t n_views) {
     if (ws->views_cap >= n_views) return RT_OK;
     cudaFree(ws->d_views);
     ws->d_views = nullptr;

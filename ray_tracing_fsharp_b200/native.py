@@ -78,6 +78,9 @@ def _declare(lib):
         "rt_multi_destroy": (None, [_vp]),
         "rt_multi_frame_begin": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), C.POINTER(_vp),
                                            C.POINTER(RtFrameProgress)]),
+        "rt_multi_render_views": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(RtRenderOpts), _vp, _vp, C.POINTER(RtStats)]),
+        "rt_multi_frame_begin_views": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(RtRenderOpts), C.POINTER(_vp),
+                                                 C.POINTER(RtFrameProgress)]),
         "rt_device_probe": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _i32, _i32, _vp, _vp, _vp,
                                       C.POINTER(RtStats)]),
         "rt_device_main": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _i32, _i32, _vp, _vp, _vp,
@@ -200,6 +203,27 @@ def device_count():
     return int(lib().rt_device_count())
 
 
+def _views_args(cameras, seeds):
+    """(n, the RtCamera array, the uint64 seeds or None) of a batch of views, as rt_render_views and its kin take them."""
+    n = len(cameras)
+    cams = (RtCamera * max(1, n))(*cameras)
+    sd = None
+    if seeds is not None:
+        if len(seeds) != n:
+            raise ValueError(f"{len(seeds)} seeds for {n} cameras")
+        sd = np.ascontiguousarray([int(x) for x in seeds], np.uint64)
+    return n, cams, sd
+
+
+def _views_frame(owner, out, progress, max_w, max_h, n):
+    """The Frame of a batch of n views opened into `out`; it holds `owner` (a SceneHandle or MultiHandle)."""
+    frame = Frame.__new__(Frame)
+    frame.scene, frame.ptr, frame.progress = owner, out, progress
+    frame.rows, frame.cols = 2 * max_h + 1, 2 * max_w + 1
+    frame.n_views = n
+    return frame
+
+
 class SceneHandle:
     """Owner of an RtScene* (rt_scene_create / rt_scene_destroy)."""
 
@@ -299,14 +323,8 @@ class SceneHandle:
         samples_per_pixel and bounce_depth), `seeds` one per view or None (then `seed` for every view).  Returns
         (uint8 [n, rows, cols, 3], int32 [n, rows, cols, 4] or None, RtStats of the batch); view v is exactly
         render(cameras[v], max_w, max_h, seed=seeds[v]).  RtError RT_ERR_INVALID_ARGUMENT for an empty batch."""
-        n = len(cameras)
+        n, cams, sd = _views_args(cameras, seeds)
         rows, cols = 2 * max_h + 1, 2 * max_w + 1
-        cams = (RtCamera * max(1, n))(*cameras)
-        sd = None
-        if seeds is not None:
-            if len(seeds) != n:
-                raise ValueError(f"{len(seeds)} seeds for {n} cameras")
-            sd = np.ascontiguousarray([int(x) for x in seeds], np.uint64)
         rgb = _frame_buffer((n, rows, cols, 3))
         sums = np.empty((n, rows, cols, 4), np.int32) if want_sums else None
         opts = RtRenderOpts(seed, int(adaptive), abi.RT_MODE_MEGAKERNEL, int(gamma), flags)
@@ -323,22 +341,12 @@ class SceneHandle:
         render_views.  A Frame whose read, noise and sums have shape [n_views, rows, cols, ...]; view v is exactly
         open_frame(cameras[v], max_w, max_h, seed=seeds[v]) at the same samples_done, and Frame.view_noise summarises
         each view.  RtError RT_ERR_INVALID_ARGUMENT for an empty batch."""
-        n = len(cameras)
-        cams = (RtCamera * max(1, n))(*cameras)
-        sd = None
-        if seeds is not None:
-            if len(seeds) != n:
-                raise ValueError(f"{len(seeds)} seeds for {n} cameras")
-            sd = np.ascontiguousarray([int(x) for x in seeds], np.uint64)
+        n, cams, sd = _views_args(cameras, seeds)
         opts = RtRenderOpts(seed, int(adaptive), abi.RT_MODE_MEGAKERNEL, 0, flags)
         out = C.c_void_p()
         progress = RtFrameProgress()
         check(lib().rt_frame_begin_views(self.ptr, cams, ptr(sd), n, max_w, max_h, C.byref(opts), C.byref(out), C.byref(progress)))
-        frame = Frame.__new__(Frame)
-        frame.scene, frame.ptr, frame.progress = self, out, progress
-        frame.rows, frame.cols = 2 * max_h + 1, 2 * max_w + 1
-        frame.n_views = n
-        return frame
+        return _views_frame(self, out, progress, max_w, max_h, n)
 
     def render_window(self, camera, max_w, max_h, window, seed=0, adaptive=True, gamma=False, flags=0, want_sums=False, rgb_out=None):
         """The window (row0, col0, rows, cols) of render(camera, max_w, max_h, ...) without tracing the rest of the frame
@@ -572,6 +580,30 @@ class MultiHandle:
         frame.scene, frame.ptr, frame.progress = self, out, progress
         frame.rows, frame.cols = 2 * max_h + 1, 2 * max_w + 1
         return frame
+
+    def render_views(self, cameras, max_w, max_h, seeds=None, adaptive=True, gamma=False, flags=0, want_sums=False, seed=0):
+        """A batch of views split over this handle's devices (rt_multi_render_views): arguments and return shapes of
+        SceneHandle.render_views, and bit for bit its images, sums and the stats' paths, rays, degenerate_paths and
+        pixels_early_out."""
+        n, cams, sd = _views_args(cameras, seeds)
+        rows, cols = 2 * max_h + 1, 2 * max_w + 1
+        rgb = _frame_buffer((n, rows, cols, 3))
+        sums = np.empty((n, rows, cols, 4), np.int32) if want_sums else None
+        opts = RtRenderOpts(seed, int(adaptive), abi.RT_MODE_MEGAKERNEL, int(gamma), flags)
+        stats = RtStats()
+        check(lib().rt_multi_render_views(self.ptr, cams, ptr(sd), n, max_w, max_h, C.byref(opts), ptr(rgb), ptr(sums), C.byref(stats)))
+        return rgb, sums, stats
+
+    def open_frame_views(self, cameras, max_w, max_h, seeds=None, seed=0, adaptive=True, flags=0):
+        """A progressive frame of a batch of views split over this handle's devices (rt_multi_frame_begin_views: runs the
+        probe), arguments as SceneHandle.open_frame_views.  A Frame that is bit for bit SceneHandle.open_frame_views' frame of
+        one device after every pass; it holds this handle, so the handle outlives it."""
+        n, cams, sd = _views_args(cameras, seeds)
+        opts = RtRenderOpts(seed, int(adaptive), abi.RT_MODE_MEGAKERNEL, 0, flags)
+        out = C.c_void_p()
+        progress = RtFrameProgress()
+        check(lib().rt_multi_frame_begin_views(self.ptr, cams, ptr(sd), n, max_w, max_h, C.byref(opts), C.byref(out), C.byref(progress)))
+        return _views_frame(self, out, progress, max_w, max_h, n)
 
 
 class CommHandle:

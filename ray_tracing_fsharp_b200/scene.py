@@ -7,9 +7,9 @@ reference's.  Everything that computes goes through the C ABI (native.py); nothi
   Scene.make            RayTracing/Scene.fs:15-28
   Scene.update          Scene.make of an edited object list, done in place on the device (rt_scene_update)
   Scene.render          RayTracing/Scene.fs:196-236
-  Scene.render_views    Scene.render of many cameras of one scene in one submission (rt_render_views)
+  Scene.render_views    Scene.render of many cameras of one scene in one submission (rt_render_views; one GPU or several)
   Scene.render_progressive  the same frame in sample passes, progress ticks as passes finish (native.Frame, one GPU or several)
-  Scene.render_views_progressive  Scene.render_views in sample passes, as one progressive frame of the batch
+  Scene.render_views_progressive  Scene.render_views in sample passes, as one progressive frame of the batch (one GPU or several)
   Scene.render_window   a window (row0, col0, rows, cols) of Scene.render's image, without tracing the rest (rt_render_window)
   Image / Image.render  RayTracing/Domain.fs:9-31
   ImageOutput.write_ppm RayTracing/ImageOutput.fs:163-197, PixelOutput.correct :11-18
@@ -210,9 +210,9 @@ class Scene:
         stereo pairs, previews), rendered together by one GPU (native.SceneHandle.render_views).  Returns (total progress,
         [Image per camera]); lazy like Scene.render: the first forced row renders every view.  The progress ticks total
         rows * len(cameras), one per row forced.  `seeds`: one RNG key per view; otherwise `seed` (None: one drawn from the
-        OS) for every view.  With the same camera and seed, view v is Scene.render's image.  `print_fn` is ignored."""
-        if not isinstance(s._handle, native.SceneHandle):
-            raise NotImplementedError("a batch of views runs on one GPU: make the scene with a single device")
+        OS) for every view.  With the same camera and seed, view v is Scene.render's image.  On a scene made with
+        devices=[...] the batch is split over those GPUs (native.MultiHandle.render_views), bit for bit the batch of one GPU.
+        `print_fn` is ignored."""
         rows, cols = 2 * max_height_coord + 1, 2 * max_width_coord + 1
         n = len(cameras)
         if seed is None and seeds is None:
@@ -365,9 +365,9 @@ class Scene:
         `converge_tolerance` every pixel of every view stops once its standard error is within it, checked at
         converge_min_samples + j * converge_interval samples (Frame.set_convergence).  Returns one uint8 [rows, cols, 3] image
         per view (before gamma): with the same camera and seed, view v is render_progressive's image of camera v with the same
-        rule, or, stopped early, that of the samples done.  `print_fn` is ignored."""
-        if not isinstance(s._handle, native.SceneHandle):
-            raise NotImplementedError("progressive frames run on one GPU: make the scene with a single device")
+        rule, or, stopped early, that of the samples done.  On a scene made with devices=[...] the frame is split over those
+        GPUs (native.MultiHandle.open_frame_views), bit for bit the frame of one GPU after every pass.  `print_fn` is
+        ignored."""
         rows, n = 2 * max_height_coord + 1, len(cameras)
         if seed is None and seeds is None:
             seed = secrets.randbits(64)

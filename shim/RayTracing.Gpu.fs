@@ -266,6 +266,14 @@ module internal Native =
     [<DllImport(Lib)>]
     extern int rt_multi_frame_begin (nativeint multi, RtCamera& camera, int maxWidthCoord, int maxHeightCoord, RtRenderOpts& opts, nativeint& frame, RtFrameProgress& progress)
 
+    // a batch of views split over the devices of an RtMulti, in one call or as a progressive frame (include/rtfs_b200.h,
+    // rt_multi_render_views; ABI 6 still: detect by the symbol)
+    [<DllImport(Lib)>]
+    extern int rt_multi_render_views (nativeint multi, RtCamera[] cameras, uint64[] seeds, int nViews, int maxWidthCoord, int maxHeightCoord, RtRenderOpts& opts, byte[] rgbOut, nativeint sumsOut, RtStats& stats)
+
+    [<DllImport(Lib)>]
+    extern int rt_multi_frame_begin_views (nativeint multi, RtCamera[] cameras, uint64[] seeds, int nViews, int maxWidthCoord, int maxHeightCoord, RtRenderOpts& opts, nativeint& frame, RtFrameProgress& progress)
+
     // one rank of a one-process-per-GPU job: the library issues the NCCL collectives itself (include/rtfs_b200.h, rt_comm_*)
     [<DllImport(Lib)>]
     extern int rt_comm_unique_id (byte[] idOut)
@@ -886,9 +894,10 @@ module SceneGpu =
         1.0<progress> * float rowsIter, Image.make rowsIter colsIter rows
 
     /// Scene.render for every camera of `cameras` (same SamplesPerPixel and BounceDepth; a turntable, a fly-through,
-    /// stereo pairs, previews), rendered together in one rt_render_views call on a single-device scene: one Image per
-    /// camera, lazy like `render` (the first forced row of any view renders them all).  Every row of every view reports
-    /// progress once: rows * cameras.Length in all.  One fresh seed per view, as `render` draws one per frame.
+    /// stereo pairs, previews), rendered together in one rt_render_views call, or on a multi-GPU scene one
+    /// rt_multi_render_views call split over its devices (bit for bit the batch of one GPU): one Image per camera, lazy
+    /// like `render` (the first forced row of any view renders them all).  Every row of every view reports progress once:
+    /// rows * cameras.Length in all.  One fresh seed per view, as `render` draws one per frame.
     let renderViews
         (progressIncrement : float<progress> -> unit)
         (_print : string -> unit)
@@ -898,9 +907,6 @@ module SceneGpu =
         (s : GpuScene)
         : float<progress> * Image array
         =
-        if s.IsMulti then
-            failwith "GPU backend: a batch of views runs on a single-device GpuScene"
-
         let rowsIter = 2 * maxHeightCoord + 1
         let colsIter = 2 * maxWidthCoord + 1
         let n = cameras.Length
@@ -914,8 +920,12 @@ module SceneGpu =
                  opts.adaptive <- 1
                  let mutable stats = Native.RtStats ()
 
-                 Native.rt_render_views (s.Handle, cams, seeds, n, maxWidthCoord, maxHeightCoord, &opts, rgb, 0n, &stats)
-                 |> Native.check
+                 if s.IsMulti then
+                     Native.rt_multi_render_views (s.Handle, cams, seeds, n, maxWidthCoord, maxHeightCoord, &opts, rgb, 0n, &stats)
+                     |> Native.check
+                 else
+                     Native.rt_render_views (s.Handle, cams, seeds, n, maxWidthCoord, maxHeightCoord, &opts, rgb, 0n, &stats)
+                     |> Native.check
 
                  rgb)
 
@@ -1036,11 +1046,9 @@ module SceneGpu =
 
     /// Opens a progressive frame of a batch of views (rt_frame_begin_views: the probe of every view runs now) with
     /// RtRenderOpts.flags `flags`: `cameras` with the same SamplesPerPixel and BounceDepth, one seed per view.  View v is
-    /// exactly the frame openFrameWith gives for cameras.[v] and seeds.[v].  Single-device scenes only.
+    /// exactly the frame openFrameWith gives for cameras.[v] and seeds.[v].  On a multi-GPU scene the frame is split over
+    /// its devices (rt_multi_frame_begin_views) and is bit for bit the frame of one GPU.
     let openFrameViews (flags : int) (maxWidthCoord : int) (maxHeightCoord : int) (cameras : Camera array) (seeds : uint64 array) (s : GpuScene) : GpuFrame =
-        if s.IsMulti then
-            failwith "GPU backend: a progressive frame of a batch of views runs on a single-device GpuScene"
-
         if seeds.Length <> cameras.Length then
             invalidArg "seeds" "one seed per camera"
 
@@ -1051,8 +1059,13 @@ module SceneGpu =
         let mutable handle = 0n
         let mutable progress = Native.RtFrameProgress ()
 
-        Native.rt_frame_begin_views (s.Handle, cams, seeds, cams.Length, maxWidthCoord, maxHeightCoord, &opts, &handle, &progress)
-        |> Native.check
+        let rc =
+            if s.IsMulti then
+                Native.rt_multi_frame_begin_views (s.Handle, cams, seeds, cams.Length, maxWidthCoord, maxHeightCoord, &opts, &handle, &progress)
+            else
+                Native.rt_frame_begin_views (s.Handle, cams, seeds, cams.Length, maxWidthCoord, maxHeightCoord, &opts, &handle, &progress)
+
+        Native.check rc
 
         new GpuFrame (handle, 2 * maxHeightCoord + 1, 2 * maxWidthCoord + 1, cameras.Length, progress)
 

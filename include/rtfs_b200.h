@@ -652,6 +652,79 @@ int rt_multi_render_views(RtMulti *multi, const RtCamera *cameras, const uint64_
 int rt_multi_frame_begin_views(RtMulti *multi, const RtCamera *cameras, const uint64_t *seeds, int32_t n_views,
                                int32_t max_width_coord, int32_t max_height_coord, const RtRenderOpts *opts,
                                RtFrame **out, RtFrameProgress *progress);
+/* ---- saving a progressive frame and resuming it ---------------------------------------------------- */
+/* A progressive frame written to bytes and opened again later, in this process or another, on one device or on an RtMulti
+ * of any device count: a frame that took minutes survives its process, and a one-GPU preview can be finished on eight.
+ *
+ * These three functions were added without a change of RT_ABI_VERSION (still 6): no existing struct or prototype changed.  A
+ * caller detects the feature by the presence of the symbol rt_frame_save.
+ *
+ * rt_frame_save writes the frame into out[0, *len).  *len is always set: out == NULL with cap == 0 only sizes the snapshot
+ *   (no device work); a cap below *len writes nothing (RT_ERR_INVALID_ARGUMENT).  It takes every frame (one camera, a batch
+ *   of views or a window, of one device or of an RtMulti) at any point: right after its opener, between passes, on a
+ *   checkpoint, after rt_frame_extend, or done.  A frame whose scene was edited since it opened is refused
+ *   (RT_ERR_INVALID_ARGUMENT), as rt_frame_advance refuses it.  The frame itself is not changed.  The copy into out is fast
+ *   if the caller pinned it (rt_host_pin).
+ * rt_frame_resume and rt_multi_frame_resume open an ordinary RtFrame from a snapshot; every rt_frame_* call takes it.
+ *   Exactness: after resuming, and after every further pass, the frame equals the saved frame continued without
+ *   interruption in everything rt_multi_frame_begin's frame equals rt_frame_begin's (sums, counts, RGB8, Q, the E map,
+ *   rt_frame_noise and rt_frame_view_noise, every RtFrameProgress and RtFrameConvergence field except the _ms fields and
+ *   passes, rt_frame_extend, rt_frame_features and rt_frame_denoise), whatever the device counts at save and at resume.
+ *   passes continues from the snapshot; last_pass_ms and device_ms cover this process only (device_ms starts with the
+ *   restore).  The first paced pass is sized from the saved device time per sample index, scaled by the ratio of the
+ *   device counts.  rt_frame_set_convergence is accepted exactly when the saved frame would have accepted it.
+ *   Refusals, before any device allocation, with *out NULL: RT_ERR_INVALID_ARGUMENT for a NULL argument, a bad magic,
+ *   version, length or checksum, and a scene whose content differs from the saved one (its fingerprint, object count or
+ *   texture count); RT_ERR_UNSUPPORTED for a scene created with device = -1, and for a window given to
+ *   rt_multi_frame_resume (windows run on one GPU); then every refusal of the frame's opener for the saved arguments.  A
+ *   snapshot that passes these checks but whose pixels break the frame's rules (below) is refused with
+ *   RT_ERR_INVALID_ARGUMENT naming the first bad pixel; the half-built frame is freed.
+ *   The scene fingerprint hashes the object array and texture table as the scene holds them now (every field but padding
+ *   and pointers, and the texels), not its tree: a snapshot taken after rt_scene_update or rt_scene_rebuild resumes on
+ *   rt_scene_create of the same arrays, bit for bit except where a closest hit is an exact tie in t (rt_scene_update).
+ *
+ * Format (little-endian; version 1).  RtSnapshotHeader, then for a batch of views n_views entries of {RtCamera, uint64
+ * seed} (the caller's cameras and seeds), then the pixel sections of n_pixels pixels (the tall frame of a batch, the
+ * window's pixels of a window):
+ *   sums    n_pixels x int32[4] {sumR, sumG, sumB, count}, as rt_frame_read gives them;
+ *   Q       n_pixels x uint64, only when opts.flags has RT_FLAG_NOISE;
+ *   flags   the pixels still being sampled, bit p % 32 of uint32 word p / 32, the words padded to an even count (zeros).
+ * checksum = sum over i of mix(i, w_i) mod 2^64, w_i the i-th little-endian uint64 word of the file with the checksum
+ *   field read as 0, and mix(i, w) = f(w + (i + 1) 0x9E3779B97F4A7C15) with splitmix64's finalizer
+ *   f(z): z = (z ^ z >> 30) 0xBF58476D1CE4E5B9; z = (z ^ z >> 27) 0x94D049BB133111EB; z ^ z >> 31.
+ * Each pixel satisfies: a pixel still being sampled has count == samples_done; any other has count == n_probe or a
+ *   checkpoint of the rule m + j k <= samples_done; each channel sum lies in [0, 255 count] and Q in [0, 3 255^2 count].
+ *   Over the frame: the counts sum to paths_done, pixels_active pixels are still sampled, and pixels_flagged pixels are
+ *   still sampled or hold more than n_probe samples.
+ * A frame with RT_FLAG_NOISE takes about 24 bytes a pixel (8.3 M pixels: about 200 MB), 16 without. */
+#define RT_SNAPSHOT_VERSION 1
+enum RtFrameKind { RT_FRAME_CAMERA = 0, RT_FRAME_VIEWS = 1, RT_FRAME_WINDOW = 2 };
+typedef struct RtSnapshotHeader {
+    char magic[8];              /* "RTFSSNAP"                                                                  */
+    uint32_t version;           /* RT_SNAPSHOT_VERSION                                                         */
+    uint32_t header_bytes;      /* sizeof(RtSnapshotHeader) = 344                                              */
+    uint64_t total_bytes;       /* the whole snapshot                                                          */
+    uint64_t checksum;          /* above                                                                       */
+    uint64_t scene_fingerprint; /* of the scene the frame traced                                               */
+    int32_t n_objects, n_textures;
+    int32_t kind;               /* RtFrameKind                                                                 */
+    int32_t n_views;            /* 1 unless kind == RT_FRAME_VIEWS                                             */
+    RtCamera camera;            /* the opener's camera (the first view's for a batch)                          */
+    int32_t max_width_coord, max_height_coord;
+    int32_t window[4];          /* RT_FRAME_WINDOW: row0, col0, rows, cols                                     */
+    RtRenderOpts opts;          /* the opener's                                                                */
+    int32_t samples_per_pixel;  /* the frame's, after any rt_frame_extend                                      */
+    int32_t samples_done, samples_target, n_probe, passes, _pad0;
+    uint64_t n_pixels, pixels_flagged, pixels_active, paths_done;
+    double conv_tolerance;      /* the convergence rule (conv_interval == 0: none)                             */
+    int32_t conv_min, conv_interval, conv_checks;
+    int32_t pace_devices;       /* the device count ms_per_sample was measured at                              */
+    double ms_per_sample;       /* the pacing estimate (< 0: none yet)                                         */
+} RtSnapshotHeader;
+int rt_frame_save(RtFrame *frame, void *out, size_t cap, size_t *len);
+int rt_frame_resume(RtScene *scene, const void *snapshot, size_t len, RtFrame **out, RtFrameProgress *progress);
+int rt_multi_frame_resume(RtMulti *multi, const void *snapshot, size_t len, RtFrame **out, RtFrameProgress *progress);
+
 /* create + render + destroy in one call */
 int rt_render_multi(const RtHittable *objects, int32_t n_objects, const RtTexture *textures,
                     int32_t n_textures, const int32_t *devices, int32_t n_devices,

@@ -202,3 +202,46 @@ class RtSceneUpdate(C.Structure):
         ("launches", C.c_int32),
         ("_pad0", C.c_int32),
     ]
+
+
+# snapshots of progressive frames (rt_frame_save / rt_frame_resume; the format is in include/rtfs_b200.h)
+RT_SNAPSHOT_VERSION = 1
+RT_FRAME_CAMERA = 0
+RT_FRAME_VIEWS = 1
+RT_FRAME_WINDOW = 2
+
+
+class RtSnapshotHeader(C.Structure):
+    _fields_ = [
+        ("magic", C.c_char * 8),
+        ("version", C.c_uint32),
+        ("header_bytes", C.c_uint32),
+        ("total_bytes", C.c_uint64),
+        ("checksum", C.c_uint64),
+        ("scene_fingerprint", C.c_uint64),
+        ("n_objects", C.c_int32),
+        ("n_textures", C.c_int32),
+        ("kind", C.c_int32),
+        ("n_views", C.c_int32),
+        ("camera", RtCamera),
+        ("max_width_coord", C.c_int32),
+        ("max_height_coord", C.c_int32),
+        ("window", C.c_int32 * 4),
+        ("opts", RtRenderOpts),
+        ("samples_per_pixel", C.c_int32),
+        ("samples_done", C.c_int32),
+        ("samples_target", C.c_int32),
+        ("n_probe", C.c_int32),
+        ("passes", C.c_int32),
+        ("_pad0", C.c_int32),
+        ("n_pixels", C.c_uint64),
+        ("pixels_flagged", C.c_uint64),
+        ("pixels_active", C.c_uint64),
+        ("paths_done", C.c_uint64),
+        ("conv_tolerance", C.c_double),
+        ("conv_min", C.c_int32),
+        ("conv_interval", C.c_int32),
+        ("conv_checks", C.c_int32),
+        ("pace_devices", C.c_int32),
+        ("ms_per_sample", C.c_double),
+    ]

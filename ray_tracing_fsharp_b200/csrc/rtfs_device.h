@@ -403,6 +403,50 @@ __host__ __device__ __forceinline__ double pixel_standard_error(int32_t n, int32
 }
 
 // ---------------------------------------------------------------------------------------------------
+// snapshots of progressive frames (rtfs_snapshot.cu; rt_frame_save, rt_frame_resume: the format is in include/rtfs_b200.h)
+// ---------------------------------------------------------------------------------------------------
+static_assert(sizeof(RtSnapshotHeader) == 344 && sizeof(RtCamera) == 152, "the snapshot header's layout is the file's");
+// the term of word i of the checksum: splitmix64's finalizer of w + (i + 1) golden; a bijection of w for every i, so one
+// flipped bit of a word changes its term and the sum
+__host__ __device__ __forceinline__ uint64_t snapshot_mix(uint64_t i, uint64_t w) {
+    uint64_t z = w + (i + 1) * 0x9E3779B97F4A7C15ull;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+// the checksum terms of bytes [0, n) (n a multiple of 8) that start at word `first_word` of the file, summed
+uint64_t snapshot_checksum(const void *bytes, size_t n, uint64_t first_word);
+// the 64-bit hash of the scene's object array and texture table (every field but padding and pointers, and the texels)
+uint64_t scene_fingerprint(const RtScene *scene);
+// The pixel sections of a snapshot in device memory, in file order: sums (2 words a pixel), Q (1 word a pixel, noise
+// only), the flags (one word per 64 pixels).  `first_word` is the file word of words[0].
+struct SnapshotSections {
+    unsigned long long *words;
+    uint64_t first_word;
+    size_t n_pixels;
+    bool noise;
+};
+__host__ __device__ __forceinline__ size_t snapshot_flag_words(size_t n_pixels) { return (n_pixels + 63) / 64; }
+inline size_t snapshot_section_words(size_t n_pixels, bool noise) { return n_pixels * (noise ? 3 : 2) + snapshot_flag_words(n_pixels); }
+// What snapshot_unpack_kernel finds: the checksum of the sections, the counts summed, the pixels still sampled, the pixels
+// flagged by the probe (still sampled or holding more than n_probe samples), and the first pixel that breaks a rule
+// (~0: none).  Zero it with first_bad = ~0 before the launch.
+struct SnapshotTally {
+    unsigned long long checksum, counts, active, flagged, first_bad;
+};
+// The frame's rules a restored pixel must satisfy (include/rtfs_b200.h): counts against samples_done, n_probe and the
+// checkpoints conv_min + j conv_interval (conv_interval == 0: no rule)
+struct SnapshotRules {
+    int32_t samples_done, n_probe, conv_min, conv_interval;
+};
+// the sections of the totals (stats, sq or null, flags) into s.words; *checksum (zeroed by the caller) += their terms
+int launch_snapshot_pack(const int32_t *stats, const unsigned long long *sq, const uint8_t *flags, const SnapshotSections &s,
+                         unsigned long long *checksum, cudaStream_t st);
+// the sections in s.words into stats, sq (noise only) and flags, checking every pixel against the rules into *tally
+int launch_snapshot_unpack(const SnapshotSections &s, const SnapshotRules &rules, int32_t *stats, unsigned long long *sq, uint8_t *flags,
+                           SnapshotTally *tally, cudaStream_t st);
+
+// ---------------------------------------------------------------------------------------------------
 // denoised previews of progressive frames (rtfs_denoise.cu; rt_frame_features, rt_frame_denoise)
 // ---------------------------------------------------------------------------------------------------
 constexpr int kMaxDenoiseIterations = 10, kMaxFeatureSamples = 64;

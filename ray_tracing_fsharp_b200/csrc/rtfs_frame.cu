@@ -20,10 +20,13 @@
 // opener, pass and end of step.  The totals, the shared flags and everything that reads them live on the first device: the
 // only part of a frame of one device traces into them directly, and over several devices the parts trace into buffers of
 // their own that the exchange kernel (rtfs_multi.cu) sums into the totals.
+// rt_frame_save writes a frame's totals, flags and counters into a snapshot, and rt_frame_resume / rt_multi_frame_resume
+// open a frame from one on any device count: frame_alloc, then a restore in place of the probe (kernels in rtfs_snapshot.cu).
 #include "rtfs_device.h"
 
 #include <algorithm>
 #include <cmath>
+#include <cstddef>
 #include <cstring>
 
 using namespace rtfs;
@@ -120,6 +123,18 @@ struct FramePart {
     cudaEvent_t listed = nullptr;   // (rank 0) the shared flags are final: the ranks may compact from them
 };
 
+// What a frame was opened with, as its opener's caller gave it: rt_frame_save writes it into the snapshot, and resuming
+// opens the frame again from it (so the snapshot does not depend on the layout of the device's tables)
+struct FrameSpec {
+    RtCamera camera{};             // the frame's camera; a batch's first
+    std::vector<RtCamera> cameras; // a batch of views: every view's camera and seed (empty otherwise)
+    std::vector<uint64_t> seeds;
+    bool has_window = false;
+    FrameWindow window{};
+    int32_t max_w = 0, max_h = 0;
+    RtRenderOpts opts{};
+};
+
 } // namespace rtfs
 
 // A frame owns everything a pass writes: sums, flags, the image and, in its parts, the flagged-pixel lists and counter
@@ -160,6 +175,8 @@ struct RtFrame {
     uint64_t generation = 0;    // the scene's edit count when the frame opened (rt_scene_update)
     std::vector<FramePart> parts;
     bool gathered = true; // the totals hold every part's samples (always, with one part)
+    FrameSpec spec;
+    uint64_t paths_base = 0; // a resumed frame: the paths of the snapshot (its parts' counter blocks start at zero)
 };
 
 namespace {
@@ -301,7 +318,7 @@ int frame_sync(RtFrame *f, FrameEvents::Which from, double *span_ms) {
         RT_CUDA(cudaMemcpyAsync(p.h_counters, p.d_counters, CN_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ds->ws->stream));
     }
     *span_ms = 0.0;
-    f->paths_done = 0;
+    f->paths_done = f->paths_base;
     for (FramePart &p : f->parts) {
         RT_CUDA(cudaSetDevice(part_scene(p)->device));
         RT_CUDA(cudaStreamSynchronize(part_scene(p)->ws->stream));
@@ -312,13 +329,19 @@ int frame_sync(RtFrame *f, FrameEvents::Which from, double *span_ms) {
     return RT_OK;
 }
 
-// Every opener, once its arguments are checked: the frame's sums, Q, flags and image on the first device, one part per
-// scene (the scene of rt_frame_begin*, or the replicas of an RtMulti in rank order), the split probe and the compaction.  A
-// batch's frame is the tall frame of rt_render_views (rtfs_views.cu) with its own table; a window's frame holds the
-// window's pixels only (rtfs_window.cu).
-int frame_open(const std::vector<RtScene *> &scenes, const RtCamera &camera, const std::vector<ViewCamera> &views, const FrameWindow *window,
-               int32_t max_w, int32_t max_h, const RtRenderOpts *opts, RtFrame **out, RtFrameProgress *progress, const char *who) {
+// The half of every opener that allocates, once its arguments are checked: the frame's sums, Q, flags and image on the
+// first device, one part per scene (the scene of rt_frame_begin*, or the replicas of an RtMulti in rank order), and every
+// part's parameters and table of views.  A batch's frame is the tall frame of rt_render_views (rtfs_views.cu) with its own
+// table; a window's frame holds the window's pixels only (rtfs_window.cu).  frame_open then probes; frame_resume restores a
+// snapshot instead.  On failure nothing is left allocated.
+int frame_alloc(const std::vector<RtScene *> &scenes, const FrameSpec &spec, RtFrame **out, const char *who) {
     const int world = int(scenes.size());
+    const RtRenderOpts *opts = &spec.opts;
+    const int32_t max_w = spec.max_w, max_h = spec.max_h;
+    const FrameWindow *window = spec.has_window ? &spec.window : nullptr;
+    const std::vector<ViewCamera> views = spec.cameras.empty() ? std::vector<ViewCamera>()
+                                                               : view_table(spec.cameras.data(), spec.seeds.data(), int32_t(spec.cameras.size()),
+                                                                            max_w, max_h, opts->seed);
     const bool noise = (opts->flags & RT_FLAG_NOISE) != 0;
     int rc;
     for (RtScene *s : scenes)
@@ -328,6 +351,7 @@ int frame_open(const std::vector<RtScene *> &scenes, const RtCamera &camera, con
     auto *f = new RtFrame();
     f->scene = scenes[0];
     f->generation = scenes[0]->generation;
+    f->spec = spec;
     auto bail = [&](int code) {
         frame_free(f);
         return code;
@@ -368,20 +392,19 @@ int frame_open(const std::vector<RtScene *> &scenes, const RtCamera &camera, con
     // the frame's parameters are one device's (the features, the filter, the pacing and rt_frame_extend read them); each
     // part has its own, of rank r of world
     auto fill = [&](FrameParams &fp, DeviceScene *ds, const ViewCamera *d_views, int r, int w) {
-        fill_frame(fp, ds, camera, max_w, max_h, *opts, r, w);
+        fill_frame(fp, ds, spec.camera, max_w, max_h, *opts, r, w);
         if (!views.empty()) set_views(fp, d_views, f->n_views, int32_t(view_pixels));
         if (window) set_window(fp, *window);
     };
     fill(f->fp, ds0, f->d_views, 0, 1);
     f->samples_done = f->fp.n_probe; // 0 without the early-out
     f->samples_target = f->fp.sample_end;
-    int launches = 0;
     for (int r = 0; r < world; ++r) {
         FramePart &p = f->parts[size_t(r)];
         DeviceScene *ds = part_scene(p);
         if (cudaSetDevice(ds->device) != cudaSuccess) return bail(fail(RT_ERR_CUDA, std::string(who) + ": cudaSetDevice failed"));
         // a batch: the rank's table on its device (from pageable memory: staged before the call returns, and the probe
-        // follows it on the stream)
+        // or the restore follows it on the stream)
         if (!views.empty() &&
             cudaMemcpyAsync(p.d_views, views.data(), views.size() * sizeof(ViewCamera), cudaMemcpyHostToDevice, ds->ws->stream) != cudaSuccess)
             return bail(fail(RT_ERR_CUDA, std::string(who) + ": view table upload failed: " + cudaGetErrorString(cudaGetLastError())));
@@ -391,6 +414,24 @@ int frame_open(const std::vector<RtScene *> &scenes, const RtCamera &camera, con
         p.fp.list = p.d_list;
         p.fp.counters = p.d_counters;
         p.fp.sq = p.d_sq; // non-null: plan_launch picks the kernels that also sum the squares
+    }
+    *out = f;
+    return RT_OK;
+}
+
+// Every opener: frame_alloc, then the split probe and the compaction.
+int frame_open(const std::vector<RtScene *> &scenes, const FrameSpec &spec, RtFrame **out, RtFrameProgress *progress, const char *who) {
+    RtFrame *f = nullptr;
+    int rc = frame_alloc(scenes, spec, &f, who);
+    if (rc != RT_OK) return rc;
+    auto bail = [&](int code) {
+        frame_free(f);
+        return code;
+    };
+    int launches = 0;
+    for (FramePart &p : f->parts) {
+        DeviceScene *ds = part_scene(p);
+        if (cudaSetDevice(ds->device) != cudaSuccess) return bail(fail(RT_ERR_CUDA, std::string(who) + ": cudaSetDevice failed"));
         // the probe of the rank's tiles; with its own counter block the rank keeps the raw "means differ" flags, also where
         // this target has no main phase: the frame can be extended
         if ((rc = frame_probe(ds, p.fp, ds->ws->stream, &p.ev, &launches)) != RT_OK) return bail(rc);
@@ -400,10 +441,30 @@ int frame_open(const std::vector<RtScene *> &scenes, const RtCamera &camera, con
     f->pixels_flagged = f->pixels_active = f->pixels_listed;
     // the probe traced n_probe samples of every pixel, a pass traces samples of the flagged pixels only; over several
     // devices the slowest rank probed 1 / world of the pixels and a pass gives it 1 / world of the indices
-    if (f->fp.adaptive) f->ms_per_sample = f->device_ms * double(f->pixels_flagged) / (double(n) * double(f->fp.n_probe));
+    if (f->fp.adaptive) f->ms_per_sample = f->device_ms * double(f->pixels_flagged) / (double(f->n_pixels) * double(f->fp.n_probe));
     *out = f;
     frame_progress(f, progress);
     return RT_OK;
+}
+
+// The spec of an opener's arguments (seeds null: every view has opts->seed)
+FrameSpec frame_spec(const RtCamera *cameras, const uint64_t *seeds, int32_t n_views, const FrameWindow *window, int32_t max_w, int32_t max_h,
+                     const RtRenderOpts *opts) {
+    FrameSpec s;
+    s.camera = cameras[0];
+    if (n_views > 0) {
+        s.cameras.assign(cameras, cameras + n_views);
+        s.seeds.assign(size_t(n_views), opts->seed);
+        if (seeds) s.seeds.assign(seeds, seeds + n_views);
+    }
+    if (window) {
+        s.has_window = true;
+        s.window = *window;
+    }
+    s.max_w = max_w;
+    s.max_h = max_h;
+    s.opts = *opts;
+    return s;
 }
 
 // one pass of every rank over [s, s + k) with s = samples_done (rank r: the indices s + r + j world) and, when it
@@ -494,6 +555,173 @@ int check_current(const RtFrame *f, const char *who) {
     return RT_OK;
 }
 
+// ---- snapshots (rt_frame_save, rt_frame_resume; the format is in include/rtfs_b200.h, the kernels in rtfs_snapshot.cu) ----
+
+constexpr char kSnapshotMagic[8] = {'R', 'T', 'F', 'S', 'S', 'N', 'A', 'P'};
+constexpr size_t kViewEntryBytes = sizeof(RtCamera) + sizeof(uint64_t); // a batch's view: the caller's camera and seed
+
+// the byte offsets of a snapshot's view table, its pixel sections and its end
+struct SnapshotLayout {
+    size_t table, sections, total;
+};
+SnapshotLayout snapshot_layout(int32_t kind, size_t n_views, size_t n_pixels, bool noise) {
+    SnapshotLayout l;
+    l.table = sizeof(RtSnapshotHeader);
+    l.sections = l.table + (kind == RT_FRAME_VIEWS ? n_views * kViewEntryBytes : 0);
+    l.total = l.sections + 8 * snapshot_section_words(n_pixels, noise);
+    return l;
+}
+
+int32_t frame_kind(const RtFrame *f) { return f->spec.has_window ? RT_FRAME_WINDOW : f->spec.cameras.empty() ? RT_FRAME_CAMERA : RT_FRAME_VIEWS; }
+
+// the sum of the checksum terms of the header (its checksum field read as 0) and the view table, bytes [0, sections)
+uint64_t snapshot_head_checksum(const uint8_t *bytes, size_t sections) {
+    RtSnapshotHeader h;
+    std::memcpy(&h, bytes, sizeof h);
+    h.checksum = 0;
+    return snapshot_checksum(&h, sizeof h, 0) + snapshot_checksum(bytes + sizeof h, sections - sizeof h, sizeof h / 8);
+}
+
+// a device allocation freed when the call returns, on whichever path
+struct StagingBuffer {
+    void *p = nullptr;
+    ~StagingBuffer() { cudaFree(p); }
+};
+
+// rt_frame_resume's and rt_multi_frame_resume's body, once the handle is checked: the header's checks, the scene's
+// fingerprint and the opener's checks, all before any device allocation; then frame_alloc, the restore of the sections
+// into the first part's sums and Q and the frame's flags (the other parts start from zero), and the relist and end of step
+// that follow a probe.
+int frame_resume(const std::vector<RtScene *> &scenes, bool multi, const void *snapshot, size_t len, RtFrame **out, RtFrameProgress *progress,
+                 const char *who) {
+    const std::string w(who);
+    RtScene *scene = scenes[0];
+    if (!scene->dev) return fail(RT_ERR_UNSUPPORTED, w + ": the scene was created without a device (device = -1)");
+    if (!snapshot || len < sizeof(RtSnapshotHeader)) return fail(RT_ERR_INVALID_ARGUMENT, w + ": the snapshot is null or shorter than its header");
+    const auto *bytes = static_cast<const uint8_t *>(snapshot);
+    RtSnapshotHeader h;
+    std::memcpy(&h, bytes, sizeof h);
+    if (std::memcmp(h.magic, kSnapshotMagic, sizeof kSnapshotMagic) != 0) return fail(RT_ERR_INVALID_ARGUMENT, w + ": not a frame snapshot (bad magic)");
+    if (h.version != RT_SNAPSHOT_VERSION)
+        return fail(RT_ERR_INVALID_ARGUMENT, w + ": snapshot format version " + std::to_string(h.version) + "; this library reads version 1");
+    const bool noise = (h.opts.flags & RT_FLAG_NOISE) != 0;
+    if (h.header_bytes != sizeof h || h.total_bytes != len || h.kind < RT_FRAME_CAMERA || h.kind > RT_FRAME_WINDOW || h.n_views < 1 ||
+        (h.kind != RT_FRAME_VIEWS && h.n_views != 1) || h.n_pixels == 0 || h.n_pixels >= (uint64_t(1) << 31) ||
+        snapshot_layout(h.kind, size_t(h.n_views), size_t(h.n_pixels), noise).total != len)
+        return fail(RT_ERR_INVALID_ARGUMENT, w + ": the snapshot's lengths do not match its header");
+    const SnapshotLayout L = snapshot_layout(h.kind, size_t(h.n_views), size_t(h.n_pixels), noise);
+    const uint64_t head_sum = snapshot_head_checksum(bytes, L.sections);
+    if (head_sum + snapshot_checksum(bytes + L.sections, len - L.sections, L.sections / 8) != h.checksum)
+        return fail(RT_ERR_INVALID_ARGUMENT, w + ": the snapshot's checksum does not match its bytes");
+    if (h.kind == RT_FRAME_WINDOW && multi)
+        return fail(RT_ERR_UNSUPPORTED, w + ": a window runs on one GPU; resume it with rt_frame_resume");
+    if (h.n_objects != int32_t(scene->objects.size()) || h.n_textures != int32_t(scene->textures.size()) ||
+        h.scene_fingerprint != scene_fingerprint(scene))
+        return fail(RT_ERR_INVALID_ARGUMENT, w + ": the scene's objects or textures differ from those of the saved frame's scene");
+
+    // the opener's arguments, and its checks
+    FrameSpec spec;
+    spec.camera = h.camera;
+    spec.max_w = h.max_width_coord;
+    spec.max_h = h.max_height_coord;
+    spec.opts = h.opts;
+    int rc;
+    if (h.kind == RT_FRAME_VIEWS) {
+        spec.cameras.resize(size_t(h.n_views));
+        spec.seeds.resize(size_t(h.n_views));
+        for (size_t v = 0; v < size_t(h.n_views); ++v) {
+            std::memcpy(&spec.cameras[v], bytes + L.table + v * kViewEntryBytes, sizeof(RtCamera));
+            std::memcpy(&spec.seeds[v], bytes + L.table + v * kViewEntryBytes + sizeof(RtCamera), sizeof(uint64_t));
+        }
+        rc = check_views(scene, spec.cameras.data(), h.n_views, spec.max_w, spec.max_h, &spec.opts, who);
+    } else if (h.kind == RT_FRAME_WINDOW) {
+        spec.has_window = true;
+        spec.window = FrameWindow{h.window[0], h.window[1], h.window[2], h.window[3]};
+        rc = check_window(spec.window, spec.max_w, spec.max_h, who);
+        if (rc == RT_OK) rc = check_frame_args(scene, &spec.camera, spec.max_w, spec.max_h, &spec.opts);
+    } else {
+        rc = check_frame_args(scene, &spec.camera, spec.max_w, spec.max_h, &spec.opts);
+    }
+    if (rc != RT_OK) return rc;
+    if ((rc = check_frame_mode(&spec.opts, who, h.kind != RT_FRAME_CAMERA)) != RT_OK) return rc;
+
+    // the frame's state against what its arguments allow (rt_frame_extend, rt_frame_set_convergence)
+    const bool adaptive = h.opts.adaptive != 0;
+    const int32_t first_trial = adaptive ? std::min(5, h.camera.samples_per_pixel / 2) : 0, n_probe = adaptive ? 2 * first_trial + 1 : 0;
+    const int32_t spp = h.samples_per_pixel, target = adaptive ? std::max(n_probe, spp) : spp;
+    const size_t view_pixels = size_t(2 * spec.max_w + 1) * size_t(2 * spec.max_h + 1);
+    const size_t n_pixels = spec.has_window ? size_t(spec.window.rows) * size_t(spec.window.cols) : view_pixels * size_t(h.n_views);
+    const bool rule_ok = h.conv_interval == 0 ? h.conv_min == 0 && h.conv_checks == 0
+                                               : noise && h.conv_interval >= 1 && h.conv_min >= 2 && h.conv_tolerance >= 0.0 && h.conv_checks >= 0;
+    if (h.n_pixels != n_pixels || h.n_probe != n_probe || spp < 1 || spp > (1 << 22) || (adaptive && std::min(5, spp / 2) != first_trial) ||
+        h.samples_target != target || h.samples_done < n_probe || h.samples_done > target || h.passes < 0 || h.pace_devices < 1 ||
+        h.pixels_active > h.pixels_flagged || h.pixels_flagged > h.n_pixels || !rule_ok)
+        return fail(RT_ERR_INVALID_ARGUMENT, w + ": the snapshot's frame state is not one its arguments allow");
+
+    RtFrame *f = nullptr;
+    if ((rc = frame_alloc(scenes, spec, &f, who)) != RT_OK) return rc;
+    auto bail = [&](int code) {
+        frame_free(f);
+        return code;
+    };
+    f->fp.cam.spp = spp; // (as rt_frame_extend leaves it)
+    f->fp.sample_end = target;
+    f->samples_done = h.samples_done;
+    f->samples_target = target;
+    f->passes = h.passes;
+    f->pixels_flagged = h.pixels_flagged;
+    f->pixels_active = h.pixels_active;
+    f->paths_base = h.paths_done;
+    f->conv_tolerance = h.conv_tolerance;
+    f->conv_min = h.conv_min;
+    f->conv_interval = h.conv_interval;
+    f->conv_checks = h.conv_checks;
+    // a pass over world devices gives each 1 / world of the indices
+    f->ms_per_sample = h.ms_per_sample > 0.0 ? h.ms_per_sample * double(h.pace_devices) / double(f->parts.size()) : h.ms_per_sample;
+
+    const size_t words = snapshot_section_words(n_pixels, noise);
+    StagingBuffer staging;
+    SnapshotTally tally{};
+    {
+        for (size_t r = 0; r < f->parts.size(); ++r) { // ZEROED: the counters (and the other parts' sums and Q) are clear
+            FramePart &p = f->parts[r];
+            DeviceScene *ds = part_scene(p);
+            cudaStream_t st = ds->ws->stream;
+            if (cudaSetDevice(ds->device) != cudaSuccess || cudaMemsetAsync(p.d_counters, 0, CN_SLOTS * sizeof(unsigned long long), st) != cudaSuccess ||
+                (r > 0 && cudaMemsetAsync(p.d_stats, 0, n_pixels * 4 * sizeof(int32_t), st) != cudaSuccess) ||
+                (r > 0 && p.d_sq && cudaMemsetAsync(p.d_sq, 0, n_pixels * sizeof(unsigned long long), st) != cudaSuccess) ||
+                p.ev.record(FrameEvents::ZEROED, st) != cudaSuccess)
+                return bail(fail(RT_ERR_CUDA, w + ": clearing the parts failed: " + cudaGetErrorString(cudaGetLastError())));
+        }
+        FramePart &p0 = f->parts[0];
+        DeviceScene *ds0 = part_scene(p0);
+        cudaStream_t st0 = ds0->ws->stream;
+        if (cudaSetDevice(ds0->device) != cudaSuccess || cudaMalloc(&staging.p, words * 8 + sizeof(SnapshotTally)) != cudaSuccess)
+            return bail(fail(RT_ERR_CUDA, w + ": allocation failed: " + cudaGetErrorString(cudaGetLastError())));
+        auto *d_words = static_cast<unsigned long long *>(staging.p);
+        auto *d_tally = reinterpret_cast<SnapshotTally *>(d_words + words);
+        if (cudaMemcpyAsync(d_words, bytes + L.sections, words * 8, cudaMemcpyHostToDevice, st0) != cudaSuccess ||
+            cudaMemsetAsync(d_tally, 0, sizeof(SnapshotTally), st0) != cudaSuccess ||
+            cudaMemsetAsync(&d_tally->first_bad, 0xff, sizeof d_tally->first_bad, st0) != cudaSuccess)
+            return bail(fail(RT_ERR_CUDA, w + ": snapshot upload failed: " + cudaGetErrorString(cudaGetLastError())));
+        const SnapshotSections sec{d_words, L.sections / 8, n_pixels, noise};
+        const SnapshotRules rules{h.samples_done, n_probe, h.conv_min, h.conv_interval};
+        if ((rc = launch_snapshot_unpack(sec, rules, p0.d_stats, p0.d_sq, f->d_flags, d_tally, st0)) != RT_OK) return bail(rc);
+        if (cudaMemcpyAsync(&tally, d_tally, sizeof tally, cudaMemcpyDeviceToHost, st0) != cudaSuccess)
+            return bail(fail(RT_ERR_CUDA, w + ": reading the restore's tally failed"));
+    }
+    if ((rc = frame_relist(f, false, false)) != RT_OK) return bail(rc);
+    if ((rc = frame_sync(f, FrameEvents::ZEROED, &f->device_ms)) != RT_OK) return bail(rc);
+    if (tally.first_bad != ~0ull)
+        return bail(fail(RT_ERR_INVALID_ARGUMENT, w + ": pixel " + std::to_string(tally.first_bad) + " of the snapshot breaks the frame's rules"));
+    if (head_sum + tally.checksum != h.checksum) return bail(fail(RT_ERR_INVALID_ARGUMENT, w + ": the sections changed on their way to the device"));
+    if (tally.counts != h.paths_done || tally.active != h.pixels_active || tally.flagged != h.pixels_flagged || f->pixels_listed != h.pixels_active)
+        return bail(fail(RT_ERR_INVALID_ARGUMENT, w + ": the snapshot's pixels do not add up to its paths_done, pixels_active and pixels_flagged"));
+    *out = f;
+    frame_progress(f, progress);
+    return RT_OK;
+}
+
 } // namespace
 
 extern "C" {
@@ -505,7 +733,7 @@ int rt_frame_begin(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_
     if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin: out is null");
     *out = nullptr;
     if ((rc = check_frame_mode(opts, "rt_frame_begin", false)) != RT_OK) return rc;
-    return frame_open({scene}, *camera, {}, nullptr, max_w, max_h, opts, out, progress, "rt_frame_begin");
+    return frame_open({scene}, frame_spec(camera, nullptr, 0, nullptr, max_w, max_h, opts), out, progress, "rt_frame_begin");
 }
 
 int rt_frame_begin_views(RtScene *scene, const RtCamera *cameras, const uint64_t *seeds, int32_t n_views, int32_t max_w, int32_t max_h,
@@ -516,8 +744,7 @@ int rt_frame_begin_views(RtScene *scene, const RtCamera *cameras, const uint64_t
     if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_begin_views: out is null");
     *out = nullptr;
     if ((rc = check_frame_mode(opts, "rt_frame_begin_views", true)) != RT_OK) return rc;
-    return frame_open({scene}, cameras[0], view_table(cameras, seeds, n_views, max_w, max_h, opts->seed), nullptr, max_w, max_h, opts, out,
-                      progress, "rt_frame_begin_views");
+    return frame_open({scene}, frame_spec(cameras, seeds, n_views, nullptr, max_w, max_h, opts), out, progress, "rt_frame_begin_views");
 }
 
 int rt_frame_begin_window(RtScene *scene, const RtCamera *camera, int32_t max_w, int32_t max_h, int32_t row0, int32_t col0, int32_t rows,
@@ -530,7 +757,7 @@ int rt_frame_begin_window(RtScene *scene, const RtCamera *camera, int32_t max_w,
     *out = nullptr;
     if ((rc = check_frame_args(scene, camera, max_w, max_h, opts)) != RT_OK) return rc;
     if ((rc = check_frame_mode(opts, "rt_frame_begin_window", true)) != RT_OK) return rc;
-    return frame_open({scene}, *camera, {}, &w, max_w, max_h, opts, out, progress, "rt_frame_begin_window");
+    return frame_open({scene}, frame_spec(camera, nullptr, 0, &w, max_w, max_h, opts), out, progress, "rt_frame_begin_window");
 }
 
 int rt_multi_frame_begin(RtMulti *multi, const RtCamera *camera, int32_t max_w, int32_t max_h, const RtRenderOpts *opts, RtFrame **out,
@@ -542,7 +769,7 @@ int rt_multi_frame_begin(RtMulti *multi, const RtCamera *camera, int32_t max_w, 
     int rc = check_frame_args(multi_scenes(multi)[0], camera, max_w, max_h, opts);
     if (rc != RT_OK) return rc;
     if ((rc = check_frame_mode(opts, "rt_multi_frame_begin", false)) != RT_OK) return rc;
-    return frame_open(multi_scenes(multi), *camera, {}, nullptr, max_w, max_h, opts, out, progress, "rt_multi_frame_begin");
+    return frame_open(multi_scenes(multi), frame_spec(camera, nullptr, 0, nullptr, max_w, max_h, opts), out, progress, "rt_multi_frame_begin");
 }
 
 int rt_multi_frame_begin_views(RtMulti *multi, const RtCamera *cameras, const uint64_t *seeds, int32_t n_views, int32_t max_w, int32_t max_h,
@@ -554,8 +781,8 @@ int rt_multi_frame_begin_views(RtMulti *multi, const RtCamera *cameras, const ui
     int rc = check_views(multi_scenes(multi)[0], cameras, n_views, max_w, max_h, opts, "rt_multi_frame_begin_views");
     if (rc != RT_OK) return rc;
     if ((rc = check_frame_mode(opts, "rt_multi_frame_begin_views", true)) != RT_OK) return rc;
-    return frame_open(multi_scenes(multi), cameras[0], view_table(cameras, seeds, n_views, max_w, max_h, opts->seed), nullptr, max_w, max_h,
-                      opts, out, progress, "rt_multi_frame_begin_views");
+    return frame_open(multi_scenes(multi), frame_spec(cameras, seeds, n_views, nullptr, max_w, max_h, opts), out, progress,
+                      "rt_multi_frame_begin_views");
 }
 
 int rt_frame_advance(RtFrame *f, int32_t max_samples, double target_ms, RtFrameProgress *progress) {
@@ -743,6 +970,96 @@ int rt_pixel_noise(const int32_t *sums, const uint64_t *sq, size_t n, float *se_
     for (size_t p = 0; p < n; ++p)
         se_out[p] = float(pixel_standard_error(sums[4 * p + 3], sums[4 * p], sums[4 * p + 1], sums[4 * p + 2], sq[p]));
     return RT_OK;
+}
+
+int rt_frame_save(RtFrame *f, void *out, size_t cap, size_t *len) {
+    if (!f || !len) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_save: null frame or len");
+    const bool noise = f->d_sq != nullptr;
+    const int32_t kind = frame_kind(f);
+    const SnapshotLayout L = snapshot_layout(kind, size_t(f->n_views), f->n_pixels, noise);
+    *len = L.total;
+    if (int rc = check_current(f, "rt_frame_save"); rc != RT_OK) return rc;
+    if (!out && cap == 0) return RT_OK; // sizing only
+    if (!out || cap < L.total)
+        return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_save: the buffer holds " + std::to_string(cap) + " bytes; the snapshot takes " + std::to_string(L.total));
+    int rc = ensure_totals(f);
+    if (rc != RT_OK) return rc;
+    auto *ds = static_cast<DeviceScene *>(f->scene->dev);
+    RT_CUDA(cudaSetDevice(ds->device));
+    cudaStream_t st = ds->ws->stream;
+    const size_t words = snapshot_section_words(f->n_pixels, noise);
+    StagingBuffer staging;
+    RT_CUDA(cudaMalloc(&staging.p, (words + 1) * 8));
+    auto *d_words = static_cast<unsigned long long *>(staging.p);
+    RT_CUDA(cudaMemsetAsync(d_words + words, 0, 8, st));
+    const SnapshotSections sec{d_words, L.sections / 8, f->n_pixels, noise};
+    if ((rc = launch_snapshot_pack(f->d_stats, f->d_sq, f->d_flags, sec, d_words + words, st)) != RT_OK) return rc;
+    auto *b = static_cast<uint8_t *>(out);
+    uint64_t sections_sum = 0;
+    RT_CUDA(cudaMemcpyAsync(b + L.sections, d_words, words * 8, cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaMemcpyAsync(&sections_sum, d_words + words, 8, cudaMemcpyDeviceToHost, st));
+
+    // the header and the view table, written while the copy runs
+    RtSnapshotHeader h;
+    std::memset(&h, 0, sizeof h);
+    std::memcpy(h.magic, kSnapshotMagic, sizeof h.magic);
+    h.version = RT_SNAPSHOT_VERSION;
+    h.header_bytes = sizeof h;
+    h.total_bytes = L.total;
+    h.scene_fingerprint = scene_fingerprint(f->scene);
+    h.n_objects = int32_t(f->scene->objects.size());
+    h.n_textures = int32_t(f->scene->textures.size());
+    h.kind = kind;
+    h.n_views = f->n_views;
+    h.camera = f->spec.camera;
+    h.max_width_coord = f->spec.max_w;
+    h.max_height_coord = f->spec.max_h;
+    if (f->spec.has_window) {
+        h.window[0] = f->spec.window.row0;
+        h.window[1] = f->spec.window.col0;
+        h.window[2] = f->spec.window.rows;
+        h.window[3] = f->spec.window.cols;
+    }
+    h.opts = f->spec.opts;
+    h.samples_per_pixel = f->fp.cam.spp;
+    h.samples_done = f->samples_done;
+    h.samples_target = f->samples_target;
+    h.n_probe = f->fp.n_probe;
+    h.passes = f->passes;
+    h.n_pixels = f->n_pixels;
+    h.pixels_flagged = f->pixels_flagged;
+    h.pixels_active = f->pixels_active;
+    h.paths_done = f->paths_done;
+    h.conv_tolerance = f->conv_tolerance;
+    h.conv_min = f->conv_min;
+    h.conv_interval = f->conv_interval;
+    h.conv_checks = f->conv_checks;
+    h.pace_devices = int32_t(f->parts.size());
+    h.ms_per_sample = f->ms_per_sample;
+    std::memcpy(b, &h, sizeof h);
+    for (size_t v = 0; v < f->spec.cameras.size(); ++v) {
+        std::memcpy(b + L.table + v * kViewEntryBytes, &f->spec.cameras[v], sizeof(RtCamera));
+        std::memcpy(b + L.table + v * kViewEntryBytes + sizeof(RtCamera), &f->spec.seeds[v], sizeof(uint64_t));
+    }
+    const uint64_t head_sum = snapshot_head_checksum(b, L.sections);
+    RT_CUDA(cudaStreamSynchronize(st));
+    h.checksum = head_sum + sections_sum;
+    std::memcpy(b + offsetof(RtSnapshotHeader, checksum), &h.checksum, sizeof h.checksum);
+    return RT_OK;
+}
+
+int rt_frame_resume(RtScene *scene, const void *snapshot, size_t len, RtFrame **out, RtFrameProgress *progress) {
+    if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_resume: out is null");
+    *out = nullptr;
+    if (!scene) return fail(RT_ERR_INVALID_ARGUMENT, "rt_frame_resume: null scene");
+    return frame_resume({scene}, false, snapshot, len, out, progress, "rt_frame_resume");
+}
+
+int rt_multi_frame_resume(RtMulti *multi, const void *snapshot, size_t len, RtFrame **out, RtFrameProgress *progress) {
+    if (!out) return fail(RT_ERR_INVALID_ARGUMENT, "rt_multi_frame_resume: out is null");
+    *out = nullptr;
+    if (!multi || multi_scenes(multi).empty()) return fail(RT_ERR_INVALID_ARGUMENT, "rt_multi_frame_resume: null handle");
+    return frame_resume(multi_scenes(multi), true, snapshot, len, out, progress, "rt_multi_frame_resume");
 }
 
 } // extern "C"

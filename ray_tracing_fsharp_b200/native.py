@@ -10,8 +10,8 @@ import os
 import numpy as np
 
 from . import abi
-from .abi import (RtCamera, RtDenoiseOpts, RtFrameConvergence, RtFrameNoise, RtFrameProgress, RtHittable, RtRenderOpts, RtSceneRebuild, RtSceneUpdate, RtStats,
-                  RtTexture)
+from .abi import (RtCamera, RtDenoiseOpts, RtFrameConvergence, RtFrameNoise, RtFrameProgress, RtHittable, RtRenderOpts, RtSceneRebuild, RtSceneUpdate,
+                  RtSnapshotHeader, RtStats, RtTexture)
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "librtfs_b200.so")
@@ -81,6 +81,9 @@ def _declare(lib):
         "rt_multi_render_views": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(RtRenderOpts), _vp, _vp, C.POINTER(RtStats)]),
         "rt_multi_frame_begin_views": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(RtRenderOpts), C.POINTER(_vp),
                                                  C.POINTER(RtFrameProgress)]),
+        "rt_frame_save": (C.c_int, [_vp, _vp, C.c_size_t, C.POINTER(C.c_size_t)]),
+        "rt_frame_resume": (C.c_int, [_vp, _vp, C.c_size_t, C.POINTER(_vp), C.POINTER(RtFrameProgress)]),
+        "rt_multi_frame_resume": (C.c_int, [_vp, _vp, C.c_size_t, C.POINTER(_vp), C.POINTER(RtFrameProgress)]),
         "rt_device_probe": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _i32, _i32, _vp, _vp, _vp,
                                       C.POINTER(RtStats)]),
         "rt_device_main": (C.c_int, [_vp, C.POINTER(RtCamera), _i32, _i32, C.POINTER(RtRenderOpts), _i32, _i32, _vp, _vp, _vp,
@@ -221,6 +224,26 @@ def _views_frame(owner, out, progress, max_w, max_h, n):
     frame.scene, frame.ptr, frame.progress = owner, out, progress
     frame.rows, frame.cols = 2 * max_h + 1, 2 * max_w + 1
     frame.n_views = n
+    return frame
+
+
+def _resume(owner, resume_fn, data):
+    """The Frame resume_fn (rt_frame_resume or rt_multi_frame_resume) opens from the snapshot `data` (bytes-like) on `owner`
+    (a SceneHandle or MultiHandle), with the shape of the frame that was saved: a tall frame for a batch of views, the
+    window's rows and cols for a window."""
+    buf = np.frombuffer(data, np.uint8)
+    out = C.c_void_p()
+    progress = RtFrameProgress()
+    check(resume_fn(owner.ptr, C.c_void_p(buf.ctypes.data if buf.size else None), buf.size, C.byref(out), C.byref(progress)))
+    h = RtSnapshotHeader.from_buffer_copy(buf[:C.sizeof(RtSnapshotHeader)].tobytes())
+    if h.kind == abi.RT_FRAME_VIEWS:
+        return _views_frame(owner, out, progress, h.max_width_coord, h.max_height_coord, h.n_views)
+    frame = Frame.__new__(Frame)
+    frame.scene, frame.ptr, frame.progress = owner, out, progress
+    if h.kind == abi.RT_FRAME_WINDOW:
+        frame.rows, frame.cols = h.window[2], h.window[3]
+    else:
+        frame.rows, frame.cols = 2 * h.max_height_coord + 1, 2 * h.max_width_coord + 1
     return frame
 
 
@@ -377,6 +400,13 @@ class SceneHandle:
         frame.rows, frame.cols = rows, cols
         return frame
 
+    def resume_frame(self, data):
+        """A progressive frame opened from a snapshot written by Frame.save (rt_frame_resume), on this scene: after every
+        further pass it is exactly the saved frame continued without interruption, whatever device count saved it.  The
+        scene must hold the objects and textures of the saved frame's scene.  RtError RT_ERR_INVALID_ARGUMENT for a damaged
+        snapshot or a scene with other content."""
+        return _resume(self, lib().rt_frame_resume, data)
+
     # ---- conformance ----
     def hit_object(self, o, d, traversal=0):
         o, d = f64(o, (-1, 3)), f64(d, (-1, 3))
@@ -517,6 +547,16 @@ class Frame:
         check(lib().rt_frame_denoise(self.ptr, C.byref(opts), ptr(rgb), ptr(linear)))
         return rgb, linear
 
+    def save(self) -> bytes:
+        """The frame as a snapshot (rt_frame_save): bytes that SceneHandle.resume_frame or MultiHandle.resume_frame open again
+        as this frame, in this process or another, on any device count.  The frame is left as it was.  RtError
+        RT_ERR_INVALID_ARGUMENT for a stale frame."""
+        n = C.c_size_t()
+        check(lib().rt_frame_save(self.ptr, None, 0, C.byref(n)))
+        buf = np.empty(n.value, np.uint8)
+        check(lib().rt_frame_save(self.ptr, ptr(buf), buf.size, C.byref(n)))
+        return buf.tobytes()
+
     def close(self):
         if getattr(self, "ptr", None):
             lib().rt_frame_destroy(self.ptr)
@@ -604,6 +644,11 @@ class MultiHandle:
         progress = RtFrameProgress()
         check(lib().rt_multi_frame_begin_views(self.ptr, cams, ptr(sd), n, max_w, max_h, C.byref(opts), C.byref(out), C.byref(progress)))
         return _views_frame(self, out, progress, max_w, max_h, n)
+
+    def resume_frame(self, data):
+        """SceneHandle.resume_frame split over this handle's devices (rt_multi_frame_resume).  A snapshot of a window raises
+        RtError RT_ERR_UNSUPPORTED: windows run on one GPU."""
+        return _resume(self, lib().rt_multi_frame_resume, data)
 
 
 class CommHandle:

@@ -10,6 +10,7 @@ reference's.  Everything that computes goes through the C ABI (native.py); nothi
   Scene.render_views    Scene.render of many cameras of one scene in one submission (rt_render_views; one GPU or several)
   Scene.render_progressive  the same frame in sample passes, progress ticks as passes finish (native.Frame, one GPU or several)
   Scene.render_views_progressive  Scene.render_views in sample passes, as one progressive frame of the batch (one GPU or several)
+  Scene.resume_progressive  a progressive frame saved by Frame.save, continued to its target (one GPU or several)
   Scene.render_window   a window (row0, col0, rows, cols) of Scene.render's image, without tracing the rest (rt_render_window)
   Image / Image.render  RayTracing/Domain.fs:9-31
   ImageOutput.write_ppm RayTracing/ImageOutput.fs:163-197, PixelOutput.correct :11-18
@@ -297,7 +298,8 @@ class Scene:
         `on_pass(progress, frame)` is called, if given: it may read the current image (`frame.read()`, exactly the frame of
         `progress.samples_done` samples per pixel) and stops the frame by returning True.  Returns the pixels (uint8
         [rows, cols, 3], before gamma): with the same seed, Scene.render's image, or that of the samples done when stopped.
-        `print_fn` is accepted and ignored as in Scene.render.
+        `print_fn` is accepted and ignored as in Scene.render.  To checkpoint the frame, `on_pass` may call `frame.save()`:
+        Scene.resume_progressive continues the snapshot later, in this process or another, bit for bit.
         With `noise_tolerance` (8-bit levels) the frame also keeps its noise estimate (abi.RT_FLAG_NOISE, Frame.noise) and
         stops at the first check where at most `noise_fraction` of the pixels still being sampled have a standard error
         of the mean above the tolerance.  The check runs after the probe and after every pass (after `on_pass`); the image
@@ -314,21 +316,8 @@ class Scene:
         rows = 2 * max_height_coord + 1 if window is None else int(window[2])
         if seed is None:
             seed = secrets.randbits(64)
-        ticks = ProgressTicks(rows)
-
-        def emit(n):
-            for _ in range(n):
-                progress_increment(1.0)
-
         if noise_tolerance is not None or converge_tolerance is not None:
             flags |= abi.RT_FLAG_NOISE
-
-        def converged(frame, progress):
-            if noise_tolerance is None or progress.done:
-                return False
-            summary, _, _ = frame.noise(noise_tolerance, want_map=False)
-            return summary.pixels_above <= noise_fraction * summary.pixels
-
         if window is None:
             opened = s._handle.open_frame(camera, max_width_coord, max_height_coord, seed=seed, adaptive=adaptive, flags=flags)
         else:
@@ -336,19 +325,7 @@ class Scene:
         with opened as frame:
             if converge_tolerance is not None:
                 frame.set_convergence(converge_tolerance, converge_min_samples, converge_interval)
-            progress = frame.progress
-            emit(ticks.update(progress.paths_done, progress.paths_target))  # the probe
-            stop = converged(frame, progress)
-            while not progress.done and not stop:
-                progress = frame.advance(target_ms=target_ms)
-                if not progress.done:
-                    emit(ticks.update(progress.paths_done, progress.paths_target))
-                if on_pass is not None and on_pass(progress, frame):
-                    break
-                stop = converged(frame, progress)
-            rgb, _ = frame.read()
-        emit(ticks.finish())  # the last pass's share, or the rest of the frame when on_pass stopped it
-        return rgb
+            return _run_passes(frame, rows, progress_increment, target_ms, on_pass, noise_tolerance, noise_fraction)
 
     @staticmethod
     def render_views_progressive(progress_increment: Callable[[float], None], print_fn: Callable[[str], None], max_width_coord: int,
@@ -371,29 +348,62 @@ class Scene:
         rows, n = 2 * max_height_coord + 1, len(cameras)
         if seed is None and seeds is None:
             seed = secrets.randbits(64)
-        ticks = ProgressTicks(rows * n)
-
-        def emit(k):
-            for _ in range(k):
-                progress_increment(1.0)
-
         if converge_tolerance is not None:
             flags |= abi.RT_FLAG_NOISE
         with s._handle.open_frame_views(list(cameras), max_width_coord, max_height_coord, seeds=seeds, seed=seed or 0, adaptive=adaptive,
                                         flags=flags) as frame:
             if converge_tolerance is not None:
                 frame.set_convergence(converge_tolerance, converge_min_samples, converge_interval)
-            progress = frame.progress
-            emit(ticks.update(progress.paths_done, progress.paths_target))  # the probe
-            while not progress.done:
-                progress = frame.advance(target_ms=target_ms)
-                if not progress.done:
-                    emit(ticks.update(progress.paths_done, progress.paths_target))
-                if on_pass is not None and on_pass(progress, frame):
-                    break
-            rgb, _ = frame.read()
-        emit(ticks.finish())
+            rgb = _run_passes(frame, rows * n, progress_increment, target_ms, on_pass, None, 0.0)
         return [rgb[v] for v in range(n)]
+
+    @staticmethod
+    def resume_progressive(progress_increment: Callable[[float], None], print_fn: Callable[[str], None], snapshot, s: "Scene",
+                           target_ms: float = 250.0, on_pass: Optional[Callable[[abi.RtFrameProgress, "native.Frame"], object]] = None,
+                           noise_tolerance: Optional[float] = None, noise_fraction: float = 0.0):
+        """Continues a frame saved by Frame.save (for instance from render_progressive's `on_pass`) to its target, on `s`,
+        which must hold the objects and textures of the scene the frame was saved from (one GPU or devices=[...], whatever
+        the device count that saved it).  Returns what render_progressive (or render_views_progressive, for a batch of
+        views) would have returned had the frame never stopped: bit for bit the same pixels.  The progress ticks total the
+        same rows (times views) as the original call; the share already done is emitted at once.  `target_ms`, `on_pass`,
+        `noise_tolerance` and `noise_fraction` act as in render_progressive (the noise stop needs a frame saved with its
+        noise estimate); the convergence rule the frame was saved with still applies.  `print_fn` is ignored."""
+        with s._handle.resume_frame(snapshot) as frame:
+            rows = frame.rows * (frame.n_views or 1)
+            rgb = _run_passes(frame, rows, progress_increment, target_ms, on_pass, noise_tolerance, noise_fraction)
+        return rgb if frame.n_views is None else [rgb[v] for v in range(frame.n_views)]
+
+
+def _run_passes(frame: "native.Frame", total_ticks: int, progress_increment: Callable[[float], None], target_ms: float, on_pass,
+                noise_tolerance: Optional[float], noise_fraction: float) -> np.ndarray:
+    """The passes of render_progressive and its kin, from the frame's current state to its target, an `on_pass` that
+    returns True, or the noise stop: `total_ticks` progress ticks spread over the paths traced (what the frame already
+    holds is emitted at once), then the frame's pixels."""
+    ticks = ProgressTicks(total_ticks)
+
+    def emit(n):
+        for _ in range(n):
+            progress_increment(1.0)
+
+    def converged(progress):
+        if noise_tolerance is None or progress.done:
+            return False
+        summary, _, _ = frame.noise(noise_tolerance, want_map=False)
+        return summary.pixels_above <= noise_fraction * summary.pixels
+
+    progress = frame.progress
+    emit(ticks.update(progress.paths_done, progress.paths_target))  # the probe (or what a resumed frame holds)
+    stop = converged(progress)
+    while not progress.done and not stop:
+        progress = frame.advance(target_ms=target_ms)
+        if not progress.done:
+            emit(ticks.update(progress.paths_done, progress.paths_target))
+        if on_pass is not None and on_pass(progress, frame):
+            break
+        stop = converged(progress)
+    rgb, _ = frame.read()
+    emit(ticks.finish())  # the last pass's share, or the rest of the frame when on_pass stopped it
+    return rgb
 
 
 def _texture_shape(t: abi.RtTexture):

@@ -252,6 +252,15 @@ module internal Native =
     extern int rt_frame_begin_window (nativeint scene, RtCamera& camera, int maxWidthCoord, int maxHeightCoord, int row0, int col0, int rows, int cols, RtRenderOpts& opts, nativeint& frame, RtFrameProgress& progress)
 
     [<DllImport(Lib)>]
+    extern int rt_frame_save (nativeint frame, byte[] out, unativeint cap, unativeint& len)
+
+    [<DllImport(Lib)>]
+    extern int rt_frame_resume (nativeint scene, byte[] snapshot, unativeint len, nativeint& frame, RtFrameProgress& progress)
+
+    [<DllImport(Lib)>]
+    extern int rt_multi_frame_resume (nativeint multi, byte[] snapshot, unativeint len, nativeint& frame, RtFrameProgress& progress)
+
+    [<DllImport(Lib)>]
     extern int rt_pixel_noise (int[] sums, uint64[] sq, unativeint n, float32[] seOut)
 
     [<DllImport(Lib)>]
@@ -725,6 +734,15 @@ type GpuFrame internal (handle : nativeint, rows : int, cols : int, views : int,
         Native.rt_frame_read (handle, (if gamma then 1 else 0), rgb, 0n) |> Native.check
         rgb
 
+    /// The frame as a snapshot (rt_frame_save): bytes SceneGpu.resumeFrame opens again as this frame, in this process or
+    /// another, on one GPU or several.  The frame is left as it was; a frame whose scene was edited since it opened fails.
+    member _.Save () : byte[] =
+        let mutable len = 0un
+        Native.rt_frame_save (handle, null, 0un, &len) |> Native.check
+        let out = Array.zeroCreate<byte> (int len)
+        Native.rt_frame_save (handle, out, len, &len) |> Native.check
+        out
+
     /// Sets the target to `samplesPerPixel`; fails if that would change the probe already run (firstTrial) or is below
     /// what the frame holds.
     member _.Extend (samplesPerPixel : int) : unit =
@@ -1089,6 +1107,28 @@ module SceneGpu =
         |> Native.check
 
         new GpuFrame (handle, rows, cols, 1, progress)
+
+    /// Opens a progressive frame from a snapshot written by GpuFrame.Save (rt_frame_resume, or rt_multi_frame_resume on a
+    /// multi-GPU scene).  After every further pass it is bit for bit the saved frame continued without interruption,
+    /// whatever device count saved it.  The scene must hold the objects and textures of the saved frame's scene; a window
+    /// resumes on a single-device scene only.  The frame's shape is read from the snapshot's header (RtSnapshotHeader).
+    let resumeFrame (s : GpuScene) (snapshot : byte[]) : GpuFrame =
+        let mutable handle = 0n
+        let mutable progress = Native.RtFrameProgress ()
+
+        let rc =
+            if s.IsMulti then
+                Native.rt_multi_frame_resume (s.Handle, snapshot, unativeint snapshot.Length, &handle, &progress)
+            else
+                Native.rt_frame_resume (s.Handle, snapshot, unativeint snapshot.Length, &handle, &progress)
+
+        Native.check rc
+        // RtSnapshotHeader: kind at byte 48, n_views at 52, max_width_coord / max_height_coord at 208 / 212, window rows and
+        // cols at 224 / 228
+        let i32 (at : int) = System.BitConverter.ToInt32 (snapshot, at)
+        let kind, views = i32 48, i32 52
+        let rows, cols = if kind = 2 then i32 224, i32 228 else 2 * i32 212 + 1, 2 * i32 208 + 1
+        new GpuFrame (handle, rows, cols, views, progress)
 
     /// The scene GpuScene.make would give for `objects` (the whole new object list), made in place on the device
     /// (rt_scene_update): the list is marshalled and diffed against the scene's current records, and only the changed objects
